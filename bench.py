@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py — Mrays/s of the RayHs ray-casting path on B200 (BASELINE.json metric).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload c4|c5]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload c4|c5] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 A step = one frame of the workload.  Default workload "c4": dragon.json with the full-res dragon.obj at
@@ -21,6 +21,12 @@ so "scaling": "strong".
 parity: the frame the timed steps rendered against the oracle (oracle/oracle.cpp, the CPU restatement of the
 reference) — c4: every row the cpu_baseline leg renders (all 2160 when the host is fast enough); c5: 16 rows x
 64 columns x 64 spp; hit ids and RGB8 bytes.
+
+--dump-outputs DIR: what the last timed step computed, as float32/float64 .npy files in DIR (at most 64 MB) — rgb.npy
+  [n, width, 3], the RGB8 values of n rows of the complete frame (all rows when they fit 48 MB as float32, else a fixed
+  seeded sample), rgb_rows.npy the indices of those rows, rays_by_class.npy [5] the frame's primary, reflect, probe,
+  exit and shadow ray counts.  The inputs are seeded, so two builds run with the same arguments can be compared file
+  for file.
 
 --impl reference times the reference's own CPU algorithm (the C++ restatement in oracle/, because GHC is not in
 this image: kind "port") with all host threads on a bounded sample of the same workload.
@@ -181,6 +187,26 @@ def c5_oracle_sample(sc, W, H, spp, seed, rows, cols, threads=0):
             f"{r['seconds']:.1f} s (+ {build_s:.0f} s for the oracle's own single-threaded tree build, not timed)", r)
 
 
+RAY_CLASSES = ("rays_primary", "rays_reflect", "rays_probe", "rays_exit", "rays_shadow")
+DUMP_FRAME_BYTES = 48_000_000   # --dump-outputs: the frame's share of the 64 MB the dump may take
+
+
+def dump_rows(H: int, W: int) -> np.ndarray:
+    """Rows of the frame --dump-outputs writes: all of them if they fit DUMP_FRAME_BYTES as float32, else a sorted
+    sample drawn with a fixed seed (the same rows in every run of the same frame size)."""
+    n = min(H, DUMP_FRAME_BYTES // (W * 3 * 4))
+    if n == H:
+        return np.arange(H)
+    return np.sort(np.random.default_rng(0).choice(H, n, replace=False))
+
+
+def dump_outputs(path: str, rgb_rows: np.ndarray, rows: np.ndarray, rays_by_class: np.ndarray) -> None:
+    os.makedirs(path, exist_ok=True)
+    np.save(os.path.join(path, "rgb.npy"), rgb_rows.astype(np.float32))
+    np.save(os.path.join(path, "rgb_rows.npy"), rows.astype(np.float64))
+    np.save(os.path.join(path, "rays_by_class.npy"), rays_by_class.astype(np.float64))
+
+
 def make_scene(rh, wl):
     if "pack" in wl:
         return rh.Scene.from_pack(os.path.join(ROOT, "tests", "golden", wl["pack"] + ".pack"))
@@ -288,7 +314,7 @@ print(json.dumps({"import_ms": 1e3 * (t1 - t0), "rh_init_ms": 1e3 * (t2 - t1), "
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=0)
+    ap.add_argument("--steps", type=int, default=None, help="timed steps (default: the workload's)")
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--workload", default="c4", choices=sorted(WORKLOADS))
@@ -299,14 +325,20 @@ def main():
     ap.add_argument("--spp", type=int, default=0)
     ap.add_argument("--tris", type=int, default=0)
     ap.add_argument("--band-height", type=int, default=0, help="rows per interleaved band at N > 1 (default: the library's choice)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step computed to DIR/<name>.npy (see the module docstring)")
     args = ap.parse_args()
     name = args.workload
     wl = dict(WORKLOADS[name])
     for k in ("width", "height", "spp", "tris"):
         if getattr(args, k):
             wl[k] = getattr(args, k)
-    if not args.steps:
+    if args.steps is None:
         args.steps = wl["steps"]
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the frame of the product path; the reference arm renders a timing-dependent row sample")
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
@@ -477,6 +509,11 @@ def main():
     launches0 = L.rh_launch_count()
     ms_dev, stats = timed(step_device, args.steps)
     launches = (L.rh_launch_count() - launches0) // args.steps
+    dumped = None
+    if args.dump_outputs and rank == 0:   # the last timed step's frame, before the calls below render into it again
+        dump_idx = dump_rows(H, W)
+        frame = rgb_dev if G == 1 else (peers.frame if use_fused[0] else full_dev)
+        dumped = frame[torch.from_numpy(dump_idx).cuda()].cpu().numpy()
     ms_e2e, stats_e2e = timed(step_e2e, args.steps)
     ms_seeded = None
     if G == 1 and not c5:  # beside e2e: the same call with the offset stream regenerated on the device from its seed (no upload)
@@ -497,6 +534,10 @@ def main():
     del dst_u8
     clocks = sampler.stop() if rank == 0 else None
     rays = total_rays(stats[-1])
+    if args.dump_outputs:
+        by_class = torch.tensor([float(stats[-1][k]) for k in RAY_CLASSES], dtype=torch.float64, device="cuda")
+        if G > 1:
+            dist.all_reduce(by_class, op=dist.ReduceOp.SUM)
     culled = torch.tensor([float(stats[-1]["rays_shadow_culled"])], dtype=torch.float64, device="cuda")
     if G > 1:
         dist.all_reduce(culled, op=dist.ReduceOp.SUM)
@@ -673,6 +714,8 @@ def main():
         if assembled_ok is not None:
             line["assembled_frame_equals_single_gpu_frame" if not c5 else "both_exchanges_assemble_the_same_frame"] = assembled_ok
             line["exchange"] = exchange
+        if dumped is not None:
+            dump_outputs(args.dump_outputs, dumped, dump_idx, by_class.cpu().numpy())
         sys.stdout.flush()
         os.dup2(saved_stdout, 1)
         print(json.dumps(line), flush=True)
