@@ -333,6 +333,35 @@ int rh_scene_light_tables(const rh_scene* scene, uint32_t* info4, float* maps_ou
 int rh_render(const rh_scene* scene, const rh_camera* camera, const rh_render_opts* opts,
               uint8_t* rgb_out, int32_t* hit_ids_out, rh_stats* stats);
 
+/* ---- batched ray queries -------------------------------------------- */
+/* Geometry.hs:39 Hit + the object and triangle that produced it (80 bytes). */
+typedef struct rh_hit {
+  double t;          /* +inf on a miss                                                                   */
+  double p[3];       /* rayAt r t (Geometry.hs:29); 0 on a miss                                           */
+  double n[3];       /* as the reference returns it: mesh normals interpolated, not renormalised (Mesh.hs:81) */
+  double uv[2];      /* mesh: Mesh.hs:81-82, plane: Geometry.hs:70-79, sphere: Geometry.hs:96             */
+  int32_t object;    /* scene index, -1 on a miss                                                         */
+  int32_t tri;       /* tri_id (index in the mesh's triangles), -1 for planes / spheres / a miss          */
+} rh_hit;
+
+/* Replaces `closestIntersection` (RayHs.hs:67-71) for n caller-built rays: the closest hit over the object list, the
+ * first object of the list winning a tie in t.  rays: double[n][6] = origin, direction (any length, zero components
+ * allowed: the reference's arithmetic decides them).  hits_out: n records.  flags: RH_FLAG_DEVICE_OUT (rays and
+ * hits_out are DEVICE pointers on the current device, 16-byte aligned) and RH_FLAG_EXACT_BOXES (validation: the
+ * reference's double slab test at every box); any other bit is RH_ERR_ARG.  Host buffers are copied through device
+ * scratch in bounded chunks, so any n works.  n == 0 is RH_OK; a null pointer with n > 0 is RH_ERR_ARG.  The call
+ * returns when the results are written.  Sphere uv goes through CUDA's atan / acos (DESIGN.md §3: within a few ulp of
+ * glibc's); every other value is bit-identical to the reference's. */
+int rh_closest_intersection(const rh_scene* scene, const double* rays, uint64_t n, rh_hit* hits_out, int32_t flags);
+/* Replaces `shadowIntersection` (RayHs.hs:74-87) towards light `light` (index into the scene's lights; out of range is
+ * RH_ERR_ARG): occluded_out[i] = 1 when some non-emitter object (isOccluder, RayHs.hs:81-82) has a hit on ray i in
+ * front of the light (inFrontOfLight, RayHs.hs:84-87: for a point light strictly nearer to the ray origin than the
+ * light, for a directional light any hit), else 0.  The caller builds the ray, as accumDiffuse does with
+ * `rayEps p ld` (RayHs.hs:93).  rays, flags, n and the buffers as for rh_closest_intersection (occluded_out needs no
+ * alignment). */
+int rh_shadow_intersection(const rh_scene* scene, uint32_t light, const double* rays, uint64_t n, uint8_t* occluded_out,
+                           int32_t flags);
+
 /* Rows owned by one shard (equal for all shards: bands are padded). */
 int rh_shard_rows(int height, int shard_count, int band_height);
 int rh_default_band_height(int height, int shard_count);

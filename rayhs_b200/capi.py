@@ -115,9 +115,14 @@ class rh_stats(C.Structure):
         return {n: getattr(self, n) for n, _ in self._fields_}
 
 
+class rh_hit(C.Structure):
+    _fields_ = [("t", C.c_double), ("p", d3), ("n", d3), ("uv", d2), ("object", C.c_int32), ("tri", C.c_int32)]
+
+
 # struct sizes the header promises (checked by tests/test_abi.py against the compiled library too)
 assert C.sizeof(rh_material) == 96 and C.sizeof(rh_light) == 64 and C.sizeof(rh_node) == 64
 assert C.sizeof(rh_tri) == 80 and C.sizeof(rh_tri_shade) == 128 and C.sizeof(rh_object) == 96
+assert C.sizeof(rh_hit) == 80
 
 vp = C.c_void_p
 
@@ -134,6 +139,8 @@ SIGNATURES = {
     "rh_scene_record_bytes": (C.c_int, [vp, C.POINTER(C.c_uint64)]),
     "rh_scene_light_tables": (C.c_int, [vp, C.POINTER(C.c_uint32), vp, vp, vp]),
     "rh_render": (C.c_int, [vp, C.POINTER(rh_camera), C.POINTER(rh_render_opts), vp, vp, C.POINTER(rh_stats)]),
+    "rh_closest_intersection": (C.c_int, [vp, vp, C.c_uint64, vp, C.c_int32]),
+    "rh_shadow_intersection": (C.c_int, [vp, C.c_uint32, vp, C.c_uint64, vp, C.c_int32]),
     "rh_shard_rows": (C.c_int, [C.c_int, C.c_int, C.c_int]),
     "rh_default_band_height": (C.c_int, [C.c_int, C.c_int]),
     "rh_deinterleave_bands": (C.c_int, [vp, vp, C.c_int, C.c_int, C.c_int, C.c_int]),

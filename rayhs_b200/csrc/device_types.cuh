@@ -269,6 +269,19 @@ struct ChunkParams {
   ShadowQueue q_hits, q_shadow;
 };
 
+// One launch of the batched ray queries (rh_closest_intersection / rh_shadow_intersection) over rays [0, n).
+struct QueryParams {
+  const double* rays;  // device, double[n][6] = origin, direction; 16-byte aligned
+  rh_hit* hits;        // closest: one record per ray; 16-byte aligned
+  uint8_t* occluded;   // shadow: 0 / 1 per ray
+  uint32_t n;
+  uint32_t light;      // shadow: index into the light table
+  int32_t exact_boxes; // RH_FLAG_EXACT_BOXES: double slab test for every ray
+  uint32_t deep_stride;
+  uint2* deep_stack;   // the render's deep-stack scratch (>= grid * block columns)
+  uint32_t* cursor;    // claim cursor, zero before the launch
+};
+
 // Launchers (kernels.cu).  `count` selects the instrumented instantiation (box/tri counters).
 // (followed by a one-thread kernel that closes the pass's range of the hit queue, ChunkCtl::hit_start)
 void launch_trace(const SceneView& S, const CameraParams& cam, const ChunkParams& P, bool count, int grid, void* stream);
@@ -277,6 +290,9 @@ void launch_trace(const SceneView& S, const CameraParams& cam, const ChunkParams
 // `classified`: a cudaEvent_t recorded after the classify kernel (or null).
 int launch_shadow(const SceneView& S, const ChunkParams& P, bool count, bool refill, int grid, void* stream, void* classified);
 void launch_resolve(const ChunkParams& P, void* stream);
+// query_closest_kernel / query_shadow_kernel: `grid` blocks of one SM each
+void launch_query_closest(const SceneView& S, const QueryParams& Q, int grid, void* stream);
+void launch_query_shadow(const SceneView& S, const QueryParams& Q, int grid, void* stream);
 void launch_deinterleave(const uint8_t* gathered, uint8_t* out, int width, int height, int shard_count, int band_height,
                          void* stream);
 int configure_kernels();  // opt in to > 48 KB dynamic shared memory; returns a cudaError_t

@@ -662,13 +662,16 @@ __device__ __noinline__ bool traverse_exact_impl(const Ctx& cx, uint32_t root, c
       RH_CNT(gnodes, 2);
       bool h0 = false, h1 = false;
       double tm0 = 0, tm1 = 0;
+      // A box that passes with tmin = +inf is not behind the bound: a zero direction component with the origin on one
+      // of the box's planes makes the reference's slab terms inf * 0 = NaN, and GHC's min / max then let the box pass
+      // with tmin = +inf whatever its real entry distance (the ray runs in the box's face).  Only a finite tmin prunes.
       if (cw.x != kEmpty) {
         RH_CNT(box, 1);
-        h0 = (refine & 1u) || (slab(r, inv, b0.x, b0.y, b1.x, b1.y, b2.x, b2.y, tm0) && !(tm0 > bound));
+        h0 = (refine & 1u) || (slab(r, inv, b0.x, b0.y, b1.x, b1.y, b2.x, b2.y, tm0) && !(tm0 > bound && !isinf(tm0)));
       }
       if (cw.y != kEmpty) {
         RH_CNT(box, 1);
-        h1 = (refine & 2u) || (slab(r, inv, b3.x, b3.y, b4.x, b4.y, b5.x, b5.y, tm1) && !(tm1 > bound));
+        h1 = (refine & 2u) || (slab(r, inv, b3.x, b3.y, b4.x, b4.y, b5.x, b5.y, tm1) && !(tm1 > bound && !isinf(tm1)));
       }
       if (h0 && h1) {
         if (tm1 < tm0) {
@@ -796,6 +799,41 @@ __device__ __forceinline__ void closest_hit(const Ctx& cx, const Ray& r, bool ex
       traverse_exact<COUNT, Closest, true>(cx, sphere_root, r, bound, best, st, cnt);
     else
       traverse<COUNT, Closest, true>(cx, sphere_root, r, f, bound, best, st, cnt);
+  }
+}
+
+// Geometry.hs:39 Hit of the primitive closest_hit chose (object `ob` of kind `okind`): the point, the normal as the
+// reference returns it (mesh normals interpolated, not renormalised: Mesh.hs:81) and, when `need_uv`, the uv.
+// (query_closest_kernel; trace_kernel keeps the same lines inline, see there.)
+template <bool COUNT>
+__device__ __forceinline__ void rebuild_hit(const SceneView& S, const DObject& ob, int okind, const Ray& r, const Closest& best,
+                                            bool need_uv, V3& p, V3& n, double& tu, double& tv, Cnt<COUNT>& cnt) {
+  p = rayAt(r, best.t);
+  if (okind == RH_OBJ_MESH) {
+    const double* sh = (const double*)(S.shade + best.slot);
+    RH_CNT(shade, 1);
+    const double wu = best.u, wv = best.v, ww = 1 - best.u - best.v;
+    // barycentricInterp u n1 v n2 (1-u-v) n0 = mul a p + mul b q + mul c r   (Mesh.hs:57, 81)
+    n = mul(wu, ld3(sh + 3)) + mul(wv, ld3(sh + 6)) + mul(ww, ld3(sh));
+    if (need_uv) {
+      tu = wu * sh[11] + wv * sh[13] + ww * sh[9];
+      tv = wu * sh[12] + wv * sh[14] + ww * sh[10];
+    }
+  } else if (okind == RH_OBJ_PLANE) {  // Geometry.hs:70-79
+    n = ld3(ob.b);
+    if (need_uv) {
+      const V3 tg = ld3(ob.c);
+      const V3 bt = cross(tg, n);
+      const V3 rel = p - ld3(ob.a);
+      tu = dot(tg, rel);
+      tv = dot(bt, rel);
+    }
+  } else {  // Geometry.hs:83-96
+    n = normalize(p - ld3(ob.a));
+    if (need_uv) {
+      tu = kPiInv * atan(n.z / n.x);
+      tv = kPiInv * acos(n.y);
+    }
   }
 }
 
@@ -1618,6 +1656,8 @@ __global__ void __launch_bounds__(kTraceBlock, kTracePerSm) trace_kernel(const _
         okind = ob.kind;
         const bool need_uv = (kind == kRayNormal) && (mkind == RH_MAT_SHOWUV ||
                                                       ((mkind == RH_MAT_DIFFUSE || mkind == RH_MAT_PLASTIC) && mat.cmap_kind != RH_CMAP_FLAT));
+        // (the same rebuild as rebuild_hit, kept inline: calling it costs this kernel 8 bytes of stack frame and 32 bytes
+        // of spill stores, DESIGN.md "Ray queries")
         p = rayAt(r, best.t);
         if (okind == RH_OBJ_MESH) {
           const double* sh = (const double*)(S.shade + best.slot);
@@ -2273,6 +2313,120 @@ __global__ void __launch_bounds__(kShadowBlock, 1) shadow_simple_kernel(const __
   flush_counters<COUNT>(cnt, P.counters, 1);
 }
 
+// ------------------------------------------------------------------ batched ray queries (caller-supplied rays)
+// query_closest_kernel: closestIntersection (RayHs.hs:67-71) + the winner's Hit; query_shadow_kernel:
+// shadowIntersection (RayHs.hs:74-87) towards one light through the general object-list form (`occluded`): the cube
+// maps and lit-triangle flags only hold for rays aimed at a light from a shaded hit.  One ray per lane, persistent warps
+// with the trace kernel's guided claims.  A warp's 32 rays (48 bytes each) arrive as coalesced 16-byte loads, three per
+// lane, through the warp's shared-memory tile, and its 32 80-byte records leave the same way, five stores per lane.
+constexpr int kQueryBlock = kTraceBlock;  // one block per SM: grid x block <= max_threads_per_launch (deep-stack scratch)
+struct QueryWarpSmem {
+  double2 tile[32 * sizeof(rh_hit) / sizeof(double2)];
+};
+static_assert(sizeof(rh_hit) == 80, "rh_hit is five 16-byte words");
+constexpr size_t kQuerySmem = sizeof(SmemTables) + (size_t)kShortStack * kQueryBlock * sizeof(uint2) +
+                              (kQueryBlock / 32) * sizeof(QueryWarpSmem);
+static_assert(kQuerySmem <= 227 * 1024, "query kernel shared memory");
+
+__device__ __forceinline__ Stack make_query_stack(const QueryParams& Q) {
+  Stack s;
+  s.col = reinterpret_cast<uint2*>(rh_smem + sizeof(SmemTables)) + threadIdx.x;
+  s.stride = kQueryBlock;
+  s.deep = Q.deep_stack + (size_t)blockIdx.x * kQueryBlock + threadIdx.x;
+  s.deep_stride = Q.deep_stride;
+  return s;
+}
+__device__ __forceinline__ double2* query_tile() {
+  return reinterpret_cast<QueryWarpSmem*>(rh_smem + sizeof(SmemTables) + (size_t)kShortStack * kQueryBlock * sizeof(uint2))[threadIdx.x >> 5].tile;
+}
+
+// The claims of one warp: body(first, count) for pieces of at most 32 consecutive rays.
+template <class Body>
+__device__ __forceinline__ void claim_rays(const QueryParams& Q, uint32_t lane, Body&& body) {
+  const uint32_t n_units = (Q.n + kSlab - 1) / kSlab * kSlabUnits, total_warps = gridDim.x * (kQueryBlock / 32);
+  uint32_t seen = (blockIdx.x * (kQueryBlock / 32) + (threadIdx.x >> 5)) * kSlabUnits;
+  for (;;) {
+    const uint2 claim = claim_units(Q.cursor, n_units, total_warps, lane, seen);
+    if (claim.x >= n_units) break;
+    const uint32_t claim_end = min(claim.x + claim.y, n_units);
+    for (uint32_t u = claim.x; u < claim_end;) {
+      uint32_t slab, b, piece_n;
+      next_piece(u, claim_end, slab, b, piece_n);
+      const uint32_t first = slab * kSlab + b;
+      if (first < Q.n) body(first, min(piece_n, Q.n - first));
+    }
+  }
+}
+
+// Ray `first + lane` of a piece (lanes >= count get whatever the tile holds and must not use it).
+__device__ __forceinline__ Ray load_query_ray(const QueryParams& Q, uint32_t first, uint32_t count, double2* tile, uint32_t lane) {
+  const double2* src = reinterpret_cast<const double2*>(Q.rays + (size_t)first * 6);
+  __syncwarp();  // the tile's previous contents have been read
+  for (uint32_t k = lane; k < 3 * count; k += 32) tile[k] = __ldcs(src + k);
+  __syncwarp();
+  const double2 a = tile[3 * lane], b = tile[3 * lane + 1], c = tile[3 * lane + 2];
+  Ray r;
+  r.o = mk(a.x, a.y, b.x);
+  r.d = mk(b.y, c.x, c.y);
+  return r;
+}
+
+__global__ void __launch_bounds__(kQueryBlock, 1) query_closest_kernel(const __grid_constant__ SceneView S,
+                                                                       const __grid_constant__ QueryParams Q) {
+  SmemTables& sm = *reinterpret_cast<SmemTables*>(rh_smem);
+  Ctx cx;
+  stage_tables(sm, S, cx);
+  Stack st = make_query_stack(Q);
+  Cnt<false> cnt;
+  const uint32_t lane = threadIdx.x & 31;
+  double2* tile = query_tile();
+  claim_rays(Q, lane, [&](uint32_t first, uint32_t count) {
+    const bool valid = lane < count;
+    const Ray r = load_query_ray(Q, first, count, tile, lane);
+    Closest best;
+    best.obj = -1;
+    if (valid) closest_hit<false>(cx, r, Q.exact_boxes || needs_exact_walk(r, S), best, st, cnt);
+    double t = __longlong_as_double(0x7ff0000000000000LL);  // a miss: t = +inf, p = n = uv = 0, ids -1
+    V3 p = mk(0, 0, 0), n = mk(0, 0, 0);
+    double tu = 0, tv = 0;
+    int tri = -1;
+    if (best.obj >= 0) {
+      const DObject& ob = cx.objects[best.obj];
+      const int okind = ob.kind;
+      t = best.t;
+      rebuild_hit<false>(S, ob, okind, r, best, true, p, n, tu, tv, cnt);
+      if (okind == RH_OBJ_MESH) tri = (int)S.tris[best.slot].tri_id;
+    }
+    __syncwarp();  // every lane has its ray out of the tile
+    double2* rec = tile + 5 * lane;
+    rec[0] = make_double2(t, p.x);
+    rec[1] = make_double2(p.y, p.z);
+    rec[2] = make_double2(n.x, n.y);
+    rec[3] = make_double2(n.z, tu);
+    rec[4] = make_double2(tv, __hiloint2double(tri, best.obj));
+    __syncwarp();
+    double2* dst = reinterpret_cast<double2*>(Q.hits + first);
+    for (uint32_t k = lane; k < 5 * count; k += 32) __stcs(dst + k, tile[k]);
+  });
+}
+
+__global__ void __launch_bounds__(kQueryBlock, 1) query_shadow_kernel(const __grid_constant__ SceneView S,
+                                                                      const __grid_constant__ QueryParams Q) {
+  SmemTables& sm = *reinterpret_cast<SmemTables*>(rh_smem);
+  Ctx cx;
+  stage_tables(sm, S, cx);
+  Stack st = make_query_stack(Q);
+  Cnt<false> cnt;
+  const uint32_t lane = threadIdx.x & 31;
+  double2* tile = query_tile();
+  const rh_light& L = cx.lights[Q.light];
+  claim_rays(Q, lane, [&](uint32_t first, uint32_t count) {
+    const Ray r = load_query_ray(Q, first, count, tile, lane);
+    if (lane < count)
+      Q.occluded[first + lane] = occluded<false>(cx, r, Q.exact_boxes || needs_exact_walk(r, S), L, st, cnt) ? 1 : 0;
+  });
+}
+
 // After pass k's trace kernel: its shaded hits are the slabs [hit_start[k], hit_start[k + 1]) of the hit queue.
 __global__ void close_hit_range_kernel(ChunkCtl* ctl, int pass) { ctl->hit_start[pass + 1] = ctl->hit_slab_next; }
 
@@ -2458,6 +2612,8 @@ int configure_kernels() {
   set((const void*)classify_kernel<false, true>, kClassifySmem);
   set((const void*)classify_kernel<true, false>, kClassifySmem);
   set((const void*)classify_kernel<false, false>, kClassifySmem);
+  set((const void*)query_closest_kernel, kQuerySmem);
+  set((const void*)query_shadow_kernel, kQuerySmem);
   if (e == cudaSuccess) {
     int dev = 0, sms = 0, nb = 0;
     cudaGetDevice(&dev);
@@ -2510,6 +2666,12 @@ int launch_shadow(const SceneView& S, const ChunkParams& P, bool count, bool ref
 void launch_resolve(const ChunkParams& P, void* stream) {
   const uint32_t n_pixels = P.n_rows * P.width;
   resolve_kernel<<<(n_pixels + kBlock - 1) / kBlock, kBlock, 0, (cudaStream_t)stream>>>(P);
+}
+void launch_query_closest(const SceneView& S, const QueryParams& Q, int grid, void* stream) {
+  query_closest_kernel<<<grid, kQueryBlock, kQuerySmem, (cudaStream_t)stream>>>(S, Q);
+}
+void launch_query_shadow(const SceneView& S, const QueryParams& Q, int grid, void* stream) {
+  query_shadow_kernel<<<grid, kQueryBlock, kQuerySmem, (cudaStream_t)stream>>>(S, Q);
 }
 void launch_deinterleave(const uint8_t* gathered, uint8_t* out, int width, int height, int shard_count, int band_height,
                          void* stream) {

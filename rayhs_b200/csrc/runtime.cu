@@ -94,6 +94,7 @@ struct Device {
     DevBuf accum, rayq[2], rayq_fill[2], hitq, hitq_words, shq, shq_words, deep, deep_shadow;
   } lane[2];
   DevBuf ctl, counters, offsets, rgb, ids;
+  DevBuf query;  // ray queries: claim cursor, then (host buffers) one chunk of rays and of results
   void* pinned = nullptr;  // ctl + counters read-back
   size_t pinned_bytes = 0;
   int max_threads = 0;  // largest grid * block of the traversal kernels (one block per SM)
@@ -146,7 +147,7 @@ struct Device {
         e = nullptr;
       }
     }
-    for (DevBuf* b : {&ctl, &counters, &offsets, &rgb, &ids})
+    for (DevBuf* b : {&ctl, &counters, &offsets, &rgb, &ids, &query})
       b->release();
     if (pinned) cudaFreeHost(pinned);
     pinned = nullptr;
@@ -1934,6 +1935,71 @@ int render_on(Device* D, const rh_scene* scene, const rh_camera* camera, const r
   }
 }
 
+// ------------------------------------------------------------------ batched ray queries
+// Rays per launch: the kernels' claim units and ray indices stay far inside 32 bits.
+constexpr uint64_t kQueryLaunch = 1ull << 24;
+// Rays per chunk of host buffers: 2 Mi x (48 + 80) bytes = 256 MB of device scratch, whatever n is.
+constexpr uint64_t kQueryChunk = 1ull << 21;
+constexpr size_t kQueryCursorBytes = 256;  // (keeps the chunk buffers 256-byte aligned)
+
+// rh_closest_intersection (light < 0) / rh_shadow_intersection (light >= 0).
+int query_on(Device* D, const rh_scene* scene, int64_t light, const double* rays, uint64_t n, void* out, int32_t flags,
+             const char* who) {
+  const std::string w(who);
+  if (!scene) return rh::set_error(RH_ERR_ARG, w + ": null scene");
+  if (scene->device != D) return rh::set_error(RH_ERR_ARG, w + ": scene lives on another device context");
+  if (flags & ~(RH_FLAG_DEVICE_OUT | RH_FLAG_EXACT_BOXES))
+    return rh::set_error(RH_ERR_ARG, w + ": flags other than RH_FLAG_DEVICE_OUT and RH_FLAG_EXACT_BOXES");
+  if (light >= 0 && (uint64_t)light >= scene->view.n_lights) return rh::set_error(RH_ERR_ARG, w + ": light index out of range");
+  if (n == 0) return RH_OK;
+  if (!rays || !out) return rh::set_error(RH_ERR_ARG, w + ": null buffer");
+  const bool shadow = light >= 0, dev = (flags & RH_FLAG_DEVICE_OUT) != 0;
+  const size_t out_bytes = shadow ? sizeof(uint8_t) : sizeof(rh_hit);
+  RH_CUDA(cudaSetDevice(D->dev));
+  if (dev) {
+    // the kernels move rays and records in 16-byte words
+    if ((uintptr_t)rays % 16 || (!shadow && (uintptr_t)out % 16))
+      return rh::set_error(RH_ERR_ARG, w + ": device buffers must be 16-byte aligned");
+    for (const void* p : {(const void*)rays, (const void*)out}) {
+      cudaPointerAttributes a{};
+      RH_CUDA(cudaPointerGetAttributes(&a, p));
+      if (a.type != cudaMemoryTypeDevice && a.type != cudaMemoryTypeManaged)
+        return rh::set_error(RH_ERR_ARG, w + ": RH_FLAG_DEVICE_OUT with a pointer that is not device memory");
+    }
+  }
+  int rc;
+  Device::Scratch& sc = D->lane[0];  // the render's deep-stack scratch covers grid x block of the query kernels
+  if ((rc = sc.deep.reserve((size_t)scene->deep_entries * D->max_threads * sizeof(uint2)))) return rc;
+  const uint64_t chunk = dev ? kQueryLaunch : kQueryChunk;
+  if ((rc = D->query.reserve(kQueryCursorBytes + (dev ? 0 : (size_t)chunk * (6 * sizeof(double) + out_bytes))))) return rc;
+  char* d_rays = (char*)D->query.p + kQueryCursorBytes;
+  char* d_out = d_rays + (size_t)chunk * 6 * sizeof(double);
+  QueryParams Q{};
+  Q.light = shadow ? (uint32_t)light : 0u;
+  Q.exact_boxes = (flags & RH_FLAG_EXACT_BOXES) ? 1 : 0;
+  Q.deep_stack = (uint2*)sc.deep.p;
+  Q.deep_stride = (uint32_t)D->max_threads;
+  Q.cursor = (uint32_t*)D->query.p;
+  for (uint64_t first = 0; first < n; first += chunk) {
+    const uint64_t m = std::min<uint64_t>(chunk, n - first);
+    const double* src = rays + first * 6;
+    char* dst = (char*)out + first * out_bytes;
+    if (!dev) RH_CUDA(cudaMemcpyAsync(d_rays, src, (size_t)m * 6 * sizeof(double), cudaMemcpyHostToDevice, D->stream));
+    Q.rays = dev ? src : (const double*)d_rays;
+    Q.n = (uint32_t)m;
+    if (shadow) Q.occluded = (uint8_t*)(dev ? dst : d_out);
+    else Q.hits = (rh_hit*)(dev ? dst : d_out);
+    RH_CUDA(cudaMemsetAsync(Q.cursor, 0, sizeof(uint32_t), D->stream));
+    if (shadow) launch_query_shadow(scene->view, Q, D->n_sms, D->stream);
+    else launch_query_closest(scene->view, Q, D->n_sms, D->stream);
+    Launch::count();
+    RH_CUDA(cudaGetLastError());
+    if (!dev) RH_CUDA(cudaMemcpyAsync(dst, d_out, (size_t)m * out_bytes, cudaMemcpyDeviceToHost, D->stream));
+  }
+  RH_CUDA(cudaStreamSynchronize(D->stream));
+  return RH_OK;
+}
+
 }  // namespace
 
 // ================================================================== C ABI
@@ -2041,6 +2107,16 @@ int rh_render(const rh_scene* scene, const rh_camera* camera, const rh_render_op
               int32_t* hit_ids_out, rh_stats* stats) {
   if (!g_dev) return rh::set_error(RH_ERR_STATE, "rh_render: call rh_init first");
   return render_on(g_dev.get(), scene, camera, opts, rgb_out, hit_ids_out, stats);
+}
+
+int rh_closest_intersection(const rh_scene* scene, const double* rays, uint64_t n, rh_hit* hits_out, int32_t flags) {
+  if (!g_dev) return rh::set_error(RH_ERR_STATE, "rh_closest_intersection: call rh_init first");
+  return query_on(g_dev.get(), scene, -1, rays, n, hits_out, flags, "rh_closest_intersection");
+}
+int rh_shadow_intersection(const rh_scene* scene, uint32_t light, const double* rays, uint64_t n, uint8_t* occluded_out,
+                           int32_t flags) {
+  if (!g_dev) return rh::set_error(RH_ERR_STATE, "rh_shadow_intersection: call rh_init first");
+  return query_on(g_dev.get(), scene, light, rays, n, occluded_out, flags, "rh_shadow_intersection");
 }
 
 int rh_default_band_height(int height, int shard_count) {

@@ -237,6 +237,99 @@ def render(job: Rendering, spp: int = 1, offsets=None, offset_tile: int = 0, wan
     return Image(job.width, rows, rgb, st.as_dict(), ids)
 
 
+# ---- batched ray queries (RayHs.hs:67-71 closestIntersection, RayHs.hs:74-87 shadowIntersection)
+
+# one rh_hit record (include/rayhs_b200.h)
+HIT_DTYPE = np.dtype([("t", "<f8"), ("p", "<f8", 3), ("n", "<f8", 3), ("uv", "<f8", 2), ("object", "<i4"), ("tri", "<i4")])
+assert HIT_DTYPE.itemsize == C.sizeof(capi.rh_hit)
+
+
+@dataclass
+class Hits:
+    """closestIntersection of a batch of rays: views of one buffer of rh_hit records (`records`), numpy arrays or CUDA
+    tensors like the rays.  t [n] (+inf on a miss), p [n, 3], n [n, 3] (mesh normals interpolated, not renormalised),
+    uv [n, 2], object [n] (scene index, -1 on a miss), tri [n] (index in the mesh's triangles, -1 for planes, spheres
+    and misses)."""
+    t: object
+    p: object
+    n: object
+    uv: object
+    object: object
+    tri: object
+    records: object
+
+
+def _query_rays(origins, directions):
+    """Checks a batch of rays and packs it as the library's [n, 6] (origin, direction) float64 array: numpy arrays (host
+    path) or CUDA tensors on the current device (device path).  Returns (rays, on_device)."""
+    if isinstance(origins, np.ndarray) and isinstance(directions, np.ndarray):
+        on_device = False
+    elif all(type(x).__module__.startswith("torch") and getattr(x, "is_cuda", False) for x in (origins, directions)):
+        import torch
+
+        on_device = True
+        if origins.device != directions.device or origins.device.index != torch.cuda.current_device():
+            raise ValueError("origins and directions must be CUDA tensors on the current device")
+    else:
+        raise ValueError("origins and directions must both be numpy arrays or both CUDA torch tensors")
+    for name, a in (("origins", origins), ("directions", directions)):
+        if str(a.dtype) not in ("float64", "torch.float64"):
+            raise ValueError(f"{name} must be float64, got {a.dtype}")
+        if a.ndim != 2 or a.shape[1] != 3:
+            raise ValueError(f"{name} must have shape [n, 3], got {tuple(a.shape)}")
+    if origins.shape[0] != directions.shape[0]:
+        raise ValueError(f"origins has {origins.shape[0]} rays, directions {directions.shape[0]}")
+    if on_device:
+        import torch
+
+        rays = torch.cat((origins, directions), dim=1).contiguous()
+        torch.cuda.current_stream().synchronize()  # the library runs on its own stream
+        return rays, True
+    rays = np.empty((origins.shape[0], 6), dtype=np.float64)
+    rays[:, :3], rays[:, 3:] = origins, directions
+    return rays, False
+
+
+def _ptr(a):
+    return a.data_ptr() if hasattr(a, "data_ptr") else a.ctypes.data
+
+
+def closestIntersection(scene, origins, directions, exact_boxes: bool = False) -> Hits:
+    """RayHs.hs:67-71 for every ray (origins[i], directions[i]): the closest hit over the scene's object list, as the
+    reference computes it.  numpy arrays in, numpy arrays out; CUDA tensors in, CUDA tensors out (no host copy).
+    `exact_boxes`: the reference's double slab test at every box (validation; same records)."""
+    rays, on_device = _query_rays(origins, directions)
+    n = rays.shape[0]
+    flags = (capi.RH_FLAG_DEVICE_OUT if on_device else 0) | (capi.RH_FLAG_EXACT_BOXES if exact_boxes else 0)
+    if on_device:
+        import torch
+
+        rec = torch.empty((n, HIT_DTYPE.itemsize), dtype=torch.uint8, device=rays.device)
+        check(lib().rh_closest_intersection(scene.device, rays.data_ptr(), n, rec.data_ptr(), flags))
+        f, i = rec.view(torch.float64), rec.view(torch.int32)
+        return Hits(f[:, 0], f[:, 1:4], f[:, 4:7], f[:, 7:9], i[:, 18], i[:, 19], rec)
+    rec = np.empty(n, dtype=HIT_DTYPE)
+    check(lib().rh_closest_intersection(scene.device, rays.ctypes.data, n, rec.ctypes.data, flags))
+    return Hits(rec["t"], rec["p"], rec["n"], rec["uv"], rec["object"], rec["tri"], rec)
+
+
+def shadowIntersection(scene, light: int, origins, directions, exact_boxes: bool = False):
+    """RayHs.hs:74-87 for every ray towards light `light` (index into the scene's lights): True where a non-emitter
+    object has a hit in front of the light.  The caller builds the rays, as accumDiffuse does with `rayEps p ld`.
+    Returns a bool numpy array or CUDA tensor, like the rays."""
+    rays, on_device = _query_rays(origins, directions)
+    n = rays.shape[0]
+    flags = (capi.RH_FLAG_DEVICE_OUT if on_device else 0) | (capi.RH_FLAG_EXACT_BOXES if exact_boxes else 0)
+    if on_device:
+        import torch
+
+        out = torch.empty(n, dtype=torch.uint8, device=rays.device)
+    else:
+        out = np.empty(n, dtype=np.uint8)
+    check(lib().rh_shadow_intersection(scene.device, int(light), _ptr(rays), n, _ptr(out), flags))
+    return out.view(torch.bool) if on_device else out.view(np.bool_)
+
+
 def scene_setup_ms(scene: Scene) -> dict:
     """Milliseconds rh_scene_create spent on its parts (host-side trees, light-space tables, uploads)."""
     ms, info = scene._info()
