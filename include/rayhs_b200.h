@@ -362,6 +362,33 @@ int rh_closest_intersection(const rh_scene* scene, const double* rays, uint64_t 
 int rh_shadow_intersection(const rh_scene* scene, uint32_t light, const double* rays, uint64_t n, uint8_t* occluded_out,
                            int32_t flags);
 
+/* ---- radiance queries ----------------------------------------------- */
+typedef struct rh_trace_opts {
+  int32_t max_depth;   /* 0 .. 30, as rh_render_opts.max_depth                                                      */
+  int32_t flags;       /* RH_FLAG_DEVICE_OUT | RH_FLAG_HIT_IDS | RH_FLAG_EXACT_BOXES | RH_FLAG_SHADOW_POOLED |
+                          RH_FLAG_SHADOW_SPLIT | RH_FLAG_NO_LIGHT_MAPS; any other bit is RH_ERR_ARG                    */
+  uint32_t chunk_rays; /* 0 = library default; else rays per wavefront chunk, in whole rows of 4096 rays (at least one) */
+  uint32_t reserved_;
+} rh_trace_opts;
+
+/* Replaces `traceRay sc 0 max_depth r` (RayHs.hs:149-154) for n caller-built rays: the full Whitted radiance of each
+ * ray (shadows, reflection, refraction, textures, the depth limit), as rh_render computes it for a camera ray.
+ * `traceRay sc d maxD` depends on d and maxD only through maxD - d (specular: depth < maxDepth; Transparent:
+ * d /= maxDepth), so a ray that starts at depth d is traced with max_depth = maxD - d.
+ * rays: double[n][6] = origin, direction, as for rh_closest_intersection.
+ * colors_out: double[n][3], the linear colour traceRay returns: not averaged, not clamped, no toIntC.  (rh_render's RGB8
+ * of a camera ray at spp = 1 is toIntC of this value.)  Colours are sums of light terms in the wavefront's order, so
+ * they may differ from the reference's in the last bits (DESIGN.md §3).
+ * hit_ids_out (RH_FLAG_HIT_IDS): int32[n][2] = (object, tri) of the ray's own closest hit, as rh_render writes them.
+ * RH_FLAG_DEVICE_OUT: rays, colors_out and hit_ids_out are DEVICE pointers on the current device (rays 16-byte aligned,
+ * colours and ids 8-byte aligned); else host buffers, streamed through device scratch.  The shadow-walk flags force a
+ * schedule; without them the call uses the one the scene's renders chose, else the pooled one.  The call never changes
+ * what later rh_render calls of the scene do.  n == 0 is RH_OK; a null buffer with n > 0 is RH_ERR_ARG.
+ * stats (optional): rays_primary = n, the other ray counts, queue_factor, shadow_split, chunks and ms_total as
+ * rh_render fills them. */
+int rh_trace_rays(const rh_scene* scene, const double* rays, uint64_t n, const rh_trace_opts* opts, double* colors_out,
+                  int32_t* hit_ids_out, rh_stats* stats);
+
 /* Rows owned by one shard (equal for all shards: bands are padded). */
 int rh_shard_rows(int height, int shard_count, int band_height);
 int rh_default_band_height(int height, int shard_count);

@@ -119,10 +119,14 @@ class rh_hit(C.Structure):
     _fields_ = [("t", C.c_double), ("p", d3), ("n", d3), ("uv", d2), ("object", C.c_int32), ("tri", C.c_int32)]
 
 
+class rh_trace_opts(C.Structure):
+    _fields_ = [("max_depth", C.c_int32), ("flags", C.c_int32), ("chunk_rays", C.c_uint32), ("reserved_", C.c_uint32)]
+
+
 # struct sizes the header promises (checked by tests/test_abi.py against the compiled library too)
 assert C.sizeof(rh_material) == 96 and C.sizeof(rh_light) == 64 and C.sizeof(rh_node) == 64
 assert C.sizeof(rh_tri) == 80 and C.sizeof(rh_tri_shade) == 128 and C.sizeof(rh_object) == 96
-assert C.sizeof(rh_hit) == 80
+assert C.sizeof(rh_hit) == 80 and C.sizeof(rh_trace_opts) == 16
 
 vp = C.c_void_p
 
@@ -141,6 +145,7 @@ SIGNATURES = {
     "rh_render": (C.c_int, [vp, C.POINTER(rh_camera), C.POINTER(rh_render_opts), vp, vp, C.POINTER(rh_stats)]),
     "rh_closest_intersection": (C.c_int, [vp, vp, C.c_uint64, vp, C.c_int32]),
     "rh_shadow_intersection": (C.c_int, [vp, C.c_uint32, vp, C.c_uint64, vp, C.c_int32]),
+    "rh_trace_rays": (C.c_int, [vp, vp, C.c_uint64, C.POINTER(rh_trace_opts), vp, vp, C.POINTER(rh_stats)]),
     "rh_shard_rows": (C.c_int, [C.c_int, C.c_int, C.c_int]),
     "rh_default_band_height": (C.c_int, [C.c_int, C.c_int]),
     "rh_deinterleave_bands": (C.c_int, [vp, vp, C.c_int, C.c_int, C.c_int, C.c_int]),

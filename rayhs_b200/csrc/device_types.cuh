@@ -232,6 +232,9 @@ struct ShadowQueue {
 
 enum { kRayNormal = 0, kRayProbe = 1 };
 enum { kOffIndexLocal = 0, kOffIndexGlobal = 1 };
+// ChunkParams::offset_mode of rh_trace_rays (not an RH_OFFSETS_* value): the pass-0 work items are caller-built rays,
+// double[6] = origin, direction, at `offsets` (ray of item i: offset_base + i), instead of camera rays.
+constexpr int kOffsetsRays = 16;
 
 struct ChunkParams {
   uint32_t first_row;     // first local (shard-compact) row of the chunk
@@ -248,7 +251,7 @@ struct ChunkParams {
   int32_t exact_boxes;    // RH_FLAG_EXACT_BOXES: double slab test for every ray (validation)
   int32_t no_light_maps;  // RH_FLAG_NO_LIGHT_MAPS: shadow rays ignore the lights' cube maps (validation, A/B)
   int32_t hit_live_pass;  // the hit queue (a ring) still holds the hits of this pass and later ones (pass, or pass - 1 when pipelined)
-  int32_t pad6_;
+  uint32_t ray_items;     // kOffsetsRays: pass-0 items of the chunk that are rays (the rest of its last row is padding)
   const void* offsets;    // device
   uint32_t offset_linear; // f64 pairs in work-item order: pair of item i at offsets[offset_base + i] (bulk-copy staging)
   uint32_t pad5_;
@@ -282,7 +285,8 @@ struct QueryParams {
   uint32_t* cursor;    // claim cursor, zero before the launch
 };
 
-// Launchers (kernels.cu).  `count` selects the instrumented instantiation (box/tri counters).
+// Launchers (kernels.cu).  `count` selects the instrumented instantiation (box/tri counters); launch_trace runs the
+// uninstrumented ray instantiation for P.offset_mode == kOffsetsRays.
 // (followed by a one-thread kernel that closes the pass's range of the hit queue, ChunkCtl::hit_start)
 void launch_trace(const SceneView& S, const CameraParams& cam, const ChunkParams& P, bool count, int grid, void* stream);
 // classify_kernel, then the walks of the hits it queued — refill: the per-lane-refill kernel (incoherent rays) instead of
@@ -290,6 +294,8 @@ void launch_trace(const SceneView& S, const CameraParams& cam, const ChunkParams
 // `classified`: a cudaEvent_t recorded after the classify kernel (or null).
 int launch_shadow(const SceneView& S, const ChunkParams& P, bool count, bool refill, int grid, void* stream, void* classified);
 void launch_resolve(const ChunkParams& P, void* stream);
+// rh_trace_rays' end of a chunk instead of the resolve: the accumulators of its rays to colors (double[n][3], all rays)
+void launch_store_colors(const ChunkParams& P, double* colors, void* stream);
 // query_closest_kernel / query_shadow_kernel: `grid` blocks of one SM each
 void launch_query_closest(const SceneView& S, const QueryParams& Q, int grid, void* stream);
 void launch_query_shadow(const SceneView& S, const QueryParams& Q, int grid, void* stream);

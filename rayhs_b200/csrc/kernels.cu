@@ -10,6 +10,7 @@
 //                         takes its next light or the next hit while its neighbours keep walking.
 //   shadow_simple_kernel  K3 for scenes with more than 32 lights.
 //   resolve_kernel        K6: average the samples of a pixel, toIntC, coalesced RGB8 store (or peer stores).
+//   store_colors_kernel   K6 of rh_trace_rays: the linear colours of caller-built rays (trace_kernel<.., RAYS = true>).
 //   deinterleave          K7: band re-assembly after the all-gather.
 //
 // All arithmetic is IEEE double in the reference's operation order and this file is compiled with -fmad=false (GHC
@@ -1484,10 +1485,20 @@ __device__ __forceinline__ bool stage_start(const ChunkParams& P, bool primary, 
 // Work item -> ray: the camera ray of a pixel sample (pass 0: pixelCoord, Image.hs:31-32, + sample offset,
 // RayHs.hs:178-181) or a queued secondary ray with its weight and tags.  False for a padding row of the last band.
 // `tile`: the item's batch was staged in shared memory (see stage_start), else it is read from global memory.
+// RAYS (rh_trace_rays, P.offset_mode == kOffsetsRays): pass 0 reads caller-built rays instead; false past the chunk's rays.
+template <bool RAYS>
 __device__ __forceinline__ bool load_item(const ChunkParams& P, const CameraParams& cam, uint32_t item, bool primary,
                                           const StageTile* tile, uint32_t lane, Ray& r, double& w, uint32_t& sample, int& depth,
                                           int& kind, uint32_t& probe_mat) {
   r.o = r.d = mk(0, 0, 1);
+  if (RAYS && primary) {
+    if (item >= P.ray_items) return false;
+    const double2* src = (const double2*)P.offsets + 3 * (P.offset_base + item);
+    const double2 a = __ldg(src), b = __ldg(src + 1), c = __ldg(src + 2);
+    r.o = mk(a.x, a.y, b.x);
+    r.d = mk(b.y, c.x, c.y);
+    return true;
+  }
   if (primary) {
     size_t idx;
     uint32_t grow, col, s;
@@ -1547,7 +1558,8 @@ static_assert(sizeof(SmemTables) % 128 == 0 || !RH_TMA_STAGE, "staging tiles nee
 static_assert(((size_t)kShortStack * kTraceBlock * sizeof(uint2)) % 128 == 0, "stack columns keep the alignment");
 static_assert(kTraceSmem <= 227 * 1024, "trace kernel shared memory");
 
-template <bool COUNT>
+// RAYS: rh_trace_rays' instantiation (caller-built rays in pass 0, see load_item); the render's is RAYS = false.
+template <bool COUNT, bool RAYS>
 __global__ void __launch_bounds__(kTraceBlock, kTracePerSm) trace_kernel(const __grid_constant__ SceneView S,
                                                                const __grid_constant__ CameraParams cam,
                                                                const __grid_constant__ ChunkParams P) {
@@ -1606,7 +1618,7 @@ __global__ void __launch_bounds__(kTraceBlock, kTracePerSm) trace_kernel(const _
         tile = &wsm.tile;
       }
 #endif
-      if (valid) valid = load_item(P, cam, item, primary, tile, lane, r, w, sample, depth, kind, probe_mat);
+      if (valid) valid = load_item<RAYS>(P, cam, item, primary, tile, lane, r, w, sample, depth, kind, probe_mat);
       else r.o = r.d = mk(0, 0, 1);
 #if RH_TMA_STAGE
       // the tile is in registers now: ask for the next batch of this claim (same slab); it lands while this one is traced
@@ -2519,6 +2531,19 @@ __global__ void __launch_bounds__(kBlock) resolve_kernel(const __grid_constant__
   }
 }
 
+// ------------------------------------------------------------------ K6': rh_trace_rays' colours (RayHs.hs:149-154)
+// One ray per sample, so the accumulators are the colours traceRay returns: the three planes of a block's rays are read
+// coalesced and leave interleaved as double[3] per ray, also coalesced, through shared memory.  No arithmetic.
+__global__ void __launch_bounds__(kBlock) store_colors_kernel(const __grid_constant__ ChunkParams P, double* __restrict__ colors) {
+  __shared__ double rgb[kBlock * 3];
+  const uint32_t first = blockIdx.x * kBlock, n_here = min((uint32_t)kBlock, P.ray_items - first);
+  if (threadIdx.x < n_here)
+    for (int c = 0; c < 3; c++) rgb[3 * threadIdx.x + c] = P.accum[(size_t)c * P.accum_stride + first + threadIdx.x];
+  __syncthreads();
+  double* dst = colors + ((size_t)P.first_row * P.width + first) * 3;
+  for (uint32_t i = threadIdx.x; i < 3 * n_here; i += kBlock) dst[i] = rgb[i];
+}
+
 // ------------------------------------------------------------------ K7: band de-interleave after the all-gather
 __global__ void deinterleave_kernel(const uint8_t* __restrict__ gathered, uint8_t* __restrict__ out, uint32_t row_bytes,
                                     uint32_t height, uint32_t shard_count, uint32_t band_height, uint32_t rows_per_shard) {
@@ -2600,8 +2625,9 @@ int configure_kernels() {
   auto set = [&](const void* fn, size_t bytes) {
     if (e == cudaSuccess) e = cudaFuncSetAttribute(fn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bytes);
   };
-  set((const void*)trace_kernel<true>, kTraceSmem);
-  set((const void*)trace_kernel<false>, kTraceSmem);
+  set((const void*)trace_kernel<true, false>, kTraceSmem);
+  set((const void*)trace_kernel<false, false>, kTraceSmem);
+  set((const void*)trace_kernel<false, true>, kTraceSmem);
   set((const void*)shadow_pooled_kernel<true>, kShadowSmem);
   set((const void*)shadow_pooled_kernel<false>, kShadowSmem);
   set((const void*)shadow_refill_kernel<true>, kWalkSmem);
@@ -2633,8 +2659,9 @@ int max_threads_per_launch(int n_sms) {
 }
 void launch_trace(const SceneView& S, const CameraParams& cam, const ChunkParams& P, bool count, int grid, void* stream) {
   cudaStream_t st = (cudaStream_t)stream;
-  if (count) trace_kernel<true><<<grid * kTracePerSm, kTraceBlock, kTraceSmem, st>>>(S, cam, P);
-  else trace_kernel<false><<<grid * kTracePerSm, kTraceBlock, kTraceSmem, st>>>(S, cam, P);
+  if (P.offset_mode == kOffsetsRays) trace_kernel<false, true><<<grid * kTracePerSm, kTraceBlock, kTraceSmem, st>>>(S, cam, P);
+  else if (count) trace_kernel<true, false><<<grid * kTracePerSm, kTraceBlock, kTraceSmem, st>>>(S, cam, P);
+  else trace_kernel<false, false><<<grid * kTracePerSm, kTraceBlock, kTraceSmem, st>>>(S, cam, P);
   close_hit_range_kernel<<<1, 1, 0, st>>>(P.ctl, P.pass);
 }
 int launch_shadow(const SceneView& S, const ChunkParams& P, bool count, bool refill, int grid, void* stream, void* classified) {
@@ -2666,6 +2693,9 @@ int launch_shadow(const SceneView& S, const ChunkParams& P, bool count, bool ref
 void launch_resolve(const ChunkParams& P, void* stream) {
   const uint32_t n_pixels = P.n_rows * P.width;
   resolve_kernel<<<(n_pixels + kBlock - 1) / kBlock, kBlock, 0, (cudaStream_t)stream>>>(P);
+}
+void launch_store_colors(const ChunkParams& P, double* colors, void* stream) {
+  store_colors_kernel<<<(P.ray_items + kBlock - 1) / kBlock, kBlock, 0, (cudaStream_t)stream>>>(P, colors);
 }
 void launch_query_closest(const SceneView& S, const QueryParams& Q, int grid, void* stream) {
   query_closest_kernel<<<grid, kQueryBlock, kQuerySmem, (cudaStream_t)stream>>>(S, Q);

@@ -1315,8 +1315,11 @@ struct Launch {
   static void count() { g_launches.fetch_add(1, std::memory_order_relaxed); }
 };
 
+// rays_n > 0: rh_trace_rays (see trace_on): the frame's pass-0 items are rays_n caller-built rays, rgb_out receives their
+// colours as double[rays_n][3] and hit_ids_out their ids; the scene's tuning state is neither used nor changed.
 int render_on(Device* D, const rh_scene* scene, const rh_camera* camera, const rh_render_opts* o, uint8_t* rgb_out,
-              int32_t* hit_ids_out, rh_stats* stats) {
+              int32_t* hit_ids_out, rh_stats* stats, uint64_t rays_n = 0) {
+  const bool rays = rays_n > 0;
   const bool peer_frames = o && (o->flags & RH_FLAG_PEER_FRAMES) != 0;
   if (!scene || !camera || !o || (!rgb_out && !peer_frames)) return rh::set_error(RH_ERR_ARG, "rh_render: null argument");
   if (peer_frames && (!o->peer_frames || o->n_peer_frames <= 0 || o->n_peer_frames > kMaxPeers))
@@ -1334,7 +1337,7 @@ int render_on(Device* D, const rh_scene* scene, const rh_camera* camera, const r
   const int bh = o->band_height > 0 ? o->band_height : rh_default_band_height(H, G);
   const int rows_local = rh_shard_rows(H, G, bh);
   const int mode = o->offset_mode;
-  if (mode < RH_OFFSETS_NONE || mode > RH_OFFSETS_SPLITMIX64) return rh::set_error(RH_ERR_ARG, "rh_render: bad offset_mode");
+  if (!rays && (mode < RH_OFFSETS_NONE || mode > RH_OFFSETS_SPLITMIX64)) return rh::set_error(RH_ERR_ARG, "rh_render: bad offset_mode");
   if (mode != RH_OFFSETS_NONE && !o->offsets) return rh::set_error(RH_ERR_ARG, "rh_render: offsets is null");
   if (mode == RH_OFFSETS_TILED_F64 && o->offset_tile <= 0) return rh::set_error(RH_ERR_ARG, "rh_render: offset_tile must be > 0");
   if ((uint64_t)W * spp > 0x7fffffffu) return rh::set_error(RH_ERR_ARG, "rh_render: row too large");
@@ -1351,10 +1354,10 @@ int render_on(Device* D, const rh_scene* scene, const rh_camera* camera, const r
   constexpr int kTuneGiveUp = 8;
   const bool refill_ok = scene->refill_possible && scene->view.n_lights <= (uint32_t)kMaskLights;
   const bool forced = (o->flags & (RH_FLAG_SHADOW_POOLED | RH_FLAG_SHADOW_SPLIT)) != 0;
-  if (!refill_ok && scene->shadow_mode == 0) scene->shadow_mode = 1;
+  if (!rays && !refill_ok && scene->shadow_mode == 0) scene->shadow_mode = 1;
   const bool decided = scene->shadow_mode != 0;
   const bool big_frame = (uint64_t)rows_local * W * spp >= (1ull << 21);
-  const bool tuning = !forced && !decided && !(o->flags & RH_FLAG_COUNT) && big_frame;
+  const bool tuning = !rays && !forced && !decided && !(o->flags & RH_FLAG_COUNT) && big_frame;
   bool use_refill = false;
   if (o->flags & RH_FLAG_SHADOW_SPLIT) use_refill = refill_ok;
   else if (o->flags & RH_FLAG_SHADOW_POOLED) use_refill = false;
@@ -1369,9 +1372,9 @@ int render_on(Device* D, const rh_scene* scene, const rh_camera* camera, const r
   // A Transparent hit inserts a probe pass per level (RayHs.hs:136-143): up to 2D + 1 passes.  Without a Transparent
   // material the rays of pass k all have depth k, and pass D emits nothing: D + 1 passes, no empty launches after them.
   const int n_passes = scene->has_transparent ? 2 * o->max_depth + 1 : o->max_depth + 1;
-  const size_t off_elem = (mode == RH_OFFSETS_F32) ? sizeof(float) * 2 : sizeof(double) * 2;
+  const size_t off_elem = rays ? sizeof(double) * 6 : (mode == RH_OFFSETS_F32) ? sizeof(float) * 2 : sizeof(double) * 2;
   const bool host_offsets =
-      (mode == RH_OFFSETS_F64 || mode == RH_OFFSETS_F32) && !(o->flags & RH_FLAG_DEVICE_OFFSETS);
+      (mode == RH_OFFSETS_F64 || mode == RH_OFFSETS_F32 || rays) && !(o->flags & RH_FLAG_DEVICE_OFFSETS);
   // Chunk plan (whole rows).  The secondary passes of a chunk are short launches whose cost is set by their slowest
   // warp, so the fewer and larger the chunks the better (measured on the bench frame with the offsets already in HBM:
   // 16 chunks 65.5 ms, 8 chunks 59.1 ms, 4 chunks 57.0 ms, 1 chunk 55.0 ms).  Default: as large as 40 % of the device
@@ -1399,7 +1402,7 @@ int render_on(Device* D, const rh_scene* scene, const rh_camera* camera, const r
     // What the last streamed frame of this shape measured: kernel time per row, and whether the kernels or the upload
     // finished last.
     const std::vector<int> shape_key = {W, H, spp, G, o->shard_index, bh};
-    know_cost = host_offsets && o->chunk_samples <= 0 && scene->cost_key == shape_key && (int)scene->row_cost.size() == rows_local;
+    know_cost = !rays && host_offsets && o->chunk_samples <= 0 && scene->cost_key == shape_key && (int)scene->row_cost.size() == rows_local;
     auto density = [&](int row0, int n) {
       double c = 0;
       for (int r = row0; r < row0 + n; r++) c += scene->row_cost[r];
@@ -1465,7 +1468,7 @@ int render_on(Device* D, const rh_scene* scene, const rh_camera* camera, const r
 
   int rc;
   uint8_t* d_rgb;
-  const size_t rgb_bytes = (size_t)rows_local * W * 3;
+  const size_t rgb_bytes = rays ? (size_t)rays_n * 3 * sizeof(double) : (size_t)rows_local * W * 3;
   if (peer_frames) d_rgb = nullptr;
   else if (dev_out) d_rgb = rgb_out;
   else {
@@ -1473,7 +1476,7 @@ int render_on(Device* D, const rh_scene* scene, const rh_camera* camera, const r
     d_rgb = (uint8_t*)D->rgb.p;
   }
   int2* d_ids = nullptr;
-  const size_t ids_bytes = (size_t)rows_local * row_samples * sizeof(int2);
+  const size_t ids_bytes = (rays ? (size_t)rays_n : (size_t)rows_local * row_samples) * sizeof(int2);
   if (want_ids) {
     if (dev_out) d_ids = (int2*)hit_ids_out;
     else {
@@ -1543,7 +1546,8 @@ int render_on(Device* D, const rh_scene* scene, const rh_camera* camera, const r
     }
   }
 
-  uint32_t factor = std::max(2u, scene->queue_factor);  // queue capacity = factor * chunk samples; doubled when a chunk overflows (and remembered)
+  // queue capacity = factor * chunk samples; doubled when a chunk overflows (and remembered by the scene's renders)
+  uint32_t factor = rays ? 2u : std::max(2u, scene->queue_factor);
   for (;;) {
     // Queue capacity in entries, a whole number of slabs: factor x the chunk's samples, plus one partly filled slab
     // per warp that can be producing (each warp leaves its last slab of a queue open).
@@ -1679,8 +1683,9 @@ int render_on(Device* D, const rh_scene* scene, const rh_camera* camera, const r
           const long long grow = ((long long)lb * G + o->shard_index) * bh + rib;
           const long long rows_ok = std::max<long long>(0, std::min<long long>(run, (long long)H - grow));
           if (rows_ok > 0) {
-            const size_t bytes = (size_t)rows_ok * row_samples * off_elem;
             const size_t src_row = shard_offsets ? (size_t)lr : (size_t)grow;
+            size_t bytes = (size_t)rows_ok * row_samples * off_elem;
+            if (rays) bytes = std::min(bytes, ((size_t)rays_n - src_row * row_samples) * off_elem);  // (a partial last row)
             RH_CUDA(cudaMemcpyAsync(slot + (size_t)(lr - first_row) * row_samples * off_elem,
                                     (const char*)o->offsets + src_row * row_samples * off_elem, bytes,
                                     cudaMemcpyHostToDevice, D->copy_stream));
@@ -1704,6 +1709,7 @@ int render_on(Device* D, const rh_scene* scene, const rh_camera* camera, const r
       // offsets in work-item order?  chunk-local slices always; the full-frame array when the frame is not sharded
       P.offset_linear = (mode == RH_OFFSETS_F64 && (P.offset_index == kOffIndexLocal || G == 1)) ? 1u : 0u;
       P.offset_base = (P.offset_index == kOffIndexLocal) ? 0ull : (unsigned long long)first_row * row_samples;
+      if (rays) P.ray_items = (uint32_t)std::min<uint64_t>(P.n_samples, rays_n - (uint64_t)first_row * row_samples);
       for (int plane = 0; plane < 3; plane++)  // (three 1-D memsets: a 2-D one is limited to 2 GB of pitch)
         RH_CUDA(cudaMemsetAsync((double*)sc.accum.p + (size_t)plane * chunk_samples, 0, (size_t)P.n_samples * sizeof(double), lane_stream));
       const int ln = i % n_lanes;
@@ -1739,7 +1745,8 @@ int render_on(Device* D, const rh_scene* scene, const rh_camera* camera, const r
       }
       cudaEvent_t a = nullptr;
       if (profile) a = prof_event();
-      launch_resolve(P, lane_stream);
+      if (rays) launch_store_colors(P, (double*)d_rgb, lane_stream);
+      else launch_resolve(P, lane_stream);
       if (profile) spans.push_back({a, prof_event(), 2});
       launches += 1;
       if (stream_offsets) {
@@ -1769,9 +1776,10 @@ int render_on(Device* D, const rh_scene* scene, const rh_camera* camera, const r
     for (int ck = 0; ck < n_chunks; ck++) overflow |= ctl[ck].overflow != 0;
     if (overflow) {
       if (cap >= 0x7fffff00u || factor >= (1u << 16))
-        return rh::set_error(RH_ERR_OVERFLOW, "rh_render: ray queue overflow; lower chunk_samples");
+        return rh::set_error(RH_ERR_OVERFLOW, rays ? "rh_trace_rays: ray queue overflow; lower chunk_rays"
+                                                   : "rh_render: ray queue overflow; lower chunk_samples");
       factor *= 2;
-      scene->queue_factor = factor;
+      if (!rays) scene->queue_factor = factor;
       continue;
     }
     if (stats) {
@@ -1787,7 +1795,7 @@ int render_on(Device* D, const rh_scene* scene, const rh_camera* camera, const r
         const long long grow = ((long long)(lr / bh) * G + o->shard_index) * bh + lr % bh;
         if (grow < H) real_rows++;
       }
-      stats->rays_primary = real_rows * row_samples;
+      stats->rays_primary = rays ? rays_n : real_rows * row_samples;
       stats->rays_reflect = fc->rays_reflect;
       stats->rays_probe = fc->rays_probe;
       stats->rays_exit = fc->rays_exit;
@@ -1897,7 +1905,7 @@ int render_on(Device* D, const rh_scene* scene, const rh_camera* camera, const r
         fprintf(stderr, "rayhs_b200:   chunk %2d lane %d rows %4d  up %6.2f  begin %6.2f  end %6.2f\n", order[i], i % n_lanes, plan[order[i]], up, kb, ke);
       }
     }
-    if (stream_offsets && o->chunk_samples <= 0 && (int)chunk_ev.size() == 2 * n_chunks && (int)copy_ev.size() == n_chunks) {
+    if (!rays && stream_offsets && o->chunk_samples <= 0 && (int)chunk_ev.size() == 2 * n_chunks && (int)copy_ev.size() == n_chunks) {
       scene->row_cost.assign(rows_local, 0.f);
       for (int i = 0; i < n_chunks; i++) {
         float ms = 0;
@@ -1928,7 +1936,7 @@ int render_on(Device* D, const rh_scene* scene, const rh_camera* camera, const r
       } else if (++scene->tune_small_frames >= kTuneGiveUp) {
         scene->shadow_mode = 1;
       }
-    } else if (!forced && !decided && !(o->flags & RH_FLAG_COUNT)) {
+    } else if (!rays && !forced && !decided && !(o->flags & RH_FLAG_COUNT)) {
       if (++scene->tune_small_frames >= kTuneGiveUp) scene->shadow_mode = 1;
     }
     return RH_OK;
@@ -1998,6 +2006,60 @@ int query_on(Device* D, const rh_scene* scene, int64_t light, const double* rays
   }
   RH_CUDA(cudaStreamSynchronize(D->stream));
   return RH_OK;
+}
+
+// ------------------------------------------------------------------ radiance queries
+// rh_trace_rays runs the render's wavefront on a frame of one sample per ray: kTraceRowRays rays per row, as many rows
+// as the rays need, unsharded.  Pass 0 reads the rays (kOffsetsRays) and the colours leave unquantised; everything in
+// between — chunk plan, queues, overflow retry, pipelined passes, counts — is render_on's.
+constexpr int kTraceRowRays = 4096;
+
+int trace_on(Device* D, const rh_scene* scene, const double* rays, uint64_t n, const rh_trace_opts* o, double* colors_out,
+             int32_t* hit_ids_out, rh_stats* stats) {
+  if (!scene || !o) return rh::set_error(RH_ERR_ARG, "rh_trace_rays: null scene or opts");
+  if (scene->device != D) return rh::set_error(RH_ERR_ARG, "rh_trace_rays: scene lives on another device context");
+  constexpr int32_t kFlags = RH_FLAG_DEVICE_OUT | RH_FLAG_HIT_IDS | RH_FLAG_EXACT_BOXES | RH_FLAG_SHADOW_POOLED |
+                             RH_FLAG_SHADOW_SPLIT | RH_FLAG_NO_LIGHT_MAPS;
+  if (o->flags & ~kFlags) return rh::set_error(RH_ERR_ARG, "rh_trace_rays: unknown flag bits");
+  if (o->max_depth < 0 || o->max_depth > kMaxDepth) return rh::set_error(RH_ERR_ARG, "rh_trace_rays: max_depth outside 0..30");
+  if (n == 0) {
+    if (stats) memset(stats, 0, sizeof *stats);
+    return RH_OK;
+  }
+  const bool want_ids = (o->flags & RH_FLAG_HIT_IDS) != 0, dev = (o->flags & RH_FLAG_DEVICE_OUT) != 0;
+  if (!rays || !colors_out) return rh::set_error(RH_ERR_ARG, "rh_trace_rays: null buffer");
+  if (want_ids && !hit_ids_out) return rh::set_error(RH_ERR_ARG, "rh_trace_rays: RH_FLAG_HIT_IDS without hit_ids_out");
+  const uint64_t rows = (n + kTraceRowRays - 1) / kTraceRowRays;
+  if (rows > 0x7fffffffu) return rh::set_error(RH_ERR_ARG, "rh_trace_rays: too many rays");
+  RH_CUDA(cudaSetDevice(D->dev));
+  if (dev) {
+    // rays are read as 16-byte words; colours and ids are written as 8-byte words
+    if ((uintptr_t)rays % 16 || (uintptr_t)colors_out % 8 || (want_ids && (uintptr_t)hit_ids_out % 8))
+      return rh::set_error(RH_ERR_ARG, "rh_trace_rays: device rays must be 16-byte aligned, colours and ids 8-byte aligned");
+    for (const void* p : {(const void*)rays, (const void*)colors_out, (const void*)(want_ids ? hit_ids_out : nullptr)}) {
+      if (!p) continue;
+      cudaPointerAttributes a{};
+      RH_CUDA(cudaPointerGetAttributes(&a, p));
+      if (a.type != cudaMemoryTypeDevice && a.type != cudaMemoryTypeManaged)
+        return rh::set_error(RH_ERR_ARG, "rh_trace_rays: RH_FLAG_DEVICE_OUT with a pointer that is not device memory");
+    }
+  }
+  rh_render_opts ro{};
+  ro.width = kTraceRowRays;
+  ro.height = (int)rows;
+  ro.max_depth = o->max_depth;
+  ro.spp = 1;
+  ro.offset_mode = kOffsetsRays;
+  ro.offsets = rays;
+  ro.shard_count = 1;
+  ro.chunk_samples = (int)std::min<uint64_t>(o->chunk_rays, 0x7fffffffu);
+  ro.flags = o->flags | (dev ? RH_FLAG_DEVICE_OFFSETS : 0);
+  rh_camera cam{};  // (no camera rays: any valid camera)
+  cam.target[2] = 1;
+  cam.up[1] = 1;
+  cam.projection = RH_PROJ_PERSPECTIVE;
+  cam.fovy = 1;
+  return render_on(D, scene, &cam, &ro, (uint8_t*)colors_out, hit_ids_out, stats, n);
 }
 
 }  // namespace
@@ -2107,6 +2169,12 @@ int rh_render(const rh_scene* scene, const rh_camera* camera, const rh_render_op
               int32_t* hit_ids_out, rh_stats* stats) {
   if (!g_dev) return rh::set_error(RH_ERR_STATE, "rh_render: call rh_init first");
   return render_on(g_dev.get(), scene, camera, opts, rgb_out, hit_ids_out, stats);
+}
+
+int rh_trace_rays(const rh_scene* scene, const double* rays, uint64_t n, const rh_trace_opts* opts, double* colors_out,
+                  int32_t* hit_ids_out, rh_stats* stats) {
+  if (!g_dev) return rh::set_error(RH_ERR_STATE, "rh_trace_rays: call rh_init first");
+  return trace_on(g_dev.get(), scene, rays, n, opts, colors_out, hit_ids_out, stats);
 }
 
 int rh_closest_intersection(const rh_scene* scene, const double* rays, uint64_t n, rh_hit* hits_out, int32_t flags) {

@@ -330,6 +330,47 @@ def shadowIntersection(scene, light: int, origins, directions, exact_boxes: bool
     return out.view(torch.bool) if on_device else out.view(np.bool_)
 
 
+# ---- radiance queries (RayHs.hs:149-154 traceRay)
+
+@dataclass
+class Radiance:
+    """traceRay of a batch of rays: colors [n, 3] float64 (linear, not clamped, no toIntC), hit_ids [n, 2] int32
+    (object, tri) of each ray's closest hit when asked for, numpy arrays or CUDA tensors like the rays, and the call's
+    rh_stats as Image carries them."""
+    colors: object
+    stats: dict = field(default_factory=dict)
+    hit_ids: object = None
+
+
+def traceRay(scene, origins, directions, max_depth: int, *, want_hit_ids: bool = False, exact_boxes: bool = False,
+             shadow: str | None = None, light_maps: bool = True, chunk_rays: int = 0) -> Radiance:
+    """RayHs.hs:149-154 `traceRay sc 0 max_depth` for every ray (origins[i], directions[i]): the full Whitted radiance
+    (shadows, reflection, refraction, textures), as the render computes it for a camera ray.  A ray that starts at depth
+    d of a tree limited to maxD is traced with max_depth = maxD - d.  numpy arrays in, numpy arrays out; CUDA tensors
+    in, CUDA tensors out.  `shadow` ('pooled' / 'split'), `exact_boxes` and `light_maps` as for render (same colours);
+    `chunk_rays`: rays per wavefront chunk (0: the library's choice)."""
+    rays, on_device = _query_rays(origins, directions)
+    if not 0 <= int(chunk_rays) < 1 << 32:
+        raise ValueError(f"chunk_rays must be in 0 .. 2^32 - 1, got {chunk_rays}")
+    n = rays.shape[0]
+    o = capi.rh_trace_opts()
+    o.max_depth, o.chunk_rays = int(max_depth), int(chunk_rays)
+    o.flags = ((capi.RH_FLAG_DEVICE_OUT if on_device else 0) | (capi.RH_FLAG_HIT_IDS if want_hit_ids else 0)
+               | (capi.RH_FLAG_EXACT_BOXES if exact_boxes else 0) | _shadow_flag(shadow) | (0 if light_maps else capi.RH_FLAG_NO_LIGHT_MAPS))
+    if on_device:
+        import torch
+
+        colors = torch.empty((n, 3), dtype=torch.float64, device=rays.device)
+        ids = torch.empty((n, 2), dtype=torch.int32, device=rays.device) if want_hit_ids else None
+    else:
+        colors = np.empty((n, 3), dtype=np.float64)
+        ids = np.empty((n, 2), dtype=np.int32) if want_hit_ids else None
+    st = capi.rh_stats()
+    check(lib().rh_trace_rays(scene.device, _ptr(rays), n, C.byref(o), _ptr(colors), _ptr(ids) if ids is not None else None,
+                              C.byref(st)))
+    return Radiance(colors, st.as_dict(), ids)
+
+
 def scene_setup_ms(scene: Scene) -> dict:
     """Milliseconds rh_scene_create spent on its parts (host-side trees, light-space tables, uploads)."""
     ms, info = scene._info()
