@@ -74,13 +74,6 @@ struct __align__(16) WideNode {
   uint32_t refine;    // bit c: child c's box is not a box the reference tests (sphere tree): the exact walk passes it
   uint32_t pad_[3];
 };
-#ifndef RH_STREAM_CHUNK_MI
-#define RH_STREAM_CHUNK_MI 16  // chunk size (Mi samples) when the sample offsets stream in from the host
-#define RH_STREAM_FIRST_MI 4   // ... and of the first chunk, whose upload nothing overlaps
-#endif
-#ifndef RH_LANES
-#define RH_LANES 2  // chunks in flight (streams with their own queues); 1 = strictly one chunk after the other
-#endif
 #ifndef RH_SUBLEAF
 #define RH_SUBLEAF 4  // triangles per leaf of the float path's cull tree (measured: 3-4 best of 2, 3, 4, 6, 8)
 #endif

@@ -20,6 +20,7 @@
 #include <cstdlib>
 #include <cstring>
 #include <deque>
+#include <initializer_list>
 #include <limits>
 #include <memory>
 #include <mutex>
@@ -30,6 +31,7 @@
 #include "common.h"
 #include "device_types.cuh"
 #include "light_geom.h"
+#include "render_plan.h"
 
 namespace rh {
 static thread_local std::string g_err;
@@ -1311,15 +1313,27 @@ CameraParams make_camera(const rh_camera& c, int width, int height) {
 }
 
 // ------------------------------------------------------------------ render
-struct Launch {
-  static void count() { g_launches.fetch_add(1, std::memory_order_relaxed); }
+// One validated frame for run_frame: a render (rh_render, one shard of rh_multi_render) or the ray frame of
+// rh_trace_rays.
+struct Frame {
+  rh_render_opts o{};        // shard_count and band_height resolved
+  CameraParams cam{};        // (renders)
+  uint8_t* out = nullptr;    // RGB8 rows, or (trace) the colours as double[n_rays][3]; null with RH_FLAG_PEER_FRAMES
+  int32_t* ids_out = nullptr;
+  size_t out_bytes = 0, ids_bytes = 0;
+  int rows_local = 0;
+  size_t off_elem = 0;       // bytes per pass-0 item of o.offsets
+  uint64_t rays_primary = 0;
+  // rh_trace_rays: pass 0 reads n_rays caller-built rays (the last row may be partial), the colours leave unquantised,
+  // and the scene's learned state (shadow-schedule tuning, queue factor, row costs) is neither used nor changed
+  bool trace = false;
+  uint64_t n_rays = 0;
+  const char* overflow_error = "rh_render: ray queue overflow; lower chunk_samples";
 };
 
-// rays_n > 0: rh_trace_rays (see trace_on): the frame's pass-0 items are rays_n caller-built rays, rgb_out receives their
-// colours as double[rays_n][3] and hit_ids_out their ids; the scene's tuning state is neither used nor changed.
-int render_on(Device* D, const rh_scene* scene, const rh_camera* camera, const rh_render_opts* o, uint8_t* rgb_out,
-              int32_t* hit_ids_out, rh_stats* stats, uint64_t rays_n = 0) {
-  const bool rays = rays_n > 0;
+// rh_render's argument checks.
+int render_frame(Device* D, const rh_scene* scene, const rh_camera* camera, const rh_render_opts* o, uint8_t* rgb_out,
+                 int32_t* hit_ids_out, Frame* f) {
   const bool peer_frames = o && (o->flags & RH_FLAG_PEER_FRAMES) != 0;
   if (!scene || !camera || !o || (!rgb_out && !peer_frames)) return rh::set_error(RH_ERR_ARG, "rh_render: null argument");
   if (peer_frames && (!o->peer_frames || o->n_peer_frames <= 0 || o->n_peer_frames > kMaxPeers))
@@ -1335,228 +1349,107 @@ int render_on(Device* D, const rh_scene* scene, const rh_camera* camera, const r
   const int G = o->shard_count <= 0 ? 1 : o->shard_count;
   if (o->shard_index < 0 || o->shard_index >= G) return rh::set_error(RH_ERR_ARG, "rh_render: shard_index out of range");
   const int bh = o->band_height > 0 ? o->band_height : rh_default_band_height(H, G);
-  const int rows_local = rh_shard_rows(H, G, bh);
   const int mode = o->offset_mode;
-  if (!rays && (mode < RH_OFFSETS_NONE || mode > RH_OFFSETS_SPLITMIX64)) return rh::set_error(RH_ERR_ARG, "rh_render: bad offset_mode");
+  if (mode < RH_OFFSETS_NONE || mode > RH_OFFSETS_SPLITMIX64) return rh::set_error(RH_ERR_ARG, "rh_render: bad offset_mode");
   if (mode != RH_OFFSETS_NONE && !o->offsets) return rh::set_error(RH_ERR_ARG, "rh_render: offsets is null");
   if (mode == RH_OFFSETS_TILED_F64 && o->offset_tile <= 0) return rh::set_error(RH_ERR_ARG, "rh_render: offset_tile must be > 0");
   if ((uint64_t)W * spp > 0x7fffffffu) return rh::set_error(RH_ERR_ARG, "rh_render: row too large");
-  const bool want_ids = (o->flags & RH_FLAG_HIT_IDS) != 0;
-  if (want_ids && !hit_ids_out) return rh::set_error(RH_ERR_ARG, "rh_render: RH_FLAG_HIT_IDS without hit_ids_out");
-  const bool dev_out = (o->flags & RH_FLAG_DEVICE_OUT) != 0;
-  const bool dev_off = (o->flags & RH_FLAG_DEVICE_OFFSETS) != 0;
-  const bool shard_offsets = (o->flags & RH_FLAG_SHARD_OFFSETS) != 0;  // offsets = this shard's rows only, shard-compact
-  const bool counting = (o->flags & RH_FLAG_COUNT) != 0;
-  // Shadow-walk schedule: forced by flags, else the scene's measured choice, else — on frames large enough to time —
-  // one of the scene's timing frames: the first is pooled and not compared (first use of freshly allocated queues), the
-  // second pooled, the third per-lane refill; the two kernels' times per walked (hit, light) pair are compared.  Small
-  // frames never take part: they run pooled, unprofiled, and after kTuneGiveUp of them the scene stays pooled.
-  constexpr int kTuneGiveUp = 8;
-  const bool refill_ok = scene->refill_possible && scene->view.n_lights <= (uint32_t)kMaskLights;
-  const bool forced = (o->flags & (RH_FLAG_SHADOW_POOLED | RH_FLAG_SHADOW_SPLIT)) != 0;
-  if (!rays && !refill_ok && scene->shadow_mode == 0) scene->shadow_mode = 1;
-  const bool decided = scene->shadow_mode != 0;
-  const bool big_frame = (uint64_t)rows_local * W * spp >= (1ull << 21);
-  const bool tuning = !rays && !forced && !decided && !(o->flags & RH_FLAG_COUNT) && big_frame;
+  if ((o->flags & RH_FLAG_HIT_IDS) && !hit_ids_out) return rh::set_error(RH_ERR_ARG, "rh_render: RH_FLAG_HIT_IDS without hit_ids_out");
+  if (mode == RH_OFFSETS_SPLITMIX64 && (o->flags & RH_FLAG_DEVICE_OFFSETS))
+    return rh::set_error(RH_ERR_ARG, "rh_render: RH_OFFSETS_SPLITMIX64 takes a host pointer to the seed");
+  f->o = *o;
+  f->o.shard_count = G;
+  f->o.band_height = bh;
+  f->cam = make_camera(*camera, W, H);
+  f->out = rgb_out;
+  f->ids_out = hit_ids_out;
+  f->rows_local = rh_shard_rows(H, G, bh);
+  f->out_bytes = (size_t)f->rows_local * W * 3;
+  f->ids_bytes = (size_t)f->rows_local * W * spp * sizeof(int2);
+  f->off_elem = (mode == RH_OFFSETS_F32) ? sizeof(float) * 2 : sizeof(double) * 2;
+  for (int lr = 0; lr < f->rows_local; lr++)  // padding rows of the last band trace nothing
+    if (((long long)(lr / bh) * G + o->shard_index) * bh + lr % bh < H) f->rays_primary += (uint64_t)W * spp;
+  return RH_OK;
+}
+
+// Shadow-walk schedule of a frame: forced by flags, else the scene's measured choice, else — on frames large enough to
+// time — one of the scene's timing frames: the first is pooled and not compared (first use of freshly allocated queues),
+// the second pooled, the third per-lane refill; the two kernels' times per walked (hit, light) pair are compared.  Small
+// frames never take part: they run pooled, unprofiled, and after kTuneGiveUp of them the scene stays pooled.  A trace
+// uses the scene's decided schedule and takes no part in the tuning.
+constexpr int kTuneGiveUp = 8;
+struct ShadowChoice {
   bool use_refill = false;
-  if (o->flags & RH_FLAG_SHADOW_SPLIT) use_refill = refill_ok;
-  else if (o->flags & RH_FLAG_SHADOW_POOLED) use_refill = false;
-  else if (decided) use_refill = scene->shadow_mode == 2;
-  else if (tuning) use_refill = scene->tune_frames == 2;
-  const bool profile = (o->flags & RH_FLAG_PROFILE) != 0 || tuning;
-  const bool exact_boxes = (o->flags & RH_FLAG_EXACT_BOXES) != 0;
+  bool untuned = false;  // the schedule is neither forced nor decided: the frame counts towards the tuning
+  bool tuning = false;   // ... and is one of the timing frames
+  bool profile = false;  // every launch is timed on its own
+};
 
-  RH_CUDA(cudaSetDevice(D->dev));
-  const CameraParams cam = make_camera(*camera, W, H);
-  const size_t row_samples = (size_t)W * spp;
-  // A Transparent hit inserts a probe pass per level (RayHs.hs:136-143): up to 2D + 1 passes.  Without a Transparent
-  // material the rays of pass k all have depth k, and pass D emits nothing: D + 1 passes, no empty launches after them.
-  const int n_passes = scene->has_transparent ? 2 * o->max_depth + 1 : o->max_depth + 1;
-  const size_t off_elem = rays ? sizeof(double) * 6 : (mode == RH_OFFSETS_F32) ? sizeof(float) * 2 : sizeof(double) * 2;
-  const bool host_offsets =
-      (mode == RH_OFFSETS_F64 || mode == RH_OFFSETS_F32 || rays) && !(o->flags & RH_FLAG_DEVICE_OFFSETS);
-  // Chunk plan (whole rows).  The secondary passes of a chunk are short launches whose cost is set by their slowest
-  // warp, so the fewer and larger the chunks the better (measured on the bench frame with the offsets already in HBM:
-  // 16 chunks 65.5 ms, 8 chunks 59.1 ms, 4 chunks 57.0 ms, 1 chunk 55.0 ms).  Default: as large as 40 % of the device
-  // memory allows (~450 bytes of queues and accumulators per sample).  When the offsets stream in from the host, chunk
-  // k+1's upload overlaps chunk k's kernels, so the chunks stay moderate (16 Mi samples) and the first one, whose
-  // upload nothing can overlap, is small.
-  std::vector<int> plan;  // rows per chunk
-  int n_tail = 0;         // chunks at the end of the plan that stay last in the processing order (streamed offsets)
-  bool know_cost = false, ramped = false;  // the rows' measured costs are known; the plan is the compute-bound one
-  int ramp_first = 0, ramp_pieces = 1;     // ... whose most expensive chunk starts at plan[ramp_first], in ramp_pieces pieces
-  {
-    size_t want = (size_t)o->chunk_samples, first = want;
-    if (o->chunk_samples <= 0) {
-      // accumulators + (two ray queues + hit queue + half a walk queue) at 2 entries per sample
-      const size_t per_sample = 3 * sizeof(double) + 2 * (2 * 4 * sizeof(double2) + (5 * sizeof(double2) + 8) + (5 * sizeof(double2) + 12) / 2);
-      want = std::min<size_t>((size_t)(0.45 * (double)D->total_mem) / per_sample, (size_t)0x3ffffff0u);
-      // a frame that needs several chunks has two of them in flight, each with its own scratch: half the budget each
-      if (RH_LANES > 1 && (size_t)rows_local * row_samples > want) want /= 2;
-      // (RAYHS_B200_STREAM_CHUNK_MI / RAYHS_B200_STREAM_FIRST_MI: A/B switches of the two sizes)
-      static const size_t stream_chunk = (size_t)(getenv("RAYHS_B200_STREAM_CHUNK_MI") ? std::max(1, atoi(getenv("RAYHS_B200_STREAM_CHUNK_MI"))) : RH_STREAM_CHUNK_MI) << 20;
-      static const size_t stream_first = (size_t)(getenv("RAYHS_B200_STREAM_FIRST_MI") ? std::max(1, atoi(getenv("RAYHS_B200_STREAM_FIRST_MI"))) : RH_STREAM_FIRST_MI) << 20;
-      if (host_offsets) want = std::min<size_t>(want, stream_chunk);
-      first = host_offsets ? std::min<size_t>(want, stream_first) : want;
-    }
-    // What the last streamed frame of this shape measured: kernel time per row, and whether the kernels or the upload
-    // finished last.
-    const std::vector<int> shape_key = {W, H, spp, G, o->shard_index, bh};
-    know_cost = !rays && host_offsets && o->chunk_samples <= 0 && scene->cost_key == shape_key && (int)scene->row_cost.size() == rows_local;
-    auto density = [&](int row0, int n) {
-      double c = 0;
-      for (int r = row0; r < row0 + n; r++) c += scene->row_cost[r];
-      return c / std::max(1, n);
-    };
-    static const bool tail_shaping = !(getenv("RAYHS_B200_TAIL") && getenv("RAYHS_B200_TAIL")[0] == '0');  // (A/B switch)
-    static const bool ramp_plan = !(getenv("RAYHS_B200_RAMP") && getenv("RAYHS_B200_RAMP")[0] == '0');     // (A/B switch)
-    if (know_cost && scene->stream_compute_bound && ramp_plan && (size_t)rows_local * row_samples > 2 * want) {
-      // Compute-bound streaming (the kernels finish after the last byte has arrived): what counts is that the GPU never
-      // waits for data once the first bytes are there.  Equal chunks, the expensive rows first (their kernels keep the GPU
-      // busy while the cheap rows arrive), and the very first chunk processed — the most expensive one — cut into
-      // 1/8, 1/8, 1/4, 1/2 so that its first piece is uploaded quickly and each piece's kernels cover the next piece's
-      // upload.  No small pieces at the end: they only help when the upload finishes last.
-      const int rows_per = (int)std::max<size_t>(1, want / row_samples);
-      for (int row = 0; row < rows_local; row += rows_per) plan.push_back(std::min(rows_per, rows_local - row));
-      if (plan.size() >= 2 && plan.back() * 4 < rows_per) {
-        plan[plan.size() - 2] += plan.back();
-        plan.pop_back();
-      }
-      size_t best = 0;
-      double best_d = -1;
-      for (size_t k = 0, row = 0; k < plan.size(); row += plan[k], k++) {
-        const double dk = density((int)row, plan[k]);
-        if (dk > best_d) { best_d = dk; best = k; }
-      }
-      const int n = plan[best];
-      ramp_first = (int)best;
-      if (n >= 16) {
-        const int e = n / 8;
-        plan[best] = e;
-        plan.insert(plan.begin() + best + 1, {e, 2 * e, n - 4 * e});
-        ramp_pieces = 4;
-      }
-      ramped = true;
-    } else {
-      int row = 0;
-      while (row < rows_local) {
-        const size_t w = plan.empty() ? first : want;
-        const int n = (int)std::max<size_t>(1, std::min<size_t>(w / row_samples, (size_t)(rows_local - row)));
-        plan.push_back(n);
-        row += n;
-      }
-      // Streamed offsets: the frame ends with the kernels of the chunk whose upload finishes last, so the frame's last
-      // chunk is cut into halves of halves (down to ~1 Mi samples): what is left to do after the last byte has arrived is
-      // a small chunk's work.
-      if (tail_shaping && host_offsets && o->chunk_samples <= 0 && plan.size() >= 4) {
-        int last = plan.back();
-        plan.pop_back();
-        const int min_rows = (int)std::max<size_t>(1, ((size_t)1 << 20) / row_samples);
-        while (last > 2 * min_rows && n_tail < 4) {
-          plan.push_back(last - last / 2);
-          last /= 2;
-          n_tail++;
-        }
-        plan.push_back(last);
-        n_tail++;
-      }
-    }
-  }
-  const int n_chunks = (int)plan.size();
-  const size_t chunk_samples = (size_t)*std::max_element(plan.begin(), plan.end()) * row_samples;  // largest chunk
-  if (chunk_samples > 0x7fffffffu) return rh::set_error(RH_ERR_ARG, "rh_render: chunk too large");
+ShadowChoice choose_shadow(const rh_scene* scene, const Frame& f) {
+  const int32_t flags = f.o.flags;
+  const bool refill_ok = scene->refill_possible && scene->view.n_lights <= (uint32_t)kMaskLights;
+  if (!f.trace && !refill_ok && scene->shadow_mode == 0) scene->shadow_mode = 1;
+  const bool forced = (flags & (RH_FLAG_SHADOW_POOLED | RH_FLAG_SHADOW_SPLIT)) != 0;
+  const bool decided = scene->shadow_mode != 0;
+  ShadowChoice c;
+  c.untuned = !f.trace && !forced && !decided && !(flags & RH_FLAG_COUNT);
+  c.tuning = c.untuned && (uint64_t)f.rows_local * f.o.width * f.o.spp >= (1ull << 21);
+  if (flags & RH_FLAG_SHADOW_SPLIT) c.use_refill = refill_ok;
+  else if (flags & RH_FLAG_SHADOW_POOLED) c.use_refill = false;
+  else if (decided) c.use_refill = scene->shadow_mode == 2;
+  else if (c.tuning) c.use_refill = scene->tune_frames == 2;
+  c.profile = (flags & RH_FLAG_PROFILE) != 0 || c.tuning;
+  return c;
+}
 
-  int rc;
-  uint8_t* d_rgb;
-  const size_t rgb_bytes = rays ? (size_t)rays_n * 3 * sizeof(double) : (size_t)rows_local * W * 3;
-  if (peer_frames) d_rgb = nullptr;
-  else if (dev_out) d_rgb = rgb_out;
-  else {
-    if ((rc = D->rgb.reserve(rgb_bytes))) return rc;
-    d_rgb = (uint8_t*)D->rgb.p;
-  }
+struct Span { cudaEvent_t a, b; int kind; };  // a timed launch: 0 trace, 1 shadow kernels, 2 resolve / store
+
+// One frame on one device: its plan and buffers, and what the enqueued chunks recorded.
+struct FrameRun {
+  Device* D;
+  const rh_scene* scene;
+  const Frame& f;
+  ShadowChoice sh;
+  rh::ChunkPlan plan;
+  size_t row_samples = 0, chunk_samples = 0;  // chunk_samples: the largest chunk's
+  int n_chunks = 0, n_passes = 0, n_lanes = 1;
+  bool counting = false, host_offsets = false, pipelined = false;
+  uint8_t* d_rgb = nullptr;
   int2* d_ids = nullptr;
-  const size_t ids_bytes = (rays ? (size_t)rays_n : (size_t)rows_local * row_samples) * sizeof(int2);
-  if (want_ids) {
-    if (dev_out) d_ids = (int2*)hit_ids_out;
-    else {
-      if ((rc = D->ids.reserve(ids_bytes))) return rc;
-      d_ids = (int2*)D->ids.p;
-    }
-  }
-  // Two chunks in flight (two streams, two sets of queues) when the frame has several: the kernels are persistent and
-  // fill the GPU, so a chunk's next kernel starts on the SMs the other chunk's kernel frees as its warps run out of
-  // work — the tail of every launch is filled instead of idle.  One lane when every launch is timed on its own.
-  const int n_lanes = (RH_LANES > 1 && n_chunks >= 2 && !profile && !counting) ? 2 : 1;
-  // Passes pipelined over two streams per lane: trace(k + 1) needs only trace(k)'s ray queue, the shadow kernels of pass k
-  // only its hits, so trace(0) trace(1) ... run on one stream and classify(0) walk(0) classify(1) ... on the other.  Every
-  // kernel is persistent and fills the GPU; what the second stream buys is that the SMs a kernel's last warps leave idle
-  // (a lone warp walks a tree at ~1 us per node: the tail of a small launch is most of it) start the other stream's
-  // next kernel.  All adds to the accumulators are made by the shadow stream in pass order: same bits as one stream.
-  static const bool pipeline_on = !(getenv("RAYHS_B200_PIPELINE") && getenv("RAYHS_B200_PIPELINE")[0] == '0');  // (A/B switch)
-  // (single-chunk frames only: a frame of several chunks has two of them in flight, which fills the same gaps, and a ring
-  // that holds two passes' hits at a time needs the queue capacity a triangle soup does not leave)
-  const bool pipelined = pipeline_on && !profile && !counting && n_passes >= 2 && n_chunks == 1;
-  for (int l = 0; l < n_lanes; l++)
-    if ((rc = D->lane[l].accum.reserve(chunk_samples * 3 * sizeof(double)))) return rc;
-  if ((rc = D->ctl.reserve((size_t)n_chunks * sizeof(ChunkCtl)))) return rc;
-  if ((rc = D->counters.reserve(sizeof(FrameCounters)))) return rc;
-  const size_t pinned_need = (size_t)n_chunks * sizeof(ChunkCtl) + sizeof(FrameCounters);
-  if (D->pinned_bytes < pinned_need) {
-    if (D->pinned) cudaFreeHost(D->pinned);
-    D->pinned = nullptr;
-    D->pinned_bytes = 0;
-    RH_CUDA(cudaMallocHost(&D->pinned, pinned_need));
-    D->pinned_bytes = pinned_need;
-  }
-  // sample offsets
   const void* d_offsets = nullptr;
   int off_index = kOffIndexLocal;
-  bool stream_offsets = false;
   unsigned long long offset_seed = 0;
-  int ring = 2;
-  if (mode == RH_OFFSETS_TILED_F64) {
-    const size_t bytes = (size_t)o->offset_tile * o->offset_tile * spp * off_elem;
-    if (dev_off) d_offsets = o->offsets;
-    else {
-      if ((rc = D->offsets.reserve(bytes))) return rc;
-      d_offsets = D->offsets.p;
-    }
-  } else if (mode == RH_OFFSETS_SPLITMIX64) {
-    if (dev_off) return rh::set_error(RH_ERR_ARG, "rh_render: RH_OFFSETS_SPLITMIX64 takes a host pointer to the seed");
-    memcpy(&offset_seed, o->offsets, sizeof offset_seed);
-  } else if (mode != RH_OFFSETS_NONE) {
-    if (dev_off) {
-      d_offsets = o->offsets;
-      off_index = shard_offsets ? kOffIndexLocal : kOffIndexGlobal;  // (compact: each chunk's slice is in work-item order)
-    } else {
-      stream_offsets = true;
-      // Upload ring: as many chunk-sized slots as 10 % of the device memory holds (all chunks, for the frames of
-      // BASELINE.json), so that the copy stream can run ahead of the kernels instead of waiting for a slot.
-      const size_t slot_bytes = chunk_samples * off_elem;
-      ring = (int)std::max<size_t>(2, std::min<size_t>((size_t)n_chunks, (size_t)(0.1 * (double)D->total_mem) / slot_bytes));
-      if ((rc = D->offsets.reserve((size_t)ring * slot_bytes))) return rc;
-      while ((int)D->ev_up.size() < ring) {
-        cudaEvent_t a, b;
-        RH_CUDA(cudaEventCreateWithFlags(&a, cudaEventDisableTiming));
-        RH_CUDA(cudaEventCreateWithFlags(&b, cudaEventDisableTiming));
-        D->ev_up.push_back(a);
-        D->ev_done.push_back(b);
-      }
-    }
-  }
+  int ring = 2;                  // slots of the offset upload ring
+  size_t cap = 0, walk_cap = 0;  // queue capacities in entries
+  // recorded by the enqueue, per attempt
+  uint32_t launches = 0;
+  size_t upload_bytes = 0, ev_used = 0;
+  std::vector<Span> spans;
+  std::vector<cudaEvent_t> chunk_ev, copy_ev;  // streamed offsets: per chunk its kernels' begin and end, its upload's end
 
-  // queue capacity = factor * chunk samples; doubled when a chunk overflows (and remembered by the scene's renders)
-  uint32_t factor = rays ? 2u : std::max(2u, scene->queue_factor);
-  for (;;) {
-    // Queue capacity in entries, a whole number of slabs: factor x the chunk's samples, plus one partly filled slab
-    // per warp that can be producing (each warp leaves its last slab of a queue open).
+  cudaEvent_t prof_event(cudaStream_t stream) {
+    if (ev_used == D->prof_events.size()) {
+      cudaEvent_t e;
+      cudaEventCreate(&e);
+      D->prof_events.push_back(e);
+    }
+    cudaEvent_t e = D->prof_events[ev_used++];
+    cudaEventRecord(e, stream);
+    return e;
+  }
+  const ChunkCtl* ctl() const { return (const ChunkCtl*)D->pinned; }
+  const FrameCounters* counters() const { return (const FrameCounters*)((const char*)D->pinned + (size_t)n_chunks * sizeof(ChunkCtl)); }
+
+  // Queue capacity in entries, a whole number of slabs: factor x the chunk's samples, plus one partly filled slab per
+  // warp that can be producing (each warp leaves its last slab of a queue open).
+  int reserve_queues(uint32_t factor) {
     const size_t producers = std::min<size_t>((size_t)D->max_threads / 32, (chunk_samples + kSlab - 1) / kSlab + 1);
-    size_t cap = std::min<size_t>((size_t)factor * chunk_samples + 2 * producers * kSlab, 0x7fffff00u);
+    cap = std::min<size_t>((size_t)factor * chunk_samples + 2 * producers * kSlab, 0x7fffff00u);
     cap = (cap + kSlab - 1) / kSlab * kSlab;
     const size_t n_slabs_cap = cap / kSlab;
-    const size_t walk_cap = std::max<size_t>((cap / 2 + kSlab - 1) / kSlab * kSlab, 2 * producers * kSlab);
+    walk_cap = std::max<size_t>((cap / 2 + kSlab - 1) / kSlab * kSlab, 2 * producers * kSlab);
     const size_t deep_bytes = (size_t)scene->deep_entries * D->max_threads * sizeof(uint2);
+    int rc;
     for (int l = 0; l < n_lanes; l++) {
       Device::Scratch& sc = D->lane[l];
       for (int k = 0; k < 2; k++) {
@@ -1571,376 +1464,468 @@ int render_on(Device* D, const rh_scene* scene, const rh_camera* camera, const r
       if ((rc = sc.deep.reserve(deep_bytes))) return rc;
       if (pipelined && (rc = sc.deep_shadow.reserve(deep_bytes))) return rc;  // (kernels of both streams run side by side)
     }
+    return RH_OK;
+  }
 
-    size_t ev_used = 0;
-    cudaStream_t lane_stream = D->stream;  // the stream of the chunk being enqueued
-    auto prof_event = [&]() -> cudaEvent_t {
-      if (ev_used == D->prof_events.size()) {
-        cudaEvent_t e;
-        cudaEventCreate(&e);
-        D->prof_events.push_back(e);
-      }
-      cudaEvent_t e = D->prof_events[ev_used++];
-      cudaEventRecord(e, lane_stream);
-      return e;
-    };
-    struct Span { cudaEvent_t a, b; int kind; };
-    std::vector<Span> spans;
-
-    RH_CUDA(cudaEventRecord(D->ev_begin, D->stream));
-    RH_CUDA(cudaMemsetAsync(D->ctl.p, 0, (size_t)n_chunks * sizeof(ChunkCtl), D->stream));
-    RH_CUDA(cudaMemsetAsync(D->counters.p, 0, sizeof(FrameCounters), D->stream));
-    if (mode == RH_OFFSETS_TILED_F64 && !dev_off)
-      RH_CUDA(cudaMemcpyAsync((void*)d_offsets, o->offsets, (size_t)o->offset_tile * o->offset_tile * spp * off_elem,
-                              cudaMemcpyHostToDevice, D->stream));
-    if (n_lanes > 1) {  // lane 1 starts after the control blocks are zeroed
-      RH_CUDA(cudaEventRecord(D->ev_lane, D->stream));
-      RH_CUDA(cudaStreamWaitEvent(D->stream2, D->ev_lane, 0));
+  // Enqueues the chunk processed i-th: its offset upload (streamed offsets), its passes and its resolve.
+  int enqueue_chunk(int i) {
+    const rh_render_opts& o = f.o;
+    const int ck = plan.order[i], first_row = plan.first_row[ck], n_rows = plan.rows[ck];
+    const int ln = i % n_lanes;
+    Device::Scratch& sc = D->lane[ln];
+    const cudaStream_t lane_stream = ln ? D->stream2 : D->stream;
+    ChunkParams P{};
+    P.first_row = first_row;
+    P.n_rows = n_rows;
+    P.n_samples = (uint32_t)((size_t)n_rows * row_samples);
+    P.spp = o.spp;
+    P.width = o.width;
+    P.height = o.height;
+    P.shard_index = o.shard_index;
+    P.shard_count = o.shard_count;
+    P.band_height = o.band_height;
+    P.max_depth = o.max_depth;
+    P.exact_boxes = (o.flags & RH_FLAG_EXACT_BOXES) ? 1 : 0;
+    P.no_light_maps = (o.flags & RH_FLAG_NO_LIGHT_MAPS) ? 1 : 0;
+    P.offset_mode = o.offset_mode;
+    P.offset_index = off_index;
+    P.offset_tile = o.offset_tile;
+    P.offsets = d_offsets;
+    P.offset_seed = offset_seed;
+    P.accum = (double*)sc.accum.p;
+    P.accum_stride = (uint32_t)chunk_samples;
+    P.hit_ids = d_ids;
+    P.rgb = d_rgb;
+    if (o.flags & RH_FLAG_PEER_FRAMES) {
+      P.n_peers = (uint32_t)o.n_peer_frames;
+      for (int g = 0; g < o.n_peer_frames; g++) P.peer[g] = (uint8_t*)o.peer_frames[g];
     }
-    uint32_t launches = 0;
-    size_t upload_bytes = 0;
+    P.ctl = (ChunkCtl*)D->ctl.p + ck;
+    P.counters = (FrameCounters*)D->counters.p;
+    P.q_hits.plane = (double2*)sc.hitq.p;
+    P.q_hits.sample = (uint32_t*)sc.hitq_words.p;
+    P.q_hits.walk = (uint32_t*)sc.hitq_words.p + cap;
+    P.q_hits.settled = nullptr;
+    P.q_hits.fill = (uint32_t*)sc.hitq_words.p + 2 * cap;
+    P.q_hits.capacity = (uint32_t)cap;
+    P.q_shadow.plane = (double2*)sc.shq.p;
+    P.q_shadow.sample = (uint32_t*)sc.shq_words.p;
+    P.q_shadow.walk = (uint32_t*)sc.shq_words.p + walk_cap;
+    P.q_shadow.settled = (uint32_t*)sc.shq_words.p + 2 * walk_cap;
+    P.q_shadow.fill = (uint32_t*)sc.shq_words.p + 3 * walk_cap;
+    P.q_shadow.capacity = (uint32_t)walk_cap;
+    P.deep_stack = (uint2*)sc.deep.p;
+    P.deep_stride = (uint32_t)D->max_threads;
 
-    // processing order of the chunks (rows are independent, Image.hs:34-36)
-    std::vector<int> first_rows(n_chunks), order(n_chunks);
-    for (int ck = 0, row = 0; ck < n_chunks; row += plan[ck], ck++) { first_rows[ck] = row; order[ck] = ck; }
-    if (stream_offsets && n_chunks > 2 && know_cost) {
-      std::vector<double> dens(n_chunks);
-      for (int ck = 0; ck < n_chunks; ck++) {
-        double c = 0;
-        for (int r = first_rows[ck]; r < first_rows[ck] + plan[ck]; r++) c += scene->row_cost[r];
-        dens[ck] = c / std::max(1, plan[ck]);
+    if (host_offsets) {
+      // upload this chunk's rows (runs of image rows that are contiguous inside one band) on the copy stream
+      const int b = i % ring, bh = o.band_height;
+      char* slot = (char*)D->offsets.p + (size_t)b * chunk_samples * f.off_elem;
+      if (i >= ring) RH_CUDA(cudaStreamWaitEvent(D->copy_stream, D->ev_done[b], 0));
+      int lr = first_row;
+      while (lr < first_row + n_rows) {
+        const int lb = lr / bh, rib = lr % bh;
+        const int run = std::min(bh - rib, first_row + n_rows - lr);
+        const long long grow = ((long long)lb * o.shard_count + o.shard_index) * bh + rib;
+        const long long rows_ok = std::max<long long>(0, std::min<long long>(run, (long long)o.height - grow));
+        if (rows_ok > 0) {
+          const size_t src_row = (o.flags & RH_FLAG_SHARD_OFFSETS) ? (size_t)lr : (size_t)grow;
+          size_t bytes = (size_t)rows_ok * row_samples * f.off_elem;
+          if (f.trace) bytes = std::min(bytes, ((size_t)f.n_rays - src_row * row_samples) * f.off_elem);  // (a partial last row)
+          RH_CUDA(cudaMemcpyAsync(slot + (size_t)(lr - first_row) * row_samples * f.off_elem,
+                                  (const char*)o.offsets + src_row * row_samples * f.off_elem, bytes,
+                                  cudaMemcpyHostToDevice, D->copy_stream));
+          upload_bytes += bytes;
+        }
+        lr += run;
       }
-      // the compute-bound plan: the pieces of the most expensive chunk first, in row order, then everything in descending
-      // cost per row; else the small first chunk stays first and the tail pieces last
-      if (ramped) {
-        order.clear();
-        for (int k = 0; k < ramp_pieces; k++) order.push_back(ramp_first + k);
-        for (int ck = 0; ck < n_chunks; ck++)
-          if (ck < ramp_first || ck >= ramp_first + ramp_pieces) order.push_back(ck);
-      }
-      std::stable_sort(order.begin() + (ramped ? ramp_pieces : 1), order.end() - n_tail, [&](int x, int y) { return dens[x] > dens[y]; });
+      RH_CUDA(cudaEventRecord(D->ev_up[b], D->copy_stream));
+      copy_ev.push_back(prof_event(D->copy_stream));  // (when each chunk's upload ended)
+      RH_CUDA(cudaStreamWaitEvent(lane_stream, D->ev_up[b], 0));
+      P.offsets = slot;
+      chunk_ev.push_back(prof_event(lane_stream));  // after the wait: the span holds kernel time only
     }
-    std::vector<cudaEvent_t> chunk_ev, copy_ev;
-    static const bool debug_timeline = getenv("RAYHS_B200_DEBUG") && strchr(getenv("RAYHS_B200_DEBUG"), 't');
-    for (int i = 0; i < n_chunks; i++) {
-      const int ck = order[i];
-      const int first_row = first_rows[ck];
-      const int n_rows = plan[ck];
-      Device::Scratch& sc = D->lane[i % n_lanes];
-      lane_stream = (i % n_lanes) ? D->stream2 : D->stream;
-      ChunkParams P{};
-      P.first_row = first_row;
-      P.n_rows = n_rows;
-      P.n_samples = (uint32_t)((size_t)n_rows * row_samples);
-      P.spp = spp;
-      P.width = W;
-      P.height = H;
-      P.shard_index = o->shard_index;
-      P.shard_count = G;
-      P.band_height = bh;
-      P.max_depth = o->max_depth;
-      P.exact_boxes = exact_boxes ? 1 : 0;
-      P.no_light_maps = (o->flags & RH_FLAG_NO_LIGHT_MAPS) ? 1 : 0;
-      P.offset_mode = mode;
-      P.offset_index = off_index;
-      P.offset_tile = o->offset_tile;
-      P.offsets = d_offsets;
-      P.offset_seed = offset_seed;
-      P.accum = (double*)sc.accum.p;
-      P.accum_stride = (uint32_t)chunk_samples;
-      P.hit_ids = d_ids;
-      P.rgb = d_rgb;
-      if (peer_frames) {
-        P.n_peers = (uint32_t)o->n_peer_frames;
-        for (int g = 0; g < o->n_peer_frames; g++) P.peer[g] = (uint8_t*)o->peer_frames[g];
-      }
-      P.ctl = (ChunkCtl*)D->ctl.p + ck;
-      P.counters = (FrameCounters*)D->counters.p;
-      P.q_hits.plane = (double2*)sc.hitq.p;
-      P.q_hits.sample = (uint32_t*)sc.hitq_words.p;
-      P.q_hits.walk = (uint32_t*)sc.hitq_words.p + cap;
-      P.q_hits.settled = nullptr;
-      P.q_hits.fill = (uint32_t*)sc.hitq_words.p + 2 * cap;
-      P.q_hits.capacity = (uint32_t)cap;
-      P.q_shadow.plane = (double2*)sc.shq.p;
-      P.q_shadow.sample = (uint32_t*)sc.shq_words.p;
-      P.q_shadow.walk = (uint32_t*)sc.shq_words.p + walk_cap;
-      P.q_shadow.settled = (uint32_t*)sc.shq_words.p + 2 * walk_cap;
-      P.q_shadow.fill = (uint32_t*)sc.shq_words.p + 3 * walk_cap;
-      P.q_shadow.capacity = (uint32_t)walk_cap;
-      P.deep_stack = (uint2*)sc.deep.p;
-      P.deep_stride = (uint32_t)D->max_threads;
 
-      if (stream_offsets) {
-        // upload this chunk's rows (runs of image rows that are contiguous inside one band) on the copy stream
-        const int b = i % ring;
-        char* slot = (char*)D->offsets.p + (size_t)b * chunk_samples * off_elem;
-        if (i >= ring) RH_CUDA(cudaStreamWaitEvent(D->copy_stream, D->ev_done[b], 0));
-        int lr = first_row;
-        while (lr < first_row + n_rows) {
-          const int lb = lr / bh, rib = lr % bh;
-          const int run = std::min(bh - rib, first_row + n_rows - lr);
-          const long long grow = ((long long)lb * G + o->shard_index) * bh + rib;
-          const long long rows_ok = std::max<long long>(0, std::min<long long>(run, (long long)H - grow));
-          if (rows_ok > 0) {
-            const size_t src_row = shard_offsets ? (size_t)lr : (size_t)grow;
-            size_t bytes = (size_t)rows_ok * row_samples * off_elem;
-            if (rays) bytes = std::min(bytes, ((size_t)rays_n - src_row * row_samples) * off_elem);  // (a partial last row)
-            RH_CUDA(cudaMemcpyAsync(slot + (size_t)(lr - first_row) * row_samples * off_elem,
-                                    (const char*)o->offsets + src_row * row_samples * off_elem, bytes,
-                                    cudaMemcpyHostToDevice, D->copy_stream));
-            upload_bytes += bytes;
-          }
-          lr += run;
-        }
-        RH_CUDA(cudaEventRecord(D->ev_up[b], D->copy_stream));
-        {  // (timing events on the copy stream: when each chunk's upload ended)
-          cudaStream_t keep = lane_stream;
-          lane_stream = D->copy_stream;
-          copy_ev.push_back(prof_event());
-          lane_stream = keep;
-        }
-        RH_CUDA(cudaStreamWaitEvent(lane_stream, D->ev_up[b], 0));
-        P.offsets = slot;
-        chunk_ev.push_back(prof_event());  // after the wait: the span holds kernel time only
-      }
-
-      if (dev_off && shard_offsets && d_offsets) P.offsets = (const char*)d_offsets + (size_t)first_row * row_samples * off_elem;
-      // offsets in work-item order?  chunk-local slices always; the full-frame array when the frame is not sharded
-      P.offset_linear = (mode == RH_OFFSETS_F64 && (P.offset_index == kOffIndexLocal || G == 1)) ? 1u : 0u;
-      P.offset_base = (P.offset_index == kOffIndexLocal) ? 0ull : (unsigned long long)first_row * row_samples;
-      if (rays) P.ray_items = (uint32_t)std::min<uint64_t>(P.n_samples, rays_n - (uint64_t)first_row * row_samples);
-      for (int plane = 0; plane < 3; plane++)  // (three 1-D memsets: a 2-D one is limited to 2 GB of pitch)
-        RH_CUDA(cudaMemsetAsync((double*)sc.accum.p + (size_t)plane * chunk_samples, 0, (size_t)P.n_samples * sizeof(double), lane_stream));
-      const int ln = i % n_lanes;
-      cudaStream_t shadow_stream = pipelined ? D->shadow_stream[ln] : lane_stream;
-      for (int pass = 0; pass < n_passes; pass++) {
-        P.pass = pass;
-        P.q_in.plane = (double2*)sc.rayq[(pass + 1) & 1].p;
-        P.q_in.fill = (uint32_t*)sc.rayq_fill[(pass + 1) & 1].p;
-        P.q_in.capacity = (uint32_t)cap;
-        P.q_out.plane = (double2*)sc.rayq[pass & 1].p;
-        P.q_out.fill = (uint32_t*)sc.rayq_fill[pass & 1].p;
-        P.q_out.capacity = (uint32_t)cap;  // (the last pass cannot emit: every ray in it has depth == maxDepth)
-        cudaEvent_t a = nullptr;
-        if (profile) a = prof_event();
-        P.deep_stack = (uint2*)sc.deep.p;
-        P.hit_live_pass = (pipelined && pass > 0) ? pass - 1 : pass;
-        if (pipelined && pass >= 2) RH_CUDA(cudaStreamWaitEvent(lane_stream, D->ev_classified[ln][pass - 2], 0));  // its slabs are free
-        launch_trace(scene->view, cam, P, counting, D->n_sms, lane_stream);
-        if (profile) { cudaEvent_t b2 = prof_event(); spans.push_back({a, b2, 0}); a = b2; }
-        if (pipelined) {
-          RH_CUDA(cudaEventRecord(D->ev_trace[ln][pass], lane_stream));
-          RH_CUDA(cudaStreamWaitEvent(shadow_stream, D->ev_trace[ln][pass], 0));
-          P.deep_stack = (uint2*)sc.deep_shadow.p;
-        }
-        const int n_shadow = launch_shadow(scene->view, P, counting, use_refill, D->n_sms, shadow_stream,
-                                           pipelined ? (void*)D->ev_classified[ln][pass] : nullptr);
-        if (profile) spans.push_back({a, prof_event(), 1});
-        launches += 2 + n_shadow;  // (trace, the one-thread kernel that closes its hit range, classify, walk)
-      }
-      if (pipelined) {  // the resolve kernel needs every pass's shadow terms
-        RH_CUDA(cudaEventRecord(D->ev_shadows[ln], shadow_stream));
-        RH_CUDA(cudaStreamWaitEvent(lane_stream, D->ev_shadows[ln], 0));
-      }
+    if ((o.flags & RH_FLAG_DEVICE_OFFSETS) && (o.flags & RH_FLAG_SHARD_OFFSETS) && d_offsets)
+      P.offsets = (const char*)d_offsets + (size_t)first_row * row_samples * f.off_elem;
+    // offsets in work-item order?  chunk-local slices always; the full-frame array when the frame is not sharded
+    P.offset_linear = (o.offset_mode == RH_OFFSETS_F64 && (P.offset_index == kOffIndexLocal || o.shard_count == 1)) ? 1u : 0u;
+    P.offset_base = (P.offset_index == kOffIndexLocal) ? 0ull : (unsigned long long)first_row * row_samples;
+    if (f.trace) P.ray_items = (uint32_t)std::min<uint64_t>(P.n_samples, f.n_rays - (uint64_t)first_row * row_samples);
+    for (int plane = 0; plane < 3; plane++)  // (three 1-D memsets: a 2-D one is limited to 2 GB of pitch)
+      RH_CUDA(cudaMemsetAsync((double*)sc.accum.p + (size_t)plane * chunk_samples, 0, (size_t)P.n_samples * sizeof(double), lane_stream));
+    const cudaStream_t shadow_stream = pipelined ? D->shadow_stream[ln] : lane_stream;
+    for (int pass = 0; pass < n_passes; pass++) {
+      P.pass = pass;
+      P.q_in.plane = (double2*)sc.rayq[(pass + 1) & 1].p;
+      P.q_in.fill = (uint32_t*)sc.rayq_fill[(pass + 1) & 1].p;
+      P.q_in.capacity = (uint32_t)cap;
+      P.q_out.plane = (double2*)sc.rayq[pass & 1].p;
+      P.q_out.fill = (uint32_t*)sc.rayq_fill[pass & 1].p;
+      P.q_out.capacity = (uint32_t)cap;  // (the last pass cannot emit: every ray in it has depth == maxDepth)
       cudaEvent_t a = nullptr;
-      if (profile) a = prof_event();
-      if (rays) launch_store_colors(P, (double*)d_rgb, lane_stream);
-      else launch_resolve(P, lane_stream);
-      if (profile) spans.push_back({a, prof_event(), 2});
-      launches += 1;
-      if (stream_offsets) {
-        RH_CUDA(cudaEventRecord(D->ev_done[i % ring], lane_stream));
-        chunk_ev.push_back(prof_event());
+      if (sh.profile) a = prof_event(lane_stream);
+      P.deep_stack = (uint2*)sc.deep.p;
+      P.hit_live_pass = (pipelined && pass > 0) ? pass - 1 : pass;
+      if (pipelined && pass >= 2) RH_CUDA(cudaStreamWaitEvent(lane_stream, D->ev_classified[ln][pass - 2], 0));  // its slabs are free
+      launch_trace(scene->view, f.cam, P, counting, D->n_sms, lane_stream);
+      if (sh.profile) { cudaEvent_t b2 = prof_event(lane_stream); spans.push_back({a, b2, 0}); a = b2; }
+      if (pipelined) {
+        RH_CUDA(cudaEventRecord(D->ev_trace[ln][pass], lane_stream));
+        RH_CUDA(cudaStreamWaitEvent(shadow_stream, D->ev_trace[ln][pass], 0));
+        P.deep_stack = (uint2*)sc.deep_shadow.p;
       }
+      const int n_shadow = launch_shadow(scene->view, P, counting, sh.use_refill, D->n_sms, shadow_stream,
+                                         pipelined ? (void*)D->ev_classified[ln][pass] : nullptr);
+      if (sh.profile) spans.push_back({a, prof_event(lane_stream), 1});
+      launches += 2 + n_shadow;  // (trace, the one-thread kernel that closes its hit range, classify, walk)
     }
-    RH_CUDA(cudaGetLastError());
-    lane_stream = D->stream;
-    if (n_lanes > 1) {  // join: everything below waits for lane 1 too
-      RH_CUDA(cudaEventRecord(D->ev_lane, D->stream2));
-      RH_CUDA(cudaStreamWaitEvent(D->stream, D->ev_lane, 0));
+    if (pipelined) {  // the resolve kernel needs every pass's shadow terms
+      RH_CUDA(cudaEventRecord(D->ev_shadows[ln], shadow_stream));
+      RH_CUDA(cudaStreamWaitEvent(lane_stream, D->ev_shadows[ln], 0));
     }
-    RH_CUDA(cudaMemcpyAsync(D->pinned, D->ctl.p, (size_t)n_chunks * sizeof(ChunkCtl), cudaMemcpyDeviceToHost, D->stream));
-    RH_CUDA(cudaMemcpyAsync((char*)D->pinned + (size_t)n_chunks * sizeof(ChunkCtl), D->counters.p, sizeof(FrameCounters),
-                            cudaMemcpyDeviceToHost, D->stream));
-    if (!dev_out && !peer_frames) {
-      RH_CUDA(cudaMemcpyAsync(rgb_out, d_rgb, rgb_bytes, cudaMemcpyDeviceToHost, D->stream));
-      if (want_ids) RH_CUDA(cudaMemcpyAsync(hit_ids_out, d_ids, ids_bytes, cudaMemcpyDeviceToHost, D->stream));
-    }
-    RH_CUDA(cudaEventRecord(D->ev_end, D->stream));
-    RH_CUDA(cudaStreamSynchronize(D->stream));
-    g_launches.fetch_add(launches, std::memory_order_relaxed);
-
-    const ChunkCtl* ctl = (const ChunkCtl*)D->pinned;
-    bool overflow = false;
-    for (int ck = 0; ck < n_chunks; ck++) overflow |= ctl[ck].overflow != 0;
-    if (overflow) {
-      if (cap >= 0x7fffff00u || factor >= (1u << 16))
-        return rh::set_error(RH_ERR_OVERFLOW, rays ? "rh_trace_rays: ray queue overflow; lower chunk_rays"
-                                                   : "rh_render: ray queue overflow; lower chunk_samples");
-      factor *= 2;
-      if (!rays) scene->queue_factor = factor;
-      continue;
-    }
-    if (stats) {
-      memset(stats, 0, sizeof *stats);
-      const FrameCounters* fc = (const FrameCounters*)((const char*)D->pinned + (size_t)n_chunks * sizeof(ChunkCtl));
-      const uint64_t shadow_tasks = fc->shaded_hits;
-      uint64_t queued_hits = 0;
-      for (int ck = 0; ck < n_chunks; ck++)
-        for (int p = 0; p < n_passes; p++) queued_hits += ctl[ck].shadow_items[p];
-      // padding rows of the last band trace nothing
-      uint64_t real_rows = 0;
-      for (int lr = 0; lr < rows_local; lr++) {
-        const long long grow = ((long long)(lr / bh) * G + o->shard_index) * bh + lr % bh;
-        if (grow < H) real_rows++;
-      }
-      stats->rays_primary = rays ? rays_n : real_rows * row_samples;
-      stats->rays_reflect = fc->rays_reflect;
-      stats->rays_probe = fc->rays_probe;
-      stats->rays_exit = fc->rays_exit;
-      stats->rays_shadow = shadow_tasks * scene->view.n_lights;  // one shadowIntersection per light (RayHs.hs:89-97)
-      stats->box_tests = fc->k[0].box_tests;
-      stats->tri_tests = fc->k[0].tri_tests;
-      stats->prim_tests = fc->k[0].prim_tests;
-      stats->shade_fetches = fc->k[0].shade_fetches;
-      stats->texel_fetches = fc->k[0].texel_fetches;
-      stats->node_visits = fc->k[0].node_visits;
-      stats->node_visits_global = fc->k[0].global_node_visits;
-      stats->shadow_node_visits_global = fc->k[1].global_node_visits;
-      stats->tri_records = fc->k[0].tri_records;
-      stats->shadow_tri_records = fc->k[1].tri_records;
-      stats->shadow_box_tests = fc->k[1].box_tests;
-      stats->shadow_tri_tests = fc->k[1].tri_tests;
-      stats->shadow_prim_tests = fc->k[1].prim_tests;
-      stats->shadow_node_visits = fc->k[1].node_visits;
-      for (int ck = 0; ck < n_chunks; ck++)
-        for (int p = 1; p < n_passes; p++) stats->queued_rays += ctl[ck].ray_items[p];
-      stats->shadow_tasks = shadow_tasks;
-      stats->shadow_tasks_queued = queued_hits;
-      stats->shadow_walk_pairs = fc->shadow_walk_pairs;
-      stats->deep_stack_pushes = fc->deep_pushes;
-      stats->rays_shadow_culled = fc->shadow_culled;
-      if (counting && getenv("RAYHS_B200_DEBUG"))
-        fprintf(stderr, "rayhs_b200: exact shadow walks %llu, most nodes visited by one shadow ray %llu; exact closest-hit walks %llu, "
-                "most nodes visited by one closest-hit ray %llu\n", fc->exact_walks, fc->max_walk_nodes, fc->exact_closest,
-                fc->max_closest_nodes);
-      if (counting && getenv("RAYHS_B200_DEBUG"))
-        for (int row = 0; row < 4; row++) {
-          fprintf(stderr, "rayhs_b200: shadow walks of pass %d%s by log2(nodes + 1) [walks / nodes]:", row, row == 3 ? "+" : "");
-          for (int b = 0; b < 20; b++)
-            if (fc->walk_hist[row][b]) fprintf(stderr, " %d:%llu/%llu", b, fc->walk_hist[row][b], fc->walk_hist_nodes[row][b]);
-          fprintf(stderr, "\n");
-        }
-#ifdef RH_WARP_TIMES
-      if (getenv("RAYHS_B200_DEBUG"))
-        for (int row = 0; row < 4; row++) {
-          std::vector<int> b, e;
-          unsigned long long tot_b = 0, tot_r = 0;
-          int slow = -1, slow_end = 0;
-          unsigned ref = 0;
-          for (int i = 0; i < 4096; i++)
-            if (fc->warp_end[row][i]) {
-              if (b.empty()) ref = fc->warp_begin[row][i];
-              b.push_back((int)(fc->warp_begin[row][i] - ref));
-              e.push_back((int)(fc->warp_end[row][i] - ref));
-              tot_b += fc->warp_batches[row][i];
-              tot_r += fc->warp_rounds[row][i];
-              if (slow < 0 || e.back() > slow_end) { slow = i; slow_end = e.back(); }
-            }
-          if (b.empty()) continue;
-          std::sort(b.begin(), b.end());
-          std::sort(e.begin(), e.end());
-          const int t0 = b.front();
-          fprintf(stderr, "rayhs_b200: pooled pass %d: %zu warps, %llu batches, %llu rounds; warp start (us after the first) p50 %.1f p99 %.1f max %.1f; "
-                  "warp end p1 %.1f p10 %.1f p50 %.1f p90 %.1f p99 %.1f max %.1f; slowest warp: %u batches %u rounds\n", row, b.size(), tot_b, tot_r,
-                  (b[b.size() / 2] - t0) / 1e3, (b[b.size() * 99 / 100] - t0) / 1e3, (b.back() - t0) / 1e3, (e[e.size() / 100] - t0) / 1e3,
-                  (e[e.size() / 10] - t0) / 1e3, (e[e.size() / 2] - t0) / 1e3, (e[e.size() * 9 / 10] - t0) / 1e3, (e[e.size() * 99 / 100] - t0) / 1e3,
-                  (e.back() - t0) / 1e3, fc->warp_batches[row][slow], fc->warp_rounds[row][slow]);
-          std::vector<std::pair<int, int>> by_end;
-          for (int i = 0; i < 4096; i++)
-            if (fc->warp_end[row][i]) by_end.push_back({(int)(fc->warp_end[row][i] - ref) - t0, i});
-          std::sort(by_end.rbegin(), by_end.rend());
-          fprintf(stderr, "rayhs_b200:   slowest warps (block.warp end-us batches rounds pairs walk-us sum-of-longest-lane nodes tris):");
-          for (size_t k = 0; k < 10 && k < by_end.size(); k++) {
-            const int i = by_end[k].second;
-            fprintf(stderr, " %d.%d %.0f %u %u %u %.0f %u %u |", i / 24, i % 24, by_end[k].first / 1e3, fc->warp_batches[row][i], fc->warp_rounds[row][i],
-                    fc->warp_pairs[row][i], fc->warp_walk_ns[row][i] / 1e3, fc->warp_max_nodes[row][i], fc->warp_max_tris[row][i]);
-          }
-          fprintf(stderr, "\n");
-          {
-            const int i = by_end[by_end.size() / 2].second;
-            fprintf(stderr, "rayhs_b200:   median warp: %d.%d %.0f %u %u %u %.0f %u %u\n", i / 24, i % 24, by_end[by_end.size() / 2].first / 1e3,
-                    fc->warp_batches[row][i], fc->warp_rounds[row][i], fc->warp_pairs[row][i], fc->warp_walk_ns[row][i] / 1e3,
-                    fc->warp_max_nodes[row][i], fc->warp_max_tris[row][i]);
-          }
-        }
-#endif
-      stats->upload_bytes = upload_bytes;
-      float ms = 0;
-      cudaEventElapsedTime(&ms, D->ev_begin, D->ev_end);
-      stats->ms_total = ms;
-      for (const Span& s : spans) {
-        float m = 0;
-        cudaEventElapsedTime(&m, s.a, s.b);
-        if (s.kind == 0) { stats->ms_trace += m; stats->trace_launches++; }
-        else if (s.kind == 1) { stats->ms_shadow += m; stats->shadow_launches++; }
-        else stats->ms_resolve += m;
-      }
-      stats->kernel_launches = launches;
-      stats->chunks = (uint32_t)n_chunks;
-      stats->negative_channels = (uint32_t)std::min<unsigned long long>(fc->negative_channels, 0xffffffffu);
-      stats->queue_factor = factor;
-      stats->shadow_split = use_refill ? 1 : 0;
-    }
-    if (debug_timeline && (int)copy_ev.size() == n_chunks && (int)chunk_ev.size() == 2 * n_chunks) {
-      float end_ms = 0;
-      cudaEventElapsedTime(&end_ms, D->ev_begin, D->ev_end);
-      fprintf(stderr, "rayhs_b200: streamed frame, %d chunks, %.2f ms; per chunk in processing order: rows, upload done, kernels begin, kernels end (ms)\n", n_chunks, end_ms);
-      for (int i = 0; i < n_chunks; i++) {
-        float up = 0, kb = 0, ke = 0;
-        cudaEventElapsedTime(&up, D->ev_begin, copy_ev[i]);
-        cudaEventElapsedTime(&kb, D->ev_begin, chunk_ev[2 * i]);
-        cudaEventElapsedTime(&ke, D->ev_begin, chunk_ev[2 * i + 1]);
-        fprintf(stderr, "rayhs_b200:   chunk %2d lane %d rows %4d  up %6.2f  begin %6.2f  end %6.2f\n", order[i], i % n_lanes, plan[order[i]], up, kb, ke);
-      }
-    }
-    if (!rays && stream_offsets && o->chunk_samples <= 0 && (int)chunk_ev.size() == 2 * n_chunks && (int)copy_ev.size() == n_chunks) {
-      scene->row_cost.assign(rows_local, 0.f);
-      for (int i = 0; i < n_chunks; i++) {
-        float ms = 0;
-        cudaEventElapsedTime(&ms, chunk_ev[2 * i], chunk_ev[2 * i + 1]);
-        const int ck = order[i];
-        for (int r = first_rows[ck]; r < first_rows[ck] + plan[ck]; r++) scene->row_cost[r] = ms / (float)std::max(1, plan[ck]);
-      }
-      // Did the last chunk's kernels have to wait for its upload, or the other way round?  Once the compute-bound plan is
-      // in use it stays until BOTH lanes were waiting for data at the end of a frame.
-      float lag = 0, lag2 = 0;
-      cudaEventElapsedTime(&lag, copy_ev[n_chunks - 1], chunk_ev[2 * (n_chunks - 1)]);
-      if (n_chunks >= 2) cudaEventElapsedTime(&lag2, copy_ev[n_chunks - 2], chunk_ev[2 * (n_chunks - 2)]);
-      scene->stream_compute_bound = ramped ? !(lag < 0.05f && lag2 < 0.05f) : lag > 0.5f;
-      scene->cost_key = {W, H, spp, G, o->shard_index, bh};
-    }
-    if (tuning) {
-      // only frames with enough walks to time say anything (256 Ki pairs ~ 0.2 ms)
-      const FrameCounters* fc = (const FrameCounters*)((const char*)D->pinned + (size_t)n_chunks * sizeof(ChunkCtl));
-      double ms = 0;
-      for (const Span& sp : spans) {
-        float m = 0;
-        cudaEventElapsedTime(&m, sp.a, sp.b);
-        if (sp.kind == 1) ms += m;
-      }
-      if (fc->shadow_walk_pairs >= (1u << 18)) {
-        if (scene->tune_frames >= 1) scene->tune_ns_per_pair[scene->tune_frames - 1] = ms * 1e6 / (double)fc->shadow_walk_pairs;
-        if (++scene->tune_frames == 3) scene->shadow_mode = scene->tune_ns_per_pair[1] < scene->tune_ns_per_pair[0] ? 2 : 1;
-      } else if (++scene->tune_small_frames >= kTuneGiveUp) {
-        scene->shadow_mode = 1;
-      }
-    } else if (!rays && !forced && !decided && !(o->flags & RH_FLAG_COUNT)) {
-      if (++scene->tune_small_frames >= kTuneGiveUp) scene->shadow_mode = 1;
+    cudaEvent_t a = nullptr;
+    if (sh.profile) a = prof_event(lane_stream);
+    if (f.trace) launch_store_colors(P, (double*)d_rgb, lane_stream);
+    else launch_resolve(P, lane_stream);
+    if (sh.profile) spans.push_back({a, prof_event(lane_stream), 2});
+    launches += 1;
+    if (host_offsets) {
+      RH_CUDA(cudaEventRecord(D->ev_done[i % ring], lane_stream));
+      chunk_ev.push_back(prof_event(lane_stream));
     }
     return RH_OK;
   }
+
+  void read_stats(rh_stats* stats, uint32_t factor) const;
+  void print_timeline() const;
+  void learn() const;
+};
+
+// RAYS_B200_DEBUG output of a counting frame (and, built with RH_WARP_TIMES, of the pooled walks' warp times).
+void print_debug_counters(const FrameCounters* fc, bool counting) {
+  if (counting && getenv("RAYHS_B200_DEBUG"))
+    fprintf(stderr, "rayhs_b200: exact shadow walks %llu, most nodes visited by one shadow ray %llu; exact closest-hit walks %llu, "
+            "most nodes visited by one closest-hit ray %llu\n", fc->exact_walks, fc->max_walk_nodes, fc->exact_closest,
+            fc->max_closest_nodes);
+  if (counting && getenv("RAYHS_B200_DEBUG"))
+    for (int row = 0; row < 4; row++) {
+      fprintf(stderr, "rayhs_b200: shadow walks of pass %d%s by log2(nodes + 1) [walks / nodes]:", row, row == 3 ? "+" : "");
+      for (int b = 0; b < 20; b++)
+        if (fc->walk_hist[row][b]) fprintf(stderr, " %d:%llu/%llu", b, fc->walk_hist[row][b], fc->walk_hist_nodes[row][b]);
+      fprintf(stderr, "\n");
+    }
+#ifdef RH_WARP_TIMES
+  if (getenv("RAYHS_B200_DEBUG"))
+    for (int row = 0; row < 4; row++) {
+      std::vector<int> b, e;
+      unsigned long long tot_b = 0, tot_r = 0;
+      int slow = -1, slow_end = 0;
+      unsigned ref = 0;
+      for (int i = 0; i < 4096; i++)
+        if (fc->warp_end[row][i]) {
+          if (b.empty()) ref = fc->warp_begin[row][i];
+          b.push_back((int)(fc->warp_begin[row][i] - ref));
+          e.push_back((int)(fc->warp_end[row][i] - ref));
+          tot_b += fc->warp_batches[row][i];
+          tot_r += fc->warp_rounds[row][i];
+          if (slow < 0 || e.back() > slow_end) { slow = i; slow_end = e.back(); }
+        }
+      if (b.empty()) continue;
+      std::sort(b.begin(), b.end());
+      std::sort(e.begin(), e.end());
+      const int t0 = b.front();
+      fprintf(stderr, "rayhs_b200: pooled pass %d: %zu warps, %llu batches, %llu rounds; warp start (us after the first) p50 %.1f p99 %.1f max %.1f; "
+              "warp end p1 %.1f p10 %.1f p50 %.1f p90 %.1f p99 %.1f max %.1f; slowest warp: %u batches %u rounds\n", row, b.size(), tot_b, tot_r,
+              (b[b.size() / 2] - t0) / 1e3, (b[b.size() * 99 / 100] - t0) / 1e3, (b.back() - t0) / 1e3, (e[e.size() / 100] - t0) / 1e3,
+              (e[e.size() / 10] - t0) / 1e3, (e[e.size() / 2] - t0) / 1e3, (e[e.size() * 9 / 10] - t0) / 1e3, (e[e.size() * 99 / 100] - t0) / 1e3,
+              (e.back() - t0) / 1e3, fc->warp_batches[row][slow], fc->warp_rounds[row][slow]);
+      std::vector<std::pair<int, int>> by_end;
+      for (int i = 0; i < 4096; i++)
+        if (fc->warp_end[row][i]) by_end.push_back({(int)(fc->warp_end[row][i] - ref) - t0, i});
+      std::sort(by_end.rbegin(), by_end.rend());
+      fprintf(stderr, "rayhs_b200:   slowest warps (block.warp end-us batches rounds pairs walk-us sum-of-longest-lane nodes tris):");
+      for (size_t k = 0; k < 10 && k < by_end.size(); k++) {
+        const int i = by_end[k].second;
+        fprintf(stderr, " %d.%d %.0f %u %u %u %.0f %u %u |", i / 24, i % 24, by_end[k].first / 1e3, fc->warp_batches[row][i], fc->warp_rounds[row][i],
+                fc->warp_pairs[row][i], fc->warp_walk_ns[row][i] / 1e3, fc->warp_max_nodes[row][i], fc->warp_max_tris[row][i]);
+      }
+      fprintf(stderr, "\n");
+      {
+        const int i = by_end[by_end.size() / 2].second;
+        fprintf(stderr, "rayhs_b200:   median warp: %d.%d %.0f %u %u %u %.0f %u %u\n", i / 24, i % 24, by_end[by_end.size() / 2].first / 1e3,
+                fc->warp_batches[row][i], fc->warp_rounds[row][i], fc->warp_pairs[row][i], fc->warp_walk_ns[row][i] / 1e3,
+                fc->warp_max_nodes[row][i], fc->warp_max_tris[row][i]);
+      }
+    }
+#endif
+}
+
+void FrameRun::read_stats(rh_stats* stats, uint32_t factor) const {
+  memset(stats, 0, sizeof *stats);
+  const FrameCounters* fc = counters();
+  const uint64_t shadow_tasks = fc->shaded_hits;
+  uint64_t queued_hits = 0;
+  for (int ck = 0; ck < n_chunks; ck++)
+    for (int p = 0; p < n_passes; p++) queued_hits += ctl()[ck].shadow_items[p];
+  stats->rays_primary = f.rays_primary;
+  stats->rays_reflect = fc->rays_reflect;
+  stats->rays_probe = fc->rays_probe;
+  stats->rays_exit = fc->rays_exit;
+  stats->rays_shadow = shadow_tasks * scene->view.n_lights;  // one shadowIntersection per light (RayHs.hs:89-97)
+  stats->box_tests = fc->k[0].box_tests;
+  stats->tri_tests = fc->k[0].tri_tests;
+  stats->prim_tests = fc->k[0].prim_tests;
+  stats->shade_fetches = fc->k[0].shade_fetches;
+  stats->texel_fetches = fc->k[0].texel_fetches;
+  stats->node_visits = fc->k[0].node_visits;
+  stats->node_visits_global = fc->k[0].global_node_visits;
+  stats->shadow_node_visits_global = fc->k[1].global_node_visits;
+  stats->tri_records = fc->k[0].tri_records;
+  stats->shadow_tri_records = fc->k[1].tri_records;
+  stats->shadow_box_tests = fc->k[1].box_tests;
+  stats->shadow_tri_tests = fc->k[1].tri_tests;
+  stats->shadow_prim_tests = fc->k[1].prim_tests;
+  stats->shadow_node_visits = fc->k[1].node_visits;
+  for (int ck = 0; ck < n_chunks; ck++)
+    for (int p = 1; p < n_passes; p++) stats->queued_rays += ctl()[ck].ray_items[p];
+  stats->shadow_tasks = shadow_tasks;
+  stats->shadow_tasks_queued = queued_hits;
+  stats->shadow_walk_pairs = fc->shadow_walk_pairs;
+  stats->deep_stack_pushes = fc->deep_pushes;
+  stats->rays_shadow_culled = fc->shadow_culled;
+  print_debug_counters(fc, counting);
+  stats->upload_bytes = upload_bytes;
+  float ms = 0;
+  cudaEventElapsedTime(&ms, D->ev_begin, D->ev_end);
+  stats->ms_total = ms;
+  for (const Span& s : spans) {
+    float m = 0;
+    cudaEventElapsedTime(&m, s.a, s.b);
+    if (s.kind == 0) { stats->ms_trace += m; stats->trace_launches++; }
+    else if (s.kind == 1) { stats->ms_shadow += m; stats->shadow_launches++; }
+    else stats->ms_resolve += m;
+  }
+  stats->kernel_launches = launches;
+  stats->chunks = (uint32_t)n_chunks;
+  stats->negative_channels = (uint32_t)std::min<unsigned long long>(fc->negative_channels, 0xffffffffu);
+  stats->queue_factor = factor;
+  stats->shadow_split = sh.use_refill ? 1 : 0;
+}
+
+// RAYHS_B200_DEBUG=t: the timeline of a streamed frame.
+void FrameRun::print_timeline() const {
+  static const bool debug_timeline = getenv("RAYHS_B200_DEBUG") && strchr(getenv("RAYHS_B200_DEBUG"), 't');
+  if (!debug_timeline || (int)copy_ev.size() != n_chunks || (int)chunk_ev.size() != 2 * n_chunks) return;
+  float end_ms = 0;
+  cudaEventElapsedTime(&end_ms, D->ev_begin, D->ev_end);
+  fprintf(stderr, "rayhs_b200: streamed frame, %d chunks, %.2f ms; per chunk in processing order: rows, upload done, kernels begin, kernels end (ms)\n", n_chunks, end_ms);
+  for (int i = 0; i < n_chunks; i++) {
+    float up = 0, kb = 0, ke = 0;
+    cudaEventElapsedTime(&up, D->ev_begin, copy_ev[i]);
+    cudaEventElapsedTime(&kb, D->ev_begin, chunk_ev[2 * i]);
+    cudaEventElapsedTime(&ke, D->ev_begin, chunk_ev[2 * i + 1]);
+    fprintf(stderr, "rayhs_b200:   chunk %2d lane %d rows %4d  up %6.2f  begin %6.2f  end %6.2f\n", plan.order[i], i % n_lanes,
+            plan.rows[plan.order[i]], up, kb, ke);
+  }
+}
+
+// The scene's learned state after a render: the row costs and the compute-bound flag of a streamed frame with the
+// default chunk plan, and the shadow-schedule tuning.
+void FrameRun::learn() const {
+  const rh_render_opts& o = f.o;
+  if (host_offsets && o.chunk_samples <= 0 && (int)chunk_ev.size() == 2 * n_chunks && (int)copy_ev.size() == n_chunks) {
+    scene->row_cost.assign(f.rows_local, 0.f);
+    for (int i = 0; i < n_chunks; i++) {
+      float ms = 0;
+      cudaEventElapsedTime(&ms, chunk_ev[2 * i], chunk_ev[2 * i + 1]);
+      const int ck = plan.order[i];
+      for (int r = plan.first_row[ck]; r < plan.first_row[ck] + plan.rows[ck]; r++) scene->row_cost[r] = ms / (float)std::max(1, plan.rows[ck]);
+    }
+    // Did the last chunk's kernels have to wait for its upload, or the other way round?  Once the compute-bound plan is
+    // in use it stays until BOTH lanes were waiting for data at the end of a frame.
+    float lag = 0, lag2 = 0;
+    cudaEventElapsedTime(&lag, copy_ev[n_chunks - 1], chunk_ev[2 * (n_chunks - 1)]);
+    if (n_chunks >= 2) cudaEventElapsedTime(&lag2, copy_ev[n_chunks - 2], chunk_ev[2 * (n_chunks - 2)]);
+    scene->stream_compute_bound = plan.ramped ? !(lag < 0.05f && lag2 < 0.05f) : lag > 0.5f;
+    scene->cost_key = {o.width, o.height, o.spp, o.shard_count, o.shard_index, o.band_height};
+  }
+  if (sh.tuning) {
+    // only frames with enough walks to time say anything (256 Ki pairs ~ 0.2 ms)
+    const FrameCounters* fc = counters();
+    double ms = 0;
+    for (const Span& sp : spans) {
+      float m = 0;
+      cudaEventElapsedTime(&m, sp.a, sp.b);
+      if (sp.kind == 1) ms += m;
+    }
+    if (fc->shadow_walk_pairs >= (1u << 18)) {
+      if (scene->tune_frames >= 1) scene->tune_ns_per_pair[scene->tune_frames - 1] = ms * 1e6 / (double)fc->shadow_walk_pairs;
+      if (++scene->tune_frames == 3) scene->shadow_mode = scene->tune_ns_per_pair[1] < scene->tune_ns_per_pair[0] ? 2 : 1;
+    } else if (++scene->tune_small_frames >= kTuneGiveUp) {
+      scene->shadow_mode = 1;
+    }
+  } else if (sh.untuned) {
+    if (++scene->tune_small_frames >= kTuneGiveUp) scene->shadow_mode = 1;
+  }
+}
+
+// Runs a validated frame: chunk plan, scratch, the chunks' launches, and — when a chunk's queues overflowed — the whole
+// frame again with twice the queue capacity.
+int run_frame(Device* D, const rh_scene* scene, const Frame& f, rh_stats* stats) {
+  const rh_render_opts& o = f.o;
+  const int mode = o.offset_mode;
+  const bool dev_out = (o.flags & RH_FLAG_DEVICE_OUT) != 0, dev_off = (o.flags & RH_FLAG_DEVICE_OFFSETS) != 0;
+  const bool peer_frames = (o.flags & RH_FLAG_PEER_FRAMES) != 0, want_ids = (o.flags & RH_FLAG_HIT_IDS) != 0;
+  RH_CUDA(cudaSetDevice(D->dev));
+  FrameRun R{D, scene, f};
+  R.sh = choose_shadow(scene, f);
+  R.counting = (o.flags & RH_FLAG_COUNT) != 0;
+  R.row_samples = (size_t)o.width * o.spp;
+  // A Transparent hit inserts a probe pass per level (RayHs.hs:136-143): up to 2D + 1 passes.  Without a Transparent
+  // material the rays of pass k all have depth k, and pass D emits nothing: D + 1 passes, no empty launches after them.
+  R.n_passes = scene->has_transparent ? 2 * o.max_depth + 1 : o.max_depth + 1;
+  R.host_offsets = (mode == RH_OFFSETS_F64 || mode == RH_OFFSETS_F32 || mode == kOffsetsRays) && !dev_off;
+  // what the last streamed frame of this shape measured: kernel time per row, and whether the kernels or the upload
+  // finished last
+  const bool know_cost = !f.trace && (int)scene->row_cost.size() == f.rows_local &&
+                         scene->cost_key == std::vector<int>{o.width, o.height, o.spp, o.shard_count, o.shard_index, o.band_height};
+  R.plan = rh::plan_chunks(f.rows_local, R.row_samples, o.chunk_samples, D->total_mem, R.host_offsets,
+                           know_cost ? scene->row_cost.data() : nullptr, scene->stream_compute_bound);
+  R.n_chunks = (int)R.plan.rows.size();
+  R.chunk_samples = (size_t)*std::max_element(R.plan.rows.begin(), R.plan.rows.end()) * R.row_samples;
+  if (R.chunk_samples > 0x7fffffffu) return rh::set_error(RH_ERR_ARG, "rh_render: chunk too large");
+
+  int rc;
+  if (peer_frames) R.d_rgb = nullptr;
+  else if (dev_out) R.d_rgb = f.out;
+  else {
+    if ((rc = D->rgb.reserve(f.out_bytes))) return rc;
+    R.d_rgb = (uint8_t*)D->rgb.p;
+  }
+  if (want_ids && dev_out) R.d_ids = (int2*)f.ids_out;
+  else if (want_ids) {
+    if ((rc = D->ids.reserve(f.ids_bytes))) return rc;
+    R.d_ids = (int2*)D->ids.p;
+  }
+  // Two chunks in flight (two streams, two sets of queues) when the frame has several: the kernels are persistent and
+  // fill the GPU, so a chunk's next kernel starts on the SMs the other chunk's kernel frees as its warps run out of
+  // work — the tail of every launch is filled instead of idle.  One lane when every launch is timed on its own.
+  R.n_lanes = (R.n_chunks >= 2 && !R.sh.profile && !R.counting) ? rh::kLanes : 1;
+  // Passes pipelined over two streams per lane: trace(k + 1) needs only trace(k)'s ray queue, the shadow kernels of pass k
+  // only its hits, so trace(0) trace(1) ... run on one stream and classify(0) walk(0) classify(1) ... on the other.  Every
+  // kernel is persistent and fills the GPU; what the second stream buys is that the SMs a kernel's last warps leave idle
+  // (a lone warp walks a tree at ~1 us per node: the tail of a small launch is most of it) start the other stream's
+  // next kernel.  All adds to the accumulators are made by the shadow stream in pass order: same bits as one stream.
+  // Single-chunk frames only: a frame of several chunks has two of them in flight, which fills the same gaps, and a ring
+  // that holds two passes' hits at a time needs the queue capacity a triangle soup does not leave.
+  R.pipelined = !R.sh.profile && !R.counting && R.n_passes >= 2 && R.n_chunks == 1;
+  for (int l = 0; l < R.n_lanes; l++)
+    if ((rc = D->lane[l].accum.reserve(R.chunk_samples * 3 * sizeof(double)))) return rc;
+  const size_t ctl_bytes = (size_t)R.n_chunks * sizeof(ChunkCtl);
+  if ((rc = D->ctl.reserve(ctl_bytes))) return rc;
+  if ((rc = D->counters.reserve(sizeof(FrameCounters)))) return rc;
+  if (D->pinned_bytes < ctl_bytes + sizeof(FrameCounters)) {
+    if (D->pinned) cudaFreeHost(D->pinned);
+    D->pinned = nullptr;
+    D->pinned_bytes = 0;
+    RH_CUDA(cudaMallocHost(&D->pinned, ctl_bytes + sizeof(FrameCounters)));
+    D->pinned_bytes = ctl_bytes + sizeof(FrameCounters);
+  }
+  // sample offsets
+  const size_t tile_bytes = (size_t)o.offset_tile * o.offset_tile * o.spp * f.off_elem;
+  if (mode == RH_OFFSETS_TILED_F64) {
+    if (dev_off) R.d_offsets = o.offsets;
+    else {
+      if ((rc = D->offsets.reserve(tile_bytes))) return rc;
+      R.d_offsets = D->offsets.p;
+    }
+  } else if (mode == RH_OFFSETS_SPLITMIX64) {
+    memcpy(&R.offset_seed, o.offsets, sizeof R.offset_seed);
+  } else if (mode != RH_OFFSETS_NONE && dev_off) {
+    R.d_offsets = o.offsets;
+    R.off_index = (o.flags & RH_FLAG_SHARD_OFFSETS) ? kOffIndexLocal : kOffIndexGlobal;  // (compact: each chunk's slice is in work-item order)
+  } else if (R.host_offsets) {
+    // Upload ring: as many chunk-sized slots as 10 % of the device memory holds (all chunks, for the frames of
+    // BASELINE.json), so that the copy stream can run ahead of the kernels instead of waiting for a slot.
+    const size_t slot_bytes = R.chunk_samples * f.off_elem;
+    R.ring = (int)std::max<size_t>(2, std::min<size_t>((size_t)R.n_chunks, (size_t)(0.1 * (double)D->total_mem) / slot_bytes));
+    if ((rc = D->offsets.reserve((size_t)R.ring * slot_bytes))) return rc;
+    while ((int)D->ev_up.size() < R.ring) {
+      cudaEvent_t a, b;
+      RH_CUDA(cudaEventCreateWithFlags(&a, cudaEventDisableTiming));
+      RH_CUDA(cudaEventCreateWithFlags(&b, cudaEventDisableTiming));
+      D->ev_up.push_back(a);
+      D->ev_done.push_back(b);
+    }
+  }
+
+  // queue capacity = factor * chunk samples; doubled when a chunk overflows (and remembered by the scene's renders)
+  uint32_t factor = f.trace ? 2u : std::max(2u, scene->queue_factor);
+  for (;;) {
+    if ((rc = R.reserve_queues(factor))) return rc;
+    R.launches = 0;
+    R.upload_bytes = R.ev_used = 0;
+    R.spans.clear();
+    R.chunk_ev.clear();
+    R.copy_ev.clear();
+    RH_CUDA(cudaEventRecord(D->ev_begin, D->stream));
+    RH_CUDA(cudaMemsetAsync(D->ctl.p, 0, ctl_bytes, D->stream));
+    RH_CUDA(cudaMemsetAsync(D->counters.p, 0, sizeof(FrameCounters), D->stream));
+    if (mode == RH_OFFSETS_TILED_F64 && !dev_off)
+      RH_CUDA(cudaMemcpyAsync((void*)R.d_offsets, o.offsets, tile_bytes, cudaMemcpyHostToDevice, D->stream));
+    if (R.n_lanes > 1) {  // lane 1 starts after the control blocks are zeroed
+      RH_CUDA(cudaEventRecord(D->ev_lane, D->stream));
+      RH_CUDA(cudaStreamWaitEvent(D->stream2, D->ev_lane, 0));
+    }
+    for (int i = 0; i < R.n_chunks; i++)
+      if ((rc = R.enqueue_chunk(i))) return rc;
+    RH_CUDA(cudaGetLastError());
+    if (R.n_lanes > 1) {  // join: everything below waits for lane 1 too
+      RH_CUDA(cudaEventRecord(D->ev_lane, D->stream2));
+      RH_CUDA(cudaStreamWaitEvent(D->stream, D->ev_lane, 0));
+    }
+    RH_CUDA(cudaMemcpyAsync(D->pinned, D->ctl.p, ctl_bytes, cudaMemcpyDeviceToHost, D->stream));
+    RH_CUDA(cudaMemcpyAsync((char*)D->pinned + ctl_bytes, D->counters.p, sizeof(FrameCounters), cudaMemcpyDeviceToHost, D->stream));
+    if (!dev_out && !peer_frames) {
+      RH_CUDA(cudaMemcpyAsync(f.out, R.d_rgb, f.out_bytes, cudaMemcpyDeviceToHost, D->stream));
+      if (want_ids) RH_CUDA(cudaMemcpyAsync(f.ids_out, R.d_ids, f.ids_bytes, cudaMemcpyDeviceToHost, D->stream));
+    }
+    RH_CUDA(cudaEventRecord(D->ev_end, D->stream));
+    RH_CUDA(cudaStreamSynchronize(D->stream));
+    g_launches.fetch_add(R.launches, std::memory_order_relaxed);
+
+    bool overflow = false;
+    for (int ck = 0; ck < R.n_chunks; ck++) overflow |= R.ctl()[ck].overflow != 0;
+    if (overflow) {
+      if (R.cap >= 0x7fffff00u || factor >= (1u << 16)) return rh::set_error(RH_ERR_OVERFLOW, f.overflow_error);
+      factor *= 2;
+      if (!f.trace) scene->queue_factor = factor;
+      continue;
+    }
+    if (stats) R.read_stats(stats, factor);
+    R.print_timeline();
+    if (!f.trace) R.learn();
+    return RH_OK;
+  }
+}
+
+int render_on(Device* D, const rh_scene* scene, const rh_camera* camera, const rh_render_opts* o, uint8_t* rgb_out,
+              int32_t* hit_ids_out, rh_stats* stats) {
+  Frame f;
+  const int rc = render_frame(D, scene, camera, o, rgb_out, hit_ids_out, &f);
+  return rc ? rc : run_frame(D, scene, f, stats);
+}
+
+// Returns RH_OK when every non-null pointer is device (or managed) memory, else the argument error `msg`.
+int check_device_pointers(std::initializer_list<const void*> ptrs, const std::string& msg) {
+  for (const void* p : ptrs) {
+    if (!p) continue;
+    cudaPointerAttributes a{};
+    RH_CUDA(cudaPointerGetAttributes(&a, p));
+    if (a.type != cudaMemoryTypeDevice && a.type != cudaMemoryTypeManaged) return rh::set_error(RH_ERR_ARG, msg);
+  }
+  return RH_OK;
 }
 
 // ------------------------------------------------------------------ batched ray queries
@@ -1968,14 +1953,10 @@ int query_on(Device* D, const rh_scene* scene, int64_t light, const double* rays
     // the kernels move rays and records in 16-byte words
     if ((uintptr_t)rays % 16 || (!shadow && (uintptr_t)out % 16))
       return rh::set_error(RH_ERR_ARG, w + ": device buffers must be 16-byte aligned");
-    for (const void* p : {(const void*)rays, (const void*)out}) {
-      cudaPointerAttributes a{};
-      RH_CUDA(cudaPointerGetAttributes(&a, p));
-      if (a.type != cudaMemoryTypeDevice && a.type != cudaMemoryTypeManaged)
-        return rh::set_error(RH_ERR_ARG, w + ": RH_FLAG_DEVICE_OUT with a pointer that is not device memory");
-    }
   }
   int rc;
+  if (dev && (rc = check_device_pointers({rays, out}, w + ": RH_FLAG_DEVICE_OUT with a pointer that is not device memory")))
+    return rc;
   Device::Scratch& sc = D->lane[0];  // the render's deep-stack scratch covers grid x block of the query kernels
   if ((rc = sc.deep.reserve((size_t)scene->deep_entries * D->max_threads * sizeof(uint2)))) return rc;
   const uint64_t chunk = dev ? kQueryLaunch : kQueryChunk;
@@ -2000,7 +1981,7 @@ int query_on(Device* D, const rh_scene* scene, int64_t light, const double* rays
     RH_CUDA(cudaMemsetAsync(Q.cursor, 0, sizeof(uint32_t), D->stream));
     if (shadow) launch_query_shadow(scene->view, Q, D->n_sms, D->stream);
     else launch_query_closest(scene->view, Q, D->n_sms, D->stream);
-    Launch::count();
+    g_launches.fetch_add(1, std::memory_order_relaxed);
     RH_CUDA(cudaGetLastError());
     if (!dev) RH_CUDA(cudaMemcpyAsync(dst, d_out, (size_t)m * out_bytes, cudaMemcpyDeviceToHost, D->stream));
   }
@@ -2011,7 +1992,7 @@ int query_on(Device* D, const rh_scene* scene, int64_t light, const double* rays
 // ------------------------------------------------------------------ radiance queries
 // rh_trace_rays runs the render's wavefront on a frame of one sample per ray: kTraceRowRays rays per row, as many rows
 // as the rays need, unsharded.  Pass 0 reads the rays (kOffsetsRays) and the colours leave unquantised; everything in
-// between — chunk plan, queues, overflow retry, pipelined passes, counts — is render_on's.
+// between — chunk plan, queues, overflow retry, pipelined passes, counts — is run_frame's.
 constexpr int kTraceRowRays = 4096;
 
 int trace_on(Device* D, const rh_scene* scene, const double* rays, uint64_t n, const rh_trace_opts* o, double* colors_out,
@@ -2036,30 +2017,30 @@ int trace_on(Device* D, const rh_scene* scene, const double* rays, uint64_t n, c
     // rays are read as 16-byte words; colours and ids are written as 8-byte words
     if ((uintptr_t)rays % 16 || (uintptr_t)colors_out % 8 || (want_ids && (uintptr_t)hit_ids_out % 8))
       return rh::set_error(RH_ERR_ARG, "rh_trace_rays: device rays must be 16-byte aligned, colours and ids 8-byte aligned");
-    for (const void* p : {(const void*)rays, (const void*)colors_out, (const void*)(want_ids ? hit_ids_out : nullptr)}) {
-      if (!p) continue;
-      cudaPointerAttributes a{};
-      RH_CUDA(cudaPointerGetAttributes(&a, p));
-      if (a.type != cudaMemoryTypeDevice && a.type != cudaMemoryTypeManaged)
-        return rh::set_error(RH_ERR_ARG, "rh_trace_rays: RH_FLAG_DEVICE_OUT with a pointer that is not device memory");
-    }
+    const int rc = check_device_pointers({rays, colors_out, want_ids ? hit_ids_out : nullptr},
+                                         "rh_trace_rays: RH_FLAG_DEVICE_OUT with a pointer that is not device memory");
+    if (rc) return rc;
   }
-  rh_render_opts ro{};
-  ro.width = kTraceRowRays;
-  ro.height = (int)rows;
-  ro.max_depth = o->max_depth;
-  ro.spp = 1;
-  ro.offset_mode = kOffsetsRays;
-  ro.offsets = rays;
-  ro.shard_count = 1;
-  ro.chunk_samples = (int)std::min<uint64_t>(o->chunk_rays, 0x7fffffffu);
-  ro.flags = o->flags | (dev ? RH_FLAG_DEVICE_OFFSETS : 0);
-  rh_camera cam{};  // (no camera rays: any valid camera)
-  cam.target[2] = 1;
-  cam.up[1] = 1;
-  cam.projection = RH_PROJ_PERSPECTIVE;
-  cam.fovy = 1;
-  return render_on(D, scene, &cam, &ro, (uint8_t*)colors_out, hit_ids_out, stats, n);
+  Frame f;
+  f.o.width = kTraceRowRays;
+  f.o.height = f.o.band_height = f.rows_local = (int)rows;
+  f.o.max_depth = o->max_depth;
+  f.o.spp = 1;
+  f.o.offset_mode = kOffsetsRays;
+  f.o.offsets = rays;
+  f.o.shard_count = 1;
+  f.o.chunk_samples = (int)std::min<uint64_t>(o->chunk_rays, 0x7fffffffu);
+  f.o.flags = o->flags | (dev ? RH_FLAG_DEVICE_OFFSETS : 0);
+  f.out = (uint8_t*)colors_out;
+  f.ids_out = hit_ids_out;
+  f.out_bytes = (size_t)n * 3 * sizeof(double);
+  f.ids_bytes = (size_t)n * sizeof(int2);
+  f.off_elem = sizeof(double) * 6;
+  f.rays_primary = n;
+  f.trace = true;
+  f.n_rays = n;
+  f.overflow_error = "rh_trace_rays: ray queue overflow; lower chunk_rays";
+  return run_frame(D, scene, f, stats);
 }
 
 }  // namespace

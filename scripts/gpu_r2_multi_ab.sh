@@ -1,5 +1,5 @@
 #!/bin/bash
-# C4 under torchrun on N GPUs: band heights (rows per interleaved band) and the pipelined passes on / off.  Short runs
+# C4 under torchrun on N GPUs: band heights (rows per interleaved band).  Short runs
 # (no CPU baseline, no cold start); one JSON line per configuration into gpurun_out/.
 N=${N:-8}
 mkdir -p gpurun_out
@@ -17,7 +17,6 @@ except Exception as e:
     print("$1 no line:", e)
 PY
 }
-run bh16 "RAYHS_B200_PIPELINE=1" "--band-height 16"
-run bh4 "RAYHS_B200_PIPELINE=1" "--band-height 4"
-run bh1 "RAYHS_B200_PIPELINE=1" "--band-height 1"
-run bh4_nopipe "RAYHS_B200_PIPELINE=0" "--band-height 4"
+run bh16 "" "--band-height 16"
+run bh4 "" "--band-height 4"
+run bh1 "" "--band-height 1"

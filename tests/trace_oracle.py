@@ -4,12 +4,11 @@ that the repository tree is never written.  TEST INFRASTRUCTURE ONLY."""
 from __future__ import annotations
 
 import ctypes as C
-import hashlib
 import os
-import subprocess
-import tempfile
 
 import numpy as np
+
+from tests.util import temp_library
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 SOURCES = [os.path.join(ROOT, "tests", "trace_oracle.cpp"), os.path.join(ROOT, "oracle", "oracle.cpp"),
@@ -23,16 +22,7 @@ _lib = None
 def lib() -> C.CDLL:
     global _lib
     if _lib is None:
-        h = hashlib.sha256(" ".join(FLAGS).encode())
-        for s in SOURCES:
-            with open(s, "rb") as f:
-                h.update(f.read())
-        path = os.path.join(tempfile.gettempdir(), f"rayhs_trace_oracle_{os.getuid()}_{h.hexdigest()[:16]}.so")
-        if not os.path.exists(path):
-            tmp = f"{path}.{os.getpid()}"
-            subprocess.check_call([os.environ.get("CXX") or "g++", *FLAGS, SOURCES[0], "-o", tmp, "-lpthread"])
-            os.replace(tmp, path)
-        L = C.CDLL(path)
+        L = temp_library("trace_oracle", SOURCES, FLAGS)
         vp = C.c_void_p
         L.orc_scene_create.restype = vp
         L.orc_scene_create.argtypes = [vp]

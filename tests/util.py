@@ -1,6 +1,10 @@
 """Shared helpers of the parity tests: scene packs, the oracle, and the comparison metrics of
 BASELINE.json (hit ids bit-exact; <= 1 LSB on >= 99.9 % of pixels; PSNR >= 50 dB)."""
+import ctypes
+import hashlib
 import os
+import subprocess
+import tempfile
 
 import numpy as np
 
@@ -12,6 +16,22 @@ def load_scene(name):
     from rayhs_b200 import Scene
 
     return Scene.from_pack(os.path.join(GOLDEN, name + ".pack"))
+
+
+def temp_library(name, sources, flags):
+    """Compiles sources[0] (which includes the rest of `sources`) with the C++ compiler into a shared library in the
+    temporary directory, named by a digest of the sources and flags, so that the repository tree is never written, and
+    loads it.  The rename makes the build safe against concurrent test processes."""
+    h = hashlib.sha256(" ".join(flags).encode())
+    for s in sources:
+        with open(s, "rb") as f:
+            h.update(f.read())
+    path = os.path.join(tempfile.gettempdir(), f"rayhs_{name}_{os.getuid()}_{h.hexdigest()[:16]}.so")
+    if not os.path.exists(path):
+        tmp = f"{path}.{os.getpid()}"
+        subprocess.check_call([os.environ.get("CXX") or "g++", *flags, sources[0], "-o", tmp, "-lpthread"])
+        os.replace(tmp, path)
+    return ctypes.CDLL(path)
 
 
 def oracle_for(scene):
