@@ -389,6 +389,37 @@ typedef struct rh_trace_opts {
 int rh_trace_rays(const rh_scene* scene, const double* rays, uint64_t n, const rh_trace_opts* opts, double* colors_out,
                   int32_t* hit_ids_out, rh_stats* stats);
 
+/* ---- progressive rendering ------------------------------------------ */
+/* Running per-pixel sums of the sample colours of one frame (or of one shard's rows of it: the rows rh_render's
+ * shard_index / shard_count / band_height select, band_height 0 resolved as rh_render resolves it), kept on the device
+ * between calls.  2 x 24 bytes per pixel of those rows.  stream_spp: samples per pixel of the SplitMix64 stream that
+ * RH_OFFSETS_SPLITMIX64 calls draw from (0: such calls are refused).  Needs rh_init (else RH_ERR_STATE). */
+typedef struct rh_accum rh_accum; /* opaque */
+int rh_accum_create(int width, int height, int shard_index, int shard_count, int band_height, uint32_t stream_spp,
+                    rh_accum** out);
+/* Back to 0 samples; the next call may use another scene, camera or max_depth. */
+int rh_accum_reset(rh_accum* acc);
+void rh_accum_destroy(rh_accum* acc);
+/* Traces opts->spp new samples per pixel exactly as rh_render would, adds them to the accumulator's sums in sample
+ * order (continuing `foldl (+) black`, RayHs.hs:169-171: K calls of s samples leave the sums of one call of K*s
+ * samples), so that the accumulator's count N grows by spp, then writes what the caller asked for:
+ *   rgb_out    RGB8 = toIntC((1/N) sum), clamped as rh_render clamps it;
+ *   linear_out double[rows][width][3] = (1/N) sum, the value toIntC is applied to (not clamped).
+ * Either may be NULL (neither: the call only accumulates).  Layouts are shard-compact, as for rh_render.
+ * Offsets: RH_OFFSETS_NONE / F64 / F32 / TILED_F64 give THIS call's samples ([pixels][spp][2] or the [tile^2][spp][2]
+ * tile), host or device, RH_FLAG_SHARD_OFFSETS as for rh_render; so slicing one stream [pixels][S][2] into
+ * consecutive sample ranges reproduces the one-shot S-sample frame.  RH_OFFSETS_SPLITMIX64 draws values 2g and 2g + 1
+ * with g = pixel * stream_spp + N_before + s: the stream of rh_sample_offsets_f64(seed, n_pixels, stream_spp, ...);
+ * N_before + spp > stream_spp is RH_ERR_ARG.  hit_ids_out (RH_FLAG_HIT_IDS): this call's samples, int32[rows][width]
+ * [spp][2].  RH_FLAG_DEVICE_OUT applies to all three outputs (linear_out 8-byte aligned).  The other flags behave as
+ * in rh_render and may change from call to call; RH_FLAG_PEER_FRAMES is refused.
+ * The first call after create or reset records the scene, the camera bytes and max_depth; a later call with others is
+ * RH_ERR_ARG (reset first).  opts must match the accumulator's size and shard.  A call that fails (argument, CUDA or
+ * RH_ERR_OVERFLOW) leaves the sums and N unchanged.  For the scene's learned state (shadow schedule, queue factor, row
+ * costs) the call is a render.  stats: this call's samples; negative_channels counts its RGB8 output. */
+int rh_render_accumulate(const rh_scene* scene, const rh_camera* camera, const rh_render_opts* opts, rh_accum* acc,
+                         uint8_t* rgb_out, double* linear_out, int32_t* hit_ids_out, rh_stats* stats);
+
 /* Rows owned by one shard (equal for all shards: bands are padded). */
 int rh_shard_rows(int height, int shard_count, int band_height);
 int rh_default_band_height(int height, int shard_count);

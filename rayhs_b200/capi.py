@@ -146,6 +146,10 @@ SIGNATURES = {
     "rh_closest_intersection": (C.c_int, [vp, vp, C.c_uint64, vp, C.c_int32]),
     "rh_shadow_intersection": (C.c_int, [vp, C.c_uint32, vp, C.c_uint64, vp, C.c_int32]),
     "rh_trace_rays": (C.c_int, [vp, vp, C.c_uint64, C.POINTER(rh_trace_opts), vp, vp, C.POINTER(rh_stats)]),
+    "rh_accum_create": (C.c_int, [C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.c_uint32, C.POINTER(vp)]),
+    "rh_accum_reset": (C.c_int, [vp]),
+    "rh_accum_destroy": (None, [vp]),
+    "rh_render_accumulate": (C.c_int, [vp, C.POINTER(rh_camera), C.POINTER(rh_render_opts), vp, vp, vp, vp, C.POINTER(rh_stats)]),
     "rh_shard_rows": (C.c_int, [C.c_int, C.c_int, C.c_int]),
     "rh_default_band_height": (C.c_int, [C.c_int, C.c_int]),
     "rh_deinterleave_bands": (C.c_int, [vp, vp, C.c_int, C.c_int, C.c_int, C.c_int]),

@@ -247,7 +247,7 @@ struct ChunkParams {
   uint32_t ray_items;     // kOffsetsRays: pass-0 items of the chunk that are rays (the rest of its last row is padding)
   const void* offsets;    // device
   uint32_t offset_linear; // f64 pairs in work-item order: pair of item i at offsets[offset_base + i] (bulk-copy staging)
-  uint32_t pad5_;
+  uint32_t stream_spp;    // RH_OFFSETS_SPLITMIX64: samples per pixel of the stream (rh_render: spp) ...
   unsigned long long offset_base;
   unsigned long long offset_seed;  // RH_OFFSETS_SPLITMIX64
   double* accum;          // 3 planes of accum_stride (r,g,b), chunk-local sample order
@@ -258,11 +258,21 @@ struct ChunkParams {
   uint8_t* rgb;           // shard-compact framebuffer (or null with peer frames)
   uint8_t* peer[kMaxPeers];  // RH_FLAG_PEER_FRAMES: full frames of all shards
   uint32_t n_peers;
-  uint32_t pad4_;
+  uint32_t stream_base;   // ... and the stream's first sample this call traces (rh_render: 0)
   ChunkCtl* ctl;
   FrameCounters* counters;
   RayQueue q_in, q_out;
   ShadowQueue q_hits, q_shadow;
+};
+
+// rh_render_accumulate's end of a chunk instead of the resolve: the running per-pixel sums of the accumulator.
+struct AccumParams {
+  const double* sum_in;  // 3 planes (r, g, b) of `plane` doubles, shard-compact pixel order; not read when n_before == 0
+  double* sum_out;       // the same layout: sum_in + this call's samples, in sample order
+  double* linear;        // shard-compact double[pixel][3] = sum / n_total, or null
+  size_t plane;
+  uint32_t n_before;     // samples in sum_in
+  uint32_t n_total;      // n_before + spp
 };
 
 // One launch of the batched ray queries (rh_closest_intersection / rh_shadow_intersection) over rays [0, n).
@@ -289,6 +299,9 @@ int launch_shadow(const SceneView& S, const ChunkParams& P, bool count, bool ref
 void launch_resolve(const ChunkParams& P, void* stream);
 // rh_trace_rays' end of a chunk instead of the resolve: the accumulators of its rays to colors (double[n][3], all rays)
 void launch_store_colors(const ChunkParams& P, double* colors, void* stream);
+// rh_render_accumulate's end of a chunk instead of the resolve: adds the chunk's samples to the running sums and writes
+// RGB8 (P.rgb, may be null) and the linear colours (A.linear, may be null) of the new sums
+void launch_accumulate_resolve(const ChunkParams& P, const AccumParams& A, void* stream);
 // query_closest_kernel / query_shadow_kernel: `grid` blocks of one SM each
 void launch_query_closest(const SceneView& S, const QueryParams& Q, int grid, void* stream);
 void launch_query_shadow(const SceneView& S, const QueryParams& Q, int grid, void* stream);

@@ -11,6 +11,7 @@
 //   shadow_simple_kernel  K3 for scenes with more than 32 lights.
 //   resolve_kernel        K6: average the samples of a pixel, toIntC, coalesced RGB8 store (or peer stores).
 //   store_colors_kernel   K6 of rh_trace_rays: the linear colours of caller-built rays (trace_kernel<.., RAYS = true>).
+//   accumulate_resolve_kernel  K6 of rh_render_accumulate: running per-pixel sums across calls, RGB8 and linear colours.
 //   deinterleave          K7: band re-assembly after the all-gather.
 //
 // All arithmetic is IEEE double in the reference's operation order and this file is compiled with -fmad=false (GHC
@@ -1506,8 +1507,9 @@ __device__ __forceinline__ bool load_item(const ChunkParams& P, const CameraPara
     if (grow >= P.height) return false;
     double ox = 0, oy = 0;
     if (P.offset_mode == RH_OFFSETS_SPLITMIX64) {
-      // values 2g and 2g+1 of the stream rh_sample_offsets_f64(seed, ...) writes (x before y, RayHs.hs:185-188)
-      const unsigned long long g = ((unsigned long long)grow * P.width + col) * P.spp + s;
+      // values 2g and 2g+1 of the stream rh_sample_offsets_f64(seed, n, stream_spp, ...) writes (x before y,
+      // RayHs.hs:185-188); a progressive call traces samples stream_base .. stream_base + spp - 1 of each pixel
+      const unsigned long long g = ((unsigned long long)grow * P.width + col) * P.stream_spp + P.stream_base + s;
       ox = splitmix01(P.offset_seed, 2 * g) - 0.5;
       oy = splitmix01(P.offset_seed, 2 * g + 1) - 0.5;
     } else if (has_array) {
@@ -2544,6 +2546,86 @@ __global__ void __launch_bounds__(kBlock) store_colors_kernel(const __grid_const
   for (uint32_t i = threadIdx.x; i < 3 * n_here; i += kBlock) dst[i] = rgb[i];
 }
 
+// ------------------------------------------------------------------ K6'': rh_render_accumulate (RayHs.hs:169-171, continued)
+// The resolve of a progressive call: each pixel's running sum (0 on the first call) continues `foldl (+) black` over the
+// chunk's samples in sample order, with resolve_kernel's loads and association, so that calls of s1, s2, ... samples
+// leave exactly the sum of one frame of s1 + s2 + ... samples.  The new sum goes to the other buffer (a retried frame
+// reads the old one again); then toIntC of (1/N) sum as RGB8 and (1/N) sum as linear double[3], both stores coalesced
+// through shared memory.  The sums are three planes, so their loads and stores coalesce as they are.
+__global__ void __launch_bounds__(kBlock) accumulate_resolve_kernel(const __grid_constant__ ChunkParams P,
+                                                                     const __grid_constant__ AccumParams A) {
+  __shared__ __align__(16) double lin[kBlock * 3];
+  __shared__ __align__(16) uint8_t bytes[kBlock * 3];
+  const uint32_t n_pixels = P.n_rows * P.width;
+  const uint32_t lp = blockIdx.x * kBlock + threadIdx.x;
+  const size_t px = (size_t)P.first_row * P.width + lp;  // pixel index in the shard's rows
+  bool negative = false;
+  if (lp < n_pixels) {
+    double sr = 0, sg = 0, sb = 0, cr = 0, cg = 0, cb = 0;
+    const uint32_t lrow = lp / P.width;
+    if (global_row(P, P.first_row + lrow) < P.height) {
+      if (A.n_before) {
+        sr = A.sum_in[px];
+        sg = A.sum_in[A.plane + px];
+        sb = A.sum_in[2 * A.plane + px];
+      }
+      const double* a = P.accum + (size_t)lp * P.spp;
+      if ((P.spp & 1u) == 0 && (P.accum_stride & 1u) == 0) {
+        const double2* a0 = (const double2*)a;
+        const double2* a1 = (const double2*)(a + P.accum_stride);
+        const double2* a2 = (const double2*)(a + 2 * (size_t)P.accum_stride);
+        for (uint32_t s = 0; s < P.spp / 2; s++) {
+          const double2 r2 = a0[s], g2 = a1[s], b2 = a2[s];
+          sr = (sr + r2.x) + r2.y;
+          sg = (sg + g2.x) + g2.y;
+          sb = (sb + b2.x) + b2.y;
+        }
+      } else {
+        for (uint32_t s = 0; s < P.spp; s++) {
+          sr = sr + a[s];
+          sg = sg + a[P.accum_stride + s];
+          sb = sb + a[2 * (size_t)P.accum_stride + s];
+        }
+      }
+      const double inv = 1.0 / (double)A.n_total;
+      cr = inv * sr;
+      cg = inv * sg;
+      cb = inv * sb;
+    }
+    A.sum_out[px] = sr;
+    A.sum_out[A.plane + px] = sg;
+    A.sum_out[2 * A.plane + px] = sb;
+    bool neg = false;  // (padding rows: 0, as resolve_kernel stores them)
+    bytes[3 * threadIdx.x] = (uint8_t)to_int_c(cr, neg);
+    bytes[3 * threadIdx.x + 1] = (uint8_t)to_int_c(cg, neg);
+    bytes[3 * threadIdx.x + 2] = (uint8_t)to_int_c(cb, neg);
+    negative = neg && P.rgb;
+    lin[3 * threadIdx.x] = cr;
+    lin[3 * threadIdx.x + 1] = cg;
+    lin[3 * threadIdx.x + 2] = cb;
+  }
+  const unsigned neg = __ballot_sync(kFull, negative);
+  if ((threadIdx.x & 31) == 0 && neg) atomicAdd(&P.counters->negative_channels, (unsigned long long)__popc(neg));
+  __syncthreads();
+  const uint32_t n_here = min((uint32_t)kBlock, n_pixels - blockIdx.x * kBlock) * 3;
+  const size_t first = (size_t)P.first_row * P.width + (size_t)blockIdx.x * kBlock;
+  if (P.rgb) {
+    uint8_t* dst = P.rgb + first * 3;
+    if ((((uintptr_t)dst) & 3) == 0) {
+      const uint32_t words = n_here / 4;
+      if (threadIdx.x < words) ((uint32_t*)dst)[threadIdx.x] = ((const uint32_t*)bytes)[threadIdx.x];
+      const uint32_t tail = words * 4 + threadIdx.x;
+      if (tail < n_here) dst[tail] = bytes[tail];
+    } else {
+      for (uint32_t i = threadIdx.x; i < n_here; i += kBlock) dst[i] = bytes[i];
+    }
+  }
+  if (A.linear) {
+    double* dst = A.linear + first * 3;
+    for (uint32_t i = threadIdx.x; i < n_here; i += kBlock) dst[i] = lin[i];
+  }
+}
+
 // ------------------------------------------------------------------ K7: band de-interleave after the all-gather
 __global__ void deinterleave_kernel(const uint8_t* __restrict__ gathered, uint8_t* __restrict__ out, uint32_t row_bytes,
                                     uint32_t height, uint32_t shard_count, uint32_t band_height, uint32_t rows_per_shard) {
@@ -2696,6 +2778,10 @@ void launch_resolve(const ChunkParams& P, void* stream) {
 }
 void launch_store_colors(const ChunkParams& P, double* colors, void* stream) {
   store_colors_kernel<<<(P.ray_items + kBlock - 1) / kBlock, kBlock, 0, (cudaStream_t)stream>>>(P, colors);
+}
+void launch_accumulate_resolve(const ChunkParams& P, const AccumParams& A, void* stream) {
+  const uint32_t n_pixels = P.n_rows * P.width;
+  accumulate_resolve_kernel<<<(n_pixels + kBlock - 1) / kBlock, kBlock, 0, (cudaStream_t)stream>>>(P, A);
 }
 void launch_query_closest(const SceneView& S, const QueryParams& Q, int grid, void* stream) {
   query_closest_kernel<<<grid, kQueryBlock, kQuerySmem, (cudaStream_t)stream>>>(S, Q);

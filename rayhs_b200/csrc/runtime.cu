@@ -46,6 +46,7 @@ using namespace rhd;
 namespace {
 
 std::atomic<uint64_t> g_launches{0};
+std::atomic<uint64_t> g_contexts{0};  // device contexts opened so far (names each one: an address can be reused)
 
 #define RH_CUDA(expr)                                                                                     \
   do {                                                                                                    \
@@ -79,6 +80,7 @@ struct DevBuf {
 // Everything the library owns on one GPU.
 struct Device {
   int dev = -1;
+  uint64_t context = 0;
   int n_sms = 0;
   size_t total_mem = 0;
   cudaStream_t stream = nullptr;       // kernels (lane 0)
@@ -95,7 +97,7 @@ struct Device {
   struct Scratch {
     DevBuf accum, rayq[2], rayq_fill[2], hitq, hitq_words, shq, shq_words, deep, deep_shadow;
   } lane[2];
-  DevBuf ctl, counters, offsets, rgb, ids;
+  DevBuf ctl, counters, offsets, rgb, ids, linear;
   DevBuf query;  // ray queries: claim cursor, then (host buffers) one chunk of rays and of results
   void* pinned = nullptr;  // ctl + counters read-back
   size_t pinned_bytes = 0;
@@ -104,6 +106,7 @@ struct Device {
 
   int open(int device) {
     dev = device;
+    context = ++g_contexts;
     RH_CUDA(cudaSetDevice(dev));
     cudaDeviceProp prop;
     RH_CUDA(cudaGetDeviceProperties(&prop, dev));
@@ -149,7 +152,7 @@ struct Device {
         e = nullptr;
       }
     }
-    for (DevBuf* b : {&ctl, &counters, &offsets, &rgb, &ids, &query})
+    for (DevBuf* b : {&ctl, &counters, &offsets, &rgb, &ids, &linear, &query})
       b->release();
     if (pinned) cudaFreeHost(pinned);
     pinned = nullptr;
@@ -200,6 +203,25 @@ struct rh_scene {
   mutable std::vector<float> row_cost;    // kernel ms per local row (its chunk's time / its chunk's rows)
   mutable uint32_t queue_factor = 2;          // the queue capacity factor the scene's last frame needed
   mutable bool stream_compute_bound = false;  // ... and in that frame the kernels, not the upload, finished last
+};
+
+// Running per-pixel sums of one progressive frame (or of one shard's rows of it): two buffers of three planes of doubles,
+// `cur` holding the sums of the n samples so far.  A call's sink reads buffer cur and writes the other; the call flips
+// them and adds its samples to n only after a frame that completed, so a failed call or an overflow retry leaves the
+// sums as they were.  The first call after create or reset fixes the view (scene, camera, max_depth).
+struct rh_accum {
+  Device* device = nullptr;
+  uint64_t context = 0;  // device->context when the accumulator was created
+  int dev = -1;
+  int width = 0, height = 0, shard_index = 0, shard_count = 1, band_height = 1, rows_local = 0;
+  uint32_t stream_spp = 0;  // RH_OFFSETS_SPLITMIX64: samples per pixel of the stream the calls draw from
+  size_t plane = 0;         // doubles per colour plane: rows_local * width
+  DevBuf sums;              // [2][3][plane]
+  int cur = 0;
+  uint32_t n = 0;
+  const rh_scene* scene = nullptr;
+  rh_camera camera{};
+  int32_t max_depth = 0;
 };
 
 namespace {
@@ -1328,41 +1350,52 @@ struct Frame {
   // and the scene's learned state (shadow-schedule tuning, queue factor, row costs) is neither used nor changed
   bool trace = false;
   uint64_t n_rays = 0;
+  // RH_OFFSETS_SPLITMIX64: the stream's samples per pixel and the first of them this frame traces
+  uint32_t stream_spp = 0, stream_base = 0;
+  // rh_render_accumulate: the sink adds the samples to the accumulator's sums (read sum_in, write sum_out) and writes
+  // RGB8 to `out` and the linear colours to `linear`, either of them optional
+  bool accumulate = false;
+  AccumParams acc{};
+  double* linear = nullptr;
+  size_t linear_bytes = 0;
   const char* overflow_error = "rh_render: ray queue overflow; lower chunk_samples";
 };
 
-// rh_render's argument checks.
+// rh_render's argument checks (`who` names the entry point in the messages).  With f->accumulate set, rgb_out may be null.
 int render_frame(Device* D, const rh_scene* scene, const rh_camera* camera, const rh_render_opts* o, uint8_t* rgb_out,
-                 int32_t* hit_ids_out, Frame* f) {
+                 int32_t* hit_ids_out, Frame* f, const char* who = "rh_render") {
+  const std::string w(who);
   const bool peer_frames = o && (o->flags & RH_FLAG_PEER_FRAMES) != 0;
-  if (!scene || !camera || !o || (!rgb_out && !peer_frames)) return rh::set_error(RH_ERR_ARG, "rh_render: null argument");
+  if (!scene || !camera || !o || (!rgb_out && !peer_frames && !f->accumulate)) return rh::set_error(RH_ERR_ARG, w + ": null argument");
   if (peer_frames && (!o->peer_frames || o->n_peer_frames <= 0 || o->n_peer_frames > kMaxPeers))
-    return rh::set_error(RH_ERR_ARG, "rh_render: RH_FLAG_PEER_FRAMES needs 1..16 peer frame pointers");
+    return rh::set_error(RH_ERR_ARG, w + ": RH_FLAG_PEER_FRAMES needs 1..16 peer frame pointers");
   if (peer_frames && (o->flags & RH_FLAG_HIT_IDS))
-    return rh::set_error(RH_ERR_ARG, "rh_render: hit ids are not exchanged; render them without RH_FLAG_PEER_FRAMES");
-  if (scene->device != D) return rh::set_error(RH_ERR_ARG, "rh_render: scene lives on another device context");
+    return rh::set_error(RH_ERR_ARG, w + ": hit ids are not exchanged; render them without RH_FLAG_PEER_FRAMES");
+  if (scene->device != D) return rh::set_error(RH_ERR_ARG, w + ": scene lives on another device context");
   const int W = o->width, H = o->height, spp = o->spp;
   if (W <= 0 || H <= 0 || spp <= 0 || o->max_depth < 0 || o->max_depth > kMaxDepth)
-    return rh::set_error(RH_ERR_ARG, "rh_render: bad width/height/spp/max_depth");
+    return rh::set_error(RH_ERR_ARG, w + ": bad width/height/spp/max_depth");
   if (camera->projection != RH_PROJ_ORTHOGRAPHIC && camera->projection != RH_PROJ_PERSPECTIVE)
-    return rh::set_error(RH_ERR_ARG, "rh_render: unknown projection");
+    return rh::set_error(RH_ERR_ARG, w + ": unknown projection");
   const int G = o->shard_count <= 0 ? 1 : o->shard_count;
-  if (o->shard_index < 0 || o->shard_index >= G) return rh::set_error(RH_ERR_ARG, "rh_render: shard_index out of range");
+  if (o->shard_index < 0 || o->shard_index >= G) return rh::set_error(RH_ERR_ARG, w + ": shard_index out of range");
   const int bh = o->band_height > 0 ? o->band_height : rh_default_band_height(H, G);
   const int mode = o->offset_mode;
-  if (mode < RH_OFFSETS_NONE || mode > RH_OFFSETS_SPLITMIX64) return rh::set_error(RH_ERR_ARG, "rh_render: bad offset_mode");
-  if (mode != RH_OFFSETS_NONE && !o->offsets) return rh::set_error(RH_ERR_ARG, "rh_render: offsets is null");
-  if (mode == RH_OFFSETS_TILED_F64 && o->offset_tile <= 0) return rh::set_error(RH_ERR_ARG, "rh_render: offset_tile must be > 0");
-  if ((uint64_t)W * spp > 0x7fffffffu) return rh::set_error(RH_ERR_ARG, "rh_render: row too large");
-  if ((o->flags & RH_FLAG_HIT_IDS) && !hit_ids_out) return rh::set_error(RH_ERR_ARG, "rh_render: RH_FLAG_HIT_IDS without hit_ids_out");
+  if (mode < RH_OFFSETS_NONE || mode > RH_OFFSETS_SPLITMIX64) return rh::set_error(RH_ERR_ARG, w + ": bad offset_mode");
+  if (mode != RH_OFFSETS_NONE && !o->offsets) return rh::set_error(RH_ERR_ARG, w + ": offsets is null");
+  if (mode == RH_OFFSETS_TILED_F64 && o->offset_tile <= 0) return rh::set_error(RH_ERR_ARG, w + ": offset_tile must be > 0");
+  if ((uint64_t)W * spp > 0x7fffffffu) return rh::set_error(RH_ERR_ARG, w + ": row too large");
+  if ((o->flags & RH_FLAG_HIT_IDS) && !hit_ids_out) return rh::set_error(RH_ERR_ARG, w + ": RH_FLAG_HIT_IDS without hit_ids_out");
   if (mode == RH_OFFSETS_SPLITMIX64 && (o->flags & RH_FLAG_DEVICE_OFFSETS))
-    return rh::set_error(RH_ERR_ARG, "rh_render: RH_OFFSETS_SPLITMIX64 takes a host pointer to the seed");
+    return rh::set_error(RH_ERR_ARG, w + ": RH_OFFSETS_SPLITMIX64 takes a host pointer to the seed");
   f->o = *o;
   f->o.shard_count = G;
   f->o.band_height = bh;
   f->cam = make_camera(*camera, W, H);
   f->out = rgb_out;
   f->ids_out = hit_ids_out;
+  f->stream_spp = (uint32_t)spp;
+  f->stream_base = 0;
   f->rows_local = rh_shard_rows(H, G, bh);
   f->out_bytes = (size_t)f->rows_local * W * 3;
   f->ids_bytes = (size_t)f->rows_local * W * spp * sizeof(int2);
@@ -1416,6 +1449,7 @@ struct FrameRun {
   bool counting = false, host_offsets = false, pipelined = false;
   uint8_t* d_rgb = nullptr;
   int2* d_ids = nullptr;
+  double* d_linear = nullptr;
   const void* d_offsets = nullptr;
   int off_index = kOffIndexLocal;
   unsigned long long offset_seed = 0;
@@ -1492,6 +1526,8 @@ struct FrameRun {
     P.offset_tile = o.offset_tile;
     P.offsets = d_offsets;
     P.offset_seed = offset_seed;
+    P.stream_spp = f.stream_spp;
+    P.stream_base = f.stream_base;
     P.accum = (double*)sc.accum.p;
     P.accum_stride = (uint32_t)chunk_samples;
     P.hit_ids = d_ids;
@@ -1586,8 +1622,15 @@ struct FrameRun {
     }
     cudaEvent_t a = nullptr;
     if (sh.profile) a = prof_event(lane_stream);
-    if (f.trace) launch_store_colors(P, (double*)d_rgb, lane_stream);
-    else launch_resolve(P, lane_stream);
+    if (f.trace) {
+      launch_store_colors(P, (double*)d_rgb, lane_stream);
+    } else if (f.accumulate) {
+      AccumParams A = f.acc;
+      A.linear = d_linear;
+      launch_accumulate_resolve(P, A, lane_stream);
+    } else {
+      launch_resolve(P, lane_stream);
+    }
     if (sh.profile) spans.push_back({a, prof_event(lane_stream), 2});
     launches += 1;
     if (host_offsets) {
@@ -1797,7 +1840,7 @@ int run_frame(Device* D, const rh_scene* scene, const Frame& f, rh_stats* stats)
   if (R.chunk_samples > 0x7fffffffu) return rh::set_error(RH_ERR_ARG, "rh_render: chunk too large");
 
   int rc;
-  if (peer_frames) R.d_rgb = nullptr;
+  if (peer_frames || !f.out) R.d_rgb = nullptr;
   else if (dev_out) R.d_rgb = f.out;
   else {
     if ((rc = D->rgb.reserve(f.out_bytes))) return rc;
@@ -1807,6 +1850,11 @@ int run_frame(Device* D, const rh_scene* scene, const Frame& f, rh_stats* stats)
   else if (want_ids) {
     if ((rc = D->ids.reserve(f.ids_bytes))) return rc;
     R.d_ids = (int2*)D->ids.p;
+  }
+  if (f.linear && dev_out) R.d_linear = f.linear;
+  else if (f.linear) {
+    if ((rc = D->linear.reserve(f.linear_bytes))) return rc;
+    R.d_linear = (double*)D->linear.p;
   }
   // Two chunks in flight (two streams, two sets of queues) when the frame has several: the kernels are persistent and
   // fill the GPU, so a chunk's next kernel starts on the SMs the other chunk's kernel frees as its warps run out of
@@ -1888,8 +1936,9 @@ int run_frame(Device* D, const rh_scene* scene, const Frame& f, rh_stats* stats)
     RH_CUDA(cudaMemcpyAsync(D->pinned, D->ctl.p, ctl_bytes, cudaMemcpyDeviceToHost, D->stream));
     RH_CUDA(cudaMemcpyAsync((char*)D->pinned + ctl_bytes, D->counters.p, sizeof(FrameCounters), cudaMemcpyDeviceToHost, D->stream));
     if (!dev_out && !peer_frames) {
-      RH_CUDA(cudaMemcpyAsync(f.out, R.d_rgb, f.out_bytes, cudaMemcpyDeviceToHost, D->stream));
+      if (f.out) RH_CUDA(cudaMemcpyAsync(f.out, R.d_rgb, f.out_bytes, cudaMemcpyDeviceToHost, D->stream));
       if (want_ids) RH_CUDA(cudaMemcpyAsync(f.ids_out, R.d_ids, f.ids_bytes, cudaMemcpyDeviceToHost, D->stream));
+      if (f.linear) RH_CUDA(cudaMemcpyAsync(f.linear, R.d_linear, f.linear_bytes, cudaMemcpyDeviceToHost, D->stream));
     }
     RH_CUDA(cudaEventRecord(D->ev_end, D->stream));
     RH_CUDA(cudaStreamSynchronize(D->stream));
@@ -1925,6 +1974,95 @@ int check_device_pointers(std::initializer_list<const void*> ptrs, const std::st
     RH_CUDA(cudaPointerGetAttributes(&a, p));
     if (a.type != cudaMemoryTypeDevice && a.type != cudaMemoryTypeManaged) return rh::set_error(RH_ERR_ARG, msg);
   }
+  return RH_OK;
+}
+
+// ------------------------------------------------------------------ progressive accumulation
+// rh_render_accumulate's argument checks: rh_render's (render_frame), then those of the accumulator.
+int accumulate_frame(Device* D, const rh_scene* scene, const rh_camera* camera, const rh_render_opts* o, rh_accum* acc,
+                     uint8_t* rgb_out, double* linear_out, int32_t* hit_ids_out, Frame* f) {
+  const std::string w = "rh_render_accumulate";
+  if (!scene || !camera || !o || !acc) return rh::set_error(RH_ERR_ARG, w + ": null argument");
+  if (acc->device != D || acc->context != D->context) return rh::set_error(RH_ERR_ARG, w + ": accumulator lives on another device context");
+  if (o->flags & RH_FLAG_PEER_FRAMES) return rh::set_error(RH_ERR_ARG, w + ": RH_FLAG_PEER_FRAMES is not supported");
+  f->accumulate = true;
+  int rc = render_frame(D, scene, camera, o, rgb_out, hit_ids_out, f, "rh_render_accumulate");
+  if (rc) return rc;
+  if (f->o.width != acc->width || f->o.height != acc->height || f->o.shard_index != acc->shard_index ||
+      f->o.shard_count != acc->shard_count || f->o.band_height != acc->band_height)
+    return rh::set_error(RH_ERR_ARG, w + ": width, height, shard_index, shard_count or band_height differ from the accumulator's");
+  const uint32_t spp = (uint32_t)o->spp;
+  if ((uint64_t)acc->n + spp > 0xffffffffu) return rh::set_error(RH_ERR_ARG, w + ": more than 2^32 - 1 samples per pixel");
+  if (o->offset_mode == RH_OFFSETS_SPLITMIX64) {
+    if (acc->stream_spp == 0)
+      return rh::set_error(RH_ERR_ARG, w + ": RH_OFFSETS_SPLITMIX64 needs an accumulator created with stream_spp > 0");
+    if ((uint64_t)acc->n + spp > acc->stream_spp)
+      return rh::set_error(RH_ERR_ARG, w + ": RH_OFFSETS_SPLITMIX64 past the end of the stream (" + std::to_string(acc->n) + " + " +
+                                           std::to_string(spp) + " > stream_spp " + std::to_string(acc->stream_spp) + ")");
+  }
+  if (acc->n > 0 && (scene != acc->scene || memcmp(camera, &acc->camera, sizeof acc->camera) != 0 || o->max_depth != acc->max_depth))
+    return rh::set_error(RH_ERR_ARG, w + ": scene, camera or max_depth differ from the accumulator's first call; rh_accum_reset it first");
+  const bool want_ids = (o->flags & RH_FLAG_HIT_IDS) != 0;
+  if (o->flags & RH_FLAG_DEVICE_OUT) {
+    if ((uintptr_t)linear_out % 8) return rh::set_error(RH_ERR_ARG, w + ": device linear_out must be 8-byte aligned");
+    RH_CUDA(cudaSetDevice(D->dev));
+    if ((rc = check_device_pointers({rgb_out, linear_out, want_ids ? hit_ids_out : nullptr},
+                                    w + ": RH_FLAG_DEVICE_OUT with a pointer that is not device memory")))
+      return rc;
+  }
+  const size_t half = 3 * acc->plane;
+  f->stream_spp = acc->stream_spp;
+  f->stream_base = acc->n;
+  f->acc.sum_in = (const double*)acc->sums.p + (size_t)acc->cur * half;
+  f->acc.sum_out = (double*)acc->sums.p + (size_t)(acc->cur ^ 1) * half;
+  f->acc.plane = acc->plane;
+  f->acc.n_before = acc->n;
+  f->acc.n_total = acc->n + spp;
+  f->linear = linear_out;
+  f->linear_bytes = (size_t)f->rows_local * f->o.width * 3 * sizeof(double);
+  f->overflow_error = "rh_render_accumulate: ray queue overflow; lower chunk_samples";
+  return RH_OK;
+}
+
+int accumulate_on(Device* D, const rh_scene* scene, const rh_camera* camera, const rh_render_opts* o, rh_accum* acc,
+                  uint8_t* rgb_out, double* linear_out, int32_t* hit_ids_out, rh_stats* stats) {
+  Frame f;
+  int rc = accumulate_frame(D, scene, camera, o, acc, rgb_out, linear_out, hit_ids_out, &f);
+  if (rc || (rc = run_frame(D, scene, f, stats))) return rc;
+  // the frame completed: its sums are the current ones
+  if (acc->n == 0) {
+    acc->scene = scene;
+    acc->camera = *camera;
+    acc->max_depth = o->max_depth;
+  }
+  acc->cur ^= 1;
+  acc->n += (uint32_t)o->spp;
+  return RH_OK;
+}
+
+int accum_create_on(Device* D, int width, int height, int shard_index, int shard_count, int band_height, uint32_t stream_spp,
+                    rh_accum** out) {
+  if (!out) return rh::set_error(RH_ERR_ARG, "rh_accum_create: null out");
+  *out = nullptr;
+  const int G = shard_count <= 0 ? 1 : shard_count;
+  if (width <= 0 || height <= 0) return rh::set_error(RH_ERR_ARG, "rh_accum_create: bad width/height");
+  if (shard_index < 0 || shard_index >= G) return rh::set_error(RH_ERR_ARG, "rh_accum_create: shard_index out of range");
+  auto A = std::make_unique<rh_accum>();
+  A->device = D;
+  A->context = D->context;
+  A->dev = D->dev;
+  A->width = width;
+  A->height = height;
+  A->shard_index = shard_index;
+  A->shard_count = G;
+  A->band_height = band_height > 0 ? band_height : rh_default_band_height(height, G);
+  A->rows_local = rh_shard_rows(height, G, A->band_height);
+  A->stream_spp = stream_spp;
+  A->plane = (size_t)A->rows_local * width;
+  RH_CUDA(cudaSetDevice(D->dev));
+  int rc = A->sums.reserve(2 * 3 * A->plane * sizeof(double));
+  if (rc) return rc;
+  *out = A.release();
   return RH_OK;
 }
 
@@ -2156,6 +2294,29 @@ int rh_trace_rays(const rh_scene* scene, const double* rays, uint64_t n, const r
                   int32_t* hit_ids_out, rh_stats* stats) {
   if (!g_dev) return rh::set_error(RH_ERR_STATE, "rh_trace_rays: call rh_init first");
   return trace_on(g_dev.get(), scene, rays, n, opts, colors_out, hit_ids_out, stats);
+}
+
+int rh_accum_create(int width, int height, int shard_index, int shard_count, int band_height, uint32_t stream_spp,
+                    rh_accum** out) {
+  if (!g_dev) return rh::set_error(RH_ERR_STATE, "rh_accum_create: call rh_init first");
+  return accum_create_on(g_dev.get(), width, height, shard_index, shard_count, band_height, stream_spp, out);
+}
+int rh_accum_reset(rh_accum* acc) {
+  if (!acc) return rh::set_error(RH_ERR_ARG, "rh_accum_reset: null accumulator");
+  acc->n = 0;
+  acc->scene = nullptr;
+  return RH_OK;
+}
+void rh_accum_destroy(rh_accum* acc) {
+  if (!acc) return;
+  if (acc->dev >= 0) cudaSetDevice(acc->dev);  // (not through acc->device: that context may have been shut down)
+  acc->sums.release();
+  delete acc;
+}
+int rh_render_accumulate(const rh_scene* scene, const rh_camera* camera, const rh_render_opts* opts, rh_accum* acc,
+                         uint8_t* rgb_out, double* linear_out, int32_t* hit_ids_out, rh_stats* stats) {
+  if (!g_dev) return rh::set_error(RH_ERR_STATE, "rh_render_accumulate: call rh_init first");
+  return accumulate_on(g_dev.get(), scene, camera, opts, acc, rgb_out, linear_out, hit_ids_out, stats);
 }
 
 int rh_closest_intersection(const rh_scene* scene, const double* rays, uint64_t n, rh_hit* hits_out, int32_t flags) {

@@ -164,12 +164,14 @@ def renderingFromScene(sc: Scene, width: int | None = None, height: int | None =
 
 @dataclass
 class Image:
-    """Image.hs:21-23, already quantised by toIntC (Image.hs:54-55): uint8 [height, width, 3]."""
+    """Image.hs:21-23, already quantised by toIntC (Image.hs:54-55): uint8 [height, width, 3].  `linear` (progressive
+    calls that ask for it): float64 [height, width, 3], the averaged colour toIntC is applied to."""
     width: int
     height: int
     pixels: np.ndarray
     stats: dict = field(default_factory=dict)
     hit_ids: np.ndarray | None = None
+    linear: np.ndarray | None = None
 
 
 def sample_offsets(n_pixels: int, spp: int, seed: int = 24, dtype=np.float64) -> np.ndarray:
@@ -583,6 +585,125 @@ def distributedRayTrace(job: Rendering, spp: int = 64, seed: int = 24, offsets=N
         n = offset_tile * offset_tile if offset_tile else job.width * job.height
         offsets = sample_offsets(n, spp, seed)
     return _trace(job, spp, offsets, offset_tile, **kw)
+
+
+class Accumulator:
+    """Progressive rendering (rh_render_accumulate): running per-pixel sums of the sample colours of one view, kept on
+    the device between calls, so that an image can be refined over several calls instead of rendered again.  Each
+    add(spp) traces spp new samples per pixel exactly as render would, continues the sums in sample order and returns
+    the image of all samples so far: K calls of s samples give the bytes of one render of K*s samples.
+
+    `stream_spp`: samples per pixel of the SplitMix64 stream that add(seed=...) draws from (sample_offsets(n, stream_spp,
+    seed) sliced into consecutive ranges); `shard_index` / `shard_count` / `band_height` as for render (the outputs are
+    shard-compact).  `device`: outputs are CUDA tensors (and `offsets` may be one); else numpy arrays.  The first add()
+    after creation or reset() fixes the scene, camera and max_depth of the job; reset() returns to 0 samples."""
+
+    def __init__(self, job: Rendering, stream_spp: int = 0, shard_index: int = 0, shard_count: int = 1, band_height: int = 0,
+                 device: bool = False):
+        L = lib()
+        init()
+        self.job, self.device = job, bool(device)
+        self.shard_index, self.shard_count = shard_index, shard_count
+        self.band_height = band_height or L.rh_default_band_height(job.height, shard_count)
+        self.rows = L.rh_shard_rows(job.height, shard_count, self.band_height)
+        self._h = C.c_void_p()
+        check(L.rh_accum_create(job.width, job.height, shard_index, shard_count, self.band_height, int(stream_spp), C.byref(self._h)))
+        self._n = 0
+
+    @property
+    def samples(self) -> int:
+        """Samples per pixel in the running sums."""
+        return self._n
+
+    def add(self, spp: int, offsets=None, seed: int | None = None, rgb: bool = True, linear: bool = True,
+            want_hit_ids: bool = False, shadow: str | None = None, exact_boxes: bool = False, light_maps: bool = True,
+            chunk_samples: int = 0, profile: bool = False) -> Image:
+        """Traces `spp` new samples per pixel and returns the Image of all samples so far: `pixels` (RGB8, when `rgb`),
+        `linear` (float64, when `linear`), `hit_ids` of this call's samples [rows, width, spp, 2] (`want_hit_ids`) and
+        this call's stats.  `offsets`: this call's samples, full-frame [width*height, spp, 2] float64 / float32 (numpy, a
+        CPU tensor or, with device=True, a CUDA tensor; a strided view such as stream[:, n:n + spp] is copied to a dense array
+        first); `seed`: the next spp samples of the accumulator's SplitMix64
+        stream instead; neither: one sample at the pixel coordinate per spp.  `profile`: time every launch on its own
+        (stats ms_trace / ms_shadow / ms_resolve; slower)."""
+        if self._h is None or not self._h:
+            raise ValueError("the accumulator is closed")
+        L = lib()
+        job = self.job
+        mode, off = _offset_mode(offsets, 0)
+        off_ptr, seed_box = None, None
+        flags = ((capi.RH_FLAG_HIT_IDS if want_hit_ids else 0) | (capi.RH_FLAG_EXACT_BOXES if exact_boxes else 0)
+                 | _shadow_flag(shadow) | (0 if light_maps else capi.RH_FLAG_NO_LIGHT_MAPS)
+                 | (capi.RH_FLAG_DEVICE_OUT if self.device else 0) | (capi.RH_FLAG_PROFILE if profile else 0))
+        if seed is not None:
+            if offsets is not None:
+                raise ValueError("pass either offsets or seed")
+            seed_box = C.c_uint64(seed)
+            mode, off_ptr = capi.RH_OFFSETS_SPLITMIX64, C.addressof(seed_box)
+        elif off is not None:
+            have = off.numel() if hasattr(off, "numel") else off.size
+            if have != job.width * job.height * spp * 2:
+                raise ValueError(f"offsets has {have} values, expected {job.width * job.height * spp * 2}")
+            if getattr(off, "is_cuda", False):
+                if not self.device:
+                    raise ValueError("CUDA offsets need an accumulator with device=True")
+                flags |= capi.RH_FLAG_DEVICE_OFFSETS
+            # a slice of one stream, offsets[:, n:n + spp], is a strided view: the library reads a dense array
+            off = off.contiguous() if hasattr(off, "contiguous") else np.ascontiguousarray(off)
+            off_ptr = _ptr(off)
+        o = _opts(job, spp, mode, off_ptr, 0, self.shard_index, self.shard_count, self.band_height, chunk_samples, flags)
+        shapes = {"rgb": (self.rows, job.width, 3), "linear": (self.rows, job.width, 3), "ids": (self.rows, job.width, spp, 2)}
+        if self.device:
+            import torch
+
+            def empty(shape, dtype):
+                return torch.empty(shape, dtype=getattr(torch, dtype), device="cuda")
+
+            torch.cuda.current_stream().synchronize()  # the library runs on its own stream
+        else:
+            def empty(shape, dtype):
+                return np.empty(shape, dtype=dtype)
+        px = empty(shapes["rgb"], "uint8") if rgb else None
+        lin = empty(shapes["linear"], "float64") if linear else None
+        ids = empty(shapes["ids"], "int32") if want_hit_ids else None
+        st = capi.rh_stats()
+        check(L.rh_render_accumulate(job.scene.device, C.byref(job.camera), C.byref(o), self._h,
+                                     *(_ptr(a) if a is not None else None for a in (px, lin, ids)), C.byref(st)))
+        self._n += spp
+        return Image(job.width, self.rows, px, st.as_dict(), ids, lin)
+
+    def reset(self) -> None:
+        """Back to 0 samples; the next add() may use another scene, camera or max_depth."""
+        check(lib().rh_accum_reset(self._h))
+        self._n = 0
+
+    def close(self) -> None:
+        if getattr(self, "_h", None):
+            lib().rh_accum_destroy(self._h)
+        self._h = None
+
+    def __del__(self):
+        try:
+            self.close()
+        except Exception:
+            pass
+
+
+def progressiveRayTrace(job: Rendering, spp: int = 64, batch: int = 8, seed: int = 24):
+    """distributedRayTrace (RayHs.hs:190-195) refined over several calls: yields the RGB8 Image of the samples so far
+    after each batch of `batch` samples per pixel (the last batch holds what is left), drawn from the SplitMix64 stream
+    distributedRayTrace(job, spp, seed) uses, so the last image is that frame byte for byte."""
+    if spp < 1 or batch < 1:
+        raise ValueError(f"spp and batch must be at least 1, got {spp} and {batch}")
+    acc = Accumulator(job, stream_spp=spp)
+    try:
+        done = 0
+        while done < spp:
+            k = min(batch, spp - done)
+            img = acc.add(k, seed=seed, linear=False)
+            done += k
+            yield img
+    finally:
+        acc.close()
 
 
 def writePPM(path: str, image: Image) -> None:
