@@ -420,6 +420,58 @@ void rh_accum_destroy(rh_accum* acc);
 int rh_render_accumulate(const rh_scene* scene, const rh_camera* camera, const rh_render_opts* opts, rh_accum* acc,
                          uint8_t* rgb_out, double* linear_out, int32_t* hit_ids_out, rh_stats* stats);
 
+/* ---- adaptive sampling ---------------------------------------------- */
+/* Progressive rendering that traces new samples only for the pixels whose standard error is still above a threshold,
+ * each pixel continuing its own slice of the SplitMix64 stream.  State per pixel p of the shard's rows (shard-compact
+ * order, rows selected as for rh_accum_create), kept on the device between calls (52 bytes per pixel, plus 52 bytes
+ * per pixel of list and staging space):
+ *   n_p      samples so far;
+ *   S_p[c]   foldl (+) 0 of the sample colours in sample order (the sum rh_render_accumulate keeps);
+ *   Q_p[c]   foldl (+) 0 of x * x, each square rounded and then added, in sample order.
+ * stream_spp >= 1: samples per pixel of the stream (no pixel goes past it).  Needs rh_init (else RH_ERR_STATE). */
+typedef struct rh_adaptive rh_adaptive; /* opaque */
+typedef struct rh_adaptive_opts {
+  double threshold;   /* >= 0, linear colour units: bound on each channel's standard error of the mean */
+  uint32_t min_spp;   /* >= 2: pixels with fewer samples are always traced                            */
+  uint32_t reserved_; /* must be 0                                                                     */
+} rh_adaptive_opts;   /* 16 bytes */
+int rh_adaptive_create(int width, int height, int shard_index, int shard_count, int band_height, uint32_t stream_spp,
+                       rh_adaptive** out);
+/* All counts and sums back to 0; the next call may use another scene, camera or max_depth. */
+int rh_adaptive_reset(rh_adaptive* ad);
+void rh_adaptive_destroy(rh_adaptive* ad); /* NULL is a no-op */
+/* One round of adaptive sampling.  opts->offset_mode must be RH_OFFSETS_SPLITMIX64 (opts->offsets: the seed); sample s of
+ * this call for pixel p draws values 2g and 2g + 1 with g = pixel * stream_spp + n_p + s (pixel: full-image index), the
+ * index rh_render_accumulate uses with the pixel's own count in place of N.  So a pixel that ends with n samples holds
+ * exactly the sums, and gives exactly the bytes, of an n-sample rh_render_accumulate (or rh_render) of that stream.
+ * Selection, on the state before the call, in this operation order (IEEE double, no fused multiply-add):
+ *   tt = threshold * threshold;  nn = (double)n * (double)(n - 1);  d_c = Q_c - S_c * (S_c / n)
+ *   p is active  iff  n + spp <= stream_spp  and  (n < min_spp  or  d_c > tt * nn for some channel c).
+ * (A NaN d_c does not keep a pixel active; a negative d_c from cancellation counts as converged.)  Each active pixel gets
+ * opts->spp new samples; the others are not traced and keep their state.  *n_active_out (optional): active pixels.  A
+ * call with no active pixel traces nothing, returns RH_OK and still writes the outputs, which cover every pixel of the
+ * shard's rows, shard-compact:
+ *   rgb_out    RGB8 = toIntC((1/n_p) S_p), clamped as rh_render clamps it (0 for a pixel with no sample yet);
+ *   linear_out double[rows][width][3] = (1/n_p) S_p (0 for a pixel with no sample yet).
+ * Either may be NULL.  RH_FLAG_DEVICE_OUT applies to both (linear_out 8-byte aligned).  RH_FLAG_HIT_IDS,
+ * RH_FLAG_PEER_FRAMES, RH_FLAG_SHARD_OFFSETS and RH_FLAG_DEVICE_OFFSETS are RH_ERR_ARG; RH_FLAG_EXACT_BOXES,
+ * RH_FLAG_NO_LIGHT_MAPS, the shadow-schedule flags, RH_FLAG_COUNT, RH_FLAG_PROFILE and chunk_samples behave as in
+ * rh_render (chunk_samples counts the samples of the active pixels).  threshold and min_spp may change from call to
+ * call.  The first call after create or reset records the scene, the camera bytes and max_depth; a later call with
+ * others is RH_ERR_ARG (reset first).  opts must match the state's size and shard.  A call that fails (argument, CUDA
+ * or RH_ERR_OVERFLOW) leaves every n_p, S_p and Q_p unchanged; a queue-overflow retry inside the call counts no sample
+ * twice.  The call uses the scene's decided shadow schedule and queue factor (else the pooled schedule and factor 2)
+ * and changes neither them nor the row costs, as rh_trace_rays does.  stats: rays_primary = n_active * spp, the other
+ * ray counts this call's; chunks, queue_factor, shadow_split and ms_total (the whole call) as in rh_render;
+ * negative_channels counts the RGB8 output; RH_FLAG_PROFILE: ms_resolve also holds the selection, commit and output
+ * kernels. */
+int rh_render_adaptive(const rh_scene* scene, const rh_camera* camera, const rh_render_opts* opts,
+                       const rh_adaptive_opts* aopts, rh_adaptive* ad, uint8_t* rgb_out, double* linear_out,
+                       uint64_t* n_active_out, rh_stats* stats);
+/* Copies the state out: counts_out uint32[rows][width] = n_p, sums_out / sumsq_out double[rows][width][3] = S_p / Q_p.
+ * Any pointer may be NULL.  flags: 0 (host buffers) or RH_FLAG_DEVICE_OUT (device buffers, the doubles 8-byte aligned). */
+int rh_adaptive_state(const rh_adaptive* ad, uint32_t* counts_out, double* sums_out, double* sumsq_out, int32_t flags);
+
 /* Rows owned by one shard (equal for all shards: bands are padded). */
 int rh_shard_rows(int height, int shard_count, int band_height);
 int rh_default_band_height(int height, int shard_count);

@@ -123,10 +123,14 @@ class rh_trace_opts(C.Structure):
     _fields_ = [("max_depth", C.c_int32), ("flags", C.c_int32), ("chunk_rays", C.c_uint32), ("reserved_", C.c_uint32)]
 
 
+class rh_adaptive_opts(C.Structure):
+    _fields_ = [("threshold", C.c_double), ("min_spp", C.c_uint32), ("reserved_", C.c_uint32)]
+
+
 # struct sizes the header promises (checked by tests/test_abi.py against the compiled library too)
 assert C.sizeof(rh_material) == 96 and C.sizeof(rh_light) == 64 and C.sizeof(rh_node) == 64
 assert C.sizeof(rh_tri) == 80 and C.sizeof(rh_tri_shade) == 128 and C.sizeof(rh_object) == 96
-assert C.sizeof(rh_hit) == 80 and C.sizeof(rh_trace_opts) == 16
+assert C.sizeof(rh_hit) == 80 and C.sizeof(rh_trace_opts) == 16 and C.sizeof(rh_adaptive_opts) == 16
 
 vp = C.c_void_p
 
@@ -150,6 +154,12 @@ SIGNATURES = {
     "rh_accum_reset": (C.c_int, [vp]),
     "rh_accum_destroy": (None, [vp]),
     "rh_render_accumulate": (C.c_int, [vp, C.POINTER(rh_camera), C.POINTER(rh_render_opts), vp, vp, vp, vp, C.POINTER(rh_stats)]),
+    "rh_adaptive_create": (C.c_int, [C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.c_uint32, C.POINTER(vp)]),
+    "rh_adaptive_reset": (C.c_int, [vp]),
+    "rh_adaptive_destroy": (None, [vp]),
+    "rh_render_adaptive": (C.c_int, [vp, C.POINTER(rh_camera), C.POINTER(rh_render_opts), C.POINTER(rh_adaptive_opts), vp, vp, vp,
+                                     C.POINTER(C.c_uint64), C.POINTER(rh_stats)]),
+    "rh_adaptive_state": (C.c_int, [vp, vp, vp, vp, C.c_int32]),
     "rh_shard_rows": (C.c_int, [C.c_int, C.c_int, C.c_int]),
     "rh_default_band_height": (C.c_int, [C.c_int, C.c_int]),
     "rh_deinterleave_bands": (C.c_int, [vp, vp, C.c_int, C.c_int, C.c_int, C.c_int]),

@@ -229,6 +229,15 @@ enum { kOffIndexLocal = 0, kOffIndexGlobal = 1 };
 // double[6] = origin, direction, at `offsets` (ray of item i: offset_base + i), instead of camera rays.
 constexpr int kOffsetsRays = 16;
 
+// rh_render_adaptive's pass-0 source: P.spp samples of each entry of a list of the shard's pixels.  The frame's rows
+// are rows of the list (P.width entries each; P.ray_items pass-0 items of the chunk are real, the rest of its last row is
+// padding), so P's geometry is the list's; the image's is here.
+struct PixelList {
+  const uint32_t* pixels;  // shard-compact pixel index of each entry, ascending; null: not a list frame
+  const uint32_t* counts;  // n_p: pixel p's samples continue the stream at pixel * stream_spp + counts[p]
+  uint32_t width, height, shard_index, shard_count, band_height;  // the image and the shard's bands
+};
+
 struct ChunkParams {
   uint32_t first_row;     // first local (shard-compact) row of the chunk
   uint32_t n_rows;        // rows in the chunk
@@ -263,6 +272,7 @@ struct ChunkParams {
   FrameCounters* counters;
   RayQueue q_in, q_out;
   ShadowQueue q_hits, q_shadow;
+  PixelList list;         // rh_render_adaptive (after the render's fields: their offsets stay as they were)
 };
 
 // rh_render_accumulate's end of a chunk instead of the resolve: the running per-pixel sums of the accumulator.
@@ -273,6 +283,26 @@ struct AccumParams {
   size_t plane;
   uint32_t n_before;     // samples in sum_in
   uint32_t n_total;      // n_before + spp
+};
+
+// rh_render_adaptive's state and the buffers of one call: the selection, the sink of the list frame, the commit and the
+// output.  State and output are in shard-compact pixel order; the list and the staging are indexed by list entry.
+struct AdaptiveParams {
+  uint32_t* counts;        // n_p, one plane
+  double* sum;             // S: 3 planes (r, g, b) of `plane` doubles
+  double* sumsq;           // Q: the same layout
+  uint32_t* list;          // active pixels, ascending (select writes it)
+  double* stage;           // 6 planes of `plane` doubles by entry: new S (r, g, b), new Q (r, g, b) (sink writes, commit reads)
+  uint32_t* warp_masks;    // select: bit i of word w = pixel 32 w + i is active
+  uint32_t* block_counts;  // select: active pixels per block, then their exclusive prefix
+  uint32_t* n_active;      // select: the total
+  unsigned long long* negative;  // output: pixels with a negative channel (RGB8 only)
+  uint8_t* rgb;            // output, or null
+  double* linear;          // output, or null
+  size_t plane;            // pixels of the shard's rows: rows * width
+  uint32_t width, height, shard_index, shard_count, band_height;  // the image and the shard's bands
+  uint32_t spp, stream_spp, min_spp;
+  double tt;               // threshold * threshold
 };
 
 // One launch of the batched ray queries (rh_closest_intersection / rh_shadow_intersection) over rays [0, n).
@@ -289,7 +319,7 @@ struct QueryParams {
 };
 
 // Launchers (kernels.cu).  `count` selects the instrumented instantiation (box/tri counters); launch_trace runs the
-// uninstrumented ray instantiation for P.offset_mode == kOffsetsRays.
+// uninstrumented ray instantiation for P.offset_mode == kOffsetsRays and the pixel-list one when P.list.pixels is set.
 // (followed by a one-thread kernel that closes the pass's range of the hit queue, ChunkCtl::hit_start)
 void launch_trace(const SceneView& S, const CameraParams& cam, const ChunkParams& P, bool count, int grid, void* stream);
 // classify_kernel, then the walks of the hits it queued — refill: the per-lane-refill kernel (incoherent rays) instead of
@@ -302,6 +332,17 @@ void launch_store_colors(const ChunkParams& P, double* colors, void* stream);
 // rh_render_accumulate's end of a chunk instead of the resolve: adds the chunk's samples to the running sums and writes
 // RGB8 (P.rgb, may be null) and the linear colours (A.linear, may be null) of the new sums
 void launch_accumulate_resolve(const ChunkParams& P, const AccumParams& A, void* stream);
+// rh_render_adaptive: the selection (evaluates the rule per pixel, writes the active pixels to A.list in pixel order
+// and their number to A.n_active); the sink of a list frame's chunk (the entries' new S and Q to A.stage); the commit of
+// a completed frame (A.stage into the state, n_p += spp for the first n_active entries); the output (RGB8 and linear
+// colours of every pixel, either optional)
+void launch_adaptive_select(const AdaptiveParams& A, void* stream);
+void launch_adaptive_fold(const ChunkParams& P, const AdaptiveParams& A, void* stream);
+void launch_adaptive_commit(const AdaptiveParams& A, uint32_t n_active, void* stream);
+void launch_adaptive_output(const AdaptiveParams& A, void* stream);
+// rh_adaptive_state: three planes of `plane` doubles to double[plane][3]
+void launch_adaptive_interleave(const double* planes, size_t plane, double* out, void* stream);
+constexpr int kSelectBlock = 256;  // pixels per block of the selection
 // query_closest_kernel / query_shadow_kernel: `grid` blocks of one SM each
 void launch_query_closest(const SceneView& S, const QueryParams& Q, int grid, void* stream);
 void launch_query_shadow(const SceneView& S, const QueryParams& Q, int grid, void* stream);

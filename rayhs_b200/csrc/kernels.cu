@@ -10,8 +10,10 @@
 //                         takes its next light or the next hit while its neighbours keep walking.
 //   shadow_simple_kernel  K3 for scenes with more than 32 lights.
 //   resolve_kernel        K6: average the samples of a pixel, toIntC, coalesced RGB8 store (or peer stores).
-//   store_colors_kernel   K6 of rh_trace_rays: the linear colours of caller-built rays (trace_kernel<.., RAYS = true>).
+//   store_colors_kernel   K6 of rh_trace_rays: the linear colours of caller-built rays (trace_kernel<.., Source::kRays>).
 //   accumulate_resolve_kernel  K6 of rh_render_accumulate: running per-pixel sums across calls, RGB8 and linear colours.
+//   adaptive_*            rh_render_adaptive: selection and compaction of the pixels still above the threshold, the
+//                         sink of their samples (trace_kernel<.., Source::kPixelList>), commit, RGB8 and linear output.
 //   deinterleave          K7: band re-assembly after the all-gather.
 //
 // All arithmetic is IEEE double in the reference's operation order and this file is compiled with -fmad=false (GHC
@@ -1486,18 +1488,42 @@ __device__ __forceinline__ bool stage_start(const ChunkParams& P, bool primary, 
 // Work item -> ray: the camera ray of a pixel sample (pass 0: pixelCoord, Image.hs:31-32, + sample offset,
 // RayHs.hs:178-181) or a queued secondary ray with its weight and tags.  False for a padding row of the last band.
 // `tile`: the item's batch was staged in shared memory (see stage_start), else it is read from global memory.
-// RAYS (rh_trace_rays, P.offset_mode == kOffsetsRays): pass 0 reads caller-built rays instead; false past the chunk's rays.
-template <bool RAYS>
+// What pass 0's work items are: camera samples of the chunk's image rows (rh_render), caller-built rays (kRays:
+// rh_trace_rays, P.offset_mode == kOffsetsRays) or samples of the entries of a pixel list (kPixelList:
+// rh_render_adaptive, P.list).  The last two are false past the chunk's items (P.ray_items).
+enum class Source { kCamera, kRays, kPixelList };
+
+// Image row of a shard-compact row of the list's image (global_row with the PixelList's bands).
+__device__ __forceinline__ uint32_t list_image_row(const PixelList& L, uint32_t local_row) {
+  const uint32_t lb = local_row / L.band_height, rib = local_row % L.band_height;
+  return (lb * L.shard_count + L.shard_index) * L.band_height + rib;
+}
+
+template <Source SRC>
 __device__ __forceinline__ bool load_item(const ChunkParams& P, const CameraParams& cam, uint32_t item, bool primary,
                                           const StageTile* tile, uint32_t lane, Ray& r, double& w, uint32_t& sample, int& depth,
                                           int& kind, uint32_t& probe_mat) {
   r.o = r.d = mk(0, 0, 1);
-  if (RAYS && primary) {
+  if (SRC == Source::kRays && primary) {
     if (item >= P.ray_items) return false;
     const double2* src = (const double2*)P.offsets + 3 * (P.offset_base + item);
     const double2 a = __ldg(src), b = __ldg(src + 1), c = __ldg(src + 2);
     r.o = mk(a.x, a.y, b.x);
     r.d = mk(b.y, c.x, c.y);
+    return true;
+  }
+  if (SRC == Source::kPixelList && primary) {
+    // sample s of list entry e: the pixel's stream continues after its n_p samples (RH_OFFSETS_SPLITMIX64 only)
+    if (item >= P.ray_items) return false;
+    const PixelList& L = P.list;
+    const uint32_t le = item / P.spp, s = item - le * P.spp;
+    const uint32_t p = __ldg(L.pixels + (size_t)P.first_row * P.width + le);
+    const uint32_t lrow = p / L.width, col = p - lrow * L.width;
+    const uint32_t grow = list_image_row(L, lrow);
+    const unsigned long long g = ((unsigned long long)grow * L.width + col) * P.stream_spp + __ldg(L.counts + p) + s;
+    const double ox = splitmix01(P.offset_seed, 2 * g) - 0.5;
+    const double oy = splitmix01(P.offset_seed, 2 * g + 1) - 0.5;
+    r = camera_ray(cam, (double)col + ox, (double)grow + oy);
     return true;
   }
   if (primary) {
@@ -1560,8 +1586,8 @@ static_assert(sizeof(SmemTables) % 128 == 0 || !RH_TMA_STAGE, "staging tiles nee
 static_assert(((size_t)kShortStack * kTraceBlock * sizeof(uint2)) % 128 == 0, "stack columns keep the alignment");
 static_assert(kTraceSmem <= 227 * 1024, "trace kernel shared memory");
 
-// RAYS: rh_trace_rays' instantiation (caller-built rays in pass 0, see load_item); the render's is RAYS = false.
-template <bool COUNT, bool RAYS>
+// SRC: what pass 0 traces (see load_item); the render's instantiations are Source::kCamera.
+template <bool COUNT, Source SRC>
 __global__ void __launch_bounds__(kTraceBlock, kTracePerSm) trace_kernel(const __grid_constant__ SceneView S,
                                                                const __grid_constant__ CameraParams cam,
                                                                const __grid_constant__ ChunkParams P) {
@@ -1620,7 +1646,7 @@ __global__ void __launch_bounds__(kTraceBlock, kTracePerSm) trace_kernel(const _
         tile = &wsm.tile;
       }
 #endif
-      if (valid) valid = load_item<RAYS>(P, cam, item, primary, tile, lane, r, w, sample, depth, kind, probe_mat);
+      if (valid) valid = load_item<SRC>(P, cam, item, primary, tile, lane, r, w, sample, depth, kind, probe_mat);
       else r.o = r.d = mk(0, 0, 1);
 #if RH_TMA_STAGE
       // the tile is in registers now: ask for the next batch of this claim (same slab); it lands while this one is traced
@@ -2626,6 +2652,207 @@ __global__ void __launch_bounds__(kBlock) accumulate_resolve_kernel(const __grid
   }
 }
 
+// ------------------------------------------------------------------ rh_render_adaptive
+// Selection rule (include/rayhs_b200.h, in its operation order): pixel p of the shard's rows is active when the stream
+// has spp more samples for it and it has fewer than min_spp samples or some channel's n(n-1) x variance of the mean,
+// d_c = Q_c - S_c (S_c / n), is above tt n (n - 1).  Padding rows of the last band are never active.
+__device__ __forceinline__ bool adaptive_active(const AdaptiveParams& A, uint32_t p) {
+  const uint32_t lrow = p / A.width;
+  const uint32_t lb = lrow / A.band_height, rib = lrow % A.band_height;
+  if ((lb * A.shard_count + A.shard_index) * A.band_height + rib >= A.height) return false;
+  const uint32_t n = A.counts[p];
+  if ((unsigned long long)n + A.spp > A.stream_spp) return false;
+  if (n < A.min_spp) return true;
+  const double dn = (double)n;
+  const double lim = A.tt * (dn * (double)(n - 1));
+  bool active = false;
+  for (int c = 0; c < 3; c++) {
+    const double S = A.sum[(size_t)c * A.plane + p], Q = A.sumsq[(size_t)c * A.plane + p];
+    const double d = Q - S * (S / dn);
+    active |= d > lim;  // (false for NaN)
+  }
+  return active;
+}
+
+// Selection, step 1 of 3: the rule per pixel; one ballot word per warp and the block's count of active pixels.  The seven
+// state planes are read at the pixel index, so the loads coalesce.
+__global__ void __launch_bounds__(kSelectBlock) adaptive_select_kernel(const __grid_constant__ AdaptiveParams A) {
+  __shared__ uint32_t warp_n[kSelectBlock / 32];
+  const uint32_t p = blockIdx.x * kSelectBlock + threadIdx.x;
+  const bool act = p < A.plane && adaptive_active(A, p);
+  const unsigned m = __ballot_sync(kFull, act);
+  const uint32_t warp = threadIdx.x >> 5;
+  if ((threadIdx.x & 31) == 0) {
+    A.warp_masks[(size_t)blockIdx.x * (kSelectBlock / 32) + warp] = m;
+    warp_n[warp] = __popc(m);
+  }
+  __syncthreads();
+  if (threadIdx.x == 0) {
+    uint32_t t = 0;
+    for (int w = 0; w < kSelectBlock / 32; w++) t += warp_n[w];
+    A.block_counts[blockIdx.x] = t;
+  }
+}
+
+// Step 2: one block turns the block counts into their exclusive prefix (each thread a run of blocks, then a scan of the
+// runs' totals in shared memory) and writes the total to n_active.
+constexpr int kScanThreads = 1024;
+__global__ void __launch_bounds__(kScanThreads) adaptive_scan_kernel(const __grid_constant__ AdaptiveParams A, uint32_t n_blocks) {
+  __shared__ uint32_t part[kScanThreads];
+  const uint32_t per = (n_blocks + kScanThreads - 1) / kScanThreads;
+  const uint32_t b0 = min(threadIdx.x * per, n_blocks), b1 = min(b0 + per, n_blocks);
+  uint32_t sum = 0;
+  for (uint32_t b = b0; b < b1; b++) sum += A.block_counts[b];
+  part[threadIdx.x] = sum;
+  __syncthreads();
+  for (uint32_t off = 1; off < kScanThreads; off <<= 1) {  // inclusive scan
+    const uint32_t v = threadIdx.x >= off ? part[threadIdx.x - off] : 0u;
+    __syncthreads();
+    part[threadIdx.x] += v;
+    __syncthreads();
+  }
+  uint32_t run = part[threadIdx.x] - sum;
+  for (uint32_t b = b0; b < b1; b++) {
+    const uint32_t c = A.block_counts[b];
+    A.block_counts[b] = run;
+    run += c;
+  }
+  if (threadIdx.x == kScanThreads - 1) *A.n_active = part[kScanThreads - 1];
+}
+
+// Step 3: each active pixel goes to list[block prefix + active warps before it in the block + active lanes before it in
+// the warp], so the list is in pixel order.
+__global__ void __launch_bounds__(kSelectBlock) adaptive_compact_kernel(const __grid_constant__ AdaptiveParams A) {
+  __shared__ uint32_t warp_base[kSelectBlock / 32];
+  const uint32_t* masks = A.warp_masks + (size_t)blockIdx.x * (kSelectBlock / 32);
+  if (threadIdx.x == 0) {
+    uint32_t run = A.block_counts[blockIdx.x];
+    for (int w = 0; w < kSelectBlock / 32; w++) {
+      warp_base[w] = run;
+      run += __popc(masks[w]);
+    }
+  }
+  __syncthreads();
+  const uint32_t warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+  const uint32_t m = masks[warp];
+  if ((m >> lane) & 1u) A.list[warp_base[warp] + __popc(m & ((1u << lane) - 1u))] = blockIdx.x * kSelectBlock + threadIdx.x;
+}
+
+// The sink of a list frame's chunk: entry e's spp samples continue its pixel's S and Q in sample order (S with
+// accumulate_resolve_kernel's loads and association, so it is bit for bit the progressive sum; Q adds each rounded
+// square).  The results go to the staging planes at e: the state is read, never written, so a retried frame reads it
+// unchanged.
+__global__ void __launch_bounds__(kBlock) adaptive_fold_kernel(const __grid_constant__ ChunkParams P,
+                                                               const __grid_constant__ AdaptiveParams A) {
+  const uint32_t le = blockIdx.x * kBlock + threadIdx.x;
+  if (le >= P.ray_items / P.spp) return;  // (padding entries of the list's last row)
+  const size_t e = (size_t)P.first_row * P.width + le;
+  const uint32_t p = A.list[e];
+  const size_t pl = A.plane;
+  double sr = A.sum[p], sg = A.sum[pl + p], sb = A.sum[2 * pl + p];
+  double qr = A.sumsq[p], qg = A.sumsq[pl + p], qb = A.sumsq[2 * pl + p];
+  const double* a = P.accum + (size_t)le * P.spp;
+  if ((P.spp & 1u) == 0 && (P.accum_stride & 1u) == 0) {
+    const double2* a0 = (const double2*)a;
+    const double2* a1 = (const double2*)(a + P.accum_stride);
+    const double2* a2 = (const double2*)(a + 2 * (size_t)P.accum_stride);
+    for (uint32_t s = 0; s < P.spp / 2; s++) {
+      const double2 r2 = a0[s], g2 = a1[s], b2 = a2[s];
+      sr = (sr + r2.x) + r2.y;
+      sg = (sg + g2.x) + g2.y;
+      sb = (sb + b2.x) + b2.y;
+      qr = (qr + r2.x * r2.x) + r2.y * r2.y;
+      qg = (qg + g2.x * g2.x) + g2.y * g2.y;
+      qb = (qb + b2.x * b2.x) + b2.y * b2.y;
+    }
+  } else {
+    for (uint32_t s = 0; s < P.spp; s++) {
+      const double r = a[s], g = a[P.accum_stride + s], b = a[2 * (size_t)P.accum_stride + s];
+      sr = sr + r;
+      sg = sg + g;
+      sb = sb + b;
+      qr = qr + r * r;
+      qg = qg + g * g;
+      qb = qb + b * b;
+    }
+  }
+  A.stage[e] = sr;
+  A.stage[pl + e] = sg;
+  A.stage[2 * pl + e] = sb;
+  A.stage[3 * pl + e] = qr;
+  A.stage[4 * pl + e] = qg;
+  A.stage[5 * pl + e] = qb;
+}
+
+// After a frame without overflow: the staged sums become the state of their pixels, which have spp more samples.
+__global__ void __launch_bounds__(kBlock) adaptive_commit_kernel(const __grid_constant__ AdaptiveParams A, uint32_t n_active) {
+  const uint32_t e = blockIdx.x * kBlock + threadIdx.x;
+  if (e >= n_active) return;
+  const uint32_t p = A.list[e];
+  const size_t pl = A.plane;
+  for (int c = 0; c < 3; c++) {
+    A.sum[c * pl + p] = A.stage[c * pl + e];
+    A.sumsq[c * pl + p] = A.stage[(3 + c) * pl + e];
+  }
+  A.counts[p] += A.spp;
+}
+
+// Every pixel's image, toIntC((1/n) S) as RGB8 and (1/n) S as linear double[3], both stores coalesced through shared
+// memory as in accumulate_resolve_kernel.  A pixel without samples (padding rows included) is 0.
+__global__ void __launch_bounds__(kBlock) adaptive_output_kernel(const __grid_constant__ AdaptiveParams A) {
+  __shared__ __align__(16) double lin[kBlock * 3];
+  __shared__ __align__(16) uint8_t bytes[kBlock * 3];
+  const uint32_t lp = blockIdx.x * kBlock + threadIdx.x;
+  bool negative = false;
+  if (lp < A.plane) {
+    double cr = 0, cg = 0, cb = 0;
+    const uint32_t n = A.counts[lp];
+    if (n) {
+      const double inv = 1.0 / (double)n;
+      cr = inv * A.sum[lp];
+      cg = inv * A.sum[A.plane + lp];
+      cb = inv * A.sum[2 * A.plane + lp];
+    }
+    bool neg = false;
+    bytes[3 * threadIdx.x] = (uint8_t)to_int_c(cr, neg);
+    bytes[3 * threadIdx.x + 1] = (uint8_t)to_int_c(cg, neg);
+    bytes[3 * threadIdx.x + 2] = (uint8_t)to_int_c(cb, neg);
+    negative = neg && A.rgb;
+    lin[3 * threadIdx.x] = cr;
+    lin[3 * threadIdx.x + 1] = cg;
+    lin[3 * threadIdx.x + 2] = cb;
+  }
+  const unsigned neg = __ballot_sync(kFull, negative);
+  if ((threadIdx.x & 31) == 0 && neg) atomicAdd(A.negative, (unsigned long long)__popc(neg));
+  __syncthreads();
+  const uint32_t n_here = min((uint32_t)kBlock, (uint32_t)A.plane - blockIdx.x * kBlock) * 3;
+  const size_t first = (size_t)blockIdx.x * kBlock;
+  if (A.rgb) {
+    uint8_t* dst = A.rgb + first * 3;
+    if ((((uintptr_t)dst) & 3) == 0) {
+      const uint32_t words = n_here / 4;
+      if (threadIdx.x < words) ((uint32_t*)dst)[threadIdx.x] = ((const uint32_t*)bytes)[threadIdx.x];
+      const uint32_t tail = words * 4 + threadIdx.x;
+      if (tail < n_here) dst[tail] = bytes[tail];
+    } else {
+      for (uint32_t i = threadIdx.x; i < n_here; i += kBlock) dst[i] = bytes[i];
+    }
+  }
+  if (A.linear) {
+    double* dst = A.linear + first * 3;
+    for (uint32_t i = threadIdx.x; i < n_here; i += kBlock) dst[i] = lin[i];
+  }
+}
+
+// rh_adaptive_state: the planes of S or Q to double[pixel][3]; the stores coalesce, the loads are three streams.
+__global__ void __launch_bounds__(kBlock) adaptive_interleave_kernel(const double* __restrict__ planes, size_t plane,
+                                                                     double* __restrict__ out) {
+  const size_t i = (size_t)blockIdx.x * kBlock + threadIdx.x;
+  if (i >= 3 * plane) return;
+  const size_t p = i / 3;
+  out[i] = planes[(i - 3 * p) * plane + p];
+}
+
 // ------------------------------------------------------------------ K7: band de-interleave after the all-gather
 __global__ void deinterleave_kernel(const uint8_t* __restrict__ gathered, uint8_t* __restrict__ out, uint32_t row_bytes,
                                     uint32_t height, uint32_t shard_count, uint32_t band_height, uint32_t rows_per_shard) {
@@ -2707,9 +2934,11 @@ int configure_kernels() {
   auto set = [&](const void* fn, size_t bytes) {
     if (e == cudaSuccess) e = cudaFuncSetAttribute(fn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bytes);
   };
-  set((const void*)trace_kernel<true, false>, kTraceSmem);
-  set((const void*)trace_kernel<false, false>, kTraceSmem);
-  set((const void*)trace_kernel<false, true>, kTraceSmem);
+  set((const void*)trace_kernel<true, Source::kCamera>, kTraceSmem);
+  set((const void*)trace_kernel<false, Source::kCamera>, kTraceSmem);
+  set((const void*)trace_kernel<false, Source::kRays>, kTraceSmem);
+  set((const void*)trace_kernel<true, Source::kPixelList>, kTraceSmem);
+  set((const void*)trace_kernel<false, Source::kPixelList>, kTraceSmem);
   set((const void*)shadow_pooled_kernel<true>, kShadowSmem);
   set((const void*)shadow_pooled_kernel<false>, kShadowSmem);
   set((const void*)shadow_refill_kernel<true>, kWalkSmem);
@@ -2741,9 +2970,11 @@ int max_threads_per_launch(int n_sms) {
 }
 void launch_trace(const SceneView& S, const CameraParams& cam, const ChunkParams& P, bool count, int grid, void* stream) {
   cudaStream_t st = (cudaStream_t)stream;
-  if (P.offset_mode == kOffsetsRays) trace_kernel<false, true><<<grid * kTracePerSm, kTraceBlock, kTraceSmem, st>>>(S, cam, P);
-  else if (count) trace_kernel<true, false><<<grid * kTracePerSm, kTraceBlock, kTraceSmem, st>>>(S, cam, P);
-  else trace_kernel<false, false><<<grid * kTracePerSm, kTraceBlock, kTraceSmem, st>>>(S, cam, P);
+  if (P.offset_mode == kOffsetsRays) trace_kernel<false, Source::kRays><<<grid * kTracePerSm, kTraceBlock, kTraceSmem, st>>>(S, cam, P);
+  else if (P.list.pixels && count) trace_kernel<true, Source::kPixelList><<<grid * kTracePerSm, kTraceBlock, kTraceSmem, st>>>(S, cam, P);
+  else if (P.list.pixels) trace_kernel<false, Source::kPixelList><<<grid * kTracePerSm, kTraceBlock, kTraceSmem, st>>>(S, cam, P);
+  else if (count) trace_kernel<true, Source::kCamera><<<grid * kTracePerSm, kTraceBlock, kTraceSmem, st>>>(S, cam, P);
+  else trace_kernel<false, Source::kCamera><<<grid * kTracePerSm, kTraceBlock, kTraceSmem, st>>>(S, cam, P);
   close_hit_range_kernel<<<1, 1, 0, st>>>(P.ctl, P.pass);
 }
 int launch_shadow(const SceneView& S, const ChunkParams& P, bool count, bool refill, int grid, void* stream, void* classified) {
@@ -2782,6 +3013,26 @@ void launch_store_colors(const ChunkParams& P, double* colors, void* stream) {
 void launch_accumulate_resolve(const ChunkParams& P, const AccumParams& A, void* stream) {
   const uint32_t n_pixels = P.n_rows * P.width;
   accumulate_resolve_kernel<<<(n_pixels + kBlock - 1) / kBlock, kBlock, 0, (cudaStream_t)stream>>>(P, A);
+}
+void launch_adaptive_select(const AdaptiveParams& A, void* stream) {
+  const cudaStream_t st = (cudaStream_t)stream;
+  const uint32_t n_blocks = (uint32_t)((A.plane + kSelectBlock - 1) / kSelectBlock);
+  adaptive_select_kernel<<<n_blocks, kSelectBlock, 0, st>>>(A);
+  adaptive_scan_kernel<<<1, kScanThreads, 0, st>>>(A, n_blocks);
+  adaptive_compact_kernel<<<n_blocks, kSelectBlock, 0, st>>>(A);
+}
+void launch_adaptive_fold(const ChunkParams& P, const AdaptiveParams& A, void* stream) {
+  const uint32_t n_entries = P.ray_items / P.spp;
+  adaptive_fold_kernel<<<(n_entries + kBlock - 1) / kBlock, kBlock, 0, (cudaStream_t)stream>>>(P, A);
+}
+void launch_adaptive_commit(const AdaptiveParams& A, uint32_t n_active, void* stream) {
+  if (n_active) adaptive_commit_kernel<<<(n_active + kBlock - 1) / kBlock, kBlock, 0, (cudaStream_t)stream>>>(A, n_active);
+}
+void launch_adaptive_output(const AdaptiveParams& A, void* stream) {
+  adaptive_output_kernel<<<(uint32_t)((A.plane + kBlock - 1) / kBlock), kBlock, 0, (cudaStream_t)stream>>>(A);
+}
+void launch_adaptive_interleave(const double* planes, size_t plane, double* out, void* stream) {
+  if (plane) adaptive_interleave_kernel<<<(uint32_t)((3 * plane + kBlock - 1) / kBlock), kBlock, 0, (cudaStream_t)stream>>>(planes, plane, out);
 }
 void launch_query_closest(const SceneView& S, const QueryParams& Q, int grid, void* stream) {
   query_closest_kernel<<<grid, kQueryBlock, kQuerySmem, (cudaStream_t)stream>>>(S, Q);

@@ -205,23 +205,41 @@ struct rh_scene {
   mutable bool stream_compute_bound = false;  // ... and in that frame the kernels, not the upload, finished last
 };
 
-// Running per-pixel sums of one progressive frame (or of one shard's rows of it): two buffers of three planes of doubles,
-// `cur` holding the sums of the n samples so far.  A call's sink reads buffer cur and writes the other; the call flips
-// them and adds its samples to n only after a frame that completed, so a failed call or an overflow retry leaves the
-// sums as they were.  The first call after create or reset fixes the view (scene, camera, max_depth).
-struct rh_accum {
+// What the per-pixel states of several calls (rh_accum, rh_adaptive) share: the frame (or shard of it) they cover, the
+// device context they live on, the SplitMix64 stream they draw from and the view their first call fixed.
+struct ShardState {
   Device* device = nullptr;
-  uint64_t context = 0;  // device->context when the accumulator was created
+  uint64_t context = 0;  // device->context when the state was created
   int dev = -1;
   int width = 0, height = 0, shard_index = 0, shard_count = 1, band_height = 1, rows_local = 0;
   uint32_t stream_spp = 0;  // RH_OFFSETS_SPLITMIX64: samples per pixel of the stream the calls draw from
   size_t plane = 0;         // doubles per colour plane: rows_local * width
-  DevBuf sums;              // [2][3][plane]
-  int cur = 0;
-  uint32_t n = 0;
   const rh_scene* scene = nullptr;
   rh_camera camera{};
   int32_t max_depth = 0;
+};
+
+// Running per-pixel sums of one progressive frame (or of one shard's rows of it): two buffers of three planes of doubles,
+// `cur` holding the sums of the n samples so far.  A call's sink reads buffer cur and writes the other; the call flips
+// them and adds its samples to n only after a frame that completed, so a failed call or an overflow retry leaves the
+// sums as they were.  The first call after create or reset fixes the view (scene, camera, max_depth).
+struct rh_accum : ShardState {
+  DevBuf sums;              // [2][3][plane]
+  int cur = 0;
+  uint32_t n = 0;
+};
+
+// Adaptive sampling state of one frame (or shard): per pixel the count n_p and the sums S_p and Q_p (state), and the
+// per-call space: the list of active pixels and the staged new sums of its entries (work), the selection's scratch.
+// A call's sink writes only the staging; the commit moves it into the state after a frame that completed, so a failed
+// call or an overflow retry leaves the state as it was.  The first call after create or reset fixes the view.
+struct rh_adaptive : ShardState {
+  DevBuf state;    // counts uint32[plane] (padded to 8 bytes), S double[3][plane], Q double[3][plane]
+  DevBuf work;     // list uint32[plane] (padded to 8 bytes), staging double[6][plane]
+  DevBuf scratch;  // negative-channel counter, n_active, block counts, warp masks
+  AdaptiveParams A{};  // the pointers into the three buffers and the geometry
+  bool fixed = false;  // the view is fixed
+  cudaEvent_t ev[4] = {nullptr, nullptr, nullptr, nullptr};  // call begin, selection end, commit begin, call end
 };
 
 namespace {
@@ -1352,6 +1370,12 @@ struct Frame {
   uint64_t n_rays = 0;
   // RH_OFFSETS_SPLITMIX64: the stream's samples per pixel and the first of them this frame traces
   uint32_t stream_spp = 0, stream_base = 0;
+  // rh_render_adaptive: pass 0 traces o.spp samples of each entry of a list of pixels (n_rays items; the frame's rows are
+  // rows of the list, the last one may be partial), the sink stages the entries' new sums (ad), and the scene's learned
+  // state is used but not changed
+  bool pixel_list = false;
+  PixelList list{};
+  AdaptiveParams ad{};
   // rh_render_accumulate: the sink adds the samples to the accumulator's sums (read sum_in, write sum_out) and writes
   // RGB8 to `out` and the linear colours to `linear`, either of them optional
   bool accumulate = false;
@@ -1359,14 +1383,17 @@ struct Frame {
   double* linear = nullptr;
   size_t linear_bytes = 0;
   const char* overflow_error = "rh_render: ray queue overflow; lower chunk_samples";
+  // renders (not traces or list frames) tune the scene's shadow schedule and record its queue factor and row costs
+  bool learns() const { return !trace && !pixel_list; }
 };
 
-// rh_render's argument checks (`who` names the entry point in the messages).  With f->accumulate set, rgb_out may be null.
+// rh_render's argument checks (`who` names the entry point in the messages).  With f->accumulate or f->pixel_list set,
+// rgb_out may be null.
 int render_frame(Device* D, const rh_scene* scene, const rh_camera* camera, const rh_render_opts* o, uint8_t* rgb_out,
                  int32_t* hit_ids_out, Frame* f, const char* who = "rh_render") {
   const std::string w(who);
   const bool peer_frames = o && (o->flags & RH_FLAG_PEER_FRAMES) != 0;
-  if (!scene || !camera || !o || (!rgb_out && !peer_frames && !f->accumulate)) return rh::set_error(RH_ERR_ARG, w + ": null argument");
+  if (!scene || !camera || !o || (!rgb_out && !peer_frames && !f->accumulate && !f->pixel_list)) return rh::set_error(RH_ERR_ARG, w + ": null argument");
   if (peer_frames && (!o->peer_frames || o->n_peer_frames <= 0 || o->n_peer_frames > kMaxPeers))
     return rh::set_error(RH_ERR_ARG, w + ": RH_FLAG_PEER_FRAMES needs 1..16 peer frame pointers");
   if (peer_frames && (o->flags & RH_FLAG_HIT_IDS))
@@ -1409,7 +1436,7 @@ int render_frame(Device* D, const rh_scene* scene, const rh_camera* camera, cons
 // time — one of the scene's timing frames: the first is pooled and not compared (first use of freshly allocated queues),
 // the second pooled, the third per-lane refill; the two kernels' times per walked (hit, light) pair are compared.  Small
 // frames never take part: they run pooled, unprofiled, and after kTuneGiveUp of them the scene stays pooled.  A trace
-// uses the scene's decided schedule and takes no part in the tuning.
+// or a list frame uses the scene's decided schedule and takes no part in the tuning.
 constexpr int kTuneGiveUp = 8;
 struct ShadowChoice {
   bool use_refill = false;
@@ -1421,11 +1448,11 @@ struct ShadowChoice {
 ShadowChoice choose_shadow(const rh_scene* scene, const Frame& f) {
   const int32_t flags = f.o.flags;
   const bool refill_ok = scene->refill_possible && scene->view.n_lights <= (uint32_t)kMaskLights;
-  if (!f.trace && !refill_ok && scene->shadow_mode == 0) scene->shadow_mode = 1;
+  if (f.learns() && !refill_ok && scene->shadow_mode == 0) scene->shadow_mode = 1;
   const bool forced = (flags & (RH_FLAG_SHADOW_POOLED | RH_FLAG_SHADOW_SPLIT)) != 0;
   const bool decided = scene->shadow_mode != 0;
   ShadowChoice c;
-  c.untuned = !f.trace && !forced && !decided && !(flags & RH_FLAG_COUNT);
+  c.untuned = f.learns() && !forced && !decided && !(flags & RH_FLAG_COUNT);
   c.tuning = c.untuned && (uint64_t)f.rows_local * f.o.width * f.o.spp >= (1ull << 21);
   if (flags & RH_FLAG_SHADOW_SPLIT) c.use_refill = refill_ok;
   else if (flags & RH_FLAG_SHADOW_POOLED) c.use_refill = false;
@@ -1587,7 +1614,8 @@ struct FrameRun {
     // offsets in work-item order?  chunk-local slices always; the full-frame array when the frame is not sharded
     P.offset_linear = (o.offset_mode == RH_OFFSETS_F64 && (P.offset_index == kOffIndexLocal || o.shard_count == 1)) ? 1u : 0u;
     P.offset_base = (P.offset_index == kOffIndexLocal) ? 0ull : (unsigned long long)first_row * row_samples;
-    if (f.trace) P.ray_items = (uint32_t)std::min<uint64_t>(P.n_samples, f.n_rays - (uint64_t)first_row * row_samples);
+    if (f.trace || f.pixel_list) P.ray_items = (uint32_t)std::min<uint64_t>(P.n_samples, f.n_rays - (uint64_t)first_row * row_samples);
+    P.list = f.list;
     for (int plane = 0; plane < 3; plane++)  // (three 1-D memsets: a 2-D one is limited to 2 GB of pitch)
       RH_CUDA(cudaMemsetAsync((double*)sc.accum.p + (size_t)plane * chunk_samples, 0, (size_t)P.n_samples * sizeof(double), lane_stream));
     const cudaStream_t shadow_stream = pipelined ? D->shadow_stream[ln] : lane_stream;
@@ -1628,6 +1656,8 @@ struct FrameRun {
       AccumParams A = f.acc;
       A.linear = d_linear;
       launch_accumulate_resolve(P, A, lane_stream);
+    } else if (f.pixel_list) {
+      launch_adaptive_fold(P, f.ad, lane_stream);
     } else {
       launch_resolve(P, lane_stream);
     }
@@ -1831,7 +1861,7 @@ int run_frame(Device* D, const rh_scene* scene, const Frame& f, rh_stats* stats)
   R.host_offsets = (mode == RH_OFFSETS_F64 || mode == RH_OFFSETS_F32 || mode == kOffsetsRays) && !dev_off;
   // what the last streamed frame of this shape measured: kernel time per row, and whether the kernels or the upload
   // finished last
-  const bool know_cost = !f.trace && (int)scene->row_cost.size() == f.rows_local &&
+  const bool know_cost = f.learns() && (int)scene->row_cost.size() == f.rows_local &&
                          scene->cost_key == std::vector<int>{o.width, o.height, o.spp, o.shard_count, o.shard_index, o.band_height};
   R.plan = rh::plan_chunks(f.rows_local, R.row_samples, o.chunk_samples, D->total_mem, R.host_offsets,
                            know_cost ? scene->row_cost.data() : nullptr, scene->stream_compute_bound);
@@ -1908,7 +1938,8 @@ int run_frame(Device* D, const rh_scene* scene, const Frame& f, rh_stats* stats)
     }
   }
 
-  // queue capacity = factor * chunk samples; doubled when a chunk overflows (and remembered by the scene's renders)
+  // queue capacity = factor * chunk samples; doubled when a chunk overflows (and remembered by the scene's renders; a
+  // trace starts from 2, a list frame from the scene's factor)
   uint32_t factor = f.trace ? 2u : std::max(2u, scene->queue_factor);
   for (;;) {
     if ((rc = R.reserve_queues(factor))) return rc;
@@ -1949,12 +1980,12 @@ int run_frame(Device* D, const rh_scene* scene, const Frame& f, rh_stats* stats)
     if (overflow) {
       if (R.cap >= 0x7fffff00u || factor >= (1u << 16)) return rh::set_error(RH_ERR_OVERFLOW, f.overflow_error);
       factor *= 2;
-      if (!f.trace) scene->queue_factor = factor;
+      if (f.learns()) scene->queue_factor = factor;
       continue;
     }
     if (stats) R.read_stats(stats, factor);
     R.print_timeline();
-    if (!f.trace) R.learn();
+    if (f.learns()) R.learn();
     return RH_OK;
   }
 }
@@ -1977,20 +2008,59 @@ int check_device_pointers(std::initializer_list<const void*> ptrs, const std::st
   return RH_OK;
 }
 
+// ------------------------------------------------------------------ per-pixel state across calls (rh_accum, rh_adaptive)
+// The checks the two kinds of state share; `noun` names the state in the messages, `reset` its reset entry point.
+int shard_state_init(ShardState* S, Device* D, int width, int height, int shard_index, int shard_count, int band_height,
+                     uint32_t stream_spp, const std::string& who) {
+  const int G = shard_count <= 0 ? 1 : shard_count;
+  if (width <= 0 || height <= 0) return rh::set_error(RH_ERR_ARG, who + ": bad width/height");
+  if (shard_index < 0 || shard_index >= G) return rh::set_error(RH_ERR_ARG, who + ": shard_index out of range");
+  S->device = D;
+  S->context = D->context;
+  S->dev = D->dev;
+  S->width = width;
+  S->height = height;
+  S->shard_index = shard_index;
+  S->shard_count = G;
+  S->band_height = band_height > 0 ? band_height : rh_default_band_height(height, G);
+  S->rows_local = rh_shard_rows(height, G, S->band_height);
+  S->stream_spp = stream_spp;
+  S->plane = (size_t)S->rows_local * width;
+  return RH_OK;
+}
+int shard_state_context(const ShardState* S, Device* D, const std::string& w, const char* noun) {
+  if (S->device != D || S->context != D->context) return rh::set_error(RH_ERR_ARG, w + ": " + noun + " lives on another device context");
+  return RH_OK;
+}
+// The frame's size and shard are the state's; once the view is fixed, so are the scene, the camera bytes and max_depth.
+int shard_state_matches(const ShardState* S, const Frame& f, bool fixed, const rh_scene* scene, const rh_camera* camera,
+                        const std::string& w, const char* noun, const char* reset) {
+  if (f.o.width != S->width || f.o.height != S->height || f.o.shard_index != S->shard_index ||
+      f.o.shard_count != S->shard_count || f.o.band_height != S->band_height)
+    return rh::set_error(RH_ERR_ARG, w + ": width, height, shard_index, shard_count or band_height differ from the " + noun + "'s");
+  if (fixed && (scene != S->scene || memcmp(camera, &S->camera, sizeof S->camera) != 0 || f.o.max_depth != S->max_depth))
+    return rh::set_error(RH_ERR_ARG, w + ": scene, camera or max_depth differ from the " + noun + "'s first call; " + reset + " it first");
+  return RH_OK;
+}
+void shard_state_fix_view(ShardState* S, const rh_scene* scene, const rh_camera* camera, int32_t max_depth) {
+  S->scene = scene;
+  S->camera = *camera;
+  S->max_depth = max_depth;
+}
+
 // ------------------------------------------------------------------ progressive accumulation
 // rh_render_accumulate's argument checks: rh_render's (render_frame), then those of the accumulator.
 int accumulate_frame(Device* D, const rh_scene* scene, const rh_camera* camera, const rh_render_opts* o, rh_accum* acc,
                      uint8_t* rgb_out, double* linear_out, int32_t* hit_ids_out, Frame* f) {
   const std::string w = "rh_render_accumulate";
   if (!scene || !camera || !o || !acc) return rh::set_error(RH_ERR_ARG, w + ": null argument");
-  if (acc->device != D || acc->context != D->context) return rh::set_error(RH_ERR_ARG, w + ": accumulator lives on another device context");
+  int rc = shard_state_context(acc, D, w, "accumulator");
+  if (rc) return rc;
   if (o->flags & RH_FLAG_PEER_FRAMES) return rh::set_error(RH_ERR_ARG, w + ": RH_FLAG_PEER_FRAMES is not supported");
   f->accumulate = true;
-  int rc = render_frame(D, scene, camera, o, rgb_out, hit_ids_out, f, "rh_render_accumulate");
+  rc = render_frame(D, scene, camera, o, rgb_out, hit_ids_out, f, "rh_render_accumulate");
   if (rc) return rc;
-  if (f->o.width != acc->width || f->o.height != acc->height || f->o.shard_index != acc->shard_index ||
-      f->o.shard_count != acc->shard_count || f->o.band_height != acc->band_height)
-    return rh::set_error(RH_ERR_ARG, w + ": width, height, shard_index, shard_count or band_height differ from the accumulator's");
+  if ((rc = shard_state_matches(acc, *f, false, scene, camera, w, "accumulator", "rh_accum_reset"))) return rc;
   const uint32_t spp = (uint32_t)o->spp;
   if ((uint64_t)acc->n + spp > 0xffffffffu) return rh::set_error(RH_ERR_ARG, w + ": more than 2^32 - 1 samples per pixel");
   if (o->offset_mode == RH_OFFSETS_SPLITMIX64) {
@@ -2000,8 +2070,7 @@ int accumulate_frame(Device* D, const rh_scene* scene, const rh_camera* camera, 
       return rh::set_error(RH_ERR_ARG, w + ": RH_OFFSETS_SPLITMIX64 past the end of the stream (" + std::to_string(acc->n) + " + " +
                                            std::to_string(spp) + " > stream_spp " + std::to_string(acc->stream_spp) + ")");
   }
-  if (acc->n > 0 && (scene != acc->scene || memcmp(camera, &acc->camera, sizeof acc->camera) != 0 || o->max_depth != acc->max_depth))
-    return rh::set_error(RH_ERR_ARG, w + ": scene, camera or max_depth differ from the accumulator's first call; rh_accum_reset it first");
+  if ((rc = shard_state_matches(acc, *f, acc->n > 0, scene, camera, w, "accumulator", "rh_accum_reset"))) return rc;
   const bool want_ids = (o->flags & RH_FLAG_HIT_IDS) != 0;
   if (o->flags & RH_FLAG_DEVICE_OUT) {
     if ((uintptr_t)linear_out % 8) return rh::set_error(RH_ERR_ARG, w + ": device linear_out must be 8-byte aligned");
@@ -2030,11 +2099,7 @@ int accumulate_on(Device* D, const rh_scene* scene, const rh_camera* camera, con
   int rc = accumulate_frame(D, scene, camera, o, acc, rgb_out, linear_out, hit_ids_out, &f);
   if (rc || (rc = run_frame(D, scene, f, stats))) return rc;
   // the frame completed: its sums are the current ones
-  if (acc->n == 0) {
-    acc->scene = scene;
-    acc->camera = *camera;
-    acc->max_depth = o->max_depth;
-  }
+  if (acc->n == 0) shard_state_fix_view(acc, scene, camera, o->max_depth);
   acc->cur ^= 1;
   acc->n += (uint32_t)o->spp;
   return RH_OK;
@@ -2044,25 +2109,224 @@ int accum_create_on(Device* D, int width, int height, int shard_index, int shard
                     rh_accum** out) {
   if (!out) return rh::set_error(RH_ERR_ARG, "rh_accum_create: null out");
   *out = nullptr;
-  const int G = shard_count <= 0 ? 1 : shard_count;
-  if (width <= 0 || height <= 0) return rh::set_error(RH_ERR_ARG, "rh_accum_create: bad width/height");
-  if (shard_index < 0 || shard_index >= G) return rh::set_error(RH_ERR_ARG, "rh_accum_create: shard_index out of range");
   auto A = std::make_unique<rh_accum>();
-  A->device = D;
-  A->context = D->context;
-  A->dev = D->dev;
-  A->width = width;
-  A->height = height;
-  A->shard_index = shard_index;
-  A->shard_count = G;
-  A->band_height = band_height > 0 ? band_height : rh_default_band_height(height, G);
-  A->rows_local = rh_shard_rows(height, G, A->band_height);
-  A->stream_spp = stream_spp;
-  A->plane = (size_t)A->rows_local * width;
+  int rc = shard_state_init(A.get(), D, width, height, shard_index, shard_count, band_height, stream_spp, "rh_accum_create");
+  if (rc) return rc;
   RH_CUDA(cudaSetDevice(D->dev));
-  int rc = A->sums.reserve(2 * 3 * A->plane * sizeof(double));
+  rc = A->sums.reserve(2 * 3 * A->plane * sizeof(double));
   if (rc) return rc;
   *out = A.release();
+  return RH_OK;
+}
+
+// ------------------------------------------------------------------ adaptive sampling
+// rh_render_adaptive's list frames: a fixed number of list entries per frame row.  Small enough that chunk_samples can
+// split a small image's list into several chunks, large enough that a 4K list has a few thousand rows.
+constexpr int kListRowEntries = 1024;
+
+// rh_render_adaptive's argument checks: rh_render's (render_frame), then those of the adaptive state.
+int adaptive_frame(Device* D, const rh_scene* scene, const rh_camera* camera, const rh_render_opts* o,
+                   const rh_adaptive_opts* ao, rh_adaptive* ad, uint8_t* rgb_out, double* linear_out, Frame* f) {
+  const std::string w = "rh_render_adaptive";
+  if (!scene || !camera || !o || !ao || !ad) return rh::set_error(RH_ERR_ARG, w + ": null argument");
+  int rc = shard_state_context(ad, D, w, "adaptive state");
+  if (rc) return rc;
+  if (o->flags & (RH_FLAG_HIT_IDS | RH_FLAG_PEER_FRAMES | RH_FLAG_SHARD_OFFSETS | RH_FLAG_DEVICE_OFFSETS))
+    return rh::set_error(RH_ERR_ARG, w + ": RH_FLAG_HIT_IDS, RH_FLAG_PEER_FRAMES, RH_FLAG_SHARD_OFFSETS and RH_FLAG_DEVICE_OFFSETS are not supported");
+  if (o->offset_mode != RH_OFFSETS_SPLITMIX64) return rh::set_error(RH_ERR_ARG, w + ": offset_mode must be RH_OFFSETS_SPLITMIX64");
+  if (!(ao->threshold >= 0)) return rh::set_error(RH_ERR_ARG, w + ": threshold must be >= 0");
+  if (ao->min_spp < 2) return rh::set_error(RH_ERR_ARG, w + ": min_spp must be >= 2");
+  if (ao->reserved_ != 0) return rh::set_error(RH_ERR_ARG, w + ": rh_adaptive_opts.reserved_ must be 0");
+  f->pixel_list = true;
+  if ((rc = render_frame(D, scene, camera, o, rgb_out, nullptr, f, "rh_render_adaptive"))) return rc;
+  if ((rc = shard_state_matches(ad, *f, ad->fixed, scene, camera, w, "adaptive state", "rh_adaptive_reset"))) return rc;
+  if (o->flags & RH_FLAG_DEVICE_OUT) {
+    if ((uintptr_t)linear_out % 8) return rh::set_error(RH_ERR_ARG, w + ": device linear_out must be 8-byte aligned");
+    RH_CUDA(cudaSetDevice(D->dev));
+    if ((rc = check_device_pointers({rgb_out, linear_out}, w + ": RH_FLAG_DEVICE_OUT with a pointer that is not device memory")))
+      return rc;
+  }
+  f->ad = ad->A;
+  f->ad.spp = (uint32_t)o->spp;
+  f->ad.min_spp = ao->min_spp;
+  f->ad.tt = ao->threshold * ao->threshold;
+  f->stream_spp = ad->stream_spp;
+  f->list = {f->ad.list, f->ad.counts, (uint32_t)ad->width, (uint32_t)ad->height, (uint32_t)ad->shard_index,
+             (uint32_t)ad->shard_count, (uint32_t)ad->band_height};
+  f->overflow_error = "rh_render_adaptive: ray queue overflow; lower chunk_samples";
+  return RH_OK;
+}
+
+// Select (library stream), read n_active back, the list frame (run_frame), commit, output.  Until the commit the state
+// is only read, so every failure before it leaves the state as it was.
+int adaptive_on(Device* D, const rh_scene* scene, const rh_camera* camera, const rh_render_opts* o, const rh_adaptive_opts* ao,
+                rh_adaptive* ad, uint8_t* rgb_out, double* linear_out, uint64_t* n_active_out, rh_stats* stats) {
+  Frame f;
+  int rc = adaptive_frame(D, scene, camera, o, ao, ad, rgb_out, linear_out, &f);
+  if (rc) return rc;
+  const bool dev_out = (o->flags & RH_FLAG_DEVICE_OUT) != 0, profile = (o->flags & RH_FLAG_PROFILE) != 0;
+  AdaptiveParams A = f.ad;
+  RH_CUDA(cudaSetDevice(D->dev));
+  RH_CUDA(cudaEventRecord(ad->ev[0], D->stream));
+  launch_adaptive_select(A, D->stream);
+  RH_CUDA(cudaEventRecord(ad->ev[1], D->stream));
+  uint32_t n_active = 0;
+  RH_CUDA(cudaMemcpyAsync(&n_active, A.n_active, sizeof n_active, cudaMemcpyDeviceToHost, D->stream));
+  RH_CUDA(cudaStreamSynchronize(D->stream));
+  uint32_t launches = 3;
+
+  // the list frame: its rows are rows of the list, unsharded; pass 0 reads the pixels through f.list
+  rh_stats fs{};
+  if (n_active) {
+    const uint64_t rows = ((uint64_t)n_active + kListRowEntries - 1) / kListRowEntries;
+    f.o.width = kListRowEntries;
+    f.o.height = f.o.band_height = f.rows_local = (int)rows;
+    f.o.shard_index = 0;
+    f.o.shard_count = 1;
+    f.out = nullptr;
+    f.out_bytes = 0;
+    f.n_rays = f.rays_primary = (uint64_t)n_active * A.spp;
+    if ((rc = run_frame(D, scene, f, &fs))) return rc;
+    RH_CUDA(cudaSetDevice(D->dev));
+  }
+
+  RH_CUDA(cudaEventRecord(ad->ev[2], D->stream));
+  launch_adaptive_commit(A, n_active, D->stream);
+  launches += n_active ? 1 : 0;
+  const size_t px = ad->plane;
+  unsigned long long negative = 0;
+  if (rgb_out || linear_out) {
+    A.rgb = rgb_out;
+    A.linear = linear_out;
+    if (!dev_out) {
+      if (rgb_out && (rc = D->rgb.reserve(px * 3))) return rc;
+      if (linear_out && (rc = D->linear.reserve(px * 3 * sizeof(double)))) return rc;
+      A.rgb = rgb_out ? (uint8_t*)D->rgb.p : nullptr;
+      A.linear = linear_out ? (double*)D->linear.p : nullptr;
+    }
+    RH_CUDA(cudaMemsetAsync(A.negative, 0, sizeof(unsigned long long), D->stream));
+    launch_adaptive_output(A, D->stream);
+    launches += 1;
+    if (!dev_out) {
+      if (rgb_out) RH_CUDA(cudaMemcpyAsync(rgb_out, A.rgb, px * 3, cudaMemcpyDeviceToHost, D->stream));
+      if (linear_out) RH_CUDA(cudaMemcpyAsync(linear_out, A.linear, px * 3 * sizeof(double), cudaMemcpyDeviceToHost, D->stream));
+    }
+    if (rgb_out) RH_CUDA(cudaMemcpyAsync(&negative, A.negative, sizeof negative, cudaMemcpyDeviceToHost, D->stream));
+  }
+  RH_CUDA(cudaEventRecord(ad->ev[3], D->stream));
+  RH_CUDA(cudaGetLastError());
+  RH_CUDA(cudaStreamSynchronize(D->stream));
+  g_launches.fetch_add(launches, std::memory_order_relaxed);
+  if (!ad->fixed) {
+    shard_state_fix_view(ad, scene, camera, o->max_depth);
+    ad->fixed = true;
+  }
+  if (n_active_out) *n_active_out = n_active;
+  if (stats) {
+    *stats = fs;  // (zero when nothing was traced)
+    float ms = 0;
+    cudaEventElapsedTime(&ms, ad->ev[0], ad->ev[3]);
+    stats->ms_total = ms;
+    if (profile) {
+      float sel = 0, post = 0;
+      cudaEventElapsedTime(&sel, ad->ev[0], ad->ev[1]);
+      cudaEventElapsedTime(&post, ad->ev[2], ad->ev[3]);
+      stats->ms_resolve += sel + post;
+    }
+    stats->kernel_launches += launches;
+    stats->negative_channels = (uint32_t)std::min<unsigned long long>(negative, 0xffffffffu);
+  }
+  return RH_OK;
+}
+
+void adaptive_release(rh_adaptive* ad) {
+  for (cudaEvent_t& e : ad->ev)
+    if (e) cudaEventDestroy(e), e = nullptr;
+  ad->state.release();
+  ad->work.release();
+  ad->scratch.release();
+}
+
+// State 52 bytes per pixel, list and staging 52, scratch one bit per pixel and a word per kSelectBlock pixels.
+int adaptive_create_on(Device* D, int width, int height, int shard_index, int shard_count, int band_height, uint32_t stream_spp,
+                       rh_adaptive** out) {
+  if (!out) return rh::set_error(RH_ERR_ARG, "rh_adaptive_create: null out");
+  *out = nullptr;
+  if (stream_spp < 1) return rh::set_error(RH_ERR_ARG, "rh_adaptive_create: stream_spp must be >= 1");
+  std::unique_ptr<rh_adaptive, void (*)(rh_adaptive*)> ad(new rh_adaptive(), [](rh_adaptive* a) { adaptive_release(a); delete a; });
+  int rc = shard_state_init(ad.get(), D, width, height, shard_index, shard_count, band_height, stream_spp, "rh_adaptive_create");
+  if (rc) return rc;
+  const size_t px = ad->plane;
+  if (px >= 0xffffffffu) return rh::set_error(RH_ERR_ARG, "rh_adaptive_create: more than 2^32 - 2 pixels per shard");
+  RH_CUDA(cudaSetDevice(D->dev));
+  const size_t words = (px + 1) / 2 * 2;  // uint32 planes padded to 8 bytes
+  const size_t n_blocks = (px + kSelectBlock - 1) / kSelectBlock;
+  const size_t state_bytes = words * 4 + 6 * px * sizeof(double);
+  if ((rc = ad->state.reserve(state_bytes))) return rc;
+  if ((rc = ad->work.reserve(words * 4 + 6 * px * sizeof(double)))) return rc;
+  if ((rc = ad->scratch.reserve(16 + (n_blocks + n_blocks * (kSelectBlock / 32)) * sizeof(uint32_t)))) return rc;
+  for (cudaEvent_t& e : ad->ev) RH_CUDA(cudaEventCreate(&e));
+  RH_CUDA(cudaMemsetAsync(ad->state.p, 0, state_bytes, D->stream));
+  RH_CUDA(cudaStreamSynchronize(D->stream));
+  AdaptiveParams& A = ad->A;
+  A.counts = (uint32_t*)ad->state.p;
+  A.sum = (double*)((char*)ad->state.p + words * 4);
+  A.sumsq = A.sum + 3 * px;
+  A.list = (uint32_t*)ad->work.p;
+  A.stage = (double*)((char*)ad->work.p + words * 4);
+  A.negative = (unsigned long long*)ad->scratch.p;
+  A.n_active = (uint32_t*)((char*)ad->scratch.p + 8);
+  A.block_counts = (uint32_t*)((char*)ad->scratch.p + 16);
+  A.warp_masks = A.block_counts + n_blocks;
+  A.plane = px;
+  A.width = (uint32_t)width;
+  A.height = (uint32_t)height;
+  A.shard_index = (uint32_t)ad->shard_index;
+  A.shard_count = (uint32_t)ad->shard_count;
+  A.band_height = (uint32_t)ad->band_height;
+  A.stream_spp = stream_spp;
+  *out = ad.release();
+  return RH_OK;
+}
+
+int adaptive_reset_on(rh_adaptive* ad) {
+  RH_CUDA(cudaSetDevice(ad->dev));
+  RH_CUDA(cudaMemset(ad->state.p, 0, (ad->plane + 1) / 2 * 2 * 4 + 6 * ad->plane * sizeof(double)));
+  RH_CUDA(cudaDeviceSynchronize());  // (the library's streams do not wait for the legacy stream)
+  ad->fixed = false;
+  ad->scene = nullptr;
+  return RH_OK;
+}
+
+// The state out: the counts as they are, S and Q from three planes to double[pixel][3] (host buffers through the
+// device scratch of the linear colours).
+int adaptive_state_on(Device* D, const rh_adaptive* ad, uint32_t* counts_out, double* sums_out, double* sumsq_out, int32_t flags) {
+  const std::string w = "rh_adaptive_state";
+  if (!ad) return rh::set_error(RH_ERR_ARG, w + ": null state");
+  int rc = shard_state_context(ad, D, w, "adaptive state");
+  if (rc) return rc;
+  if (flags & ~RH_FLAG_DEVICE_OUT) return rh::set_error(RH_ERR_ARG, w + ": flags must be 0 or RH_FLAG_DEVICE_OUT");
+  const bool dev = (flags & RH_FLAG_DEVICE_OUT) != 0;
+  RH_CUDA(cudaSetDevice(D->dev));
+  if (dev) {
+    if ((uintptr_t)sums_out % 8 || (uintptr_t)sumsq_out % 8)
+      return rh::set_error(RH_ERR_ARG, w + ": device sums_out and sumsq_out must be 8-byte aligned");
+    if ((rc = check_device_pointers({counts_out, sums_out, sumsq_out}, w + ": RH_FLAG_DEVICE_OUT with a pointer that is not device memory")))
+      return rc;
+  }
+  const size_t px = ad->plane, bytes = px * 3 * sizeof(double);
+  if (counts_out)
+    RH_CUDA(cudaMemcpyAsync(counts_out, ad->A.counts, px * sizeof(uint32_t), dev ? cudaMemcpyDeviceToDevice : cudaMemcpyDeviceToHost, D->stream));
+  if (!dev && (sums_out || sumsq_out) && (rc = D->linear.reserve(bytes))) return rc;
+  const double* planes[2] = {ad->A.sum, ad->A.sumsq};
+  double* outs[2] = {sums_out, sumsq_out};
+  for (int k = 0; k < 2; k++) {
+    if (!outs[k]) continue;
+    launch_adaptive_interleave(planes[k], px, dev ? outs[k] : (double*)D->linear.p, D->stream);
+    if (!dev) RH_CUDA(cudaMemcpyAsync(outs[k], D->linear.p, bytes, cudaMemcpyDeviceToHost, D->stream));
+  }
+  RH_CUDA(cudaGetLastError());
+  RH_CUDA(cudaStreamSynchronize(D->stream));
   return RH_OK;
 }
 
@@ -2317,6 +2581,31 @@ int rh_render_accumulate(const rh_scene* scene, const rh_camera* camera, const r
                          uint8_t* rgb_out, double* linear_out, int32_t* hit_ids_out, rh_stats* stats) {
   if (!g_dev) return rh::set_error(RH_ERR_STATE, "rh_render_accumulate: call rh_init first");
   return accumulate_on(g_dev.get(), scene, camera, opts, acc, rgb_out, linear_out, hit_ids_out, stats);
+}
+
+int rh_adaptive_create(int width, int height, int shard_index, int shard_count, int band_height, uint32_t stream_spp,
+                       rh_adaptive** out) {
+  if (!g_dev) return rh::set_error(RH_ERR_STATE, "rh_adaptive_create: call rh_init first");
+  return adaptive_create_on(g_dev.get(), width, height, shard_index, shard_count, band_height, stream_spp, out);
+}
+int rh_adaptive_reset(rh_adaptive* ad) {
+  if (!ad) return rh::set_error(RH_ERR_ARG, "rh_adaptive_reset: null state");
+  return adaptive_reset_on(ad);
+}
+void rh_adaptive_destroy(rh_adaptive* ad) {
+  if (!ad) return;
+  if (ad->dev >= 0) cudaSetDevice(ad->dev);  // (not through ad->device: that context may have been shut down)
+  adaptive_release(ad);
+  delete ad;
+}
+int rh_render_adaptive(const rh_scene* scene, const rh_camera* camera, const rh_render_opts* opts, const rh_adaptive_opts* aopts,
+                       rh_adaptive* ad, uint8_t* rgb_out, double* linear_out, uint64_t* n_active_out, rh_stats* stats) {
+  if (!g_dev) return rh::set_error(RH_ERR_STATE, "rh_render_adaptive: call rh_init first");
+  return adaptive_on(g_dev.get(), scene, camera, opts, aopts, ad, rgb_out, linear_out, n_active_out, stats);
+}
+int rh_adaptive_state(const rh_adaptive* ad, uint32_t* counts_out, double* sums_out, double* sumsq_out, int32_t flags) {
+  if (!g_dev) return rh::set_error(RH_ERR_STATE, "rh_adaptive_state: call rh_init first");
+  return adaptive_state_on(g_dev.get(), ad, counts_out, sums_out, sumsq_out, flags);
 }
 
 int rh_closest_intersection(const rh_scene* scene, const double* rays, uint64_t n, rh_hit* hits_out, int32_t flags) {

@@ -706,6 +706,126 @@ def progressiveRayTrace(job: Rendering, spp: int = 64, batch: int = 8, seed: int
         acc.close()
 
 
+class AdaptiveAccumulator:
+    """Adaptive sampling (rh_render_adaptive): progressive rendering that traces new samples only for the pixels whose
+    standard error of the mean is still above a threshold in some channel.  Every pixel continues its own slice of the
+    SplitMix64 stream sample_offsets(n, stream_spp, seed), so a pixel that ends with n samples has exactly the bytes of
+    an n-sample render of that stream.  The state per pixel (count, sums of the colours and of their squares) stays on
+    the device between calls.
+
+    `shard_index` / `shard_count` / `band_height` as for render (the outputs are shard-compact).  `device`: outputs are
+    CUDA tensors, else numpy arrays.  The first add() after creation or reset() fixes the scene, camera and max_depth."""
+
+    def __init__(self, job: Rendering, stream_spp: int, shard_index: int = 0, shard_count: int = 1, band_height: int = 0,
+                 device: bool = False):
+        L = lib()
+        init()
+        self.job, self.device, self.stream_spp = job, bool(device), int(stream_spp)
+        self.shard_index, self.shard_count = shard_index, shard_count
+        self.band_height = band_height or L.rh_default_band_height(job.height, shard_count)
+        self.rows = L.rh_shard_rows(job.height, shard_count, self.band_height)
+        self._h = C.c_void_p()
+        check(L.rh_adaptive_create(job.width, job.height, shard_index, shard_count, self.band_height, self.stream_spp,
+                                   C.byref(self._h)))
+
+    def add(self, spp: int, seed: int, threshold: float, min_spp: int = 8, rgb: bool = True, linear: bool = True,
+            shadow: str | None = None, exact_boxes: bool = False, light_maps: bool = True, chunk_samples: int = 0,
+            profile: bool = False, count: bool = False) -> Image:
+        """One round: `spp` new samples for each pixel that is active by the rule of include/rayhs_b200.h (fewer than
+        `min_spp` samples, or a channel's standard error above `threshold`, and room left in the stream).  Returns the
+        Image of every pixel's samples so far: `pixels` (RGB8, when `rgb`), `linear` (float64, when `linear`) and this
+        call's stats, with stats["n_active"] the number of pixels traced."""
+        if self._h is None or not self._h:
+            raise ValueError("the adaptive accumulator is closed")
+        L = lib()
+        job = self.job
+        seed_box = C.c_uint64(seed)
+        flags = ((capi.RH_FLAG_EXACT_BOXES if exact_boxes else 0) | _shadow_flag(shadow)
+                 | (0 if light_maps else capi.RH_FLAG_NO_LIGHT_MAPS) | (capi.RH_FLAG_DEVICE_OUT if self.device else 0)
+                 | (capi.RH_FLAG_PROFILE if profile else 0) | (capi.RH_FLAG_COUNT if count else 0))
+        o = _opts(job, spp, capi.RH_OFFSETS_SPLITMIX64, C.addressof(seed_box), 0, self.shard_index, self.shard_count,
+                  self.band_height, chunk_samples, flags)
+        ao = capi.rh_adaptive_opts()
+        ao.threshold, ao.min_spp = float(threshold), int(min_spp)
+        shape = (self.rows, job.width, 3)
+        if self.device:
+            import torch
+
+            torch.cuda.current_stream().synchronize()  # the library runs on its own stream
+            px = torch.empty(shape, dtype=torch.uint8, device="cuda") if rgb else None
+            lin = torch.empty(shape, dtype=torch.float64, device="cuda") if linear else None
+        else:
+            px = np.empty(shape, dtype=np.uint8) if rgb else None
+            lin = np.empty(shape, dtype=np.float64) if linear else None
+        n_active = C.c_uint64()
+        st = capi.rh_stats()
+        check(L.rh_render_adaptive(job.scene.device, C.byref(job.camera), C.byref(o), C.byref(ao), self._h,
+                                   _ptr(px) if px is not None else None, _ptr(lin) if lin is not None else None,
+                                   C.byref(n_active), C.byref(st)))
+        stats = st.as_dict()
+        stats["n_active"] = n_active.value
+        return Image(job.width, self.rows, px, stats, None, lin)
+
+    def state(self):
+        """(counts uint32 [rows, width], sums float64 [rows, width, 3], sums of squares float64 [rows, width, 3]), numpy
+        arrays or, with device=True, CUDA tensors."""
+        shape = (self.rows, self.job.width)
+        if self.device:
+            import torch
+
+            counts = torch.empty(shape, dtype=torch.int32, device="cuda")  # (torch has no uint32 arithmetic to speak of)
+            sums = torch.empty(shape + (3,), dtype=torch.float64, device="cuda")
+            sumsq = torch.empty(shape + (3,), dtype=torch.float64, device="cuda")
+            torch.cuda.current_stream().synchronize()
+            flags = capi.RH_FLAG_DEVICE_OUT
+        else:
+            counts = np.empty(shape, dtype=np.uint32)
+            sums = np.empty(shape + (3,), dtype=np.float64)
+            sumsq = np.empty(shape + (3,), dtype=np.float64)
+            flags = 0
+        check(lib().rh_adaptive_state(self._h, _ptr(counts), _ptr(sums), _ptr(sumsq), flags))
+        return counts, sums, sumsq
+
+    def reset(self) -> None:
+        """Every count and sum back to 0; the next add() may use another scene, camera or max_depth."""
+        check(lib().rh_adaptive_reset(self._h))
+
+    def close(self) -> None:
+        if getattr(self, "_h", None):
+            lib().rh_adaptive_destroy(self._h)
+        self._h = None
+
+    def __del__(self):
+        try:
+            self.close()
+        except Exception:
+            pass
+
+
+def adaptiveRayTrace(job: Rendering, max_spp: int = 64, batch: int = 4, min_spp: int = 8, threshold: float = 0.5 / 255,
+                     seed: int = 24):
+    """distributedRayTrace (RayHs.hs:190-195) refined adaptively: yields the RGB8 Image (stats["n_active"]: pixels traced
+    in that round) after each round of `batch` new samples for every pixel still active, until no pixel is.  A pixel
+    gets at least min(min_spp, max_spp) samples rounded up to whole batches and at most max_spp; it stops once every
+    channel's standard error of the mean is at most `threshold`.  The default, half an RGB8 step (0.5 / 255), stops a
+    pixel when one standard error of its mean no longer reaches the next quantisation step from the middle of one, so
+    more samples would rarely change its byte.  Samples come from the stream distributedRayTrace(job, max_spp, seed)
+    uses: a pixel that reaches max_spp has that frame's bytes."""
+    if max_spp < 1 or batch < 1 or batch > max_spp:
+        raise ValueError(f"need 1 <= batch <= max_spp, got batch {batch} and max_spp {max_spp}")
+    if min_spp < 2:
+        raise ValueError(f"min_spp must be at least 2, got {min_spp}")
+    ad = AdaptiveAccumulator(job, stream_spp=max_spp)
+    try:
+        while True:
+            img = ad.add(batch, seed, threshold, min_spp=min_spp, linear=False)
+            if img.stats["n_active"] == 0:
+                return
+            yield img
+    finally:
+        ad.close()
+
+
 def writePPM(path: str, image: Image) -> None:
     """Image.hs:70-75 — byte-identical P3 text."""
     px = np.ascontiguousarray(image.pixels, dtype=np.uint8)
