@@ -322,6 +322,33 @@ int rh_scene_record_bytes(const rh_scene* scene, uint64_t* bytes5);
  * map or 0xFFFFFFFF); lit_out: one uint16 per triangle slot.  Any pointer may be NULL. */
 int rh_scene_light_tables(const rh_scene* scene, uint32_t* info4, float* maps_out, uint32_t* index_out, uint16_t* lit_out);
 
+/* ---- scene updates --------------------------------------------------- */
+/* What rh_scene_update rebuilt (24 bytes). */
+typedef struct rh_update_info {
+  uint32_t colours_only;      /* 1: nothing but light color / radius and material color1 / color2 / size changed  */
+  uint32_t occluders_rebuilt; /* 1: the set of emitter objects changed (occluder tables and all light tables rebuilt) */
+  uint32_t maps_rasterised;   /* cube maps built anew                                                                */
+  uint32_t maps_kept;         /* cube maps carried over from the previous tables by device copies                    */
+  uint64_t lit_queries;       /* (triangle, light) lit-triangle queries made                                          */
+} rh_update_info;
+/* Replaces the scene's material and light tables in place; the geometry (objects, their material indices, meshes,
+ * textures) stays.  materials: n_materials entries, which must equal the scene's material count, or NULL (keep the
+ * table); lights: n_lights entries (n_lights may differ from the scene's; 0 removes every light), or NULL (keep the
+ * table, n_lights ignored).  Entries are checked as rh_scene_create checks them.  After RH_OK every call on the scene
+ * behaves as on rh_scene_create of the same description with the new tables (set-up times aside), including
+ * rh_scene_info's info4, rh_scene_light_tables and rh_scene_record_bytes.  Only what the edit touches is rebuilt: an
+ * update of colours only (light color / radius, material color1 / color2 / size) uploads the two tables; one that turns
+ * an object into an emitter or back rebuilds the occluder tables and every light table; any other rebuilds the cube
+ * maps of the lights that are new or moved (kind or vec) and their lit-triangle bits, and carries the other maps over.
+ * Beyond a colours-only update the scene's learned state (shadow schedule, queue factor, row costs) starts over as a
+ * fresh scene's.  An update that changes no byte is a no-op.  Every other update makes rh_render_accumulate and
+ * rh_render_adaptive refuse a state whose view was fixed before it (reset it first).  The call returns when the device
+ * work is done and must not overlap another call on the scene.  On failure (argument, RH_ERR_OOM, RH_ERR_CUDA) the
+ * scene is unchanged and usable: the new tables are built beside the old ones and swapped in at the end, so the peak
+ * memory is both sets.  info (optional): what was rebuilt. */
+int rh_scene_update(rh_scene* scene, const rh_material* materials, uint32_t n_materials, const rh_light* lights,
+                    uint32_t n_lights, rh_update_info* info);
+
 /* Replaces `rayTrace` (RayHs.hs:161-166) / `distributedRayTrace` (RayHs.hs:190-195).
  * rgb_out: RGB8, row-major.  For shard_count == 1 it is width*height*3 bytes.
  * For shard_count > 1 it is the COMPACT band buffer of this shard:
@@ -414,7 +441,8 @@ void rh_accum_destroy(rh_accum* acc);
  * [spp][2].  RH_FLAG_DEVICE_OUT applies to all three outputs (linear_out 8-byte aligned).  The other flags behave as
  * in rh_render and may change from call to call; RH_FLAG_PEER_FRAMES is refused.
  * The first call after create or reset records the scene, the camera bytes and max_depth; a later call with others is
- * RH_ERR_ARG (reset first).  opts must match the accumulator's size and shard.  A call that fails (argument, CUDA or
+ * RH_ERR_ARG (reset first), and so is a call after an rh_scene_update of that scene that changed bytes.  opts must
+ * match the accumulator's size and shard.  A call that fails (argument, CUDA or
  * RH_ERR_OVERFLOW) leaves the sums and N unchanged.  For the scene's learned state (shadow schedule, queue factor, row
  * costs) the call is a render.  stats: this call's samples; negative_channels counts its RGB8 output. */
 int rh_render_accumulate(const rh_scene* scene, const rh_camera* camera, const rh_render_opts* opts, rh_accum* acc,
@@ -458,7 +486,8 @@ void rh_adaptive_destroy(rh_adaptive* ad); /* NULL is a no-op */
  * RH_FLAG_NO_LIGHT_MAPS, the shadow-schedule flags, RH_FLAG_COUNT, RH_FLAG_PROFILE and chunk_samples behave as in
  * rh_render (chunk_samples counts the samples of the active pixels).  threshold and min_spp may change from call to
  * call.  The first call after create or reset records the scene, the camera bytes and max_depth; a later call with
- * others is RH_ERR_ARG (reset first).  opts must match the state's size and shard.  A call that fails (argument, CUDA
+ * others is RH_ERR_ARG (reset first), and so is a call after an rh_scene_update of that scene that changed bytes.
+ * opts must match the state's size and shard.  A call that fails (argument, CUDA
  * or RH_ERR_OVERFLOW) leaves every n_p, S_p and Q_p unchanged; a queue-overflow retry inside the call counts no sample
  * twice.  The call uses the scene's decided shadow schedule and queue factor (else the pooled schedule and factor 2)
  * and changes neither them nor the row costs, as rh_trace_rays does.  stats: rays_primary = n_active * spp, the other
@@ -495,6 +524,10 @@ void rh_multi_shutdown(void);
 int rh_multi_gpu_count(void);
 int rh_multi_scene_create(const rh_scene_desc* desc, rh_multi_scene** out);
 void rh_multi_scene_destroy(rh_multi_scene* scene);
+/* rh_scene_update on every replica: all are prepared before any is swapped in, so the update takes on every GPU or on
+ * none.  info: replica 0's. */
+int rh_multi_scene_update(rh_multi_scene* scene, const rh_material* materials, uint32_t n_materials, const rh_light* lights,
+                          uint32_t n_lights, rh_update_info* info);
 int rh_multi_render(const rh_multi_scene* scene, const rh_camera* camera, const rh_render_opts* opts, uint8_t* rgb_out,
                     rh_stats* stats);
 

@@ -35,7 +35,7 @@ CXX_FLAGS = ["-std=c++17", "-O2", "-fPIC", "-ffp-contract=off", "-Wall", "-Wno-u
 
 CUDA_SOURCES = ["kernels.cu", "runtime.cu", "setup_kernels.cu"]
 CXX_SOURCES = ["frontend.cpp", "host_build.cpp", "light_maps.cpp"]
-HEADERS = [os.path.join(CSRC, h) for h in ("device_types.cuh", "common.h", "light_geom.h", "render_plan.h")] + [os.path.join(ROOT, "include", "rayhs_b200.h")]
+HEADERS = [os.path.join(CSRC, h) for h in ("device_types.cuh", "common.h", "light_geom.h", "render_plan.h", "scene_update.h")] + [os.path.join(ROOT, "include", "rayhs_b200.h")]
 
 
 def _digest(deps: list[str], flags: list[str]) -> str:

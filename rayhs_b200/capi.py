@@ -127,10 +127,16 @@ class rh_adaptive_opts(C.Structure):
     _fields_ = [("threshold", C.c_double), ("min_spp", C.c_uint32), ("reserved_", C.c_uint32)]
 
 
+class rh_update_info(C.Structure):
+    _fields_ = [("colours_only", C.c_uint32), ("occluders_rebuilt", C.c_uint32), ("maps_rasterised", C.c_uint32),
+                ("maps_kept", C.c_uint32), ("lit_queries", C.c_uint64)]
+
+
 # struct sizes the header promises (checked by tests/test_abi.py against the compiled library too)
 assert C.sizeof(rh_material) == 96 and C.sizeof(rh_light) == 64 and C.sizeof(rh_node) == 64
 assert C.sizeof(rh_tri) == 80 and C.sizeof(rh_tri_shade) == 128 and C.sizeof(rh_object) == 96
 assert C.sizeof(rh_hit) == 80 and C.sizeof(rh_trace_opts) == 16 and C.sizeof(rh_adaptive_opts) == 16
+assert C.sizeof(rh_update_info) == 24
 
 vp = C.c_void_p
 
@@ -146,6 +152,7 @@ SIGNATURES = {
     "rh_scene_info": (C.c_int, [vp, C.POINTER(C.c_double), C.POINTER(C.c_int32)]),
     "rh_scene_record_bytes": (C.c_int, [vp, C.POINTER(C.c_uint64)]),
     "rh_scene_light_tables": (C.c_int, [vp, C.POINTER(C.c_uint32), vp, vp, vp]),
+    "rh_scene_update": (C.c_int, [vp, C.POINTER(rh_material), C.c_uint32, C.POINTER(rh_light), C.c_uint32, C.POINTER(rh_update_info)]),
     "rh_render": (C.c_int, [vp, C.POINTER(rh_camera), C.POINTER(rh_render_opts), vp, vp, C.POINTER(rh_stats)]),
     "rh_closest_intersection": (C.c_int, [vp, vp, C.c_uint64, vp, C.c_int32]),
     "rh_shadow_intersection": (C.c_int, [vp, C.c_uint32, vp, C.c_uint64, vp, C.c_int32]),
@@ -168,6 +175,8 @@ SIGNATURES = {
     "rh_multi_gpu_count": (C.c_int, []),
     "rh_multi_scene_create": (C.c_int, [C.POINTER(rh_scene_desc), C.POINTER(vp)]),
     "rh_multi_scene_destroy": (None, [vp]),
+    "rh_multi_scene_update": (C.c_int, [vp, C.POINTER(rh_material), C.c_uint32, C.POINTER(rh_light), C.c_uint32,
+                                        C.POINTER(rh_update_info)]),
     "rh_multi_render": (C.c_int, [vp, C.POINTER(rh_camera), C.POINTER(rh_render_opts), vp, C.POINTER(rh_stats)]),
     "rh_peer_alloc": (C.c_int, [C.c_size_t, C.POINTER(vp), C.c_char_p]),
     "rh_peer_open": (C.c_int, [C.c_char_p, C.POINTER(vp)]),

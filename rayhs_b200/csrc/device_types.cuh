@@ -355,7 +355,7 @@ int preload_setup_kernels();
 int device_light_map(const double L[3], const rh_tri* d_tris, const uint32_t* d_slots, size_t n, int R, float* d_out, double min_empty,
                      unsigned long long* d_words, int* useful, double* empty_fraction, void* stream);
 int device_lit_flags(const rh_tri* d_tris, const WideNode32* d_nodes, const double center[3], uint32_t root, const uint32_t* d_slots,
-                     uint32_t n_slots, const rh_light* d_lights, uint32_t n_lights, uint32_t mesh, uint16_t* d_lit,
+                     uint32_t n_slots, const rh_light* d_lights, uint32_t n_lights, uint32_t mask, uint32_t mesh, uint16_t* d_lit,
                      unsigned long long* d_flagged, void* stream);
 // micro-benchmarks
 void launch_gather_bench(const double2* buf, uint64_t n_records, uint32_t loads_per_thread, double2* sink, int grid, int block,

@@ -32,6 +32,7 @@
 #include "device_types.cuh"
 #include "light_geom.h"
 #include "render_plan.h"
+#include "scene_update.h"
 
 namespace rh {
 static thread_local std::string g_err;
@@ -203,6 +204,26 @@ struct rh_scene {
   mutable std::vector<float> row_cost;    // kernel ms per local row (its chunk's time / its chunk's rows)
   mutable uint32_t queue_factor = 2;          // the queue capacity factor the scene's last frame needed
   mutable bool stream_compute_bound = false;  // ... and in that frame the kernels, not the upload, finished last
+  // What derive_tables needs to rebuild the material- and light-derived tables for rh_scene_update (DESIGN.md "Scene
+  // updates"), on the host: the object records, the linear object list, the sphere-tree root, both tree depths, the
+  // texture table, the current material and light tables, and each mesh's triangle slots (4 bytes per triangle) in
+  // the order the light-table builders walk its cull tree.
+  std::vector<DObject> objs_host;
+  std::vector<uint32_t> lin_objs_host;
+  uint32_t sphere_root = kEmpty, ref_depth = 0, cull_depth = 0;
+  std::vector<rh_texture> textures_host;
+  uint64_t n_texels = 0;
+  std::vector<rh_material> materials_host;
+  std::vector<rh_light> lights_host;
+  std::vector<uint32_t> mesh_slots;  // object i's slots: mesh_slots[slot_begin[i] .. slot_begin[i + 1])
+  std::vector<size_t> slot_begin;
+  // The light tables as derive_tables left them: the cube-map resolution (0: no tables), the host copy of
+  // light_map_index, per occluder mesh whether it got lit-triangle queries, and whether the device builders made them.
+  uint32_t tables_res = 0;
+  std::vector<uint32_t> map_index_host;
+  std::vector<uint8_t> mesh_lit;
+  bool tables_on_device = false;
+  uint64_t generation = 0;  // rh_scene_update calls that changed bytes
 };
 
 // What the per-pixel states of several calls (rh_accum, rh_adaptive) share: the frame (or shard of it) they cover, the
@@ -215,6 +236,7 @@ struct ShardState {
   uint32_t stream_spp = 0;  // RH_OFFSETS_SPLITMIX64: samples per pixel of the stream the calls draw from
   size_t plane = 0;         // doubles per colour plane: rows_local * width
   const rh_scene* scene = nullptr;
+  uint64_t scene_generation = 0;  // scene->generation when the view was fixed
   rh_camera camera{};
   int32_t max_depth = 0;
 };
@@ -804,30 +826,46 @@ int upload(DevBuf& b, const T* src, size_t n) {
   return RH_OK;
 }
 
+// rh_scene_create's checks of the material and light tables (rh_scene_update makes the same ones).
+int check_tables(const rh_material* mats, uint32_t n_materials, const rh_texture* textures, uint32_t n_textures, uint64_t n_texels,
+                 const rh_light* lights, uint32_t n_lights, const std::string& w) {
+  for (uint32_t i = 0; i < n_materials; i++) {
+    const rh_material& m = mats[i];
+    if (m.kind < RH_MAT_MIRROR || m.kind > RH_MAT_SHOWUV) return rh::set_error(RH_ERR_ARG, w + ": unknown material kind");
+    if ((m.kind == RH_MAT_DIFFUSE || m.kind == RH_MAT_PLASTIC)) {
+      if (m.cmap_kind < RH_CMAP_FLAT || m.cmap_kind > RH_CMAP_TEXTURE) return rh::set_error(RH_ERR_ARG, w + ": unknown colour-map kind");
+      if (m.cmap_kind == RH_CMAP_TEXTURE) {
+        if (m.texture < 0 || (uint32_t)m.texture >= n_textures) return rh::set_error(RH_ERR_ARG, w + ": texture index out of range");
+        const rh_texture& t = textures[m.texture];
+        if (t.w <= 0 || t.h <= 0 || t.offset + (uint64_t)t.w * t.h > n_texels)
+          return rh::set_error(RH_ERR_ARG, w + ": texture outside the texel array");
+      }
+    }
+  }
+  for (uint32_t i = 0; i < n_lights; i++)
+    if (lights[i].kind != RH_LIGHT_DIRECTIONAL && lights[i].kind != RH_LIGHT_POINT) return rh::set_error(RH_ERR_ARG, w + ": unknown light kind");
+  return RH_OK;
+}
+
+// RAYHS_B200_SETUP=host: rh_scene_create's host builders of the light tables (light_maps.cpp) read the cull tree and the
+// triangle records on the host.
+struct HostGeometry {
+  const std::vector<WideNode>* cull;
+  const TriVec* tris;
+};
+
+int derive_tables(Device* D, const rh_scene& G, const rh_material* mats, uint32_t n_materials, const rh_light* lights,
+                  uint32_t n_lights, const HostGeometry* host, const rh_scene* old, rh_scene* T, rh_update_info* info,
+                  const std::string& w);
+
 int scene_create_on(Device* D, const rh_scene_desc* d, rh_scene** out) {
   if (!d || !out) return rh::set_error(RH_ERR_ARG, "rh_scene_create: null argument");
   if (d->n_materials > 0x7fff) return rh::set_error(RH_ERR_ARG, "rh_scene_create: more than 32767 materials");
   if ((d->n_nodes && !d->nodes) || (d->n_tris && (!d->tris || !d->tri_shade)) || (d->n_objects && !d->objects) ||
       (d->n_materials && !d->materials) || (d->n_lights && !d->lights))
     return rh::set_error(RH_ERR_ARG, "rh_scene_create: null array with non-zero count");
-  for (uint32_t i = 0; i < d->n_materials; i++) {
-    const rh_material& m = d->materials[i];
-    if (m.kind < RH_MAT_MIRROR || m.kind > RH_MAT_SHOWUV) return rh::set_error(RH_ERR_ARG, "rh_scene_create: unknown material kind");
-    if ((m.kind == RH_MAT_DIFFUSE || m.kind == RH_MAT_PLASTIC)) {
-      if (m.cmap_kind < RH_CMAP_FLAT || m.cmap_kind > RH_CMAP_TEXTURE)
-        return rh::set_error(RH_ERR_ARG, "rh_scene_create: unknown colour-map kind");
-      if (m.cmap_kind == RH_CMAP_TEXTURE) {
-        if (m.texture < 0 || (uint32_t)m.texture >= d->n_textures)
-          return rh::set_error(RH_ERR_ARG, "rh_scene_create: texture index out of range");
-        const rh_texture& t = d->textures[m.texture];
-        if (t.w <= 0 || t.h <= 0 || t.offset + (uint64_t)t.w * t.h > d->n_texels)
-          return rh::set_error(RH_ERR_ARG, "rh_scene_create: texture outside the texel array");
-      }
-    }
-  }
-  for (uint32_t i = 0; i < d->n_lights; i++)
-    if (d->lights[i].kind != RH_LIGHT_DIRECTIONAL && d->lights[i].kind != RH_LIGHT_POINT)
-      return rh::set_error(RH_ERR_ARG, "rh_scene_create: unknown light kind");
+  if (int rc = check_tables(d->materials, d->n_materials, d->textures, d->n_textures, d->n_texels, d->lights, d->n_lights, "rh_scene_create"))
+    return rc;
   using clk = std::chrono::steady_clock;
   auto ms_since = [](clk::time_point t) { return std::chrono::duration<double, std::milli>(clk::now() - t).count(); };
   const clk::time_point t_begin = clk::now();
@@ -934,7 +972,6 @@ int scene_create_on(Device* D, const rh_scene_desc* d, rh_scene** out) {
   auto S = std::make_unique<rh_scene>();
   S->device = D;
   S->max_tree_depth = std::max(depth, cull_depth);
-  for (uint32_t i = 0; i < d->n_materials; i++) S->has_transparent |= d->materials[i].kind == RH_MAT_TRANSPARENT;
   int rc;
   // conservative float copy of the boxes: lower bounds rounded down, upper bounds rounded up
   // ... stored relative to the middle of all boxes, so that a scene far from the coordinate origin keeps float's full
@@ -1006,172 +1043,283 @@ int scene_create_on(Device* D, const rh_scene_desc* d, rh_scene** out) {
   if ((rc = upload(S->wide32, wide32.data(), wide32.size()))) return rc;
   if ((rc = upload(S->tris, dtris.data(), dtris.size()))) return rc;
   if ((rc = upload(S->shade, dshade.data(), dshade.size()))) return rc;
-  if ((rc = upload(S->objects, objs.data(), objs.size()))) return rc;
-  if ((rc = upload(S->materials, d->materials, d->n_materials))) return rc;
-  if ((rc = upload(S->lights, d->lights, d->n_lights))) return rc;
   if ((rc = upload(S->textures, d->textures, d->n_textures))) return rc;
   if ((rc = upload(S->texels, d->texels, (size_t)d->n_texels * 3))) return rc;
   if ((rc = upload(S->lin_objs, lin_objs.data(), lin_objs.size()))) return rc;
   if ((rc = upload(S->sphere_refs, sphere_refs.data(), sphere_refs.size()))) return rc;
   if ((rc = upload(S->exact_index, exact_index.data(), exact_index.size()))) return rc;
-  // occluder tables (isOccluder, RayHs.hs:81-82: everything but Emmit objects)
+  SceneView& v = S->view;
+  v.wide = (const WideNode*)S->wide.p;
+  v.wide32 = (const WideNode32*)S->wide32.p;
+  v.abs_max = abs_max;
+  for (int k = 0; k < 3; k++) v.center[k] = center[k];
+  v.tris = (const rh_tri*)S->tris.p;
+  v.shade = (const rh_tri_shade*)S->shade.p;
+  v.textures = (const rh_texture*)S->textures.p;
+  v.texels = (const double*)S->texels.p;
+  v.n_wide = (uint32_t)cull.size();
+  v.n_tris = (uint32_t)dtris.size();  // triangle slots on the device (the meshes' triangles, in cull-tree leaf order)
+  v.n_objects = d->n_objects;
+  v.n_textures = d->n_textures;
+  v.lin_objs = (const uint32_t*)S->lin_objs.p;
+  v.sphere_refs = (const uint32_t*)S->sphere_refs.p;
+  v.exact_index = exact_index.empty() ? nullptr : (const uint32_t*)S->exact_index.p;
+  v.n_lin = (uint32_t)lin_objs.size();
+  v.sphere_root = sphere_root;
+  v.n_smem_nodes = std::min<uint32_t>(v.n_wide, kSmemNodes);
+  S->ms_upload = ms_since(t_mark);
+  // what derive_tables reads, now and on every rh_scene_update
+  try {
+    S->objs_host.swap(objs);
+    S->lin_objs_host.swap(lin_objs);
+    S->sphere_root = sphere_root;
+    S->ref_depth = depth;
+    S->cull_depth = cull_depth;
+    S->textures_host.assign(d->textures, d->textures + d->n_textures);
+    S->n_texels = d->n_texels;
+    S->slot_begin.assign((size_t)d->n_objects + 1, 0);
+    std::vector<uint32_t> dfs;
+    for (uint32_t i = 0; i < d->n_objects; i++) {
+      S->slot_begin[i] = S->mesh_slots.size();
+      if (S->objs_host[i].kind != RH_OBJ_MESH || S->objs_host[i].root == kEmpty) continue;
+      dfs.assign(1, S->objs_host[i].root);  // the mesh's triangles: leaves of its cull tree
+      while (!dfs.empty()) {
+        const WideNode& w = cull[dfs.back()];
+        dfs.pop_back();
+        for (int c = 0; c < 2; c++) {
+          if (w.child[c] == kEmpty) continue;
+          if (w.child[c] & kLeafBit)
+            for (uint32_t k = 0; k < (w.child[c] & kCountMask); k++) S->mesh_slots.push_back(w.first[c] + k);
+          else dfs.push_back(w.child[c]);
+        }
+      }
+    }
+    S->slot_begin[d->n_objects] = S->mesh_slots.size();
+  } catch (const std::bad_alloc&) {
+    return rh::set_error(RH_ERR_OOM, "rh_scene_create: out of host memory");
+  }
+  const char* env_setup = getenv("RAYHS_B200_SETUP");
+  const HostGeometry on_host{&cull, &dtris};
+  if ((rc = derive_tables(D, *S, d->materials, d->n_materials, d->lights, d->n_lights,
+                          env_setup && strcmp(env_setup, "host") == 0 ? &on_host : nullptr, nullptr, S.get(), nullptr, "rh_scene_create")))
+    return rc;
+  *out = S.release();
+  return RH_OK;
+}
+
+// Device buffers of one table build that do not outlive it.
+struct ScratchBufs {
+  std::vector<DevBuf> bufs;
+  ~ScratchBufs() {
+    for (DevBuf& b : bufs) b.release();
+  }
+};
+
+// Everything rh_scene_create derives from the material and light tables: the object records (is_emitter), the occluder
+// tables and what depends on them (shadow_fast, refill_possible, deep_entries), has_transparent, tables_in_smem, and the
+// light-space tables of the shadow kernels.  G is the scene whose geometry the tables are for.  They go into T's buffers,
+// view and host copies: T is G in rh_scene_create, a fresh scene in rh_scene_update, which swaps them in on success.
+// old (rh_scene_update with an unchanged occluder set): earlier device-built tables of G whose cube maps and lit-triangle
+// bits are carried over where the light they belong to did not move; else every table is built anew.  host: build the
+// light tables with the host builders (rh_scene_create only); null: on the device.
+int derive_tables(Device* D, const rh_scene& G, const rh_material* mats, uint32_t n_materials, const rh_light* lights,
+                  uint32_t n_lights, const HostGeometry* host, const rh_scene* old, rh_scene* T, rh_update_info* info,
+                  const std::string& w) {
+  using clk = std::chrono::steady_clock;
+  const clk::time_point t_begin = clk::now();
+  RH_CUDA(cudaSetDevice(D->dev));
+  int rc;
+  std::vector<DObject> objs;
   std::vector<OccPlane> occ_planes;
   std::vector<OccSphere> occ_spheres;
-  std::vector<uint32_t> occ_meshes;
-  for (uint32_t i : lin_objs) {
-    const DObject& o = objs[i];
-    if (o.is_emitter) continue;
-    if (o.kind == RH_OBJ_PLANE) {
-      OccPlane q;
-      memcpy(q.p, o.a, sizeof q.p);
-      memcpy(q.n, o.b, sizeof q.n);
-      occ_planes.push_back(q);
-    } else if (o.kind == RH_OBJ_SPHERE) {
-      OccSphere q;
-      memcpy(q.c, o.a, sizeof q.c);
-      q.r = o.b[0];
-      occ_spheres.push_back(q);
-    } else if (o.root != kEmpty) {
-      occ_meshes.push_back(o.root);
+  std::vector<uint32_t> occ_meshes, occ_objs;  // occluder meshes: super-root, object index
+  try {
+    objs = G.objs_host;
+    for (DObject& o : objs) o.is_emitter = mats[o.material].kind == RH_MAT_EMMIT;
+    T->materials_host.assign(mats, mats + n_materials);
+    T->lights_host.assign(lights, lights + n_lights);
+    // occluder tables (isOccluder, RayHs.hs:81-82: everything but Emmit objects)
+    for (uint32_t i : G.lin_objs_host) {
+      const DObject& o = objs[i];
+      if (o.is_emitter) continue;
+      if (o.kind == RH_OBJ_PLANE) {
+        OccPlane q;
+        memcpy(q.p, o.a, sizeof q.p);
+        memcpy(q.n, o.b, sizeof q.n);
+        occ_planes.push_back(q);
+      } else if (o.kind == RH_OBJ_SPHERE) {
+        OccSphere q;
+        memcpy(q.c, o.a, sizeof q.c);
+        q.r = o.b[0];
+        occ_spheres.push_back(q);
+      } else if (o.root != kEmpty) {
+        occ_meshes.push_back(o.root);
+        occ_objs.push_back(i);
+      }
     }
+  } catch (const std::bad_alloc&) {
+    return rh::set_error(RH_ERR_OOM, w + ": out of host memory");
   }
-  if ((rc = upload(S->occ_planes, occ_planes.data(), occ_planes.size()))) return rc;
-  if ((rc = upload(S->occ_spheres, occ_spheres.data(), occ_spheres.size()))) return rc;
-  if ((rc = upload(S->occ_meshes, occ_meshes.data(), occ_meshes.size()))) return rc;
-  SceneView& v = S->view;
-  v.occ_planes = (const OccPlane*)S->occ_planes.p;
-  v.occ_spheres = (const OccSphere*)S->occ_spheres.p;
-  v.occ_meshes = (const uint32_t*)S->occ_meshes.p;
+  if ((rc = upload(T->objects, objs.data(), objs.size()))) return rc;
+  if ((rc = upload(T->materials, mats, n_materials))) return rc;
+  if ((rc = upload(T->lights, lights, n_lights))) return rc;
+  if ((rc = upload(T->occ_planes, occ_planes.data(), occ_planes.size()))) return rc;
+  if ((rc = upload(T->occ_spheres, occ_spheres.data(), occ_spheres.size()))) return rc;
+  if ((rc = upload(T->occ_meshes, occ_meshes.data(), occ_meshes.size()))) return rc;
+  SceneView& v = T->view;
+  v.objects = (const DObject*)T->objects.p;
+  v.materials = (const rh_material*)T->materials.p;
+  v.lights = (const rh_light*)T->lights.p;
+  v.n_materials = n_materials;
+  v.n_lights = n_lights;
+  v.occ_planes = (const OccPlane*)T->occ_planes.p;
+  v.occ_spheres = (const OccSphere*)T->occ_spheres.p;
+  v.occ_meshes = (const uint32_t*)T->occ_meshes.p;
   v.n_occ_planes = (uint32_t)occ_planes.size();
   v.n_occ_spheres = (uint32_t)occ_spheres.size();
   v.n_occ_meshes = (uint32_t)occ_meshes.size();
   v.shadow_fast = occ_planes.size() <= (size_t)kOccPlanes && occ_spheres.size() <= (size_t)kOccSpheres &&
-                  occ_meshes.size() <= (size_t)kOccMeshes && d->n_lights <= (uint32_t)kFastLights;
+                  occ_meshes.size() <= (size_t)kOccMeshes && n_lights <= (uint32_t)kFastLights;
+  v.tables_in_smem = (objs.size() <= (size_t)kSmemObjects && n_materials <= (uint32_t)kSmemObjects && n_lights <= (uint32_t)kSmemLights);
+  T->has_transparent = false;
+  for (uint32_t i = 0; i < n_materials; i++) T->has_transparent |= mats[i].kind == RH_MAT_TRANSPARENT;
   {
     // Deep-stack scratch (entries beyond the shared-memory short stack, and the exact walk's whole stack): a walk
     // stacks at most one entry per level of its tree; the per-lane-refill shadow kernel also stacks the other roots.
-    const uint32_t n_roots = (uint32_t)occ_meshes.size() + (sphere_root != kEmpty ? 1u : 0u);
-    S->refill_possible = n_roots <= 64;
-    const uint32_t float_need = cull_depth + (S->refill_possible ? n_roots : 1u) + 4;
-    S->deep_entries = std::max<uint32_t>(depth + 4, float_need > (uint32_t)kShortStack ? float_need - kShortStack : 1u);
+    const uint32_t n_roots = (uint32_t)occ_meshes.size() + (G.sphere_root != kEmpty ? 1u : 0u);
+    T->refill_possible = n_roots <= 64;
+    const uint32_t float_need = G.cull_depth + (T->refill_possible ? n_roots : 1u) + 4;
+    T->deep_entries = std::max<uint32_t>(G.ref_depth + 4, float_need > (uint32_t)kShortStack ? float_need - kShortStack : 1u);
   }
   // Light-space tables of the shadow kernels (light_maps.cpp): cube maps of the nearest possible occluder distance, one
   // per (point light, occluder mesh), and lit-triangle flags per (triangle, light of either kind).  Only the
   // shared-memory-table shadow kernels read them; RAYHS_B200_LIGHT_MAPS=0 switches the build off.
-  S->ms_upload = ms_since(t_mark);
-  t_mark = clk::now();
   v.light_maps = nullptr;
   v.lit_flags = nullptr;
   v.light_map_index = nullptr;
   v.light_map_res = 0;
+  T->n_light_maps = 0;
+  T->tables_res = 0;
+  T->map_index_host.clear();
+  T->mesh_lit.clear();
+  T->tables_on_device = host == nullptr;
+  const rh_tri* d_tris = (const rh_tri*)G.tris.p;
+  auto mesh_slots = [&](size_t m) { return G.mesh_slots.data() + G.slot_begin[occ_objs[m]]; };
+  auto mesh_n_slots = [&](size_t m) { return G.slot_begin[occ_objs[m] + 1] - G.slot_begin[occ_objs[m]]; };
   {
     const char* env = getenv("RAYHS_B200_LIGHT_MAPS");
     const char* env_res = getenv("RAYHS_B200_LIGHT_MAP_RES");
     const char* env_lit = getenv("RAYHS_B200_LIT_TRIANGLES");  // 0: no lit-triangle flags (A/B)
-    size_t n_pairs = 0;
-    for (uint32_t li = 0; li < d->n_lights; li++)
-      if (d->lights[li].kind == RH_LIGHT_POINT) n_pairs += occ_meshes.size();
-    if (v.shadow_fast && !occ_meshes.empty() && d->n_lights && !(env && env[0] == '0')) {
+    uint32_t n_point = 0;
+    for (uint32_t li = 0; li < n_lights; li++) n_point += lights[li].kind == RH_LIGHT_POINT;
+    const size_t n_pairs = (size_t)n_point * occ_meshes.size();
+    if (v.shadow_fast && !occ_meshes.empty() && n_lights && !(env && env[0] == '0')) {
       int R = env_res ? std::max(16, std::min(4096, atoi(env_res))) : kLightMapRes;
       while (R > 64 && std::max<size_t>(n_pairs, 1) * 6 * (size_t)R * R * sizeof(float) > kLightMapBudget) R /= 2;
       const size_t cells = (size_t)6 * R * R;
       try {
-        std::vector<uint32_t> index((size_t)d->n_lights * kOccMeshes, kEmpty);
-        std::vector<float> maps, one(cells);
-        std::vector<uint16_t> lit;
+        std::vector<uint32_t> index((size_t)n_lights * kOccMeshes, kEmpty);
         uint32_t n_maps = 0;
-        size_t n_lit = 0;
         // The tables are built on the GPU (setup_kernels.cu: the triangle records and the cull tree are already in
         // HBM); RAYHS_B200_SETUP=host keeps the host builders of light_maps.cpp — same geometry code (light_geom.h),
         // same tables bit for bit (tests/test_round2_gpu.py).
-        const char* env_setup = getenv("RAYHS_B200_SETUP");
-        const bool on_device = !(env_setup && strcmp(env_setup, "host") == 0);
-        std::vector<DevBuf> slot_bufs(on_device ? occ_meshes.size() : 0);
-        DevBuf words;
-        bool any_lit_query = false;
-        if (on_device) {
+        if (!host) {
+          // Maps of a light that did not move (same kind and position, at any index) are copied from the old tables
+          // into their place in the new numbering, with their old verdict; so are lit bits of unchanged light indices.
+          const bool reuse_maps = old && old->tables_on_device && old->tables_res == (uint32_t)R;
+          const std::vector<rh::MapStep> steps =
+              rh::plan_maps(reuse_maps ? old->map_index_host : std::vector<uint32_t>(),
+                            old ? rh::match_point_lights(old->lights_host.data(), (uint32_t)old->lights_host.size(), lights, n_lights)
+                                : std::vector<int32_t>(n_lights, -1),
+                            lights, n_lights, (uint32_t)occ_meshes.size());
+          ScratchBufs scratch;
+          scratch.bufs.resize(occ_meshes.size() + 1);
+          DevBuf& words = scratch.bufs.back();
+          std::vector<uint8_t> want(occ_meshes.size(), 0);
           if ((rc = words.reserve(64))) return rc;
           RH_CUDA(cudaMemsetAsync(words.p, 0, 64, D->stream));
-          if (n_pairs && (rc = S->light_maps.reserve(n_pairs * cells * sizeof(float)))) return rc;
-        }
-        for (size_t m = 0; on_device && m < occ_meshes.size(); m++) {
-          std::vector<uint32_t> slots, dfs{occ_meshes[m]};  // the mesh's triangles: leaves of its cull tree
-          while (!dfs.empty()) {
-            const WideNode& w = cull[dfs.back()];
-            dfs.pop_back();
-            for (int c = 0; c < 2; c++) {
-              if (w.child[c] == kEmpty) continue;
-              if (w.child[c] & kLeafBit)
-                for (uint32_t k = 0; k < (w.child[c] & kCountMask); k++) slots.push_back(w.first[c] + k);
-              else dfs.push_back(w.child[c]);
+          if (n_pairs && (rc = T->light_maps.reserve(n_pairs * cells * sizeof(float)))) return rc;
+          for (size_t m = 0; m < occ_meshes.size(); m++) {
+            const size_t n_slots = mesh_n_slots(m);
+            if (!n_slots) continue;
+            if ((rc = upload(scratch.bufs[m], mesh_slots(m), n_slots))) return rc;
+            const uint32_t* d_slots = (const uint32_t*)scratch.bufs[m].p;
+            // the cube maps first: a mesh none of whose maps is worth having is a triangle soup around its lights, where
+            // nearly every triangle is shadowed by another one — the lit-triangle queries (long hulls through the whole
+            // soup, ~0.25 us each on the GPU) are not made either
+            uint32_t useful_maps = 0;
+            for (uint32_t j = 0; j < n_point; j++) {
+              const rh::MapStep& st = steps[m * n_point + j];
+              float* dst = (float*)T->light_maps.p + (size_t)n_maps * cells;
+              int useful = 0;
+              if (st.raster) {
+                double empty = 0;
+                RH_CUDA((cudaError_t)device_light_map(lights[st.light].vec, d_tris, d_slots, n_slots, R, dst, kLightMapMinEmpty,
+                                                      (unsigned long long*)words.p, &useful, &empty, D->stream));
+                if (info) info->maps_rasterised++;
+              } else if (st.old_map != kEmpty) {
+                RH_CUDA(cudaMemcpyAsync(dst, (const float*)old->light_maps.p + (size_t)st.old_map * cells, cells * sizeof(float),
+                                        cudaMemcpyDeviceToDevice, D->stream));
+                useful = 1;
+                if (info) info->maps_kept++;
+              }
+              if (useful) {
+                index[(size_t)st.light * kOccMeshes + m] = n_maps++;
+                useful_maps++;
+              }
             }
+            want[m] = n_slots * (size_t)n_lights <= kLitMaxQueriesDevice && !(env_lit && env_lit[0] == '0') &&
+                      (n_point == 0 || useful_maps > 0);
           }
-          if (slots.empty()) continue;
-          if ((rc = upload(slot_bufs[m], slots.data(), slots.size()))) return rc;
-          const uint32_t* d_slots = (const uint32_t*)slot_bufs[m].p;
-          // the cube maps first: a mesh none of whose maps is worth having is a triangle soup around its lights, where
-          // nearly every triangle is shadowed by another one — the lit-triangle queries (long hulls through the whole
-          // soup, ~0.25 us each on the GPU) are not made either
-          uint32_t point_lights = 0, useful_maps = 0;
-          for (uint32_t li = 0; li < d->n_lights; li++) {
-            if (d->lights[li].kind != RH_LIGHT_POINT) continue;
-            point_lights++;
-            int useful = 0;
-            double empty = 0;
-            RH_CUDA((cudaError_t)device_light_map(d->lights[li].vec, (const rh_tri*)S->tris.p, d_slots, slots.size(), R,
-                                                  (float*)S->light_maps.p + (size_t)n_maps * cells, kLightMapMinEmpty,
-                                                  (unsigned long long*)words.p, &useful, &empty, D->stream));
-            if (useful) {
-              index[(size_t)li * kOccMeshes + m] = n_maps++;
-              useful_maps++;
+          // lit triangles: the old bits of every light index whose light kept its kind and position stay, as long as
+          // every mesh that had bits still has them (a mesh that gains them is queried for every light)
+          const uint32_t all = n_lights >= 12 ? 0x0fffu : (1u << n_lights) - 1;
+          bool reuse_lit = old && old->tables_on_device && old->tables_res && old->lit_flags.p && old->mesh_lit.size() == occ_meshes.size();
+          for (size_t m = 0; reuse_lit && m < occ_meshes.size(); m++) reuse_lit = !(old->mesh_lit[m] && !want[m]);
+          const uint32_t changed =
+              reuse_lit ? rh::lit_changed_mask(old->lights_host.data(), (uint32_t)old->lights_host.size(), lights, n_lights) : all;
+          for (size_t m = 0; m < occ_meshes.size(); m++) {
+            if (!want[m]) continue;
+            if (!T->lit_flags.p) {
+              const size_t lit_bytes = ((G.view.n_tris + 1) / 2) * 4;  // (whole 32-bit words: the kernel sets bits with atomicOr)
+              if ((rc = T->lit_flags.reserve(std::max<size_t>(lit_bytes, 256)))) return rc;
+              if (reuse_lit)
+                RH_CUDA(cudaMemcpyAsync(T->lit_flags.p, old->lit_flags.p, T->lit_flags.bytes, cudaMemcpyDeviceToDevice, D->stream));
+              else
+                RH_CUDA(cudaMemsetAsync(T->lit_flags.p, 0, T->lit_flags.bytes, D->stream));
             }
+            const uint32_t mask = reuse_lit && old->mesh_lit[m] ? changed : all;
+            RH_CUDA((cudaError_t)device_lit_flags(d_tris, (const WideNode32*)G.wide32.p, G.view.center, occ_meshes[m],
+                                                  (const uint32_t*)scratch.bufs[m].p, (uint32_t)mesh_n_slots(m),
+                                                  (const rh_light*)T->lights.p, n_lights, mask, (uint32_t)m, (uint16_t*)T->lit_flags.p,
+                                                  (unsigned long long*)words.p + 2, D->stream));
+            if (info) info->lit_queries += (uint64_t)mesh_n_slots(m) * (uint64_t)__builtin_popcount(mask & all);
           }
-          const bool want_lit = slots.size() * (size_t)d->n_lights <= kLitMaxQueriesDevice && !(env_lit && env_lit[0] == '0') &&
-                                (point_lights == 0 || useful_maps > 0);
-          if (want_lit) {
-            if (!any_lit_query) {
-              const size_t lit_bytes = ((dtris.size() + 1) / 2) * 4;  // (whole 32-bit words: the kernel sets bits with atomicOr)
-              if ((rc = S->lit_flags.reserve(std::max<size_t>(lit_bytes, 256)))) return rc;
-              RH_CUDA(cudaMemsetAsync(S->lit_flags.p, 0, S->lit_flags.bytes, D->stream));
-              any_lit_query = true;
-            }
-            RH_CUDA((cudaError_t)device_lit_flags((const rh_tri*)S->tris.p, (const WideNode32*)S->wide32.p, center, occ_meshes[m], d_slots,
-                                                  (uint32_t)slots.size(), (const rh_light*)S->lights.p, d->n_lights, (uint32_t)m,
-                                                  (uint16_t*)S->lit_flags.p, (unsigned long long*)words.p + 2, D->stream));
-          }
-        }
-        if (on_device) {
           unsigned long long flagged = 0;
           RH_CUDA(cudaMemcpyAsync(&flagged, (unsigned long long*)words.p + 2, 8, cudaMemcpyDeviceToHost, D->stream));
           RH_CUDA(cudaStreamSynchronize(D->stream));
-          for (DevBuf& b : slot_bufs) b.release();
-          words.release();
-          if (flagged) v.lit_flags = (const uint16_t*)S->lit_flags.p;
-          else S->lit_flags.release();
+          if (flagged) v.lit_flags = (const uint16_t*)T->lit_flags.p;
+          else T->lit_flags.release();
           if (n_maps) {
-            if ((rc = upload(S->light_map_index, index.data(), index.size()))) return rc;
-            v.light_maps = (const float*)S->light_maps.p;
-            v.light_map_index = (const uint32_t*)S->light_map_index.p;
+            if ((rc = upload(T->light_map_index, index.data(), index.size()))) return rc;
+            v.light_maps = (const float*)T->light_maps.p;
+            v.light_map_index = (const uint32_t*)T->light_map_index.p;
             v.light_map_res = (uint32_t)R;
           } else {
-            S->light_maps.release();
+            T->light_maps.release();
           }
-        }
-        for (size_t m = 0; !on_device && m < occ_meshes.size(); m++) {
-          std::vector<uint32_t> slots, dfs{occ_meshes[m]};  // the mesh's triangles: leaves of its cull tree
-          while (!dfs.empty()) {
-            const WideNode& w = cull[dfs.back()];
-            dfs.pop_back();
-            for (int c = 0; c < 2; c++) {
-              if (w.child[c] == kEmpty) continue;
-              if (w.child[c] & kLeafBit)
-                for (uint32_t k = 0; k < (w.child[c] & kCountMask); k++) slots.push_back(w.first[c] + k);
-              else dfs.push_back(w.child[c]);
-            }
-          }
+          T->mesh_lit = want;
+        } else {
+          const std::vector<WideNode>& cull = *host->cull;
+          const TriVec& dtris = *host->tris;
+          std::vector<float> maps, one(cells);
+          std::vector<uint16_t> lit;
+          size_t n_lit = 0;
+          for (size_t m = 0; m < occ_meshes.size(); m++) {
+            const std::vector<uint32_t> slots(mesh_slots(m), mesh_slots(m) + mesh_n_slots(m));
           // lit triangles: per triangle and light, can another triangle of this mesh shadow it at all?  The queries
           // run on their own threads while this one builds the mesh's cube maps.
-          const bool want_lit = slots.size() * (size_t)d->n_lights <= kLitMaxQueries && !(env_lit && env_lit[0] == '0');
+          const bool want_lit = slots.size() * (size_t)n_lights <= kLitMaxQueries && !(env_lit && env_lit[0] == '0');
           if (want_lit && lit.empty()) lit.assign(dtris.size(), 0);
           size_t lit_found = 0;
           bool lit_failed = false;
@@ -1189,9 +1337,9 @@ int scene_create_on(Device* D, const rh_scene_desc* d, rh_scene** out) {
                 for (size_t at = begin; at < std::min(begin + 256, slots.size()); at++) {
                   const uint32_t s0 = slots[at];
                   uint32_t bits = 0;
-                  for (uint32_t li = 0; li < d->n_lights && li < 12; li++) {
+                  for (uint32_t li = 0; li < n_lights && li < 12; li++) {
                     rh::LitQuery q;
-                    if (!rh::lit_query_make(dtris[s0], d->lights[li].vec, d->lights[li].kind == RH_LIGHT_DIRECTIONAL, &q)) continue;
+                    if (!rh::lit_query_make(dtris[s0], lights[li].vec, lights[li].kind == RH_LIGHT_DIRECTIONAL, &q)) continue;
                     bool blocked = false;
                     walk.assign(1, occ_meshes[m]);
                     while (!walk.empty() && !blocked) {
@@ -1237,11 +1385,11 @@ int scene_create_on(Device* D, const rh_scene_desc* d, rh_scene** out) {
           bool maps_failed = false;
           uint32_t point_lights = 0, useful_maps = 0;
           try {
-            for (uint32_t li = 0; li < d->n_lights; li++) {
-              if (d->lights[li].kind != RH_LIGHT_POINT) continue;
+            for (uint32_t li = 0; li < n_lights; li++) {
+              if (lights[li].kind != RH_LIGHT_POINT) continue;
               point_lights++;
               double empty = 0;
-              if (!rh::build_light_map(d->lights[li].vec, dtris.data(), slots.data(), slots.size(), R, one.data(), kLightMapMinEmpty, &empty))
+              if (!rh::build_light_map(lights[li].vec, dtris.data(), slots.data(), slots.size(), R, one.data(), kLightMapMinEmpty, &empty))
                 continue;
               index[(size_t)li * kOccMeshes + m] = n_maps++;
               useful_maps++;
@@ -1255,57 +1403,30 @@ int scene_create_on(Device* D, const rh_scene_desc* d, rh_scene** out) {
           if (lit_thread.joinable()) lit_thread.join();
           if (lit_failed || maps_failed) throw std::bad_alloc();
           n_lit += lit_found;
+          }
+          if (n_lit) {
+            if ((rc = upload(T->lit_flags, lit.data(), lit.size()))) return rc;
+            v.lit_flags = (const uint16_t*)T->lit_flags.p;
+          }
+          if (n_maps) {
+            if ((rc = upload(T->light_maps, maps.data(), maps.size()))) return rc;
+            if ((rc = upload(T->light_map_index, index.data(), index.size()))) return rc;
+            v.light_maps = (const float*)T->light_maps.p;
+            v.light_map_index = (const uint32_t*)T->light_map_index.p;
+            v.light_map_res = (uint32_t)R;
+          }
         }
-        if (!on_device && n_lit) {
-          if ((rc = upload(S->lit_flags, lit.data(), lit.size()))) return rc;
-          v.lit_flags = (const uint16_t*)S->lit_flags.p;
-        }
-        if (!on_device && n_maps) {
-          if ((rc = upload(S->light_maps, maps.data(), maps.size()))) return rc;
-          if ((rc = upload(S->light_map_index, index.data(), index.size()))) return rc;
-          v.light_maps = (const float*)S->light_maps.p;
-          v.light_map_index = (const uint32_t*)S->light_map_index.p;
-          v.light_map_res = (uint32_t)R;
-        }
+        for (uint32_t x : index)
+          if (x != kEmpty) T->n_light_maps = std::max(T->n_light_maps, x + 1);
+        T->tables_res = (uint32_t)R;
+        T->map_index_host.swap(index);
       } catch (const std::bad_alloc&) {
-        return rh::set_error(RH_ERR_OOM, "rh_scene_create: out of host memory");
+        return rh::set_error(RH_ERR_OOM, w + ": out of host memory");
       }
     }
   }
-  S->ms_light_tables = ms_since(t_mark);
-  S->n_light_maps = 0;
-  if (v.light_map_index) {
-    std::vector<uint32_t> idx((size_t)d->n_lights * kOccMeshes);
-    RH_CUDA(cudaMemcpy(idx.data(), v.light_map_index, idx.size() * sizeof(uint32_t), cudaMemcpyDeviceToHost));
-    for (uint32_t x : idx)
-      if (x != kEmpty) S->n_light_maps = std::max(S->n_light_maps, x + 1);
-  }
-  v.wide = (const WideNode*)S->wide.p;
-  v.wide32 = (const WideNode32*)S->wide32.p;
-  v.abs_max = abs_max;
-  for (int k = 0; k < 3; k++) v.center[k] = center[k];
-  v.tris = (const rh_tri*)S->tris.p;
-  v.shade = (const rh_tri_shade*)S->shade.p;
-  v.objects = (const DObject*)S->objects.p;
-  v.materials = (const rh_material*)S->materials.p;
-  v.lights = (const rh_light*)S->lights.p;
-  v.textures = (const rh_texture*)S->textures.p;
-  v.texels = (const double*)S->texels.p;
-  v.n_wide = (uint32_t)cull.size();
-  v.n_tris = (uint32_t)dtris.size();  // triangle slots on the device (the meshes' triangles, in cull-tree leaf order)
-  v.n_objects = d->n_objects;
-  v.n_materials = d->n_materials;
-  v.n_lights = d->n_lights;
-  v.n_textures = d->n_textures;
-  v.lin_objs = (const uint32_t*)S->lin_objs.p;
-  v.sphere_refs = (const uint32_t*)S->sphere_refs.p;
-  v.exact_index = exact_index.empty() ? nullptr : (const uint32_t*)S->exact_index.p;
-  v.n_lin = (uint32_t)lin_objs.size();
-  v.sphere_root = sphere_root;
-  v.n_smem_nodes = std::min<uint32_t>(v.n_wide, kSmemNodes);
-  v.tables_in_smem = (d->n_objects <= (uint32_t)kSmemObjects && d->n_materials <= (uint32_t)kSmemObjects &&
-                      d->n_lights <= (uint32_t)kSmemLights);
-  *out = S.release();
+  T->objs_host.swap(objs);
+  T->ms_light_tables = std::chrono::duration<double, std::milli>(clk::now() - t_begin).count();
   return RH_OK;
 }
 
@@ -1317,6 +1438,120 @@ void scene_destroy(rh_scene* s) {
                     &s->light_map_index, &s->lit_flags})
     b->release();
   delete s;
+}
+
+// ------------------------------------------------------------------ scene updates (DESIGN.md "Scene updates")
+// The fields derive_tables fills: a prepared update is swapped in with them, and the old tables leave with the scratch
+// scene.
+void swap_tables(rh_scene& a, rh_scene& b) {
+  for (auto f : {&rh_scene::objects, &rh_scene::materials, &rh_scene::lights, &rh_scene::occ_planes, &rh_scene::occ_spheres,
+                 &rh_scene::occ_meshes, &rh_scene::light_maps, &rh_scene::light_map_index, &rh_scene::lit_flags})
+    std::swap(a.*f, b.*f);
+  std::swap(a.deep_entries, b.deep_entries);
+  std::swap(a.refill_possible, b.refill_possible);
+  std::swap(a.has_transparent, b.has_transparent);
+  std::swap(a.n_light_maps, b.n_light_maps);
+  std::swap(a.ms_light_tables, b.ms_light_tables);
+  std::swap(a.objs_host, b.objs_host);
+  std::swap(a.materials_host, b.materials_host);
+  std::swap(a.lights_host, b.lights_host);
+  std::swap(a.tables_res, b.tables_res);
+  std::swap(a.map_index_host, b.map_index_host);
+  std::swap(a.mesh_lit, b.mesh_lit);
+  std::swap(a.tables_on_device, b.tables_on_device);
+  SceneView &x = a.view, &y = b.view;
+  std::swap(x.objects, y.objects);
+  std::swap(x.materials, y.materials);
+  std::swap(x.lights, y.lights);
+  std::swap(x.occ_planes, y.occ_planes);
+  std::swap(x.occ_spheres, y.occ_spheres);
+  std::swap(x.occ_meshes, y.occ_meshes);
+  std::swap(x.light_maps, y.light_maps);
+  std::swap(x.light_map_index, y.light_map_index);
+  std::swap(x.lit_flags, y.lit_flags);
+  for (auto f : {&SceneView::n_materials, &SceneView::n_lights, &SceneView::n_occ_planes, &SceneView::n_occ_spheres,
+                 &SceneView::n_occ_meshes, &SceneView::shadow_fast, &SceneView::tables_in_smem, &SceneView::light_map_res})
+    std::swap(x.*f, y.*f);
+}
+
+// Validates an update of S and builds its new tables into a fresh scene *out (null when nothing changed); S is not
+// touched.  *cls: the update's class (scene_update.h).
+int scene_update_prepare(rh_scene* S, const rh_material* materials, uint32_t n_materials, const rh_light* lights, uint32_t n_lights,
+                         rh_update_info* info, const std::string& w, int* cls, std::unique_ptr<rh_scene>* out) {
+  out->reset();
+  *cls = rh::kUpdateNone;
+  if (info) memset(info, 0, sizeof *info);
+  if (n_materials != S->materials_host.size())
+    return rh::set_error(RH_ERR_ARG, w + ": n_materials (" + std::to_string(n_materials) + ") differs from the scene's material count (" +
+                                         std::to_string(S->materials_host.size()) + ")");
+  const rh_material* mats = materials ? materials : S->materials_host.data();
+  if (!lights) {
+    lights = S->lights_host.data();
+    n_lights = (uint32_t)S->lights_host.size();
+  }
+  int rc = check_tables(mats, n_materials, S->textures_host.data(), (uint32_t)S->textures_host.size(), S->n_texels, lights, n_lights, w);
+  if (rc) return rc;
+  std::vector<int32_t> object_material;
+  try {
+    for (const DObject& o : S->objs_host) object_material.push_back(o.material);
+  } catch (const std::bad_alloc&) {
+    return rh::set_error(RH_ERR_OOM, w + ": out of host memory");
+  }
+  *cls = rh::classify_update(S->materials_host.data(), mats, n_materials, S->lights_host.data(), (uint32_t)S->lights_host.size(), lights,
+                             n_lights, object_material);
+  if (*cls == rh::kUpdateNone) return RH_OK;
+  auto N = std::make_unique<rh_scene>();
+  N->device = S->device;
+  if (*cls == rh::kUpdateColours) {
+    // the kernels read these two tables on every call; nothing is derived from the fields that changed
+    if (info) info->colours_only = 1;
+    try {
+      N->materials_host.assign(mats, mats + n_materials);
+      N->lights_host.assign(lights, lights + n_lights);
+    } catch (const std::bad_alloc&) {
+      return rh::set_error(RH_ERR_OOM, w + ": out of host memory");
+    }
+    RH_CUDA(cudaSetDevice(S->device->dev));
+    if ((rc = upload(N->materials, mats, n_materials)) || (rc = upload(N->lights, lights, n_lights))) {
+      scene_destroy(N.release());
+      return rc;
+    }
+  } else {
+    if (info) info->occluders_rebuilt = *cls == rh::kUpdateEmitters;
+    rc = derive_tables(S->device, *S, mats, n_materials, lights, n_lights, nullptr, *cls == rh::kUpdateTables ? S : nullptr, N.get(),
+                       info, w);
+    if (rc) {
+      scene_destroy(N.release());
+      return rc;
+    }
+  }
+  *out = std::move(N);
+  return RH_OK;
+}
+
+// Swaps a prepared update in and releases the old tables.  Frames after a change of the light tables or the occluders
+// cast other rays, so the scene's learned state (shadow schedule, queue factor, row costs) starts over as a fresh scene's.
+void scene_update_commit(rh_scene* S, std::unique_ptr<rh_scene> N, int cls) {
+  if (!N) return;
+  if (cls == rh::kUpdateColours) {
+    std::swap(S->materials, N->materials);
+    std::swap(S->lights, N->lights);
+    std::swap(S->materials_host, N->materials_host);
+    std::swap(S->lights_host, N->lights_host);
+    S->view.materials = (const rh_material*)S->materials.p;
+    S->view.lights = (const rh_light*)S->lights.p;
+  } else {
+    swap_tables(*S, *N);
+    S->shadow_mode = 0;
+    S->tune_frames = S->tune_small_frames = 0;
+    S->tune_ns_per_pair[0] = S->tune_ns_per_pair[1] = 0;
+    S->cost_key.clear();
+    S->row_cost.clear();
+    S->queue_factor = 2;
+    S->stream_compute_bound = false;
+  }
+  S->generation++;
+  scene_destroy(N.release());
 }
 
 // ------------------------------------------------------------------ camera (Projection.hs:22-46, Mat.hs:83-93)
@@ -2040,10 +2275,13 @@ int shard_state_matches(const ShardState* S, const Frame& f, bool fixed, const r
     return rh::set_error(RH_ERR_ARG, w + ": width, height, shard_index, shard_count or band_height differ from the " + noun + "'s");
   if (fixed && (scene != S->scene || memcmp(camera, &S->camera, sizeof S->camera) != 0 || f.o.max_depth != S->max_depth))
     return rh::set_error(RH_ERR_ARG, w + ": scene, camera or max_depth differ from the " + noun + "'s first call; " + reset + " it first");
+  if (fixed && scene->generation != S->scene_generation)
+    return rh::set_error(RH_ERR_ARG, w + ": the scene was updated since the " + noun + "'s first call; " + reset + " it first");
   return RH_OK;
 }
 void shard_state_fix_view(ShardState* S, const rh_scene* scene, const rh_camera* camera, int32_t max_depth) {
   S->scene = scene;
+  S->scene_generation = scene->generation;
   S->camera = *camera;
   S->max_depth = max_depth;
 }
@@ -2516,6 +2754,18 @@ int rh_scene_light_tables(const rh_scene* scene, uint32_t* info4, float* maps_ou
   return RH_OK;
 }
 
+int rh_scene_update(rh_scene* scene, const rh_material* materials, uint32_t n_materials, const rh_light* lights, uint32_t n_lights,
+                    rh_update_info* info) {
+  const std::string w = "rh_scene_update";
+  if (!scene) return rh::set_error(RH_ERR_ARG, w + ": null scene");
+  int cls = 0;
+  std::unique_ptr<rh_scene> N;
+  int rc = scene_update_prepare(scene, materials, n_materials, lights, n_lights, info, w, &cls, &N);
+  if (rc) return rc;
+  scene_update_commit(scene, std::move(N), cls);
+  return RH_OK;
+}
+
 int rh_cull_tree_build(const rh_tri* tris, uint32_t n_tris, uint32_t* order_out, rh_node* nodes_out, uint32_t* n_nodes_out,
                        uint32_t* depth_out) {
   if ((!tris && n_tris) || !order_out || !nodes_out || !n_nodes_out) return rh::set_error(RH_ERR_ARG, "rh_cull_tree_build: null argument");
@@ -2727,6 +2977,25 @@ void rh_multi_scene_destroy(rh_multi_scene* scene) {
   if (!scene) return;
   for (rh_scene* r : scene->replica) scene_destroy(r);
   delete scene;
+}
+
+int rh_multi_scene_update(rh_multi_scene* scene, const rh_material* materials, uint32_t n_materials, const rh_light* lights,
+                          uint32_t n_lights, rh_update_info* info) {
+  const std::string w = "rh_multi_scene_update";
+  if (!scene || scene->replica.empty()) return rh::set_error(RH_ERR_ARG, w + ": null scene");
+  // every replica is prepared before any is swapped: the update takes on all GPUs or on none
+  std::vector<std::unique_ptr<rh_scene>> prepared(scene->replica.size());
+  int cls = 0;
+  for (size_t g = 0; g < scene->replica.size(); g++) {
+    int rc = scene_update_prepare(scene->replica[g], materials, n_materials, lights, n_lights, g == 0 ? info : nullptr, w, &cls, &prepared[g]);
+    if (rc) {
+      for (auto& p : prepared)
+        if (p) scene_destroy(p.release());
+      return rc;
+    }
+  }
+  for (size_t g = 0; g < scene->replica.size(); g++) scene_update_commit(scene->replica[g], std::move(prepared[g]), cls);
+  return RH_OK;
 }
 
 int rh_multi_render(const rh_multi_scene* scene, const rh_camera* camera, const rh_render_opts* opts, uint8_t* rgb_out,

@@ -70,21 +70,26 @@ __global__ void count_empty_kernel(const uint32_t* __restrict__ cells, size_t n,
   if ((threadIdx.x & 31) == 0 && mine) atomicAdd(out, mine);
 }
 
-// Lit flags of one mesh: lit[slot] = mesh << 12 first, then one thread per (triangle of the mesh, light) clears nothing
-// and sets bit `light` when no other triangle of the mesh meets the triangle's query region K.
-__global__ void lit_init_kernel(const uint32_t* __restrict__ slots, uint32_t n_slots, uint32_t mesh, uint16_t* __restrict__ lit) {
+// Lit flags of one mesh for the lights in `mask`: lit[slot] gets the mesh in bits 12-15 and loses the mask's light bits
+// first (the other lights' bits stay), then one thread per (triangle of the mesh, light of the mask) clears nothing and
+// sets bit `light` when no other triangle of the mesh meets the triangle's query region K.
+__global__ void lit_init_kernel(const uint32_t* __restrict__ slots, uint32_t n_slots, uint32_t mesh, uint32_t mask,
+                                uint16_t* __restrict__ lit) {
   const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
-  if (i < n_slots) lit[slots[i]] = (uint16_t)(mesh << 12);
+  if (i < n_slots) lit[slots[i]] = (uint16_t)((lit[slots[i]] & 0x0fffu & ~mask) | (mesh << 12));
 }
 
 __global__ void __launch_bounds__(128) lit_query_kernel(const rh_tri* __restrict__ tris, const WideNode32* __restrict__ nodes,
                                                         double cx, double cy, double cz, uint32_t root,
                                                         const uint32_t* __restrict__ slots, uint32_t n_slots,
-                                                        const rh_light* __restrict__ lights, uint32_t n_lights,
+                                                        const rh_light* __restrict__ lights, uint32_t mask, uint32_t n_mask,
                                                         uint32_t* __restrict__ lit_words) {
   const uint32_t idx = blockIdx.x * blockDim.x + threadIdx.x;
-  const uint32_t at = idx / n_lights, li = idx - at * n_lights;
+  const uint32_t at = idx / n_mask;
   if (at >= n_slots) return;
+  uint32_t rest = mask;  // the light: set bit number (idx - at * n_mask) of the mask
+  for (uint32_t k = idx - at * n_mask; k; k--) rest &= rest - 1;
+  const uint32_t li = (uint32_t)__ffs(rest) - 1;
   const uint32_t s0 = slots[at];
   rh::LitQuery q;
   const rh_light L = lights[li];
@@ -194,19 +199,24 @@ int device_light_map(const double L[3], const rh_tri* d_tris, const uint32_t* d_
   return 0;
 }
 
-// Device version of the lit-triangle queries of one mesh (runtime.cu's host loop): enqueues only; the flags of the
-// mesh's slots are complete when the stream has run.  d_flagged: device counter, incremented by the number of
-// triangles of this mesh with at least one flag.
+// Device version of the lit-triangle queries of one mesh (runtime.cu's host loop) for the light indices in `mask` (bits
+// below 12): clears those bits on the mesh's slots, writes the mesh into bits 12-15 and queries those of the lights
+// 0 .. n_lights-1 only; the other bits stay.  mask 0 only counts.  Enqueues only; the flags of the mesh's slots are
+// complete when the stream has run.  d_flagged: device counter, incremented by the number of triangles of this mesh with
+// at least one flag.
 int device_lit_flags(const rh_tri* d_tris, const WideNode32* d_nodes, const double center[3], uint32_t root, const uint32_t* d_slots,
-                     uint32_t n_slots, const rh_light* d_lights, uint32_t n_lights, uint32_t mesh, uint16_t* d_lit,
+                     uint32_t n_slots, const rh_light* d_lights, uint32_t n_lights, uint32_t mask, uint32_t mesh, uint16_t* d_lit,
                      unsigned long long* d_flagged, void* stream_) {
   cudaStream_t st = (cudaStream_t)stream_;
-  if (!n_slots || !n_lights) return 0;
-  const uint32_t nl = n_lights < 12 ? n_lights : 12;
-  lit_init_kernel<<<(n_slots + 255) / 256, 256, 0, st>>>(d_slots, n_slots, mesh, d_lit);
-  const unsigned long long threads = (unsigned long long)n_slots * nl;
-  lit_query_kernel<<<(unsigned)((threads + 127) / 128), 128, 0, st>>>(d_tris, d_nodes, center[0], center[1], center[2], root, d_slots, n_slots,
-                                                                      d_lights, nl, (uint32_t*)d_lit);
+  if (!n_slots) return 0;
+  mask &= 0x0fffu;
+  const uint32_t query = mask & (n_lights >= 12 ? 0x0fffu : (1u << n_lights) - 1), n_query = (uint32_t)__builtin_popcount(query);
+  if (mask) lit_init_kernel<<<(n_slots + 255) / 256, 256, 0, st>>>(d_slots, n_slots, mesh, mask, d_lit);
+  if (n_query) {
+    const unsigned long long threads = (unsigned long long)n_slots * n_query;
+    lit_query_kernel<<<(unsigned)((threads + 127) / 128), 128, 0, st>>>(d_tris, d_nodes, center[0], center[1], center[2], root, d_slots,
+                                                                        n_slots, d_lights, query, n_query, (uint32_t*)d_lit);
+  }
   lit_count_kernel<<<(n_slots + 255) / 256, 256, 0, st>>>(d_slots, n_slots, d_lit, d_flagged);
   return (int)cudaGetLastError();
 }

@@ -49,6 +49,8 @@ class Scene:
         L.rh_loaded_size(loaded, C.byref(w), C.byref(h), C.byref(d))
         self.width, self.height, self.max_depth = w.value, h.value, d.value
         self.camera = capi.rh_camera.from_buffer_copy(L.rh_loaded_camera(loaded).contents)
+        self._tables = None  # (materials, lights) ctypes arrays after update(): what raw and flat describe from then on
+        self._raw_view = self._flat_view = None
 
     # ---- construction (front end)
     @staticmethod
@@ -76,15 +78,75 @@ class Scene:
     # ---- views
     @property
     def raw(self):
-        """POINTER(rh_raw_scene): the scene before any tree build (what the oracle is fed)."""
-        return lib().rh_loaded_raw(self._loaded)
+        """POINTER(rh_raw_scene): the scene before any tree build (what the oracle is fed), with the tables of the last
+        update()."""
+        r = lib().rh_loaded_raw(self._loaded)
+        if self._tables is None:
+            return r
+        self._raw_view = self._patched(capi.rh_raw_scene, r)
+        return C.pointer(self._raw_view)
 
     @property
     def flat(self):
-        """POINTER(rh_scene_desc): KDTree.hs:68-90 build + flattening, on the host."""
+        """POINTER(rh_scene_desc): KDTree.hs:68-90 build + flattening, on the host, with the tables of the last update()."""
         if not self._flat:
             check(lib().rh_flatten(self.raw, C.byref(self._flat)))
-        return lib().rh_flat_desc(self._flat)
+        d = lib().rh_flat_desc(self._flat)
+        if self._tables is None:
+            return d
+        self._flat_view = self._patched(capi.rh_scene_desc, d)
+        return C.pointer(self._flat_view)
+
+    def _patched(self, struct, ptr):
+        """A copy of the library's description whose material and light tables are this Scene's (kept alive by it)."""
+        mats, lights = self._tables
+        c = struct.from_buffer_copy(ptr.contents)
+        c.materials = C.cast(mats, C.POINTER(capi.rh_material))
+        c.lights = C.cast(lights, C.POINTER(capi.rh_light)) if len(lights) else None
+        c.n_lights = len(lights)
+        return c
+
+    @property
+    def materials(self):
+        """A copy of the current material table (ctypes array of rh_material)."""
+        r = self.raw.contents
+        return (capi.rh_material * r.n_materials).from_buffer_copy(
+            C.string_at(r.materials, r.n_materials * C.sizeof(capi.rh_material)) if r.n_materials else b"")
+
+    @property
+    def lights(self):
+        """A copy of the current light table (ctypes array of rh_light)."""
+        r = self.raw.contents
+        return (capi.rh_light * r.n_lights).from_buffer_copy(
+            C.string_at(r.lights, r.n_lights * C.sizeof(capi.rh_light)) if r.n_lights else b"")
+
+    def update(self, materials=None, lights=None) -> dict:
+        """rh_scene_update: replaces the material table (same length) and / or the light table (any length; None keeps
+        a table) of the device copy, of the multi-GPU replica render_multi made, and of raw / flat.  Before the device
+        copy exists only the description changes.  Returns the library's rh_update_info as a dict."""
+        def table(kind, rows):
+            if isinstance(rows, C.Array) and rows._type_ is kind:
+                return (kind * len(rows)).from_buffer_copy(rows)
+            rows = list(rows)
+            if not all(isinstance(x, kind) for x in rows):
+                raise TypeError(f"expected {kind.__name__} entries")
+            return (kind * len(rows))(*rows)
+
+        cur_m, cur_l = self.materials, self.lights
+        mats = cur_m if materials is None else table(capi.rh_material, materials)
+        lts = cur_l if lights is None else table(capi.rh_light, lights)
+        if len(mats) != len(cur_m):
+            raise ValueError(f"{len(mats)} materials for a scene with {len(cur_m)}: objects keep their material indices")
+        info = capi.rh_update_info()
+        args = (None if materials is None else mats, len(mats), None if lights is None else (lts if len(lts) else (capi.rh_light * 1)()),
+                len(lts))
+        L = lib()
+        if self._dev:
+            check(L.rh_scene_update(self._dev, *args, C.byref(info)))
+        if getattr(self, "_multi", None):
+            check(L.rh_multi_scene_update(self._multi, *args, None if self._dev else C.byref(info)))
+        self._tables = (mats, lts)
+        return {n: int(getattr(info, n)) for n, _ in info._fields_}
 
     @property
     def device(self) -> C.c_void_p:
