@@ -50,9 +50,6 @@ constexpr int kMaxPeers = 16;
 #ifndef RH_REFILL_MIN
 #define RH_REFILL_MIN 16
 #endif
-#ifndef RH_TMA_STAGE
-#define RH_TMA_STAGE 0  // trace kernel: the next batch's sample offsets (1) or also the next batch of queued rays (2) arrive by a bulk async copy (cp.async.bulk + mbarrier) while the current batch is traced; 0 = plain loads.  Measured on the bench frame: 0 = 41.3 ms, 1 = 42.4 ms, 2 = 42.8 ms — the loads it replaces are one coalesced LDG.128 per lane whose latency the other warps of the SM already hide, while the tile, the mbarrier handshake and the shared memory taken from L1 cost more than they save: off by default
-#endif
 #ifndef RH_TRACE_PER_SM
 #define RH_TRACE_PER_SM 1   // resident blocks per SM of the trace kernel (block size x this = threads per SM)
 #endif
@@ -255,7 +252,7 @@ struct ChunkParams {
   int32_t hit_live_pass;  // the hit queue (a ring) still holds the hits of this pass and later ones (pass, or pass - 1 when pipelined)
   uint32_t ray_items;     // kOffsetsRays: pass-0 items of the chunk that are rays (the rest of its last row is padding)
   const void* offsets;    // device
-  uint32_t offset_linear; // f64 pairs in work-item order: pair of item i at offsets[offset_base + i] (bulk-copy staging)
+  uint32_t reserved_;     // padding: keeps the offsets of the fields below
   uint32_t stream_spp;    // RH_OFFSETS_SPLITMIX64: samples per pixel of the stream (rh_render: spp) ...
   unsigned long long offset_base;
   unsigned long long offset_seed;  // RH_OFFSETS_SPLITMIX64

@@ -24,8 +24,7 @@
 //
 // B200 specifics: persistent warps (one block per SM); the traversal stack is a per-thread column of SHARED memory
 // (8-byte entries), never local memory; queues are arrays of 128-entry slabs that a warp reserves or claims with one
-// atomic; the trace kernel's next batch of queue entries / sample offsets arrives by bulk async copy
-// (cp.async.bulk.shared::cluster.global + mbarrier, SASS: UBLKCP / SYNCS) while the current batch is traced.
+// atomic.
 #include <cuda_runtime.h>
 
 #include <cstdint>
@@ -461,14 +460,6 @@ struct AnyHit {
   __device__ __forceinline__ bool offer_object(const Ray& r, double tt, int, double&) const { return in_front(r, tt); }
 };
 
-// Prefetches (RH_PREFETCH bit 0: the lines of a leaf's triangle records beyond the first when the leaf is entered; bit 1:
-// the node record of a child that is stacked for later).  A lone warp walks at the latency of its loads — an L2 hit is
-// ~250 cycles, an L1 hit ~32 — and the records a walk will need next are known one step ahead.
-#ifndef RH_PREFETCH
-#define RH_PREFETCH 0
-#endif
-__device__ __forceinline__ void prefetch_l1(const void* p) { asm volatile("prefetch.global.L1 [%0];" ::"l"(p)); }
-
 // Mesh.hs:59-82 triangleIntersection over the `count` triangles of one leaf (Geometry.hs:54-57).
 // The accept/reject decision is the reference's expression evaluated on the reference's values
 // of det, u, v, t.  Before the division, a triangle is dropped early only when that expression is
@@ -480,12 +471,6 @@ __device__ __forceinline__ void prefetch_l1(const void* p) { asm volatile("prefe
 template <bool COUNT, class Sink>
 __device__ __forceinline__ bool test_leaf(const rh_tri* __restrict__ tris, uint32_t first, uint32_t count, const Ray& r,
                                           Sink& sink, double& bound, Cnt<COUNT>& cnt, const uint32_t* __restrict__ index = nullptr) {
-#if RH_PREFETCH & 1
-  if (!index && count > 1) {  // the records are consecutive: first .. first + count - 1, 80 bytes each
-    const char* base = (const char*)(tris + first);
-    for (uint32_t off = 128; off < count * (uint32_t)sizeof(rh_tri) + 127u; off += 128) prefetch_l1(base + off);
-  }
-#endif
   for (uint32_t k = 0; k < count; k++) {
     const uint32_t slot = index ? __ldg(index + first + k) : first + k;  // (exact walk over the reference tree's leaves)
     const double2* tp = (const double2*)(tris + slot);
@@ -582,16 +567,6 @@ __device__ __forceinline__ bool node_step(const Ctx& cx, uint32_t& ref, const Ra
       st.push(sp, cw.y, tm1);
       ref = cw.x;
     }
-#if RH_PREFETCH & 2
-    {
-      const uint32_t far = (tm1 < tm0) ? cw.x : cw.y;  // popped later: its record (or its first triangle) can be on its way
-      if (far & kLeafBit) {
-        if (!(far & kSphereLeafBit)) prefetch_l1(cx.S->tris + (far & kLeafFirstMask));
-      } else if (far >= cx.S->n_smem_nodes) {
-        prefetch_l1(&cx.S->wide32[far]);
-      }
-    }
-#endif
     return true;
   }
   if (h0) {
@@ -1093,34 +1068,6 @@ __device__ __forceinline__ void accumulate(const ChunkParams& P, uint32_t sample
   atomicAdd(a + 2 * (size_t)P.accum_stride, w * c.z);
 }
 
-// ------------------------------------------------------------------ bulk async copies (TMA unit, 1-D form)
-// cp.async.bulk.shared::cluster.global with mbarrier completion: one elected lane starts the copy of a contiguous
-// tile, the data lands in shared memory without occupying registers or LSU slots, every lane waits on the mbarrier's
-// phase before reading.  SASS: UBLKCP, SYNCS.ARRIVE.TRANS64, SYNCS.PHASECHK.
-__device__ __forceinline__ uint32_t smem_u32(const void* p) { return (uint32_t)__cvta_generic_to_shared(p); }
-__device__ __forceinline__ void mbar_init(unsigned long long* bar) {
-  asm volatile("mbarrier.init.shared::cta.b64 [%0], 1;" ::"r"(smem_u32(bar)) : "memory");
-  asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-}
-__device__ __forceinline__ void mbar_expect(unsigned long long* bar, uint32_t bytes) {
-  asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(smem_u32(bar)), "r"(bytes) : "memory");
-}
-__device__ __forceinline__ void bulk_g2s(void* dst_smem, const void* src_global, uint32_t bytes, unsigned long long* bar) {
-  asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];" ::"r"(smem_u32(dst_smem)),
-               "l"(src_global), "r"(bytes), "r"(smem_u32(bar))
-               : "memory");
-}
-__device__ __forceinline__ void mbar_wait(unsigned long long* bar, uint32_t parity) {
-  uint32_t ok = 0;
-  while (!ok) {
-    asm volatile(
-        "{ .reg .pred p; mbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2; selp.u32 %0, 1, 0, p; }"
-        : "=r"(ok)
-        : "r"(smem_u32(bar)), "r"(parity)
-        : "memory");
-  }
-}
-
 // Image row of a shard-compact row (SURVEY 8e): band b = row / band_height goes to shard b mod G.
 __device__ __forceinline__ uint32_t global_row(const ChunkParams& P, uint32_t local_row) {
   const uint32_t lb = local_row / P.band_height, rib = local_row % P.band_height;
@@ -1443,51 +1390,8 @@ __device__ __forceinline__ bool offset_slot(const ChunkParams& P, uint32_t item,
   return P.offset_mode == RH_OFFSETS_F64 || P.offset_mode == RH_OFFSETS_F32 || P.offset_mode == RH_OFFSETS_TILED_F64;
 }
 
-// One warp's staging tile for the NEXT batch of 32 work items: the four planes of a ray-queue batch (pass >= 1) or the
-// f64 offset pairs of 32 pixel samples (pass 0, plane 0 only), filled by bulk async copies.
-#if RH_TMA_STAGE >= 2
-constexpr int kStagePlanes = 4;  // also the four planes of a ray-queue batch (passes >= 1)
-#else
-constexpr int kStagePlanes = 1;  // the sample offsets of pass 0 only: 512 bytes per warp
-#endif
-struct __align__(128) StageTile {
-  double2 plane[kStagePlanes][32];
-};
-struct Staged {
-  uint32_t first;   // first work item of the staged batch, kEmpty = nothing staged
-  uint32_t parity;  // phase of the warp's mbarrier the next wait uses
-};
-
-// Start the copy of the batch of `n` items beginning at `first` (lane 0 only calls this).  Pass 0: only when the
-// offsets are per-sample f64 pairs laid out in work-item order (P.offset_linear: chunk-local slices, or the full-frame
-// array of an unsharded frame), so that the batch's pairs are one contiguous run.
-// `dep`: a value derived from what this lane just read out of the tile; the copy's byte count is made to depend on
-// it, so the warp's shared-memory reads of the previous batch have returned before the copy engine may overwrite them.
-__device__ __forceinline__ bool stage_start(const ChunkParams& P, bool primary, uint32_t first, uint32_t n, StageTile* tile,
-                                            unsigned long long* bar, uint32_t dep) {
-  uint32_t zero;
-  asm volatile("and.b32 %0, %1, 0;" : "=r"(zero) : "r"(dep));
-  n += zero;
-  if (primary) {
-    if (!P.offset_linear) return false;
-    mbar_expect(bar, n * 16u);
-    bulk_g2s(tile->plane[0], (const double2*)P.offsets + P.offset_base + first, n * 16u, bar);
-    return true;
-  }
-#if RH_TMA_STAGE >= 2
-  const size_t cap = P.q_in.capacity;
-  mbar_expect(bar, 4u * n * 16u);
-#pragma unroll
-  for (int k = 0; k < 4; k++) bulk_g2s(tile->plane[k], P.q_in.plane + (size_t)k * cap + first, n * 16u, bar);
-  return true;
-#else
-  return false;
-#endif
-}
-
 // Work item -> ray: the camera ray of a pixel sample (pass 0: pixelCoord, Image.hs:31-32, + sample offset,
 // RayHs.hs:178-181) or a queued secondary ray with its weight and tags.  False for a padding row of the last band.
-// `tile`: the item's batch was staged in shared memory (see stage_start), else it is read from global memory.
 // What pass 0's work items are: camera samples of the chunk's image rows (rh_render), caller-built rays (kRays:
 // rh_trace_rays, P.offset_mode == kOffsetsRays) or samples of the entries of a pixel list (kPixelList:
 // rh_render_adaptive, P.list).  The last two are false past the chunk's items (P.ray_items).
@@ -1501,8 +1405,7 @@ __device__ __forceinline__ uint32_t list_image_row(const PixelList& L, uint32_t 
 
 template <Source SRC>
 __device__ __forceinline__ bool load_item(const ChunkParams& P, const CameraParams& cam, uint32_t item, bool primary,
-                                          const StageTile* tile, uint32_t lane, Ray& r, double& w, uint32_t& sample, int& depth,
-                                          int& kind, uint32_t& probe_mat) {
+                                          Ray& r, double& w, uint32_t& sample, int& depth, int& kind, uint32_t& probe_mat) {
   r.o = r.d = mk(0, 0, 1);
   if (SRC == Source::kRays && primary) {
     if (item >= P.ray_items) return false;
@@ -1544,7 +1447,7 @@ __device__ __forceinline__ bool load_item(const ChunkParams& P, const CameraPara
         ox = (double)o2.x;
         oy = (double)o2.y;
       } else {
-        const double2 o2 = tile ? tile->plane[0][lane] : __ldg((const double2*)P.offsets + idx);
+        const double2 o2 = __ldg((const double2*)P.offsets + idx);
         ox = o2.x;
         oy = o2.y;
       }
@@ -1552,13 +1455,8 @@ __device__ __forceinline__ bool load_item(const ChunkParams& P, const CameraPara
     r = camera_ray(cam, (double)col + ox, (double)grow + oy);
     return true;
   }
-  double2 a, b, c, d;
-  if (RH_TMA_STAGE >= 2 && tile) {
-    a = tile->plane[0][lane], b = tile->plane[1 % kStagePlanes][lane], c = tile->plane[2 % kStagePlanes][lane], d = tile->plane[3 % kStagePlanes][lane];
-  } else {
-    const size_t cap = P.q_in.capacity;
-    a = P.q_in.plane[item], b = P.q_in.plane[cap + item], c = P.q_in.plane[2 * cap + item], d = P.q_in.plane[3 * cap + item];
-  }
+  const size_t cap = P.q_in.capacity;
+  const double2 a = P.q_in.plane[item], b = P.q_in.plane[cap + item], c = P.q_in.plane[2 * cap + item], d = P.q_in.plane[3 * cap + item];
   r.o = mk(a.x, a.y, b.x);
   r.d = mk(b.y, c.x, c.y);
   w = d.x;
@@ -1572,17 +1470,13 @@ __device__ __forceinline__ bool load_item(const ChunkParams& P, const CameraPara
 
 // ------------------------------------------------------------------ K1/K2/K4/K5
 struct TraceWarpSmem {
-#if RH_TMA_STAGE
-  StageTile tile;
-#endif
-  unsigned long long bar;
+  unsigned long long reserved_;     // padding: keeps the offsets of the fields below
   SlabWriter out_rays, out_shadow;  // the warp's open slabs of the two output queues
   unsigned long long pad_[12];
 };
-static_assert(sizeof(TraceWarpSmem) % 128 == 0, "staging tiles stay 128-byte aligned");
+static_assert(sizeof(TraceWarpSmem) == 128, "one 128-byte line per warp");
 constexpr size_t kTraceSmem = sizeof(SmemTables) + (size_t)kShortStack * kTraceBlock * sizeof(uint2) +
                               (kTraceBlock / 32) * sizeof(TraceWarpSmem);
-static_assert(sizeof(SmemTables) % 128 == 0 || !RH_TMA_STAGE, "staging tiles need 128-byte alignment after the tables");
 static_assert(((size_t)kShortStack * kTraceBlock * sizeof(uint2)) % 128 == 0, "stack columns keep the alignment");
 static_assert(kTraceSmem <= 227 * 1024, "trace kernel shared memory");
 
@@ -1612,12 +1506,6 @@ __global__ void __launch_bounds__(kTraceBlock, kTracePerSm) trace_kernel(const _
     out_rays.init();
     out_shadow.init();
   }
-#if RH_TMA_STAGE
-  if (lane == 0) mbar_init(&wsm.bar);
-  Staged staged;
-  staged.first = kEmpty;
-  staged.parity = 0;
-#endif
   __syncwarp();
 
   const uint32_t n_units = n_slabs * kSlabUnits, total_warps = gridDim.x * (kTraceBlock / 32);
@@ -1638,27 +1526,8 @@ __global__ void __launch_bounds__(kTraceBlock, kTracePerSm) trace_kernel(const _
       double w = 1;
       uint32_t sample = item, probe_mat = 0;
       int depth = 0, kind = kRayNormal;
-      const StageTile* tile = nullptr;
-#if RH_TMA_STAGE
-      if (staged.first == slab_first + b) {  // this batch was asked for while the previous one was traced
-        mbar_wait(&wsm.bar, staged.parity);
-        staged.parity ^= 1u;
-        tile = &wsm.tile;
-      }
-#endif
-      if (valid) valid = load_item<SRC>(P, cam, item, primary, tile, lane, r, w, sample, depth, kind, probe_mat);
+      if (valid) valid = load_item<SRC>(P, cam, item, primary, r, w, sample, depth, kind, probe_mat);
       else r.o = r.d = mk(0, 0, 1);
-#if RH_TMA_STAGE
-      // the tile is in registers now: ask for the next batch of this claim (same slab); it lands while this one is traced
-      __syncwarp();
-      staged.first = kEmpty;
-      if (piece_n == 32 && b + 32 < count && u < claim_end && u % kSlabUnits != 0) {
-        uint32_t ok = 0;
-        const uint32_t dep = (uint32_t)(__double2loint(r.o.x) ^ __double2loint(r.d.x) ^ __double2loint(w));
-        if (lane == 0) ok = stage_start(P, primary, slab_first + b + 32, min(32u, count - b - 32), &wsm.tile, &wsm.bar, dep) ? 1u : 0u;
-        if (__shfl_sync(kFull, ok, 0)) staged.first = slab_first + b + 32;
-      }
-#endif
 
       Closest best;
       best.obj = -1;

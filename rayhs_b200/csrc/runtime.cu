@@ -1193,7 +1193,7 @@ int derive_tables(Device* D, const rh_scene& G, const rh_material* mats, uint32_
   }
   // Light-space tables of the shadow kernels (light_maps.cpp): cube maps of the nearest possible occluder distance, one
   // per (point light, occluder mesh), and lit-triangle flags per (triangle, light of either kind).  Only the
-  // shared-memory-table shadow kernels read them; RAYHS_B200_LIGHT_MAPS=0 switches the build off.
+  // shared-memory-table shadow kernels read them.
   v.light_maps = nullptr;
   v.lit_flags = nullptr;
   v.light_map_index = nullptr;
@@ -1207,14 +1207,11 @@ int derive_tables(Device* D, const rh_scene& G, const rh_material* mats, uint32_
   auto mesh_slots = [&](size_t m) { return G.mesh_slots.data() + G.slot_begin[occ_objs[m]]; };
   auto mesh_n_slots = [&](size_t m) { return G.slot_begin[occ_objs[m] + 1] - G.slot_begin[occ_objs[m]]; };
   {
-    const char* env = getenv("RAYHS_B200_LIGHT_MAPS");
-    const char* env_res = getenv("RAYHS_B200_LIGHT_MAP_RES");
-    const char* env_lit = getenv("RAYHS_B200_LIT_TRIANGLES");  // 0: no lit-triangle flags (A/B)
     uint32_t n_point = 0;
     for (uint32_t li = 0; li < n_lights; li++) n_point += lights[li].kind == RH_LIGHT_POINT;
     const size_t n_pairs = (size_t)n_point * occ_meshes.size();
-    if (v.shadow_fast && !occ_meshes.empty() && n_lights && !(env && env[0] == '0')) {
-      int R = env_res ? std::max(16, std::min(4096, atoi(env_res))) : kLightMapRes;
+    if (v.shadow_fast && !occ_meshes.empty() && n_lights) {
+      int R = kLightMapRes;
       while (R > 64 && std::max<size_t>(n_pairs, 1) * 6 * (size_t)R * R * sizeof(float) > kLightMapBudget) R /= 2;
       const size_t cells = (size_t)6 * R * R;
       try {
@@ -1268,8 +1265,7 @@ int derive_tables(Device* D, const rh_scene& G, const rh_material* mats, uint32_
                 useful_maps++;
               }
             }
-            want[m] = n_slots * (size_t)n_lights <= kLitMaxQueriesDevice && !(env_lit && env_lit[0] == '0') &&
-                      (n_point == 0 || useful_maps > 0);
+            want[m] = n_slots * (size_t)n_lights <= kLitMaxQueriesDevice && (n_point == 0 || useful_maps > 0);
           }
           // lit triangles: the old bits of every light index whose light kept its kind and position stay, as long as
           // every mesh that had bits still has them (a mesh that gains them is queried for every light)
@@ -1319,7 +1315,7 @@ int derive_tables(Device* D, const rh_scene& G, const rh_material* mats, uint32_
             const std::vector<uint32_t> slots(mesh_slots(m), mesh_slots(m) + mesh_n_slots(m));
           // lit triangles: per triangle and light, can another triangle of this mesh shadow it at all?  The queries
           // run on their own threads while this one builds the mesh's cube maps.
-          const bool want_lit = slots.size() * (size_t)n_lights <= kLitMaxQueries && !(env_lit && env_lit[0] == '0');
+          const bool want_lit = slots.size() * (size_t)n_lights <= kLitMaxQueries;
           if (want_lit && lit.empty()) lit.assign(dtris.size(), 0);
           size_t lit_found = 0;
           bool lit_failed = false;
@@ -1846,8 +1842,6 @@ struct FrameRun {
 
     if ((o.flags & RH_FLAG_DEVICE_OFFSETS) && (o.flags & RH_FLAG_SHARD_OFFSETS) && d_offsets)
       P.offsets = (const char*)d_offsets + (size_t)first_row * row_samples * f.off_elem;
-    // offsets in work-item order?  chunk-local slices always; the full-frame array when the frame is not sharded
-    P.offset_linear = (o.offset_mode == RH_OFFSETS_F64 && (P.offset_index == kOffIndexLocal || o.shard_count == 1)) ? 1u : 0u;
     P.offset_base = (P.offset_index == kOffIndexLocal) ? 0ull : (unsigned long long)first_row * row_samples;
     if (f.trace || f.pixel_list) P.ray_items = (uint32_t)std::min<uint64_t>(P.n_samples, f.n_rays - (uint64_t)first_row * row_samples);
     P.list = f.list;
