@@ -501,6 +501,40 @@ int rh_render_adaptive(const rh_scene* scene, const rh_camera* camera, const rh_
  * Any pointer may be NULL.  flags: 0 (host buffers) or RH_FLAG_DEVICE_OUT (device buffers, the doubles 8-byte aligned). */
 int rh_adaptive_state(const rh_adaptive* ad, uint32_t* counts_out, double* sums_out, double* sumsq_out, int32_t flags);
 
+/* ---- feature buffers ------------------------------------------------ */
+/* Per-pixel buffers of the camera rays' first hits, for denoisers (albedo, normal) and compositing (depth, coverage).
+ * Layouts are shard-compact rows, as rh_render's rgb_out; any pointer may be NULL. */
+typedef struct rh_features {
+  double* albedo;        /* double[rows][width][3], or NULL                                        */
+  double* normal;        /* double[rows][width][3], or NULL                                        */
+  double* depth;         /* double[rows][width], or NULL                                           */
+  uint32_t* hits;        /* uint32[rows][width], or NULL                                           */
+  uint32_t stream_spp;   /* RH_OFFSETS_SPLITMIX64 only: samples per pixel of the stream; 0 = opts->spp */
+  uint32_t stream_base;  /* RH_OFFSETS_SPLITMIX64 only: the pixel's first stream sample this call uses */
+} rh_features;           /* 40 bytes */
+/* Casts exactly the camera rays rh_render casts for the same scene, camera and opts (offset modes, device and shard
+ * offsets, shard and band selection), without shading them.  RH_OFFSETS_SPLITMIX64: sample s of pixel p uses stream
+ * index g = p * stream_spp + stream_base + s, the index rh_render_accumulate uses; stream_base + spp > stream_spp, or a
+ * nonzero stream field with another offset mode, is RH_ERR_ARG.  Each ray's closest hit is the one rh_render's
+ * RH_FLAG_HIT_IDS reports.  Per sample s: t_s and n_s as rh_closest_intersection's rh_hit gives them (mesh normals
+ * interpolated, not renormalised); the albedo a_s is colorAt of the material at the hit's uv for Diffuse and Plastic
+ * (the colour the render shades with, textures included), color1 for Emmit, n_s for ShowNormal, (u, v, 0) for ShowUV and
+ * (1, 1, 1) for Mirror and Transparent; a miss has a_s = n_s = 0 and no t_s.  Per pixel, with foldl (+) 0 over the
+ * samples in sample order, per channel, in IEEE double without fused multiply-add, and inv = 1.0 / spp:
+ *   albedo = inv * sum a_s;   normal = inv * sum n_s (not renormalised: a half-covered pixel has a shorter normal);
+ *   hits = h, the samples that hit;   depth = (1.0 / h) * (sum of t_s over the hitting samples), +inf when h = 0.
+ * Padding rows of the last band are pixels without hits.  hit_ids_out (RH_FLAG_HIT_IDS): int32[rows][width][spp][2] as
+ * rh_render writes it.  RH_FLAG_DEVICE_OUT: every output is a device pointer on the current device, 8-byte aligned;
+ * else host buffers, written through device scratch in bounded chunks (so are host offsets).  RH_FLAG_DEVICE_OFFSETS,
+ * RH_FLAG_SHARD_OFFSETS and RH_FLAG_EXACT_BOXES behave as in rh_render; the shadow-schedule flags, RH_FLAG_NO_LIGHT_MAPS,
+ * chunk_samples and max_depth (checked as in rh_render) have no effect, so a render's opts can be passed unchanged;
+ * RH_FLAG_PEER_FRAMES, RH_FLAG_COUNT and RH_FLAG_PROFILE are RH_ERR_ARG, and so is a call that asks for no output.  The
+ * call neither reads nor changes the scene's learned state (shadow schedule, queue factor, row costs), reflects the
+ * scene's latest rh_scene_update, and returns when the outputs are written.  stats: rays_primary (the samples traced),
+ * chunks, kernel_launches and ms_total; every other field 0. */
+int rh_render_features(const rh_scene* scene, const rh_camera* camera, const rh_render_opts* opts, const rh_features* features,
+                       int32_t* hit_ids_out, rh_stats* stats);
+
 /* Rows owned by one shard (equal for all shards: bands are padded). */
 int rh_shard_rows(int height, int shard_count, int band_height);
 int rh_default_band_height(int height, int shard_count);

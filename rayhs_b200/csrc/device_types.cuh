@@ -315,6 +315,16 @@ struct QueryParams {
   uint32_t* cursor;    // claim cursor, zero before the launch
 };
 
+// rh_render_features' outputs of one launch, indexed by the launch's pixels (pixel 0 = first pixel of ChunkParams::
+// first_row); any may be null.
+struct FeatureParams {
+  double* albedo;   // double[pixel][3]
+  double* normal;   // double[pixel][3]
+  double* depth;    // double[pixel]
+  uint32_t* hits;   // uint32[pixel]
+  int2* hit_ids;    // int2[pixel][spp]
+};
+
 // Launchers (kernels.cu).  `count` selects the instrumented instantiation (box/tri counters); launch_trace runs the
 // uninstrumented ray instantiation for P.offset_mode == kOffsetsRays and the pixel-list one when P.list.pixels is set.
 // (followed by a one-thread kernel that closes the pass's range of the hit queue, ChunkCtl::hit_start)
@@ -343,6 +353,10 @@ constexpr int kSelectBlock = 256;  // pixels per block of the selection
 // query_closest_kernel / query_shadow_kernel: `grid` blocks of one SM each
 void launch_query_closest(const SceneView& S, const QueryParams& Q, int grid, void* stream);
 void launch_query_shadow(const SceneView& S, const QueryParams& Q, int grid, void* stream);
+// feature_kernel (rh_render_features): the Q.n pixels of the rows of P (first_row, width, spp, offsets and the shard as
+// for the render's pass 0; Q: claim cursor, deep stack, exact boxes) into F; `grid` blocks of one SM each
+void launch_features(const SceneView& S, const CameraParams& cam, const ChunkParams& P, const QueryParams& Q, const FeatureParams& F,
+                     int grid, void* stream);
 void launch_deinterleave(const uint8_t* gathered, uint8_t* out, int width, int height, int shard_count, int band_height,
                          void* stream);
 int configure_kernels();  // opt in to > 48 KB dynamic shared memory; returns a cudaError_t

@@ -14,6 +14,8 @@
 //   accumulate_resolve_kernel  K6 of rh_render_accumulate: running per-pixel sums across calls, RGB8 and linear colours.
 //   adaptive_*            rh_render_adaptive: selection and compaction of the pixels still above the threshold, the
 //                         sink of their samples (trace_kernel<.., Source::kPixelList>), commit, RGB8 and linear output.
+//   feature_kernel        rh_render_features: per pixel the albedo, normal, depth and hit count of its camera rays' first
+//                         hits (closest hit + Hit + colorAt, no shading), for denoisers and compositing.
 //   deinterleave          K7: band re-assembly after the all-gather.
 //
 // All arithmetic is IEEE double in the reference's operation order and this file is compiled with -fmad=false (GHC
@@ -2336,6 +2338,84 @@ __global__ void __launch_bounds__(kQueryBlock, 1) query_shadow_kernel(const __gr
   });
 }
 
+// ------------------------------------------------------------------ feature buffers (rh_render_features)
+// One pixel per lane, the query kernels' persistent warps and shared-memory layout: the pixel's spp camera rays in sample
+// order (load_item, as the render's pass 0 makes them), the closest hit of each, its Hit (rebuild_hit) and albedo
+// (color_at for Diffuse / Plastic), and per channel `foldl (+) 0` of the samples' albedos and normals (a miss adds 0) and
+// of the hitting samples' t, all in registers.  The warp's 32 albedo and normal triples leave through its tile as
+// coalesced stores; depth and hit count are one word per lane.  A padding row of the last band is a pixel without hits.
+__global__ void __launch_bounds__(kQueryBlock, 1) feature_kernel(const __grid_constant__ SceneView S,
+                                                                 const __grid_constant__ CameraParams cam,
+                                                                 const __grid_constant__ ChunkParams P,
+                                                                 const __grid_constant__ QueryParams Q,
+                                                                 const __grid_constant__ FeatureParams F) {
+  SmemTables& sm = *reinterpret_cast<SmemTables*>(rh_smem);
+  Ctx cx;
+  stage_tables(sm, S, cx);
+  Stack st = make_query_stack(Q);
+  Cnt<false> cnt;
+  const uint32_t lane = threadIdx.x & 31;
+  double* tile = reinterpret_cast<double*>(query_tile());
+  const double inv = 1.0 / (double)P.spp;
+  claim_rays(Q, lane, [&](uint32_t first, uint32_t count) {
+    const uint32_t px = first + lane;
+    double ar = 0, ag = 0, ab = 0, nx = 0, ny = 0, nz = 0, ts = 0;
+    uint32_t h = 0;
+    for (uint32_t s = 0; s < P.spp; s++) {
+      Ray r;
+      double w;
+      uint32_t sample, probe_mat;
+      int depth, kind;
+      const bool valid = lane < count && load_item<Source::kCamera>(P, cam, px * P.spp + s, true, r, w, sample, depth, kind, probe_mat);
+      Closest best;
+      best.obj = -1;
+      if (valid) closest_hit<false>(cx, r, Q.exact_boxes || needs_exact_walk(r, S), best, st, cnt);
+      V3 a = mk(0, 0, 0), n = mk(0, 0, 0);
+      int tri = -1;
+      if (best.obj >= 0) {
+        const DObject& ob = cx.objects[best.obj];
+        const rh_material& mat = cx.materials[ob.material];
+        const int mkind = mat.kind;
+        const bool shaded = mkind == RH_MAT_DIFFUSE || mkind == RH_MAT_PLASTIC;
+        V3 p;
+        double tu = 0, tv = 0;
+        rebuild_hit<false>(S, ob, ob.kind, r, best, mkind == RH_MAT_SHOWUV || (shaded && mat.cmap_kind != RH_CMAP_FLAT), p, n, tu, tv, cnt);
+        if (shaded) a = color_at<false>(S, mat, tu, tv, cnt);
+        else if (mkind == RH_MAT_EMMIT) a = ld3(mat.color1);
+        else if (mkind == RH_MAT_SHOWNORMAL) a = n;
+        else if (mkind == RH_MAT_SHOWUV) a = mk(tu, tv, 0);
+        else a = mk(1, 1, 1);  // Mirror, Transparent
+        if (ob.kind == RH_OBJ_MESH) tri = (int)S.tris[best.slot].tri_id;
+        ts = ts + best.t;
+        h++;
+      }
+      ar = ar + a.x;
+      ag = ag + a.y;
+      ab = ab + a.z;
+      nx = nx + n.x;
+      ny = ny + n.y;
+      nz = nz + n.z;
+      if (F.hit_ids && lane < count) F.hit_ids[(size_t)px * P.spp + s] = make_int2(best.obj, tri);
+    }
+    __syncwarp();  // the tile's previous contents have been stored
+    tile[3 * lane] = inv * ar;
+    tile[3 * lane + 1] = inv * ag;
+    tile[3 * lane + 2] = inv * ab;
+    tile[96 + 3 * lane] = inv * nx;
+    tile[96 + 3 * lane + 1] = inv * ny;
+    tile[96 + 3 * lane + 2] = inv * nz;
+    __syncwarp();
+    for (uint32_t k = lane; k < 3 * count; k += 32) {
+      if (F.albedo) __stcs(F.albedo + (size_t)3 * first + k, tile[k]);
+      if (F.normal) __stcs(F.normal + (size_t)3 * first + k, tile[96 + k]);
+    }
+    if (lane < count) {
+      if (F.depth) __stcs(F.depth + px, h ? (1.0 / (double)h) * ts : __longlong_as_double(0x7ff0000000000000LL));
+      if (F.hits) __stcs(F.hits + px, h);
+    }
+  });
+}
+
 // After pass k's trace kernel: its shaded hits are the slabs [hit_start[k], hit_start[k + 1]) of the hit queue.
 __global__ void close_hit_range_kernel(ChunkCtl* ctl, int pass) { ctl->hit_start[pass + 1] = ctl->hit_slab_next; }
 
@@ -2820,6 +2900,7 @@ int configure_kernels() {
   set((const void*)classify_kernel<false, false>, kClassifySmem);
   set((const void*)query_closest_kernel, kQuerySmem);
   set((const void*)query_shadow_kernel, kQuerySmem);
+  set((const void*)feature_kernel, kQuerySmem);
   if (e == cudaSuccess) {
     int dev = 0, sms = 0, nb = 0;
     cudaGetDevice(&dev);
@@ -2908,6 +2989,10 @@ void launch_query_closest(const SceneView& S, const QueryParams& Q, int grid, vo
 }
 void launch_query_shadow(const SceneView& S, const QueryParams& Q, int grid, void* stream) {
   query_shadow_kernel<<<grid, kQueryBlock, kQuerySmem, (cudaStream_t)stream>>>(S, Q);
+}
+void launch_features(const SceneView& S, const CameraParams& cam, const ChunkParams& P, const QueryParams& Q, const FeatureParams& F,
+                     int grid, void* stream) {
+  feature_kernel<<<grid, kQueryBlock, kQuerySmem, (cudaStream_t)stream>>>(S, cam, P, Q, F);
 }
 void launch_deinterleave(const uint8_t* gathered, uint8_t* out, int width, int height, int shard_count, int band_height,
                          void* stream) {

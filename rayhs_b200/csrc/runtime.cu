@@ -1613,18 +1613,21 @@ struct Frame {
   AccumParams acc{};
   double* linear = nullptr;
   size_t linear_bytes = 0;
+  // rh_render_features: render_frame's checks and geometry only (features_on runs the frame, not run_frame); no RGB8 sink
+  bool features = false;
   const char* overflow_error = "rh_render: ray queue overflow; lower chunk_samples";
   // renders (not traces or list frames) tune the scene's shadow schedule and record its queue factor and row costs
   bool learns() const { return !trace && !pixel_list; }
 };
 
-// rh_render's argument checks (`who` names the entry point in the messages).  With f->accumulate or f->pixel_list set,
-// rgb_out may be null.
+// rh_render's argument checks (`who` names the entry point in the messages).  With f->accumulate, f->pixel_list or
+// f->features set, rgb_out may be null.
 int render_frame(Device* D, const rh_scene* scene, const rh_camera* camera, const rh_render_opts* o, uint8_t* rgb_out,
                  int32_t* hit_ids_out, Frame* f, const char* who = "rh_render") {
   const std::string w(who);
   const bool peer_frames = o && (o->flags & RH_FLAG_PEER_FRAMES) != 0;
-  if (!scene || !camera || !o || (!rgb_out && !peer_frames && !f->accumulate && !f->pixel_list)) return rh::set_error(RH_ERR_ARG, w + ": null argument");
+  if (!scene || !camera || !o || (!rgb_out && !peer_frames && !f->accumulate && !f->pixel_list && !f->features))
+    return rh::set_error(RH_ERR_ARG, w + ": null argument");
   if (peer_frames && (!o->peer_frames || o->n_peer_frames <= 0 || o->n_peer_frames > kMaxPeers))
     return rh::set_error(RH_ERR_ARG, w + ": RH_FLAG_PEER_FRAMES needs 1..16 peer frame pointers");
   if (peer_frames && (o->flags & RH_FLAG_HIT_IDS))
@@ -1694,6 +1697,31 @@ ShadowChoice choose_shadow(const rh_scene* scene, const Frame& f) {
 }
 
 struct Span { cudaEvent_t a, b; int kind; };  // a timed launch: 0 trace, 1 shadow kernels, 2 resolve / store
+
+// Copies the host sample offsets of the frame's local rows [first_row, first_row + n_rows) to `slot` in work-item order:
+// one copy per run of image rows that are contiguous inside one band, none for padding rows.  A trace frame's last row
+// may be partial.  Adds the bytes copied to *bytes.
+int upload_offset_rows(const Frame& f, size_t row_samples, int first_row, int n_rows, char* slot, cudaStream_t stream, size_t* bytes) {
+  const rh_render_opts& o = f.o;
+  const int bh = o.band_height;
+  int lr = first_row;
+  while (lr < first_row + n_rows) {
+    const int lb = lr / bh, rib = lr % bh;
+    const int run = std::min(bh - rib, first_row + n_rows - lr);
+    const long long grow = ((long long)lb * o.shard_count + o.shard_index) * bh + rib;
+    const long long rows_ok = std::max<long long>(0, std::min<long long>(run, (long long)o.height - grow));
+    if (rows_ok > 0) {
+      const size_t src_row = (o.flags & RH_FLAG_SHARD_OFFSETS) ? (size_t)lr : (size_t)grow;
+      size_t n = (size_t)rows_ok * row_samples * f.off_elem;
+      if (f.trace) n = std::min(n, ((size_t)f.n_rays - src_row * row_samples) * f.off_elem);  // (a partial last row)
+      RH_CUDA(cudaMemcpyAsync(slot + (size_t)(lr - first_row) * row_samples * f.off_elem,
+                              (const char*)o.offsets + src_row * row_samples * f.off_elem, n, cudaMemcpyHostToDevice, stream));
+      *bytes += n;
+    }
+    lr += run;
+  }
+  return RH_OK;
+}
 
 // One frame on one device: its plan and buffers, and what the enqueued chunks recorded.
 struct FrameRun {
@@ -1812,27 +1840,12 @@ struct FrameRun {
     P.deep_stride = (uint32_t)D->max_threads;
 
     if (host_offsets) {
-      // upload this chunk's rows (runs of image rows that are contiguous inside one band) on the copy stream
-      const int b = i % ring, bh = o.band_height;
+      // upload this chunk's rows on the copy stream
+      const int b = i % ring;
       char* slot = (char*)D->offsets.p + (size_t)b * chunk_samples * f.off_elem;
       if (i >= ring) RH_CUDA(cudaStreamWaitEvent(D->copy_stream, D->ev_done[b], 0));
-      int lr = first_row;
-      while (lr < first_row + n_rows) {
-        const int lb = lr / bh, rib = lr % bh;
-        const int run = std::min(bh - rib, first_row + n_rows - lr);
-        const long long grow = ((long long)lb * o.shard_count + o.shard_index) * bh + rib;
-        const long long rows_ok = std::max<long long>(0, std::min<long long>(run, (long long)o.height - grow));
-        if (rows_ok > 0) {
-          const size_t src_row = (o.flags & RH_FLAG_SHARD_OFFSETS) ? (size_t)lr : (size_t)grow;
-          size_t bytes = (size_t)rows_ok * row_samples * f.off_elem;
-          if (f.trace) bytes = std::min(bytes, ((size_t)f.n_rays - src_row * row_samples) * f.off_elem);  // (a partial last row)
-          RH_CUDA(cudaMemcpyAsync(slot + (size_t)(lr - first_row) * row_samples * f.off_elem,
-                                  (const char*)o.offsets + src_row * row_samples * f.off_elem, bytes,
-                                  cudaMemcpyHostToDevice, D->copy_stream));
-          upload_bytes += bytes;
-        }
-        lr += run;
-      }
+      const int rc = upload_offset_rows(f, row_samples, first_row, n_rows, slot, D->copy_stream, &upload_bytes);
+      if (rc) return rc;
       RH_CUDA(cudaEventRecord(D->ev_up[b], D->copy_stream));
       copy_ev.push_back(prof_event(D->copy_stream));  // (when each chunk's upload ended)
       RH_CUDA(cudaStreamWaitEvent(lane_stream, D->ev_up[b], 0));
@@ -2677,6 +2690,150 @@ int trace_on(Device* D, const rh_scene* scene, const double* rays, uint64_t n, c
   return run_frame(D, scene, f, stats);
 }
 
+// ------------------------------------------------------------------ feature buffers
+// rh_render_features casts the render's camera rays (render_frame's checks and geometry, load_item's offsets) through
+// feature_kernel, chunk after chunk of rows on the library stream.  Device outputs with device (or no) offsets are used
+// in place, in chunks as large as one launch takes; host offsets and host outputs go through device scratch in smaller
+// chunks, so that a 4K x 16-spp offset array (2.1 GB) is never staged at once.
+constexpr uint64_t kFeatureLaunchSamples = 1ull << 30;  // camera samples per launch: item indices stay far inside 32 bits
+constexpr uint64_t kFeatureChunkSamples = 1ull << 21;   // ... per chunk through scratch: 32 MB of F64 offsets, 16 MB of ids
+
+int features_on(Device* D, const rh_scene* scene, const rh_camera* camera, const rh_render_opts* o, const rh_features* ft,
+                int32_t* hit_ids_out, rh_stats* stats) {
+  const std::string w = "rh_render_features";
+  if (!scene || !camera || !o || !ft) return rh::set_error(RH_ERR_ARG, w + ": null argument");
+  if (o->flags & (RH_FLAG_PEER_FRAMES | RH_FLAG_COUNT | RH_FLAG_PROFILE))
+    return rh::set_error(RH_ERR_ARG, w + ": RH_FLAG_PEER_FRAMES, RH_FLAG_COUNT and RH_FLAG_PROFILE are not supported");
+  const bool want_ids = (o->flags & RH_FLAG_HIT_IDS) != 0;
+  if (!ft->albedo && !ft->normal && !ft->depth && !ft->hits && !want_ids) return rh::set_error(RH_ERR_ARG, w + ": no output requested");
+  if (o->offset_mode != RH_OFFSETS_SPLITMIX64 && (ft->stream_spp || ft->stream_base))
+    return rh::set_error(RH_ERR_ARG, w + ": stream_spp and stream_base are for RH_OFFSETS_SPLITMIX64 only");
+  Frame f;
+  f.features = true;
+  int rc = render_frame(D, scene, camera, o, nullptr, hit_ids_out, &f, "rh_render_features");
+  if (rc) return rc;
+  const uint32_t spp = (uint32_t)o->spp;
+  if (ft->stream_spp) f.stream_spp = ft->stream_spp;
+  f.stream_base = ft->stream_base;
+  if ((uint64_t)f.stream_base + spp > f.stream_spp)
+    return rh::set_error(RH_ERR_ARG, w + ": RH_OFFSETS_SPLITMIX64 past the end of the stream (stream_base " + std::to_string(f.stream_base) +
+                                         " + spp " + std::to_string(spp) + " > stream_spp " + std::to_string(f.stream_spp) + ")");
+  const int mode = o->offset_mode;
+  const bool dev = (o->flags & RH_FLAG_DEVICE_OUT) != 0, dev_off = (o->flags & RH_FLAG_DEVICE_OFFSETS) != 0;
+  RH_CUDA(cudaSetDevice(D->dev));
+  if (dev) {
+    for (const void* p : {(const void*)ft->albedo, (const void*)ft->normal, (const void*)ft->depth, (const void*)ft->hits,
+                          (const void*)(want_ids ? hit_ids_out : nullptr)})
+      if ((uintptr_t)p % 8) return rh::set_error(RH_ERR_ARG, w + ": device outputs must be 8-byte aligned");
+    if ((rc = check_device_pointers({ft->albedo, ft->normal, ft->depth, ft->hits, want_ids ? hit_ids_out : nullptr},
+                                    w + ": RH_FLAG_DEVICE_OUT with a pointer that is not device memory")))
+      return rc;
+  }
+  const bool host_offsets = (mode == RH_OFFSETS_F64 || mode == RH_OFFSETS_F32) && !dev_off;
+  const size_t W = (size_t)o->width, row_samples = W * spp;
+  const int rows = f.rows_local;
+  const uint64_t per_chunk = (host_offsets || !dev) ? kFeatureChunkSamples : kFeatureLaunchSamples;
+  const int chunk_rows = (int)std::max<uint64_t>(1, std::min<uint64_t>((uint64_t)rows, per_chunk / row_samples));
+  const size_t chunk_px = (size_t)chunk_rows * W, chunk_samples = chunk_px * spp;
+  const size_t tile_bytes = mode == RH_OFFSETS_TILED_F64 && !dev_off ? (size_t)o->offset_tile * o->offset_tile * spp * f.off_elem : 0;
+
+  // scratch: claim cursor, then (host buffers) the tile, one chunk of offsets and one chunk of each host output
+  Device::Scratch& sc = D->lane[0];  // the render's deep-stack scratch covers grid x block of feature_kernel
+  if ((rc = sc.deep.reserve((size_t)scene->deep_entries * D->max_threads * sizeof(uint2)))) return rc;
+  size_t at = kQueryCursorBytes;
+  auto carve = [&](bool need, size_t bytes) {
+    const size_t here = at;
+    if (need) at += (bytes + 255) / 256 * 256;
+    return need ? here : 0;
+  };
+  const size_t s_tile = carve(tile_bytes > 0, tile_bytes), s_off = carve(host_offsets, chunk_samples * f.off_elem);
+  const size_t s_albedo = carve(!dev && ft->albedo, chunk_px * 3 * sizeof(double)), s_normal = carve(!dev && ft->normal, chunk_px * 3 * sizeof(double));
+  const size_t s_depth = carve(!dev && ft->depth, chunk_px * sizeof(double)), s_hits = carve(!dev && ft->hits, chunk_px * sizeof(uint32_t));
+  const size_t s_ids = carve(!dev && want_ids, chunk_samples * sizeof(int2));
+  if ((rc = D->query.reserve(at))) return rc;
+  char* scratch = (char*)D->query.p;
+
+  ChunkParams P{};
+  P.spp = spp;
+  P.width = o->width;
+  P.height = o->height;
+  P.shard_index = f.o.shard_index;
+  P.shard_count = f.o.shard_count;
+  P.band_height = f.o.band_height;
+  P.offset_mode = mode;
+  P.offset_tile = o->offset_tile;
+  P.stream_spp = f.stream_spp;
+  P.stream_base = f.stream_base;
+  if (mode == RH_OFFSETS_SPLITMIX64) memcpy(&P.offset_seed, o->offsets, sizeof P.offset_seed);
+  QueryParams Q{};
+  Q.exact_boxes = (o->flags & RH_FLAG_EXACT_BOXES) ? 1 : 0;
+  Q.deep_stack = (uint2*)sc.deep.p;
+  Q.deep_stride = (uint32_t)D->max_threads;
+  Q.cursor = (uint32_t*)scratch;
+  uint32_t launches = 0, chunks = 0;
+  size_t uploaded = 0;
+  RH_CUDA(cudaEventRecord(D->ev_begin, D->stream));
+  if (tile_bytes) RH_CUDA(cudaMemcpyAsync(scratch + s_tile, o->offsets, tile_bytes, cudaMemcpyHostToDevice, D->stream));
+  for (int r0 = 0; r0 < rows; r0 += chunk_rows) {
+    const int n_rows = std::min(chunk_rows, rows - r0);
+    const size_t px0 = (size_t)r0 * W, n_px = (size_t)n_rows * W;
+    P.first_row = (uint32_t)r0;
+    P.n_rows = (uint32_t)n_rows;
+    P.n_samples = (uint32_t)(n_px * spp);
+    P.offset_index = kOffIndexLocal;
+    if (mode == RH_OFFSETS_TILED_F64) {
+      P.offsets = dev_off ? o->offsets : scratch + s_tile;
+    } else if (host_offsets) {
+      if ((rc = upload_offset_rows(f, row_samples, r0, n_rows, scratch + s_off, D->stream, &uploaded))) return rc;
+      P.offsets = scratch + s_off;
+    } else if (mode == RH_OFFSETS_F64 || mode == RH_OFFSETS_F32) {  // device offsets: the shard's compact rows or the frame's
+      if (o->flags & RH_FLAG_SHARD_OFFSETS) P.offsets = (const char*)o->offsets + px0 * spp * f.off_elem;
+      else {
+        P.offsets = o->offsets;
+        P.offset_index = kOffIndexGlobal;
+      }
+    }
+    auto out = [&](void* user, size_t px_bytes, size_t s) -> void* {
+      return !user ? nullptr : dev ? (void*)((char*)user + px0 * px_bytes) : (void*)(scratch + s);
+    };
+    FeatureParams F{};
+    F.albedo = (double*)out(ft->albedo, 3 * sizeof(double), s_albedo);
+    F.normal = (double*)out(ft->normal, 3 * sizeof(double), s_normal);
+    F.depth = (double*)out(ft->depth, sizeof(double), s_depth);
+    F.hits = (uint32_t*)out(ft->hits, sizeof(uint32_t), s_hits);
+    F.hit_ids = (int2*)out(want_ids ? hit_ids_out : nullptr, spp * sizeof(int2), s_ids);
+    Q.n = (uint32_t)n_px;
+    RH_CUDA(cudaMemsetAsync(Q.cursor, 0, sizeof(uint32_t), D->stream));
+    launch_features(scene->view, f.cam, P, Q, F, D->n_sms, D->stream);
+    RH_CUDA(cudaGetLastError());
+    launches++;
+    chunks++;
+    if (!dev) {
+      auto back = [&](void* user, size_t px_bytes, const void* src) -> int {
+        if (user) RH_CUDA(cudaMemcpyAsync((char*)user + px0 * px_bytes, src, n_px * px_bytes, cudaMemcpyDeviceToHost, D->stream));
+        return RH_OK;
+      };
+      if ((rc = back(ft->albedo, 3 * sizeof(double), F.albedo)) || (rc = back(ft->normal, 3 * sizeof(double), F.normal)) ||
+          (rc = back(ft->depth, sizeof(double), F.depth)) || (rc = back(ft->hits, sizeof(uint32_t), F.hits)) ||
+          (rc = back(want_ids ? hit_ids_out : nullptr, spp * sizeof(int2), F.hit_ids)))
+        return rc;
+    }
+  }
+  RH_CUDA(cudaEventRecord(D->ev_end, D->stream));
+  RH_CUDA(cudaStreamSynchronize(D->stream));
+  g_launches.fetch_add(launches, std::memory_order_relaxed);
+  if (stats) {
+    memset(stats, 0, sizeof *stats);
+    stats->rays_primary = f.rays_primary;
+    stats->chunks = chunks;
+    stats->kernel_launches = launches;
+    float ms = 0;
+    cudaEventElapsedTime(&ms, D->ev_begin, D->ev_end);
+    stats->ms_total = ms;
+  }
+  return RH_OK;
+}
+
 }  // namespace
 
 // ================================================================== C ABI
@@ -2860,6 +3017,12 @@ int rh_shadow_intersection(const rh_scene* scene, uint32_t light, const double* 
                            int32_t flags) {
   if (!g_dev) return rh::set_error(RH_ERR_STATE, "rh_shadow_intersection: call rh_init first");
   return query_on(g_dev.get(), scene, light, rays, n, occluded_out, flags, "rh_shadow_intersection");
+}
+
+int rh_render_features(const rh_scene* scene, const rh_camera* camera, const rh_render_opts* opts, const rh_features* features,
+                       int32_t* hit_ids_out, rh_stats* stats) {
+  if (!g_dev) return rh::set_error(RH_ERR_STATE, "rh_render_features: call rh_init first");
+  return features_on(g_dev.get(), scene, camera, opts, features, hit_ids_out, stats);
 }
 
 int rh_default_band_height(int height, int shard_count) {

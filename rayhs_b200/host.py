@@ -435,6 +435,83 @@ def traceRay(scene, origins, directions, max_depth: int, *, want_hit_ids: bool =
     return Radiance(colors, st.as_dict(), ids)
 
 
+# ---- feature buffers (first hits of the camera rays, for denoisers and compositing)
+
+@dataclass
+class Features:
+    """rh_render_features of one view: per pixel of the (shard-compact) rows, the mean over its samples of the albedo
+    albedo [rows, w, 3] and of the normal normal [rows, w, 3] of each camera ray's closest hit (0 for a miss; normals are
+    not renormalised), the mean t of the hitting samples depth [rows, w] (+inf without one), the number of hitting samples
+    hits [rows, w] (uint32; int32 on the device), the hit ids [rows, w, spp, 2] when asked for, and the call's stats.
+    numpy arrays, or CUDA tensors with device=True."""
+    albedo: object
+    normal: object
+    depth: object
+    hits: object
+    hit_ids: object = None
+    stats: dict = field(default_factory=dict)
+
+
+def renderFeatures(job: Rendering, spp: int = 1, offsets=None, seed: int | None = None, offset_tile: int = 0, stream_spp: int = 0,
+                   stream_base: int = 0, want_hit_ids: bool = False, shard_index: int = 0, shard_count: int = 1,
+                   band_height: int = 0, exact_boxes: bool = False, device: bool = False) -> Features:
+    """Feature buffers of the camera rays render(job, spp, offsets / seed, ...) casts.  `offsets`: full-frame
+    [width*height, spp, 2] float64 / float32 (or the [tile*tile, spp, 2] tile with `offset_tile`), numpy, a CPU tensor
+    or, with device=True, a CUDA tensor (a strided view is copied to a dense array first); `seed`: the SplitMix64 stream
+    instead, samples stream_base .. stream_base + spp - 1 of a stream of `stream_spp` samples per pixel (0: spp), as an
+    Accumulator holding stream_base samples draws them.  `device`: outputs are CUDA tensors."""
+    L = lib()
+    mode, off = _offset_mode(offsets, offset_tile)
+    off_ptr, seed_box = None, None
+    flags = ((capi.RH_FLAG_HIT_IDS if want_hit_ids else 0) | (capi.RH_FLAG_EXACT_BOXES if exact_boxes else 0)
+             | (capi.RH_FLAG_DEVICE_OUT if device else 0))
+    if seed is not None:
+        if offsets is not None:
+            raise ValueError("pass either offsets or seed")
+        seed_box = C.c_uint64(seed)
+        mode, off_ptr = capi.RH_OFFSETS_SPLITMIX64, C.addressof(seed_box)
+    elif stream_spp or stream_base:
+        raise ValueError("stream_spp and stream_base go with seed")
+    elif off is not None:
+        need = (offset_tile * offset_tile if offset_tile else job.width * job.height) * spp * 2
+        have = off.numel() if hasattr(off, "numel") else off.size
+        if have != need:
+            raise ValueError(f"offsets has {have} values, expected {need}")
+        if getattr(off, "is_cuda", False):
+            if not device:
+                raise ValueError("CUDA offsets need device=True")
+            flags |= capi.RH_FLAG_DEVICE_OFFSETS
+        off = off.contiguous() if hasattr(off, "contiguous") else np.ascontiguousarray(off)
+        off_ptr = _ptr(off)
+    bh = band_height or L.rh_default_band_height(job.height, shard_count)
+    rows = L.rh_shard_rows(job.height, shard_count, bh)
+    o = _opts(job, spp, mode, off_ptr, offset_tile, shard_index, shard_count, bh, 0, flags)
+    shape = (rows, job.width)
+    if device:
+        import torch
+
+        def empty(s, dtype):
+            return torch.empty(s, dtype=getattr(torch, dtype), device="cuda")
+
+        hits_dtype = "int32"  # (torch has no uint32 arithmetic to speak of)
+        torch.cuda.current_stream().synchronize()  # the library runs on its own stream
+    else:
+        def empty(s, dtype):
+            return np.empty(s, dtype=dtype)
+
+        hits_dtype = "uint32"
+    fe = Features(empty(shape + (3,), "float64"), empty(shape + (3,), "float64"), empty(shape, "float64"), empty(shape, hits_dtype),
+                  empty(shape + (spp, 2), "int32") if want_hit_ids else None)
+    ft = capi.rh_features()
+    ft.albedo, ft.normal, ft.depth, ft.hits = (_ptr(a) for a in (fe.albedo, fe.normal, fe.depth, fe.hits))
+    ft.stream_spp, ft.stream_base = int(stream_spp), int(stream_base)
+    st = capi.rh_stats()
+    check(L.rh_render_features(job.scene.device, C.byref(job.camera), C.byref(o), C.byref(ft),
+                               _ptr(fe.hit_ids) if want_hit_ids else None, C.byref(st)))
+    fe.stats = st.as_dict()
+    return fe
+
+
 def scene_setup_ms(scene: Scene) -> dict:
     """Milliseconds rh_scene_create spent on its parts (host-side trees, light-space tables, uploads)."""
     ms, info = scene._info()
