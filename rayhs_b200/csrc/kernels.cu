@@ -921,8 +921,11 @@ __device__ __noinline__ V3 color_at(const SceneView& S, const rh_material& m, do
 }
 
 // ------------------------------------------------------------------ queues: slabs, warp-aggregated compaction
-__device__ __forceinline__ uint64_t pack_bits(uint32_t sample, int depth, int kind, uint32_t mat) {
-  return (uint64_t)sample | ((uint64_t)(depth & 0xff) << 32) | ((uint64_t)(kind & 0xff) << 40) | ((uint64_t)(mat & 0xffff) << 48);
+// Bit 63 (`taint`, above the 15-bit material index): a factor between the ray's value and the nearest enclosing addition
+// of the reference's expression is inf or NaN (see trace_kernel's black terms).
+__device__ __forceinline__ uint64_t pack_bits(uint32_t sample, int depth, int kind, uint32_t mat, bool taint = false) {
+  return (uint64_t)sample | ((uint64_t)(depth & 0xff) << 32) | ((uint64_t)(kind & 0xff) << 40) | ((uint64_t)(mat & 0x7fff) << 48) |
+         ((uint64_t)taint << 63);
 }
 
 // A warp's open slab of an output queue: entries [base, base + used) are written.  One per warp, in shared memory.
@@ -1036,7 +1039,7 @@ __device__ __forceinline__ void push_ray(bool has, const Ray& r, double w, uint6
 }
 
 // `walk` word of a hit-queue entry: the hit triangle's lit flags (16 bits), or kHitDirect: the entry's colour is a finished
-// term (Emmit / ShowNormal / ShowUV) that is added as it is
+// term (Emmit / ShowNormal / ShowUV, or black under a non-finite weight) that is added as it is
 constexpr uint32_t kHitDirect = 0x80000000u;
 struct ShadowTask {
   V3 p, n, cd;
@@ -1155,10 +1158,16 @@ __device__ __forceinline__ AnyHit make_any_hit(const LightPair& q) {
 }
 
 // Is the Lambert cull exact for this light?  diffuse (Material.hs:31-33) = (max (l.n) 0 / pi) * (cd (*) lc) is +-0 for
-// l.n <= 0 only while cd (*) lc is finite: 0 * inf = NaN in the reference, which prints as channel 255.
+// l.n <= 0 only while cd (*) lc is finite: 0 * inf = NaN in the reference, which prints as channel 255.  Finite is not
+// enough — 1e200 * 1e200 overflows — so both sides are bounded: |lc_k| <= |c_k| <= 2^511 (the falloff of a radius in
+// [0, inf) is in [0, 1]; radius < 0 can make it 1 / 0, and radius inf makes it inf / inf = NaN for a light at dd = inf)
+// and |cd_k| <= 2^511 (colour_is_tame) keep every channel of the product within 2^1022.
+constexpr double kTameColour = 6.703903964971299e153;  // 2^511
+__device__ __forceinline__ bool colour_is_tame(const V3& c) {
+  return fabs(c.x) <= kTameColour && fabs(c.y) <= kTameColour && fabs(c.z) <= kTameColour;  // (false for NaN)
+}
 __device__ __forceinline__ bool light_is_tame(const rh_light& L) {
-  const bool colour = isfinite(L.color[0]) && isfinite(L.color[1]) && isfinite(L.color[2]);
-  return colour && (L.kind == RH_LIGHT_DIRECTIONAL || L.radius >= 0);  // radius < 0 can make the falloff 1 / 0
+  return colour_is_tame(ld3(L.color)) && (L.kind == RH_LIGHT_DIRECTIONAL || (L.radius >= 0 && isfinite(L.radius)));
 }
 
 // Planes and linear spheres of shadowIntersection (RayHs.hs:74-87) for one pair; true = occluded.
@@ -1307,7 +1316,7 @@ __device__ __forceinline__ LightFold fold_lights(const SmemTables& sm, const Ctx
   const rh_light* lights = fast ? sm.lights : cx.lights;
   const uint32_t n_roots = S.n_occ_meshes + (S.sphere_root != kEmpty ? 1u : 0u);
   const bool use_maps = S.light_map_index != nullptr && !P.no_light_maps;
-  const bool cd_finite = isfinite(cd.x) && isfinite(cd.y) && isfinite(cd.z);
+  const bool cd_tame = colour_is_tame(cd);
   // Plane sides, once per hit instead of once per (hit, light).  f(x) = pn.(x - pp) is affine, so a plane can only hold a
   // point of the shadow ray between its origin o and a point light L when f(o) and f(L) differ in sign.  o is within
   // 1e-6 |ld| of the hit p, so |f(o) - f(p)| <= 1e-6 |pn|_1; with |f(p)| and |f(L)| both above the margin
@@ -1332,7 +1341,7 @@ __device__ __forceinline__ LightFold fold_lights(const SmemTables& sm, const Ctx
     const rh_light& L = lights[li];
     const LightPair q = make_light_pair(L, p);
     const double ldn = dot(q.ld, n);
-    if (ldn <= 0 && cd_finite && light_is_tame(L)) {
+    if (ldn <= 0 && cd_tame && light_is_tame(L)) {
       F.culled++;
       F.settled |= 1u << li;
       continue;
@@ -1466,7 +1475,7 @@ __device__ __forceinline__ bool load_item(const ChunkParams& P, const CameraPara
   sample = (uint32_t)bits;
   depth = (int)((bits >> 32) & 0xff);
   kind = (int)((bits >> 40) & 0xff);
-  probe_mat = (uint32_t)((bits >> 48) & 0x7fff);
+  probe_mat = (uint32_t)((bits >> 48) & 0xffff);  // (bit 15: pack_bits' taint)
   return true;
 }
 
@@ -1530,6 +1539,8 @@ __global__ void __launch_bounds__(kTraceBlock, kTracePerSm) trace_kernel(const _
       int depth = 0, kind = kRayNormal;
       if (valid) valid = load_item<SRC>(P, cam, item, primary, r, w, sample, depth, kind, probe_mat);
       else r.o = r.d = mk(0, 0, 1);
+      const bool taint = (probe_mat >> 15) != 0;
+      probe_mat &= 0x7fff;
 
       Closest best;
       best.obj = -1;
@@ -1615,7 +1626,7 @@ __global__ void __launch_bounds__(kTraceBlock, kTracePerSm) trace_kernel(const _
             has = is_exit = true;
             ra = rayEps(p, outDir);
             wa = w;
-            bits = pack_bits(sample, depth, kRayNormal, 0);
+            bits = pack_bits(sample, depth, kRayNormal, 0, taint);  // (the probe's taint: mul (1 - r0) radiance)
           }
         } else if (surface && (mkind == RH_MAT_PLASTIC || mkind == RH_MAT_MIRROR || mkind == RH_MAT_TRANSPARENT) && depth < P.max_depth) {
           const double ior = cx.materials[mat_index].ior;
@@ -1623,8 +1634,16 @@ __global__ void __launch_bounds__(kTraceBlock, kTracePerSm) trace_kernel(const _
           const double f = fresnel(ior, dot(n, neg(r.d)));
           has = true;
           ra = rayEps(p, rd);
-          wa = w * (f * dot(rd, n));
-          bits = pack_bits(sample, depth + 1, kRayNormal, 0);
+          const double fd = f * dot(rd, n);
+          wa = w * fd;
+          // the child's taint: Plastic adds (diff + spec) and a Transparent whose probe is made adds (radiance + spec), so
+          // the chain of factors starts again there; a Mirror, and a Transparent that cannot enter, pass theirs on
+          bool chained = mkind == RH_MAT_MIRROR;
+          if (mkind == RH_MAT_TRANSPARENT && taint) {
+            V3 refDir;
+            chained = !refract(r.d, n, 1.0, ior, refDir);
+          }
+          bits = pack_bits(sample, depth + 1, kRayNormal, 0, (chained && taint) || !isfinite(fd));
         }
         if (has) {
           if (is_exit) n_exit++;
@@ -1645,8 +1664,9 @@ __global__ void __launch_bounds__(kTraceBlock, kTracePerSm) trace_kernel(const _
           if (refract(r.d, n, 1.0, ior, refDir)) {
             has = true;
             rb = rayEps(p, refDir);
-            wb = w * (1 - r0f(ior, 1.0));
-            bits = pack_bits(sample, depth + 1, kRayProbe, mat_index);
+            const double k = 1 - r0f(ior, 1.0);
+            wb = w * k;
+            bits = pack_bits(sample, depth + 1, kRayProbe, mat_index, !isfinite(k));
             n_probe++;
           }
         }
@@ -1656,16 +1676,28 @@ __global__ void __launch_bounds__(kTraceBlock, kTracePerSm) trace_kernel(const _
       // ambient + accumDiffuse terms (RayHs.hs:111-119) classify_kernel folds: both go to the hit queue.  Every add to a
       // sample's accumulator is made by the shadow kernels, pass after pass, so the order of a sample's terms does not
       // depend on how far the next pass's trace kernel — which runs on its own stream — has got.
+      // A black term is NaN, not nothing, when a factor between it and the nearest enclosing addition of the reference's
+      // expression is inf or NaN (0 * inf = NaN; an addition absorbs a +-0 term, and the weights above it multiply the
+      // other summand, as the wavefront's w does).  The reference multiplies black by the factors of a reflection or exit
+      // ray that misses (mul (l.n) black, mul (1 - r0) black: RayHs.hs:99-104, 140-143; the ray's taint bit carries
+      // the factors since the last addition) and by the fresnel factor of a Plastic / Mirror / Transparent hit at
+      // maxDepth (specular = black; Plastic adds it to diff right there, the other two pass it up).  Such a term is added
+      // like Emmit's, with a NaN weight; a Plastic hit carries that weight in its own entry (w * local + NaN = NaN in every
+      // channel, in any order).  A probe that misses adds nothing (have = False).  Finite factors never take this branch.
       {
+        bool black = valid && !hit && kind == kRayNormal && taint;  // (camera rays are untainted)
+        if (surface && (mkind == RH_MAT_PLASTIC || mkind == RH_MAT_MIRROR || mkind == RH_MAT_TRANSPARENT) && depth == P.max_depth)
+          black = !isfinite(fresnel(cx.materials[mat_index].ior, dot(n, neg(r.d)))) || (taint && mkind != RH_MAT_PLASTIC);
         const bool lit_surface = surface && (mkind == RH_MAT_DIFFUSE || mkind == RH_MAT_PLASTIC);
-        const bool direct = surface && (mkind == RH_MAT_EMMIT || mkind == RH_MAT_SHOWNORMAL || mkind == RH_MAT_SHOWUV);
+        const bool direct = (surface && (mkind == RH_MAT_EMMIT || mkind == RH_MAT_SHOWNORMAL || mkind == RH_MAT_SHOWUV)) ||
+                            (black && !lit_surface);
         ShadowTask task;
         if (lit_surface) {
           n_shaded++;
           task.p = p;
           task.n = n;
           task.cd = color_at<COUNT>(S, cx.materials[mat_index], tu, tv, cnt);
-          task.w = w;
+          task.w = black ? __longlong_as_double(0x7ff8000000000000LL) : w;
           task.sample = sample | (mkind == RH_MAT_DIFFUSE ? 0x80000000u : 0u);
           // lit-triangle flags of the hit triangle (light_maps.cpp) travel in the `walk` word of the hit queue
           task.walk = (okind == RH_OBJ_MESH && S.lit_flags && !P.no_light_maps) ? (uint32_t)__ldg(S.lit_flags + best.slot) : 0u;
@@ -1673,8 +1705,8 @@ __global__ void __launch_bounds__(kTraceBlock, kTracePerSm) trace_kernel(const _
         } else if (direct) {
           task.p = p;
           task.n = n;
-          task.cd = mkind == RH_MAT_EMMIT ? ld3(cx.materials[mat_index].color1) : (mkind == RH_MAT_SHOWNORMAL ? n : mk(tu, tv, 0));
-          task.w = w;
+          task.cd = black ? mk(0, 0, 0) : mkind == RH_MAT_EMMIT ? ld3(cx.materials[mat_index].color1) : (mkind == RH_MAT_SHOWNORMAL ? n : mk(tu, tv, 0));
+          task.w = black ? __longlong_as_double(0x7ff8000000000000LL) : w;
           task.sample = sample;
           task.walk = kHitDirect;
           task.settled = 0;
@@ -2194,20 +2226,20 @@ __global__ void __launch_bounds__(kShadowBlock, 1) shadow_simple_kernel(const __
       const uint32_t sbits = P.q_hits.sample[item];
       const V3 p = mk(a.x, a.y, b.x), n = mk(b.y, c.x, c.y), cd = mk(d.x, d.y, e.x);
       const double w = e.y;
-      if (P.q_hits.walk[item] & kHitDirect) {  // a finished term (Emmit / ShowNormal / ShowUV)
+      if (P.q_hits.walk[item] & kHitDirect) {  // a finished term (Emmit / ShowNormal / ShowUV / black)
         accumulate(P, sbits & 0x7fffffffu, w, cd);
         continue;
       }
-      const bool cd_finite = isfinite(cd.x) && isfinite(cd.y) && isfinite(cd.z);
+      const bool cd_tame = colour_is_tame(cd);
       V3 acc = mk(0, 0, 0);  // foldl ... black lts
       for (uint32_t li = 0; li < S.n_lights; li++) {
         const rh_light& L = cx.lights[li];
         V3 ld, lc;
         light_at(L, p, ld, lc);
-        // diffuse (Material.hs:31-33) = (max (l.n) 0 / pi) * (cd (*) lc): exactly zero when l.n <= 0 (and the colours
-        // are finite), whether or not the point is shadowed, so the occlusion query cannot change the sum
+        // diffuse (Material.hs:31-33) = (max (l.n) 0 / pi) * (cd (*) lc): exactly zero when l.n <= 0 (and cd (*) lc is
+        // finite, light_is_tame), whether or not the point is shadowed, so the occlusion query cannot change the sum
         const double ldn = dot(ld, n);
-        if (ldn <= 0 && cd_finite && light_is_tame(L)) {
+        if (ldn <= 0 && cd_tame && light_is_tame(L)) {
           n_culled++;
           continue;
         }

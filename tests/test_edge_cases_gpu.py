@@ -6,7 +6,7 @@ import pytest
 
 import rayhs_b200 as rh
 from oracle.orc import OracleScene
-from tests.util import RawScene, assert_parity
+from tests.util import RawScene, assert_parity, grid_mesh
 
 pytestmark = pytest.mark.gpu
 
@@ -32,21 +32,6 @@ def both(rs, w, h, depth=None, spp=1, offsets=None, **kw):
 
 QUAD = dict(positions=[(-1, -1, 0), (1, -1, 0), (1, 1, 0), (-1, 1, 0)], normals=[(0, 0, -1)] * 4,
             uvs=[(0, 0), (1, 0), (1, 1), (0, 1)], indices=[0, 1, 2, 0, 2, 3])
-
-
-def grid_mesh(n, z=0.0, wobble=0.0, seed=1):
-    """n x n quads (2 n^2 triangles) on [-1,1]^2: enough triangles for a real tree (>= 20 per split)."""
-    rng = np.random.RandomState(seed)
-    xs = np.linspace(-1, 1, n + 1)
-    pos = np.array([(x, y, z + wobble * rng.uniform(-1, 1)) for y in xs for x in xs])
-    nrm = np.tile((0.0, 0.0, -1.0), (len(pos), 1)) + 0.2 * rng.uniform(-1, 1, size=(len(pos), 3))
-    uv = (pos[:, :2] + 1) / 2
-    idx = []
-    for j in range(n):
-        for i in range(n):
-            a = j * (n + 1) + i
-            idx += [a, a + 1, a + n + 2, a, a + n + 2, a + n + 1]
-    return dict(positions=pos, normals=nrm, uvs=uv, indices=idx)
 
 
 def test_empty_scene_and_no_lights():

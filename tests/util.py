@@ -163,3 +163,18 @@ class RawScene:
             self._dev = C.c_void_p()
             capi.check(capi.lib().rh_scene_create(self.flat, C.byref(self._dev)))
         return self._dev
+
+
+def grid_mesh(n, z=0.0, wobble=0.0, seed=1):
+    """n x n quads (2 n^2 triangles) on [-1,1]^2: enough triangles for a real tree (>= 20 per split)."""
+    rng = np.random.RandomState(seed)
+    xs = np.linspace(-1, 1, n + 1)
+    pos = np.array([(x, y, z + wobble * rng.uniform(-1, 1)) for y in xs for x in xs])
+    nrm = np.tile((0.0, 0.0, -1.0), (len(pos), 1)) + 0.2 * rng.uniform(-1, 1, size=(len(pos), 3))
+    uv = (pos[:, :2] + 1) / 2
+    idx = []
+    for j in range(n):
+        for i in range(n):
+            a = j * (n + 1) + i
+            idx += [a, a + 1, a + n + 2, a, a + n + 2, a + n + 1]
+    return dict(positions=pos, normals=nrm, uvs=uv, indices=idx)
