@@ -535,6 +535,35 @@ typedef struct rh_features {
 int rh_render_features(const rh_scene* scene, const rh_camera* camera, const rh_render_opts* opts, const rh_features* features,
                        int32_t* hit_ids_out, rh_stats* stats);
 
+/* ---- light groups --------------------------------------------------- */
+/* One linear image per group of lights, plus one of everything else (the remainder), for relighting in compositing:
+ * scaling group g's image by k_g is scaling those lights' colours by k_g. */
+typedef struct rh_light_groups {
+  const uint8_t* group_of_light; /* n_lights entries (host memory), each < n_groups; may be NULL for a scene without lights */
+  uint32_t n_groups;             /* 1 .. 16                                                                 */
+  uint32_t reserved_;            /* must be 0                                                               */
+  double* out;                   /* double[n_groups + 1][rows][width][3], shard-compact rows; last = remainder */
+} rh_light_groups;               /* 24 bytes */
+/* Renders exactly as rh_render does for the same scene, camera and opts (the same rays, every offset mode, device and
+ * shard offsets, shard and band selection) and also writes the light groups.  Per shaded hit with weight w:
+ *   group g:   w * foldl (+) black [diffuse_l | l <- lights in order, group_of_light[l] == g, l visible], added only when
+ *              one of g's lights is visible; culled (l.n <= 0) and occluded pairs add nothing, as in the render;
+ *   remainder: Diffuse's ambient term w * 0.2 cd, and every finished term (Emmit, ShowNormal, ShowUV, and the NaN terms of
+ *              tainted rays).
+ * A sample's group sums add these terms in pass order; a pixel is foldl (+) 0 of its samples in sample order, times
+ * inv = 1.0 / spp, in IEEE double without fused multiply-add.  Padding rows of the last band are 0.  So the groups and
+ * the remainder add up to the render's linear colour only up to rounding, group g is linear in its lights' colours
+ * only up to rounding, and Transparent forks wobble in the last bit as everywhere else; a group without lights is 0.
+ * rgb_out (optional: may be NULL) receives rh_render's bytes and hit_ids_out (RH_FLAG_HIT_IDS) its ids.
+ * RH_FLAG_DEVICE_OUT covers all outputs (out 8-byte aligned); host outputs go through device scratch in bounded chunks.
+ * RH_FLAG_PEER_FRAMES and RH_FLAG_COUNT are RH_ERR_ARG, and so is a scene with more than 32 lights; RH_FLAG_EXACT_BOXES,
+ * RH_FLAG_NO_LIGHT_MAPS, the shadow-schedule flags, RH_FLAG_PROFILE and chunk_samples behave as in rh_render.  The call
+ * uses the scene's decided shadow schedule and queue factor (else pooled and 2) and changes neither of them nor the row
+ * costs.  stats as rh_render fills them (negative_channels counts rgb_out).  A call refused for its arguments writes
+ * nothing. */
+int rh_render_light_groups(const rh_scene* scene, const rh_camera* camera, const rh_render_opts* opts,
+                           const rh_light_groups* groups, uint8_t* rgb_out, int32_t* hit_ids_out, rh_stats* stats);
+
 /* Rows owned by one shard (equal for all shards: bands are padded). */
 int rh_shard_rows(int height, int shard_count, int band_height);
 int rh_default_band_height(int height, int shard_count);

@@ -105,6 +105,7 @@ struct OccPlane { double p[3], n[3]; };   // Geometry.hs:62
 struct OccSphere { double c[3], r; };     // Geometry.hs:63
 constexpr int kOccPlanes = 16, kOccSpheres = 16, kOccMeshes = 8, kFastLights = 12;
 constexpr int kMaskLights = 32;  // lights whose per-hit state fits the 32-bit walk / settled masks of a shadow task
+constexpr int kMaxGroups = 16;   // light groups of rh_render_light_groups
 
 struct SceneView {
   const WideNode* wide;      // exact double boxes: rays with a zero direction component, RH_FLAG_EXACT_BOXES
@@ -270,6 +271,13 @@ struct ChunkParams {
   RayQueue q_in, q_out;
   ShadowQueue q_hits, q_shadow;
   PixelList list;         // rh_render_adaptive (after the render's fields: their offsets stay as they were)
+  // rh_render_light_groups (after the render's fields: their offsets stay as they were): the shadow kernels also add a
+  // hit's terms split by light group to (n_groups + 1) x 3 planes of group_stride doubles, chunk-local sample order
+  // (plane 3 g + c: group g, channel c; group n_groups: the remainder).  Null for every other frame.
+  double* groups;
+  uint32_t group_stride;
+  uint32_t n_groups;
+  uint32_t group_mask[kMaxGroups];  // bit l: light l is in group g
 };
 
 // rh_render_accumulate's end of a chunk instead of the resolve: the running per-pixel sums of the accumulator.
@@ -330,10 +338,15 @@ struct FeatureParams {
 // (followed by a one-thread kernel that closes the pass's range of the hit queue, ChunkCtl::hit_start)
 void launch_trace(const SceneView& S, const CameraParams& cam, const ChunkParams& P, bool count, int grid, void* stream);
 // classify_kernel, then the walks of the hits it queued — refill: the per-lane-refill kernel (incoherent rays) instead of
-// the pooled one (coherent rays).  Returns the number of launches.
+// the pooled one (coherent rays).  Returns the number of launches.  P.groups set: the instantiations that also add the
+// light-group terms (count must be false).
 // `classified`: a cudaEvent_t recorded after the classify kernel (or null).
 int launch_shadow(const SceneView& S, const ChunkParams& P, bool count, bool refill, int grid, void* stream, void* classified);
 void launch_resolve(const ChunkParams& P, void* stream);
+// rh_render_light_groups' sink, beside the resolve: each group's (and the remainder's) per-sample sums of the chunk,
+// folded per pixel in sample order and times 1 / spp, to out + g * out_group_stride + (out_px0 + pixel) * 3, where
+// pixel is chunk-local (padding rows: 0)
+void launch_light_groups_resolve(const ChunkParams& P, double* out, size_t out_group_stride, size_t out_px0, void* stream);
 // rh_trace_rays' end of a chunk instead of the resolve: the accumulators of its rays to colors (double[n][3], all rays)
 void launch_store_colors(const ChunkParams& P, double* colors, void* stream);
 // rh_render_accumulate's end of a chunk instead of the resolve: adds the chunk's samples to the running sums and writes

@@ -1073,6 +1073,14 @@ __device__ __forceinline__ void accumulate(const ChunkParams& P, uint32_t sample
   atomicAdd(a + 2 * (size_t)P.accum_stride, w * c.z);
 }
 
+// rh_render_light_groups: the term w * c of group g (g = n_groups: the remainder) beside the sample's accumulator
+__device__ __forceinline__ void accumulate_group(const ChunkParams& P, uint32_t g, uint32_t sample, double w, V3 c) {
+  double* a = P.groups + (size_t)3 * g * P.group_stride + sample;
+  atomicAdd(a, w * c.x);
+  atomicAdd(a + P.group_stride, w * c.y);
+  atomicAdd(a + 2 * (size_t)P.group_stride, w * c.z);
+}
+
 // Image row of a shard-compact row (SURVEY 8e): band b = row / band_height goes to shard b mod G.
 __device__ __forceinline__ uint32_t global_row(const ChunkParams& P, uint32_t local_row) {
   const uint32_t lb = local_row / P.band_height, rib = local_row % P.band_height;
@@ -1383,6 +1391,20 @@ __device__ __forceinline__ V3 fold_visible(const Ctx& cx, uint32_t n_lights, uin
     acc = acc + mul(hs_max(dot(ld, n), 0) * kPiInv, cmul(cd, lc));  // diffuse, Material.hs:31-33
   }
   return acc;
+}
+
+// rh_render_light_groups, beside a folded hit's add to its sample: the same fold restricted to each group's lights (a
+// group without a visible light adds nothing), and Diffuse's ambient term to the remainder.  `sbits`: the queue's sample
+// word (bit 31: ambient term).
+__device__ __forceinline__ void accumulate_groups(const Ctx& cx, const ChunkParams& P, uint32_t n_lights, uint32_t vis, uint32_t sbits,
+                                                  const V3& p, const V3& n, const V3& cd, double w) {
+  const uint32_t sample = sbits & 0x7fffffffu;
+#pragma unroll 1
+  for (uint32_t g = 0; g < P.n_groups; g++) {
+    const uint32_t mask = P.group_mask[g];
+    if (mask & ~vis) accumulate_group(P, g, sample, w, fold_visible(cx, n_lights, vis | ~mask, p, n, cd));
+  }
+  if (sbits & 0x80000000u) accumulate_group(P, P.n_groups, sample, w, mul(0.2, cd));
 }
 
 // Index of a pixel sample's offset pair in the offset array, or false when the mode has no array.
@@ -1747,7 +1769,9 @@ struct ClassifyWarpSmem {
 };
 constexpr size_t kClassifySmem = sizeof(SmemTables) + (kClassifyBlock / 32) * sizeof(ClassifyWarpSmem);
 
-template <bool COUNT, bool FAST>
+// GROUPS (rh_render_light_groups): a hit folded here also adds its light-group terms (accumulate_groups; a finished
+// kHitDirect term goes to the remainder).
+template <bool COUNT, bool FAST, bool GROUPS = false>
 __global__ void __launch_bounds__(kClassifyBlock, RH_CLASSIFY_MINB) classify_kernel(const __grid_constant__ SceneView S,
                                                                      const __grid_constant__ ChunkParams P) {
   SmemTables& sm = *reinterpret_cast<SmemTables*>(rh_smem);
@@ -1805,6 +1829,10 @@ __global__ void __launch_bounds__(kClassifyBlock, RH_CLASSIFY_MINB) classify_ker
         } else {
           const V3 total = (task.sample & 0x80000000u) ? mul(0.2, task.cd) + F.acc : F.acc;  // Diffuse adds the ambient term, RayHs.hs:111-114
           accumulate(P, task.sample & 0x7fffffffu, task.w, total);
+          if constexpr (GROUPS) {
+            if (lit & kHitDirect) accumulate_group(P, P.n_groups, task.sample, task.w, task.cd);
+            else accumulate_groups(cx, P, S.n_lights, F.settled, task.sample, task.p, task.n, task.cd, task.w);
+          }
         }
       }
       push_shadow(queue, task, P.q_shadow, out, &ctl->shadow_slabs[P.pass], &ctl->overflow, lane);
@@ -1883,7 +1911,7 @@ constexpr size_t kShadowSmem = sizeof(WalkTables) + (kShadowBlock / 32) * sizeof
                                (size_t)kShortStack * kShadowBlock * sizeof(uint2);
 static_assert(kShadowSmem <= 227 * 1024, "pooled shadow kernel shared memory");
 
-template <bool COUNT>
+template <bool COUNT, bool GROUPS = false>  // GROUPS: phase 3 also adds the light-group terms
 __global__ void __launch_bounds__(kShadowBlock, kShadowPerSm) shadow_pooled_kernel(const __grid_constant__ SceneView S,
                                                                         const __grid_constant__ ChunkParams P) {
   WalkTables& sm = *reinterpret_cast<WalkTables*>(rh_smem);
@@ -2008,6 +2036,7 @@ __global__ void __launch_bounds__(kShadowBlock, kShadowPerSm) shadow_pooled_kern
       const V3 acc = fold_visible(cx, n_lights, ws.vis[j], p, n, cd);
       const V3 total = (sbits & 0x80000000u) ? mul(0.2, cd) + acc : acc;  // Diffuse adds the ambient term, RayHs.hs:111-114
       accumulate(P, sbits & 0x7fffffffu, e.y, total);
+      if constexpr (GROUPS) accumulate_groups(cx, P, n_lights, ws.vis[j], sbits, p, n, cd, e.y);
     }
     __syncwarp();
   }
@@ -2042,7 +2071,7 @@ constexpr size_t kWalkSmem = sizeof(WalkTables) + (size_t)kWalkColumns * kWalkBl
                              (size_t)kShortStack * kWalkBlock * sizeof(uint2);
 static_assert(kWalkSmem <= 227 * 1024, "refill shadow kernel shared memory");
 
-template <bool COUNT>
+template <bool COUNT, bool GROUPS = false>  // GROUPS: the final fold also adds the light-group terms
 __global__ void __launch_bounds__(kWalkBlock, 1) shadow_refill_kernel(const __grid_constant__ SceneView S,
                                                                       const __grid_constant__ ChunkParams P) {
   WalkTables& sm = *reinterpret_cast<WalkTables*>(rh_smem);
@@ -2086,6 +2115,7 @@ __global__ void __launch_bounds__(kWalkBlock, 1) shadow_refill_kernel(const __gr
         const V3 acc = fold_visible(cx, n_lights, vis, p, n, cd);
         const V3 total = (sbits & 0x80000000u) ? mul(0.2, cd) + acc : acc;  // Diffuse adds the ambient term, RayHs.hs:111-114
         accumulate(P, sbits & 0x7fffffffu, e.y, total);
+        if constexpr (GROUPS) accumulate_groups(cx, P, n_lights, vis, sbits, p, n, cd, e.y);
         has_task = false;
       }
       const unsigned empty = __ballot_sync(kFull, !has_task);
@@ -2633,6 +2663,56 @@ __global__ void __launch_bounds__(kBlock) accumulate_resolve_kernel(const __grid
   }
 }
 
+// ------------------------------------------------------------------ K6''': rh_render_light_groups' images
+// Beside resolve_kernel: per group (and the remainder), each pixel's samples folded in sample order with resolve_kernel's
+// loads and association, times 1 / spp; the linear triples leave coalesced through shared memory, as in
+// accumulate_resolve_kernel.  Padding rows are 0.
+__global__ void __launch_bounds__(kBlock) light_groups_resolve_kernel(const __grid_constant__ ChunkParams P, double* __restrict__ out,
+                                                                      size_t out_group_stride, size_t out_px0) {
+  __shared__ __align__(16) double lin[kBlock * 3];
+  const uint32_t n_pixels = P.n_rows * P.width;
+  const uint32_t lp = blockIdx.x * kBlock + threadIdx.x;
+  const bool real = lp < n_pixels && global_row(P, P.first_row + lp / P.width) < P.height;
+  const uint32_t n_here = min((uint32_t)kBlock, n_pixels - blockIdx.x * kBlock) * 3;
+  const double inv = 1.0 / (double)P.spp;
+#pragma unroll 1
+  for (uint32_t g = 0; g <= P.n_groups; g++) {
+    double sr = 0, sg = 0, sb = 0;  // foldl (+) black
+    if (real) {
+      const double* a = P.groups + (size_t)3 * g * P.group_stride + (size_t)lp * P.spp;
+      if ((P.spp & 1u) == 0 && (P.group_stride & 1u) == 0) {
+        const double2* a0 = (const double2*)a;
+        const double2* a1 = (const double2*)(a + P.group_stride);
+        const double2* a2 = (const double2*)(a + 2 * (size_t)P.group_stride);
+        for (uint32_t s = 0; s < P.spp / 2; s++) {
+          const double2 r2 = a0[s], g2 = a1[s], b2 = a2[s];
+          sr = (sr + r2.x) + r2.y;
+          sg = (sg + g2.x) + g2.y;
+          sb = (sb + b2.x) + b2.y;
+        }
+      } else {
+        for (uint32_t s = 0; s < P.spp; s++) {
+          sr = sr + a[s];
+          sg = sg + a[P.group_stride + s];
+          sb = sb + a[2 * (size_t)P.group_stride + s];
+        }
+      }
+      sr = inv * sr;
+      sg = inv * sg;
+      sb = inv * sb;
+    }
+    if (lp < n_pixels) {
+      lin[3 * threadIdx.x] = sr;
+      lin[3 * threadIdx.x + 1] = sg;
+      lin[3 * threadIdx.x + 2] = sb;
+    }
+    __syncthreads();
+    double* dst = out + g * out_group_stride + (out_px0 + (size_t)blockIdx.x * kBlock) * 3;
+    for (uint32_t i = threadIdx.x; i < n_here; i += kBlock) dst[i] = lin[i];
+    __syncthreads();
+  }
+}
+
 // ------------------------------------------------------------------ rh_render_adaptive
 // Selection rule (include/rayhs_b200.h, in its operation order): pixel p of the shard's rows is active when the stream
 // has spp more samples for it and it has fewer than min_spp samples or some channel's n(n-1) x variance of the mean,
@@ -2910,6 +2990,7 @@ __global__ void stream_bench_kernel(const double2* __restrict__ buf, uint64_t n_
 
 // ------------------------------------------------------------------ launchers
 static int g_classify_grid[2] = {148, 148};
+static int g_groups_classify_grid[2] = {148, 148};  // classify_kernel<false, FAST, true>, by FAST
 int configure_kernels() {
   cudaError_t e = cudaSuccess;
   auto set = [&](const void* fn, size_t bytes) {
@@ -2930,6 +3011,10 @@ int configure_kernels() {
   set((const void*)classify_kernel<false, true>, kClassifySmem);
   set((const void*)classify_kernel<true, false>, kClassifySmem);
   set((const void*)classify_kernel<false, false>, kClassifySmem);
+  set((const void*)shadow_pooled_kernel<false, true>, kShadowSmem);
+  set((const void*)shadow_refill_kernel<false, true>, kWalkSmem);
+  set((const void*)classify_kernel<false, true, true>, kClassifySmem);
+  set((const void*)classify_kernel<false, false, true>, kClassifySmem);
   set((const void*)query_closest_kernel, kQuerySmem);
   set((const void*)query_shadow_kernel, kQuerySmem);
   set((const void*)feature_kernel, kQuerySmem);
@@ -2941,6 +3026,12 @@ int configure_kernels() {
       if (c) cudaOccupancyMaxActiveBlocksPerMultiprocessor(&nb, classify_kernel<true, true>, kClassifyBlock, kClassifySmem);
       else cudaOccupancyMaxActiveBlocksPerMultiprocessor(&nb, classify_kernel<false, true>, kClassifyBlock, kClassifySmem);
       g_classify_grid[c] = sms * (nb > 0 ? nb : 1);
+    }
+    for (int fast = 0; fast < 2; fast++) {
+      nb = 0;
+      if (fast) cudaOccupancyMaxActiveBlocksPerMultiprocessor(&nb, classify_kernel<false, true, true>, kClassifyBlock, kClassifySmem);
+      else cudaOccupancyMaxActiveBlocksPerMultiprocessor(&nb, classify_kernel<false, false, true>, kClassifyBlock, kClassifySmem);
+      g_groups_classify_grid[fast] = sms * (nb > 0 ? nb : 1);
     }
   }
   return (int)e;
@@ -2967,6 +3058,14 @@ int launch_shadow(const SceneView& S, const ChunkParams& P, bool count, bool ref
     if (classified) cudaEventRecord((cudaEvent_t)classified, st);
     return 1;
   }
+  if (P.groups) {  // rh_render_light_groups (never counting)
+    if (S.shadow_fast) classify_kernel<false, true, true><<<g_groups_classify_grid[1], kClassifyBlock, kClassifySmem, st>>>(S, P);
+    else classify_kernel<false, false, true><<<g_groups_classify_grid[0], kClassifyBlock, kClassifySmem, st>>>(S, P);
+    if (classified) cudaEventRecord((cudaEvent_t)classified, st);
+    if (refill) shadow_refill_kernel<false, true><<<grid, kWalkBlock, kWalkSmem, st>>>(S, P);
+    else shadow_pooled_kernel<false, true><<<grid * kShadowPerSm, kShadowBlock, kShadowSmem, st>>>(S, P);
+    return 2;
+  }
   // FAST: the occluder tables are the staged shared-memory ones (SceneView::shadow_fast)
   if (S.shadow_fast) {
     if (count) classify_kernel<true, true><<<g_classify_grid[1], kClassifyBlock, kClassifySmem, st>>>(S, P);
@@ -2988,6 +3087,10 @@ int launch_shadow(const SceneView& S, const ChunkParams& P, bool count, bool ref
 void launch_resolve(const ChunkParams& P, void* stream) {
   const uint32_t n_pixels = P.n_rows * P.width;
   resolve_kernel<<<(n_pixels + kBlock - 1) / kBlock, kBlock, 0, (cudaStream_t)stream>>>(P);
+}
+void launch_light_groups_resolve(const ChunkParams& P, double* out, size_t out_group_stride, size_t out_px0, void* stream) {
+  const uint32_t n_pixels = P.n_rows * P.width;
+  light_groups_resolve_kernel<<<(n_pixels + kBlock - 1) / kBlock, kBlock, 0, (cudaStream_t)stream>>>(P, out, out_group_stride, out_px0);
 }
 void launch_store_colors(const ChunkParams& P, double* colors, void* stream) {
   store_colors_kernel<<<(P.ray_items + kBlock - 1) / kBlock, kBlock, 0, (cudaStream_t)stream>>>(P, colors);

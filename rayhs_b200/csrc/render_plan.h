@@ -38,14 +38,15 @@ inline double cost_density(const float* row_cost, int row0, int n) {
 // the chunks the better (measured on the bench frame with the offsets already in HBM: 16 chunks 65.5 ms, 8 chunks
 // 59.1 ms, 4 chunks 57.0 ms, 1 chunk 55.0 ms).  Default: as large as 45 % of the device memory allows.  When the
 // offsets stream in from the host, chunk k+1's upload overlaps chunk k's kernels, so the chunks stay moderate and the
-// first one, whose upload nothing can overlap, is small.
+// first one, whose upload nothing can overlap, is small.  bytes_per_sample: the device scratch a sample of a chunk needs
+// (a frame with more per-sample state than the render's passes its own count).
 inline ChunkPlan plan_chunks(int rows_local, size_t row_samples, int chunk_samples, size_t device_mem, bool host_offsets,
-                             const float* row_cost, bool compute_bound) {
+                             const float* row_cost, bool compute_bound, size_t bytes_per_sample = kBytesPerSample) {
   ChunkPlan p;
   std::vector<int>& plan = p.rows;
   size_t want = (size_t)chunk_samples, first = want;
   if (chunk_samples <= 0) {
-    want = std::min<size_t>((size_t)(0.45 * (double)device_mem) / kBytesPerSample, (size_t)0x3ffffff0u);
+    want = std::min<size_t>((size_t)(0.45 * (double)device_mem) / bytes_per_sample, (size_t)0x3ffffff0u);
     // a frame that needs several chunks has two of them in flight, each with its own scratch: half the budget each
     if ((size_t)rows_local * row_samples > want) want /= kLanes;
     if (host_offsets) want = std::min<size_t>(want, kStreamChunk);

@@ -97,6 +97,7 @@ struct Device {
   // per-lane scratch: a chunk's accumulators and queues
   struct Scratch {
     DevBuf accum, rayq[2], rayq_fill[2], hitq, hitq_words, shq, shq_words, deep, deep_shadow;
+    DevBuf groups, group_out;  // rh_render_light_groups: per-sample group sums; one chunk of host output
   } lane[2];
   DevBuf ctl, counters, offsets, rgb, ids, linear;
   DevBuf query;  // ray queries: claim cursor, then (host buffers) one chunk of rays and of results
@@ -137,7 +138,8 @@ struct Device {
     if (dev < 0) return;
     cudaSetDevice(dev);
     for (Scratch& sc : lane)
-      for (DevBuf* b : {&sc.accum, &sc.rayq[0], &sc.rayq[1], &sc.rayq_fill[0], &sc.rayq_fill[1], &sc.hitq, &sc.hitq_words, &sc.shq, &sc.shq_words, &sc.deep, &sc.deep_shadow})
+      for (DevBuf* b : {&sc.accum, &sc.rayq[0], &sc.rayq[1], &sc.rayq_fill[0], &sc.rayq_fill[1], &sc.hitq, &sc.hitq_words, &sc.shq, &sc.shq_words, &sc.deep, &sc.deep_shadow,
+                        &sc.groups, &sc.group_out})
         b->release();
     for (int l = 0; l < 2; l++) {
       if (shadow_stream[l]) cudaStreamDestroy(shadow_stream[l]);
@@ -1615,18 +1617,24 @@ struct Frame {
   size_t linear_bytes = 0;
   // rh_render_features: render_frame's checks and geometry only (features_on runs the frame, not run_frame); no RGB8 sink
   bool features = false;
+  // rh_render_light_groups: the shadow kernels also add each group's terms, and a sink beside the resolve writes the
+  // group images to group_out (device, or host through a chunk of scratch); RGB8 is optional
+  uint32_t n_groups = 0;
+  uint32_t group_mask[kMaxGroups] = {};
+  double* group_out = nullptr;
   const char* overflow_error = "rh_render: ray queue overflow; lower chunk_samples";
-  // renders (not traces or list frames) tune the scene's shadow schedule and record its queue factor and row costs
-  bool learns() const { return !trace && !pixel_list; }
+  // renders (not traces, list frames or light-group frames) tune the scene's shadow schedule and record its queue factor
+  // and row costs
+  bool learns() const { return !trace && !pixel_list && !n_groups; }
 };
 
-// rh_render's argument checks (`who` names the entry point in the messages).  With f->accumulate, f->pixel_list or
-// f->features set, rgb_out may be null.
+// rh_render's argument checks (`who` names the entry point in the messages).  With f->accumulate, f->pixel_list,
+// f->features or f->n_groups set, rgb_out may be null.
 int render_frame(Device* D, const rh_scene* scene, const rh_camera* camera, const rh_render_opts* o, uint8_t* rgb_out,
                  int32_t* hit_ids_out, Frame* f, const char* who = "rh_render") {
   const std::string w(who);
   const bool peer_frames = o && (o->flags & RH_FLAG_PEER_FRAMES) != 0;
-  if (!scene || !camera || !o || (!rgb_out && !peer_frames && !f->accumulate && !f->pixel_list && !f->features))
+  if (!scene || !camera || !o || (!rgb_out && !peer_frames && !f->accumulate && !f->pixel_list && !f->features && !f->n_groups))
     return rh::set_error(RH_ERR_ARG, w + ": null argument");
   if (peer_frames && (!o->peer_frames || o->n_peer_frames <= 0 || o->n_peer_frames > kMaxPeers))
     return rh::set_error(RH_ERR_ARG, w + ": RH_FLAG_PEER_FRAMES needs 1..16 peer frame pointers");
@@ -1736,6 +1744,10 @@ struct FrameRun {
   uint8_t* d_rgb = nullptr;
   int2* d_ids = nullptr;
   double* d_linear = nullptr;
+  // light-group frames: where the group sink writes (the caller's device buffer, else the lane's chunk of scratch), and
+  // the doubles between two group images there
+  bool group_out_dev = false;
+  size_t group_out_stride = 0;
   const void* d_offsets = nullptr;
   int off_index = kOffIndexLocal;
   unsigned long long offset_seed = 0;
@@ -1794,6 +1806,7 @@ struct FrameRun {
     const int ln = i % n_lanes;
     Device::Scratch& sc = D->lane[ln];
     const cudaStream_t lane_stream = ln ? D->stream2 : D->stream;
+    double* group_out = group_out_dev ? f.group_out : (double*)sc.group_out.p;
     ChunkParams P{};
     P.first_row = first_row;
     P.n_rows = n_rows;
@@ -1860,6 +1873,14 @@ struct FrameRun {
     P.list = f.list;
     for (int plane = 0; plane < 3; plane++)  // (three 1-D memsets: a 2-D one is limited to 2 GB of pitch)
       RH_CUDA(cudaMemsetAsync((double*)sc.accum.p + (size_t)plane * chunk_samples, 0, (size_t)P.n_samples * sizeof(double), lane_stream));
+    if (f.n_groups) {
+      P.groups = (double*)sc.groups.p;
+      P.group_stride = (uint32_t)chunk_samples;
+      P.n_groups = f.n_groups;
+      memcpy(P.group_mask, f.group_mask, sizeof P.group_mask);
+      // the 3 (n_groups + 1) planes follow each other: one memset up to the last plane's n_samples
+      RH_CUDA(cudaMemsetAsync(P.groups, 0, ((size_t)(3 * f.n_groups + 2) * chunk_samples + P.n_samples) * sizeof(double), lane_stream));
+    }
     const cudaStream_t shadow_stream = pipelined ? D->shadow_stream[ln] : lane_stream;
     for (int pass = 0; pass < n_passes; pass++) {
       P.pass = pass;
@@ -1900,11 +1921,23 @@ struct FrameRun {
       launch_accumulate_resolve(P, A, lane_stream);
     } else if (f.pixel_list) {
       launch_adaptive_fold(P, f.ad, lane_stream);
-    } else {
+    } else if (!f.n_groups) {
       launch_resolve(P, lane_stream);
+    } else {
+      if (d_rgb) {  // (a light-group frame without RGB8 output has no use for the resolve)
+        launch_resolve(P, lane_stream);
+        launches += 1;
+      }
+      launch_light_groups_resolve(P, group_out, group_out_stride, group_out_dev ? (size_t)first_row * o.width : 0, lane_stream);
     }
     if (sh.profile) spans.push_back({a, prof_event(lane_stream), 2});
     launches += 1;
+    if (f.n_groups && !group_out_dev) {  // host output: the chunk's rows of every group image
+      const size_t plane = (size_t)f.rows_local * o.width * 3, at = (size_t)first_row * o.width * 3;
+      for (uint32_t g = 0; g <= f.n_groups; g++)
+        RH_CUDA(cudaMemcpyAsync(f.group_out + g * plane + at, group_out + g * group_out_stride, (size_t)n_rows * o.width * 3 * sizeof(double),
+                                cudaMemcpyDeviceToHost, lane_stream));
+    }
     if (host_offsets) {
       RH_CUDA(cudaEventRecord(D->ev_done[i % ring], lane_stream));
       chunk_ev.push_back(prof_event(lane_stream));
@@ -2105,8 +2138,12 @@ int run_frame(Device* D, const rh_scene* scene, const Frame& f, rh_stats* stats)
   // finished last
   const bool know_cost = f.learns() && (int)scene->row_cost.size() == f.rows_local &&
                          scene->cost_key == std::vector<int>{o.width, o.height, o.spp, o.shard_count, o.shard_index, o.band_height};
+  // a light-group frame's chunks also hold 3 doubles per group and sample, and (host output) per group and pixel
+  const size_t group_bytes = f.n_groups ? 3 * sizeof(double) * (f.n_groups + 1) : 0;
+  R.group_out_dev = dev_out;
   R.plan = rh::plan_chunks(f.rows_local, R.row_samples, o.chunk_samples, D->total_mem, R.host_offsets,
-                           know_cost ? scene->row_cost.data() : nullptr, scene->stream_compute_bound);
+                           know_cost ? scene->row_cost.data() : nullptr, scene->stream_compute_bound,
+                           rh::kBytesPerSample + group_bytes * (dev_out ? 1 : 2));
   R.n_chunks = (int)R.plan.rows.size();
   R.chunk_samples = (size_t)*std::max_element(R.plan.rows.begin(), R.plan.rows.end()) * R.row_samples;
   if (R.chunk_samples > 0x7fffffffu) return rh::set_error(RH_ERR_ARG, "rh_render: chunk too large");
@@ -2142,6 +2179,14 @@ int run_frame(Device* D, const rh_scene* scene, const Frame& f, rh_stats* stats)
   R.pipelined = !R.sh.profile && !R.counting && R.n_passes >= 2 && R.n_chunks == 1;
   for (int l = 0; l < R.n_lanes; l++)
     if ((rc = D->lane[l].accum.reserve(R.chunk_samples * 3 * sizeof(double)))) return rc;
+  if (f.n_groups) {
+    const size_t chunk_px = R.chunk_samples / o.spp;
+    R.group_out_stride = dev_out ? (size_t)f.rows_local * o.width * 3 : chunk_px * 3;
+    for (int l = 0; l < R.n_lanes; l++) {
+      if ((rc = D->lane[l].groups.reserve(R.chunk_samples * group_bytes))) return rc;
+      if (!dev_out && (rc = D->lane[l].group_out.reserve(chunk_px * group_bytes))) return rc;
+    }
+  }
   const size_t ctl_bytes = (size_t)R.n_chunks * sizeof(ChunkCtl);
   if ((rc = D->ctl.reserve(ctl_bytes))) return rc;
   if ((rc = D->counters.reserve(sizeof(FrameCounters)))) return rc;
@@ -2834,6 +2879,42 @@ int features_on(Device* D, const rh_scene* scene, const rh_camera* camera, const
   return RH_OK;
 }
 
+// ------------------------------------------------------------------ light groups
+// rh_render_light_groups is a render (render_frame's checks, run_frame's plan, queues, overflow retry and passes) whose
+// shadow kernels also add each group's terms beside the sample's, and whose chunks end with the group sink beside the
+// resolve.  Like a list frame it uses the scene's learned state without changing it.
+int light_groups_on(Device* D, const rh_scene* scene, const rh_camera* camera, const rh_render_opts* o, const rh_light_groups* lg,
+                    uint8_t* rgb_out, int32_t* hit_ids_out, rh_stats* stats) {
+  const std::string w = "rh_render_light_groups";
+  if (!lg) return rh::set_error(RH_ERR_ARG, w + ": null argument");
+  if (o && (o->flags & (RH_FLAG_PEER_FRAMES | RH_FLAG_COUNT)))
+    return rh::set_error(RH_ERR_ARG, w + ": RH_FLAG_PEER_FRAMES and RH_FLAG_COUNT are not supported");
+  if (lg->n_groups < 1 || lg->n_groups > (uint32_t)kMaxGroups) return rh::set_error(RH_ERR_ARG, w + ": n_groups must be 1..16");
+  if (lg->reserved_) return rh::set_error(RH_ERR_ARG, w + ": reserved_ must be 0");
+  if (!lg->out) return rh::set_error(RH_ERR_ARG, w + ": out is null");
+  Frame f;
+  f.n_groups = lg->n_groups;
+  int rc = render_frame(D, scene, camera, o, rgb_out, hit_ids_out, &f, "rh_render_light_groups");
+  if (rc) return rc;
+  const uint32_t n_lights = scene->view.n_lights;
+  if (n_lights > (uint32_t)kMaskLights) return rh::set_error(RH_ERR_ARG, w + ": scenes with more than 32 lights are not supported");
+  if (n_lights && !lg->group_of_light) return rh::set_error(RH_ERR_ARG, w + ": group_of_light is null");
+  for (uint32_t l = 0; l < n_lights; l++) {
+    const uint32_t g = lg->group_of_light[l];
+    if (g >= lg->n_groups)
+      return rh::set_error(RH_ERR_ARG, w + ": group_of_light[" + std::to_string(l) + "] = " + std::to_string(g) + " is not below n_groups");
+    f.group_mask[g] |= 1u << l;
+  }
+  f.group_out = lg->out;
+  f.overflow_error = "rh_render_light_groups: ray queue overflow; lower chunk_samples";
+  if (o->flags & RH_FLAG_DEVICE_OUT) {
+    if ((uintptr_t)lg->out % 8) return rh::set_error(RH_ERR_ARG, w + ": device out must be 8-byte aligned");
+    RH_CUDA(cudaSetDevice(D->dev));
+    if ((rc = check_device_pointers({lg->out}, w + ": RH_FLAG_DEVICE_OUT with a pointer that is not device memory"))) return rc;
+  }
+  return run_frame(D, scene, f, stats);
+}
+
 }  // namespace
 
 // ================================================================== C ABI
@@ -3023,6 +3104,12 @@ int rh_render_features(const rh_scene* scene, const rh_camera* camera, const rh_
                        int32_t* hit_ids_out, rh_stats* stats) {
   if (!g_dev) return rh::set_error(RH_ERR_STATE, "rh_render_features: call rh_init first");
   return features_on(g_dev.get(), scene, camera, opts, features, hit_ids_out, stats);
+}
+
+int rh_render_light_groups(const rh_scene* scene, const rh_camera* camera, const rh_render_opts* opts,
+                           const rh_light_groups* groups, uint8_t* rgb_out, int32_t* hit_ids_out, rh_stats* stats) {
+  if (!g_dev) return rh::set_error(RH_ERR_STATE, "rh_render_light_groups: call rh_init first");
+  return light_groups_on(g_dev.get(), scene, camera, opts, groups, rgb_out, hit_ids_out, stats);
 }
 
 int rh_default_band_height(int height, int shard_count) {

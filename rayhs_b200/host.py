@@ -512,6 +512,100 @@ def renderFeatures(job: Rendering, spp: int = 1, offsets=None, seed: int | None 
     return fe
 
 
+# ---- light groups (one linear image per group of lights, for relighting in compositing)
+
+@dataclass
+class LightGroups:
+    """rh_render_light_groups of one view: groups [G, rows, w, 3] float64, the linear image of each group of lights;
+    rest [rows, w, 3], what no light adds (Diffuse's ambient term, Emmit, ShowNormal, ShowUV); image, the render's RGB8
+    rows (None unless asked for); hit_ids [rows, w, spp, 2] when asked for; and the call's stats.  numpy arrays, or CUDA
+    tensors for a call with device outputs."""
+    groups: object
+    rest: object
+    image: object = None
+    hit_ids: object = None
+    stats: dict = field(default_factory=dict)
+
+    def relight(self, scales):
+        """sum over g of scales[g] * groups[g] (per channel, in group order), plus rest: the image with the colours of
+        group g's lights multiplied by scales[g], up to rounding.  scales: [G, 3]."""
+        on_device = getattr(self.groups, "is_cuda", False)
+        if on_device:
+            import torch
+
+            s = torch.as_tensor(scales, dtype=torch.float64).to(self.groups.device)
+        else:
+            s = np.asarray(scales, dtype=np.float64)
+        G = self.groups.shape[0]
+        if tuple(s.shape) != (G, 3):
+            raise ValueError(f"scales must have shape [{G}, 3], got {tuple(s.shape)}")
+        out = s[0] * self.groups[0]
+        for g in range(1, G):
+            out = out + s[g] * self.groups[g]
+        return out + self.rest
+
+
+def renderLightGroups(job: Rendering, spp: int = 1, offsets=None, seed: int | None = None, groups=None, rgb: bool = True,
+                      want_hit_ids: bool = False, shadow: str | None = None, exact_boxes: bool = False, light_maps: bool = True,
+                      chunk_samples: int = 0, shard_index: int = 0, shard_count: int = 1, band_height: int = 0,
+                      device: bool = False, profile: bool = False) -> LightGroups:
+    """The light groups of the frame render(job, spp, offsets / seed, ...) renders.  `groups`: the group of each of the
+    scene's lights (a sequence of ints, G = largest + 1 <= 16); None: one group per light.  `offsets`: full-frame
+    [width*height, spp, 2] float64 / float32, numpy, a CPU tensor or a CUDA tensor; `seed`: the SplitMix64 stream
+    instead.  CUDA offsets or device=True: the outputs are CUDA tensors.  `rgb`: also return the render's RGB8 rows."""
+    L = lib()
+    n_lights = job.scene.raw.contents.n_lights
+    if groups is None:
+        groups = list(range(n_lights))
+    groups = [int(g) for g in groups]
+    if len(groups) != n_lights:
+        raise ValueError(f"groups has {len(groups)} entries for a scene with {n_lights} lights")
+    if any(not 0 <= g < 16 for g in groups):
+        raise ValueError("group indices must be in 0 .. 15")
+    G = max(groups, default=0) + 1
+    mode, off = _offset_mode(offsets, 0)
+    off_ptr, seed_box = None, None
+    if seed is not None:
+        if offsets is not None:
+            raise ValueError("pass either offsets or seed")
+        seed_box = C.c_uint64(seed)
+        mode, off_ptr = capi.RH_OFFSETS_SPLITMIX64, C.addressof(seed_box)
+    dev_off = getattr(off, "is_cuda", False)
+    device = device or dev_off
+    if off is not None:
+        have = off.numel() if hasattr(off, "numel") else off.size
+        if have != job.width * job.height * spp * 2:
+            raise ValueError(f"offsets has {have} values, expected {job.width * job.height * spp * 2}")
+        off = off.contiguous() if hasattr(off, "contiguous") else np.ascontiguousarray(off)
+        off_ptr = _ptr(off)
+    flags = ((capi.RH_FLAG_HIT_IDS if want_hit_ids else 0) | (capi.RH_FLAG_EXACT_BOXES if exact_boxes else 0) | _shadow_flag(shadow)
+             | (0 if light_maps else capi.RH_FLAG_NO_LIGHT_MAPS) | (capi.RH_FLAG_PROFILE if profile else 0)
+             | (capi.RH_FLAG_DEVICE_OUT if device else 0) | (capi.RH_FLAG_DEVICE_OFFSETS if dev_off else 0))
+    bh = band_height or L.rh_default_band_height(job.height, shard_count)
+    rows = L.rh_shard_rows(job.height, shard_count, bh)
+    o = _opts(job, spp, mode, off_ptr, 0, shard_index, shard_count, bh, chunk_samples, flags)
+    if device:
+        import torch
+
+        def empty(s, dtype):
+            return torch.empty(s, dtype=getattr(torch, dtype), device="cuda")
+
+        torch.cuda.current_stream().synchronize()  # the library runs on its own stream
+    else:
+        def empty(s, dtype):
+            return np.empty(s, dtype=dtype)
+    out = empty((G + 1, rows, job.width, 3), "float64")
+    image = empty((rows, job.width, 3), "uint8") if rgb else None
+    ids = empty((rows, job.width, spp, 2), "int32") if want_hit_ids else None
+    map_ = (C.c_uint8 * max(n_lights, 1))(*groups)
+    lg = capi.rh_light_groups()
+    lg.group_of_light, lg.n_groups, lg.out = C.addressof(map_), G, _ptr(out)
+    st = capi.rh_stats()
+    check(L.rh_render_light_groups(job.scene.device, C.byref(job.camera), C.byref(o), C.byref(lg),
+                                   _ptr(image) if rgb else None, _ptr(ids) if want_hit_ids else None, C.byref(st)))
+    return LightGroups(out[:G], out[G], image, ids, st.as_dict())
+
+
 def scene_setup_ms(scene: Scene) -> dict:
     """Milliseconds rh_scene_create spent on its parts (host-side trees, light-space tables, uploads)."""
     ms, info = scene._info()
