@@ -255,14 +255,59 @@ def _opts(job: Rendering, spp: int, mode: int, offsets_ptr, tile: int, shard_ind
     return o
 
 
-def _offset_mode(offsets, tile: int):
+def _ptr(a):
+    return a.data_ptr() if hasattr(a, "data_ptr") else a.ctypes.data
+
+
+def _offsets(job: Rendering, spp: int, offsets, seed: int | None, tile: int, shard_rows: int | None = None):
+    """The sample source of one call: `offsets` (float64 / float32 values of the full frame, [width*height, spp, 2]; of
+    a tile, [tile*tile, spp, 2]; or with `shard_rows` of this shard's rows only, [shard_rows*width, spp, 2]: numpy, a
+    CPU tensor or a CUDA tensor), `seed` (the SplitMix64 stream the library regenerates) or neither (pixel centres).
+    Returns (mode, pointer, keep, on_device): `keep` holds what the pointer refers to (the seed, or the dense copy of a
+    strided view, which the library could not read) and must outlive the call; `on_device`: the offsets are CUDA."""
+    if seed is not None:
+        if offsets is not None:
+            raise ValueError("pass either offsets or seed")
+        box = C.c_uint64(seed)
+        return capi.RH_OFFSETS_SPLITMIX64, C.addressof(box), box, False
     if offsets is None:
-        return capi.RH_OFFSETS_NONE, None
-    if tile:
-        return capi.RH_OFFSETS_TILED_F64, offsets
-    if hasattr(offsets, "dtype") and str(offsets.dtype).endswith("float32"):
-        return capi.RH_OFFSETS_F32, offsets
-    return capi.RH_OFFSETS_F64, offsets
+        return capi.RH_OFFSETS_NONE, None, None, False
+    need = (tile * tile if tile else (job.height if shard_rows is None else shard_rows) * job.width) * spp * 2
+    have = offsets.numel() if hasattr(offsets, "numel") else offsets.size
+    if have != need:
+        raise ValueError(f"offsets has {have} values, expected {need}")
+    mode = (capi.RH_OFFSETS_TILED_F64 if tile else capi.RH_OFFSETS_F32 if str(offsets.dtype).endswith("float32")
+            else capi.RH_OFFSETS_F64)
+    off = offsets.contiguous() if hasattr(offsets, "contiguous") else np.ascontiguousarray(offsets)
+    return mode, _ptr(off), off, bool(getattr(off, "is_cuda", False))
+
+
+def _flags(*, want_hit_ids: bool = False, device: bool = False, count: bool = False, profile: bool = False,
+           exact_boxes: bool = False, shadow: str | None = None, light_maps: bool = True) -> int:
+    """RH_FLAG_* bits of the keyword arguments the entry points share.  `shadow`, the shadow-walk schedule: None = the
+    library's per-scene choice, 'pooled' / 'split' (per-lane refill) = forced (same image)."""
+    return ((capi.RH_FLAG_HIT_IDS if want_hit_ids else 0) | (capi.RH_FLAG_DEVICE_OUT if device else 0)
+            | (capi.RH_FLAG_COUNT if count else 0) | (capi.RH_FLAG_PROFILE if profile else 0)
+            | (capi.RH_FLAG_EXACT_BOXES if exact_boxes else 0) | (0 if light_maps else capi.RH_FLAG_NO_LIGHT_MAPS)
+            | (0 if shadow is None else {"pooled": capi.RH_FLAG_SHADOW_POOLED, "split": capi.RH_FLAG_SHADOW_SPLIT}[shadow]))
+
+
+def _shard_rows(job: Rendering, shard_count: int, band_height: int):
+    """(band height, rows of one shard): `band_height` 0 is the library's choice."""
+    L = lib()
+    bh = band_height or L.rh_default_band_height(job.height, shard_count)
+    return bh, L.rh_shard_rows(job.height, shard_count, bh)
+
+
+def _alloc(device: bool):
+    """empty(shape, dtype name) for a call's outputs: numpy arrays, or CUDA tensors with `device`.  On the device the
+    current torch stream is synchronised first, since the library runs on its own stream."""
+    if not device:
+        return lambda shape, dtype: np.empty(shape, dtype=dtype)
+    import torch
+
+    torch.cuda.current_stream().synchronize()
+    return lambda shape, dtype: torch.empty(shape, dtype=getattr(torch, dtype), device="cuda")
 
 
 def render(job: Rendering, spp: int = 1, offsets=None, offset_tile: int = 0, want_hit_ids: bool = False,
@@ -272,32 +317,18 @@ def render(job: Rendering, spp: int = 1, offsets=None, offset_tile: int = 0, wan
     """One rh_render call with HOST buffers (numpy or pinned torch CPU tensors for `offsets`).
     `seed` (instead of `offsets`): the kernel regenerates sample_offsets(width*height, spp, seed) on the device.
     Returns the shard-compact RGB8 rows when shard_count > 1."""
-    L = lib()
-    mode, off = _offset_mode(offsets, offset_tile)
-    off_ptr = None
-    seed_box = None
-    if seed is not None:
-        if offsets is not None:
-            raise ValueError("pass either offsets or seed")
-        seed_box = C.c_uint64(seed)
-        mode, off, off_ptr = capi.RH_OFFSETS_SPLITMIX64, None, C.addressof(seed_box)
-    if off is not None:
-        off_ptr = off.data_ptr() if hasattr(off, "data_ptr") else off.ctypes.data
-        need = (offset_tile * offset_tile if offset_tile else job.width * job.height) * spp * 2
-        have = off.numel() if hasattr(off, "numel") else off.size
-        if have != need:
-            raise ValueError(f"offsets has {have} values, expected {need}")
-    bh = band_height or L.rh_default_band_height(job.height, shard_count)
-    rows = L.rh_shard_rows(job.height, shard_count, bh)
-    flags = ((capi.RH_FLAG_HIT_IDS if want_hit_ids else 0) | (capi.RH_FLAG_COUNT if count else 0)
-             | (capi.RH_FLAG_PROFILE if profile else 0) | (capi.RH_FLAG_EXACT_BOXES if exact_boxes else 0) | _shadow_flag(shadow)
-             | (0 if light_maps else capi.RH_FLAG_NO_LIGHT_MAPS))
+    mode, off_ptr, keep, on_device = _offsets(job, spp, offsets, seed, offset_tile)
+    if on_device:
+        raise ValueError("CUDA offsets go to render_device; render takes host offsets")
+    bh, rows = _shard_rows(job, shard_count, band_height)
+    flags = _flags(want_hit_ids=want_hit_ids, count=count, profile=profile, exact_boxes=exact_boxes, shadow=shadow,
+                   light_maps=light_maps)
     o = _opts(job, spp, mode, off_ptr, offset_tile, shard_index, shard_count, bh, chunk_samples, flags)
     rgb = out if out is not None else np.empty((rows, job.width, 3), dtype=np.uint8)
     ids = np.empty((rows, job.width, spp, 2), dtype=np.int32) if want_hit_ids else None
     st = capi.rh_stats()
-    check(L.rh_render(job.scene.device, C.byref(job.camera), C.byref(o), rgb.ctypes.data,
-                      ids.ctypes.data if ids is not None else None, C.byref(st)))
+    check(lib().rh_render(job.scene.device, C.byref(job.camera), C.byref(o), rgb.ctypes.data,
+                          ids.ctypes.data if ids is not None else None, C.byref(st)))
     return Image(job.width, rows, rgb, st.as_dict(), ids)
 
 
@@ -325,7 +356,8 @@ class Hits:
 
 def _query_rays(origins, directions):
     """Checks a batch of rays and packs it as the library's [n, 6] (origin, direction) float64 array: numpy arrays (host
-    path) or CUDA tensors on the current device (device path).  Returns (rays, on_device)."""
+    path) or CUDA tensors on the current device (device path; _alloc(True) synchronises the packing).  Returns (rays,
+    on_device)."""
     if isinstance(origins, np.ndarray) and isinstance(directions, np.ndarray):
         on_device = False
     elif all(type(x).__module__.startswith("torch") and getattr(x, "is_cuda", False) for x in (origins, directions)):
@@ -346,16 +378,10 @@ def _query_rays(origins, directions):
     if on_device:
         import torch
 
-        rays = torch.cat((origins, directions), dim=1).contiguous()
-        torch.cuda.current_stream().synchronize()  # the library runs on its own stream
-        return rays, True
+        return torch.cat((origins, directions), dim=1).contiguous(), True
     rays = np.empty((origins.shape[0], 6), dtype=np.float64)
     rays[:, :3], rays[:, 3:] = origins, directions
     return rays, False
-
-
-def _ptr(a):
-    return a.data_ptr() if hasattr(a, "data_ptr") else a.ctypes.data
 
 
 def closestIntersection(scene, origins, directions, exact_boxes: bool = False) -> Hits:
@@ -364,16 +390,14 @@ def closestIntersection(scene, origins, directions, exact_boxes: bool = False) -
     `exact_boxes`: the reference's double slab test at every box (validation; same records)."""
     rays, on_device = _query_rays(origins, directions)
     n = rays.shape[0]
-    flags = (capi.RH_FLAG_DEVICE_OUT if on_device else 0) | (capi.RH_FLAG_EXACT_BOXES if exact_boxes else 0)
+    rec = _alloc(on_device)((n, HIT_DTYPE.itemsize), "uint8")
+    check(lib().rh_closest_intersection(scene.device, _ptr(rays), n, _ptr(rec), _flags(device=on_device, exact_boxes=exact_boxes)))
     if on_device:
         import torch
 
-        rec = torch.empty((n, HIT_DTYPE.itemsize), dtype=torch.uint8, device=rays.device)
-        check(lib().rh_closest_intersection(scene.device, rays.data_ptr(), n, rec.data_ptr(), flags))
         f, i = rec.view(torch.float64), rec.view(torch.int32)
         return Hits(f[:, 0], f[:, 1:4], f[:, 4:7], f[:, 7:9], i[:, 18], i[:, 19], rec)
-    rec = np.empty(n, dtype=HIT_DTYPE)
-    check(lib().rh_closest_intersection(scene.device, rays.ctypes.data, n, rec.ctypes.data, flags))
+    rec = rec.view(HIT_DTYPE).reshape(n)
     return Hits(rec["t"], rec["p"], rec["n"], rec["uv"], rec["object"], rec["tri"], rec)
 
 
@@ -383,15 +407,13 @@ def shadowIntersection(scene, light: int, origins, directions, exact_boxes: bool
     Returns a bool numpy array or CUDA tensor, like the rays."""
     rays, on_device = _query_rays(origins, directions)
     n = rays.shape[0]
-    flags = (capi.RH_FLAG_DEVICE_OUT if on_device else 0) | (capi.RH_FLAG_EXACT_BOXES if exact_boxes else 0)
+    out = _alloc(on_device)(n, "uint8")
+    check(lib().rh_shadow_intersection(scene.device, int(light), _ptr(rays), n, _ptr(out), _flags(device=on_device, exact_boxes=exact_boxes)))
     if on_device:
         import torch
 
-        out = torch.empty(n, dtype=torch.uint8, device=rays.device)
-    else:
-        out = np.empty(n, dtype=np.uint8)
-    check(lib().rh_shadow_intersection(scene.device, int(light), _ptr(rays), n, _ptr(out), flags))
-    return out.view(torch.bool) if on_device else out.view(np.bool_)
+        return out.view(torch.bool)
+    return out.view(np.bool_)
 
 
 # ---- radiance queries (RayHs.hs:149-154 traceRay)
@@ -419,16 +441,10 @@ def traceRay(scene, origins, directions, max_depth: int, *, want_hit_ids: bool =
     n = rays.shape[0]
     o = capi.rh_trace_opts()
     o.max_depth, o.chunk_rays = int(max_depth), int(chunk_rays)
-    o.flags = ((capi.RH_FLAG_DEVICE_OUT if on_device else 0) | (capi.RH_FLAG_HIT_IDS if want_hit_ids else 0)
-               | (capi.RH_FLAG_EXACT_BOXES if exact_boxes else 0) | _shadow_flag(shadow) | (0 if light_maps else capi.RH_FLAG_NO_LIGHT_MAPS))
-    if on_device:
-        import torch
-
-        colors = torch.empty((n, 3), dtype=torch.float64, device=rays.device)
-        ids = torch.empty((n, 2), dtype=torch.int32, device=rays.device) if want_hit_ids else None
-    else:
-        colors = np.empty((n, 3), dtype=np.float64)
-        ids = np.empty((n, 2), dtype=np.int32) if want_hit_ids else None
+    o.flags = _flags(device=on_device, want_hit_ids=want_hit_ids, exact_boxes=exact_boxes, shadow=shadow, light_maps=light_maps)
+    empty = _alloc(on_device)
+    colors = empty((n, 3), "float64")
+    ids = empty((n, 2), "int32") if want_hit_ids else None
     st = capi.rh_stats()
     check(lib().rh_trace_rays(scene.device, _ptr(rays), n, C.byref(o), _ptr(colors), _ptr(ids) if ids is not None else None,
                               C.byref(st)))
@@ -460,54 +476,25 @@ def renderFeatures(job: Rendering, spp: int = 1, offsets=None, seed: int | None 
     or, with device=True, a CUDA tensor (a strided view is copied to a dense array first); `seed`: the SplitMix64 stream
     instead, samples stream_base .. stream_base + spp - 1 of a stream of `stream_spp` samples per pixel (0: spp), as an
     Accumulator holding stream_base samples draws them.  `device`: outputs are CUDA tensors."""
-    L = lib()
-    mode, off = _offset_mode(offsets, offset_tile)
-    off_ptr, seed_box = None, None
-    flags = ((capi.RH_FLAG_HIT_IDS if want_hit_ids else 0) | (capi.RH_FLAG_EXACT_BOXES if exact_boxes else 0)
-             | (capi.RH_FLAG_DEVICE_OUT if device else 0))
-    if seed is not None:
-        if offsets is not None:
-            raise ValueError("pass either offsets or seed")
-        seed_box = C.c_uint64(seed)
-        mode, off_ptr = capi.RH_OFFSETS_SPLITMIX64, C.addressof(seed_box)
-    elif stream_spp or stream_base:
+    if seed is None and (stream_spp or stream_base):
         raise ValueError("stream_spp and stream_base go with seed")
-    elif off is not None:
-        need = (offset_tile * offset_tile if offset_tile else job.width * job.height) * spp * 2
-        have = off.numel() if hasattr(off, "numel") else off.size
-        if have != need:
-            raise ValueError(f"offsets has {have} values, expected {need}")
-        if getattr(off, "is_cuda", False):
-            if not device:
-                raise ValueError("CUDA offsets need device=True")
-            flags |= capi.RH_FLAG_DEVICE_OFFSETS
-        off = off.contiguous() if hasattr(off, "contiguous") else np.ascontiguousarray(off)
-        off_ptr = _ptr(off)
-    bh = band_height or L.rh_default_band_height(job.height, shard_count)
-    rows = L.rh_shard_rows(job.height, shard_count, bh)
+    mode, off_ptr, keep, dev_off = _offsets(job, spp, offsets, seed, offset_tile)
+    if dev_off and not device:
+        raise ValueError("CUDA offsets need device=True")
+    flags = _flags(want_hit_ids=want_hit_ids, exact_boxes=exact_boxes, device=device) | (capi.RH_FLAG_DEVICE_OFFSETS if dev_off else 0)
+    bh, rows = _shard_rows(job, shard_count, band_height)
     o = _opts(job, spp, mode, off_ptr, offset_tile, shard_index, shard_count, bh, 0, flags)
     shape = (rows, job.width)
-    if device:
-        import torch
-
-        def empty(s, dtype):
-            return torch.empty(s, dtype=getattr(torch, dtype), device="cuda")
-
-        hits_dtype = "int32"  # (torch has no uint32 arithmetic to speak of)
-        torch.cuda.current_stream().synchronize()  # the library runs on its own stream
-    else:
-        def empty(s, dtype):
-            return np.empty(s, dtype=dtype)
-
-        hits_dtype = "uint32"
+    empty = _alloc(device)
+    hits_dtype = "int32" if device else "uint32"  # (torch has no uint32 arithmetic to speak of)
     fe = Features(empty(shape + (3,), "float64"), empty(shape + (3,), "float64"), empty(shape, "float64"), empty(shape, hits_dtype),
                   empty(shape + (spp, 2), "int32") if want_hit_ids else None)
     ft = capi.rh_features()
     ft.albedo, ft.normal, ft.depth, ft.hits = (_ptr(a) for a in (fe.albedo, fe.normal, fe.depth, fe.hits))
     ft.stream_spp, ft.stream_base = int(stream_spp), int(stream_base)
     st = capi.rh_stats()
-    check(L.rh_render_features(job.scene.device, C.byref(job.camera), C.byref(o), C.byref(ft),
-                               _ptr(fe.hit_ids) if want_hit_ids else None, C.byref(st)))
+    check(lib().rh_render_features(job.scene.device, C.byref(job.camera), C.byref(o), C.byref(ft),
+                                   _ptr(fe.hit_ids) if want_hit_ids else None, C.byref(st)))
     fe.stats = st.as_dict()
     return fe
 
@@ -553,7 +540,6 @@ def renderLightGroups(job: Rendering, spp: int = 1, offsets=None, seed: int | No
     scene's lights (a sequence of ints, G = largest + 1 <= 16); None: one group per light.  `offsets`: full-frame
     [width*height, spp, 2] float64 / float32, numpy, a CPU tensor or a CUDA tensor; `seed`: the SplitMix64 stream
     instead.  CUDA offsets or device=True: the outputs are CUDA tensors.  `rgb`: also return the render's RGB8 rows."""
-    L = lib()
     n_lights = job.scene.raw.contents.n_lights
     if groups is None:
         groups = list(range(n_lights))
@@ -563,37 +549,13 @@ def renderLightGroups(job: Rendering, spp: int = 1, offsets=None, seed: int | No
     if any(not 0 <= g < 16 for g in groups):
         raise ValueError("group indices must be in 0 .. 15")
     G = max(groups, default=0) + 1
-    mode, off = _offset_mode(offsets, 0)
-    off_ptr, seed_box = None, None
-    if seed is not None:
-        if offsets is not None:
-            raise ValueError("pass either offsets or seed")
-        seed_box = C.c_uint64(seed)
-        mode, off_ptr = capi.RH_OFFSETS_SPLITMIX64, C.addressof(seed_box)
-    dev_off = getattr(off, "is_cuda", False)
+    mode, off_ptr, keep, dev_off = _offsets(job, spp, offsets, seed, 0)
     device = device or dev_off
-    if off is not None:
-        have = off.numel() if hasattr(off, "numel") else off.size
-        if have != job.width * job.height * spp * 2:
-            raise ValueError(f"offsets has {have} values, expected {job.width * job.height * spp * 2}")
-        off = off.contiguous() if hasattr(off, "contiguous") else np.ascontiguousarray(off)
-        off_ptr = _ptr(off)
-    flags = ((capi.RH_FLAG_HIT_IDS if want_hit_ids else 0) | (capi.RH_FLAG_EXACT_BOXES if exact_boxes else 0) | _shadow_flag(shadow)
-             | (0 if light_maps else capi.RH_FLAG_NO_LIGHT_MAPS) | (capi.RH_FLAG_PROFILE if profile else 0)
-             | (capi.RH_FLAG_DEVICE_OUT if device else 0) | (capi.RH_FLAG_DEVICE_OFFSETS if dev_off else 0))
-    bh = band_height or L.rh_default_band_height(job.height, shard_count)
-    rows = L.rh_shard_rows(job.height, shard_count, bh)
+    flags = (_flags(want_hit_ids=want_hit_ids, exact_boxes=exact_boxes, shadow=shadow, light_maps=light_maps, profile=profile,
+                    device=device) | (capi.RH_FLAG_DEVICE_OFFSETS if dev_off else 0))
+    bh, rows = _shard_rows(job, shard_count, band_height)
     o = _opts(job, spp, mode, off_ptr, 0, shard_index, shard_count, bh, chunk_samples, flags)
-    if device:
-        import torch
-
-        def empty(s, dtype):
-            return torch.empty(s, dtype=getattr(torch, dtype), device="cuda")
-
-        torch.cuda.current_stream().synchronize()  # the library runs on its own stream
-    else:
-        def empty(s, dtype):
-            return np.empty(s, dtype=dtype)
+    empty = _alloc(device)
     out = empty((G + 1, rows, job.width, 3), "float64")
     image = empty((rows, job.width, 3), "uint8") if rgb else None
     ids = empty((rows, job.width, spp, 2), "int32") if want_hit_ids else None
@@ -601,8 +563,8 @@ def renderLightGroups(job: Rendering, spp: int = 1, offsets=None, seed: int | No
     lg = capi.rh_light_groups()
     lg.group_of_light, lg.n_groups, lg.out = C.addressof(map_), G, _ptr(out)
     st = capi.rh_stats()
-    check(L.rh_render_light_groups(job.scene.device, C.byref(job.camera), C.byref(o), C.byref(lg),
-                                   _ptr(image) if rgb else None, _ptr(ids) if want_hit_ids else None, C.byref(st)))
+    check(lib().rh_render_light_groups(job.scene.device, C.byref(job.camera), C.byref(o), C.byref(lg),
+                                       _ptr(image) if rgb else None, _ptr(ids) if want_hit_ids else None, C.byref(st)))
     return LightGroups(out[:G], out[G], image, ids, st.as_dict())
 
 
@@ -610,14 +572,6 @@ def scene_setup_ms(scene: Scene) -> dict:
     """Milliseconds rh_scene_create spent on its parts (host-side trees, light-space tables, uploads)."""
     ms, info = scene._info()
     return {"trees": ms[0], "light_tables": ms[1], "upload": ms[2], "deep_stack_entries_per_thread": info[3], "max_tree_depth": info[2]}
-
-
-def _shadow_flag(shadow: str | None) -> int:
-    """Shadow-walk schedule: None = the library's per-scene choice, 'pooled' / 'split' (per-lane refill) = forced
-    (same image)."""
-    if shadow is None:
-        return 0
-    return {"pooled": capi.RH_FLAG_SHADOW_POOLED, "split": capi.RH_FLAG_SHADOW_SPLIT}[shadow]
 
 
 def render_device(job: Rendering, rgb_dev, spp: int = 1, offsets_dev=None, offset_tile: int = 0, shard_index: int = 0,
@@ -631,23 +585,15 @@ def render_device(job: Rendering, rgb_dev, spp: int = 1, offsets_dev=None, offse
     [rows*width*spp, 2] for the primary hit ids.  The call returns after the frame is complete."""
     import torch
 
-    L = lib()
-    mode, off = _offset_mode(offsets_dev, offset_tile)
-    bh = band_height or L.rh_default_band_height(job.height, shard_count)
-    rows = L.rh_shard_rows(job.height, shard_count, bh)
+    bh, rows = _shard_rows(job, shard_count, band_height)
     if peer_frames is None and (tuple(rgb_dev.shape) != (rows, job.width, 3) or rgb_dev.dtype != torch.uint8 or not rgb_dev.is_cuda):
         raise ValueError("rgb_dev must be a CUDA uint8 tensor of shape [rows, width, 3]")
-    flags = (capi.RH_FLAG_DEVICE_OUT | (capi.RH_FLAG_COUNT if count else 0) | (capi.RH_FLAG_PROFILE if profile else 0)
-             | _shadow_flag(shadow) | (0 if light_maps else capi.RH_FLAG_NO_LIGHT_MAPS)
-             | (capi.RH_FLAG_SHARD_OFFSETS if shard_offsets else 0) | (capi.RH_FLAG_HIT_IDS if hit_ids_dev is not None else 0))
-    if off is not None and off.is_cuda:
+    mode, off_ptr, keep, dev_off = _offsets(job, spp, offsets_dev, seed, offset_tile, rows if shard_offsets else None)
+    flags = (_flags(device=True, count=count, profile=profile, shadow=shadow, light_maps=light_maps, want_hit_ids=hit_ids_dev is not None)
+             | (capi.RH_FLAG_SHARD_OFFSETS if shard_offsets else 0))
+    if dev_off:
         flags |= capi.RH_FLAG_DEVICE_OFFSETS
         torch.cuda.current_stream().synchronize()
-    off_ptr = off.data_ptr() if off is not None else None
-    seed_box = None
-    if seed is not None:  # the kernel regenerates sample_offsets(width*height, spp, seed) on the device
-        seed_box = C.c_uint64(seed)
-        mode, off_ptr = capi.RH_OFFSETS_SPLITMIX64, C.addressof(seed_box)
     ptrs = None
     if peer_frames is not None:  # fused exchange: rows go straight into every shard's full frame (PeerFrames.pointers)
         flags |= capi.RH_FLAG_PEER_FRAMES
@@ -656,8 +602,8 @@ def render_device(job: Rendering, rgb_dev, spp: int = 1, offsets_dev=None, offse
     if ptrs is not None:
         o.n_peer_frames, o.peer_frames = len(peer_frames), ptrs
     st = capi.rh_stats()
-    check(L.rh_render(job.scene.device, C.byref(job.camera), C.byref(o), rgb_dev.data_ptr() if rgb_dev is not None else None,
-                      hit_ids_dev.data_ptr() if hit_ids_dev is not None else None, C.byref(st)))
+    check(lib().rh_render(job.scene.device, C.byref(job.camera), C.byref(o), rgb_dev.data_ptr() if rgb_dev is not None else None,
+                          hit_ids_dev.data_ptr() if hit_ids_dev is not None else None, C.byref(st)))
     return st.as_dict()
 
 
@@ -666,6 +612,9 @@ def render_multi(job: Rendering, n_gpus: int, spp: int = 1, offsets=None, seed: 
     """rh_multi_render: the whole frame on `n_gpus` GPUs of this process (one host thread per GPU, row bands interleaved,
     finished rows stored into one frame on GPU 0 over NVLink) — what a single-process host such as the Haskell
     front end calls.  The multi context and the replicated scene are created on first use."""
+    mode, off_ptr, keep, on_device = _offsets(job, spp, offsets, seed, 0)
+    if on_device:
+        raise ValueError("CUDA offsets go to render_device; render_multi takes host offsets")
     L = lib()
     if L.rh_multi_gpu_count() == 0:
         check(L.rh_multi_init(int(n_gpus)))
@@ -675,15 +624,7 @@ def render_multi(job: Rendering, n_gpus: int, spp: int = 1, offsets=None, seed: 
     if getattr(sc, "_multi", None) is None:
         sc._multi = C.c_void_p()
         check(L.rh_multi_scene_create(sc.flat, C.byref(sc._multi)))
-    mode, off = _offset_mode(offsets, 0)
-    off_ptr = None
-    seed_box = None
-    if seed is not None:
-        seed_box = C.c_uint64(seed)
-        mode, off_ptr = capi.RH_OFFSETS_SPLITMIX64, C.addressof(seed_box)
-    elif off is not None:
-        off_ptr = off.data_ptr() if hasattr(off, "data_ptr") else off.ctypes.data
-    o = _opts(job, spp, mode, off_ptr, 0, 0, 1, band_height, 0, _shadow_flag(shadow))
+    o = _opts(job, spp, mode, off_ptr, 0, 0, 1, band_height, 0, _flags(shadow=shadow))
     rgb = np.empty((job.height, job.width, 3), dtype=np.uint8)
     st = capi.rh_stats()
     check(L.rh_multi_render(sc._multi, C.byref(job.camera), C.byref(o), rgb.ctypes.data, C.byref(st)))
@@ -786,10 +727,8 @@ def _trace(job: Rendering, spp: int, offsets, offset_tile: int, **kw) -> Image:
     # one process per GPU: each rank renders its interleaved row bands, then one NCCL all-gather
     import torch
 
-    L = lib()
     G, rank = dist.get_world_size(), dist.get_rank()
-    bh = kw.pop("band_height", 0) or L.rh_default_band_height(job.height, G)
-    rows = L.rh_shard_rows(job.height, G, bh)
+    bh, rows = _shard_rows(job, G, kw.pop("band_height", 0))
     img = render(job, spp=spp, offsets=offsets, offset_tile=offset_tile, shard_index=rank, shard_count=G, band_height=bh, **kw)
     if dist.get_backend() == "nccl":
         mine = torch.from_numpy(img.pixels).cuda()
@@ -797,7 +736,7 @@ def _trace(job: Rendering, spp: int, offsets, offset_tile: int, **kw) -> Image:
         dist.all_gather_into_tensor(gathered, mine)
         full = torch.empty((job.height, job.width, 3), dtype=torch.uint8, device=mine.device)
         torch.cuda.current_stream().synchronize()
-        check(L.rh_deinterleave_bands(gathered.data_ptr(), full.data_ptr(), job.width, job.height, G, bh))
+        check(lib().rh_deinterleave_bands(gathered.data_ptr(), full.data_ptr(), job.width, job.height, G, bh))
         pixels = full.cpu().numpy()
     else:  # gloo (CPU tests of the shard logic)
         mine = torch.from_numpy(img.pixels)
@@ -820,7 +759,38 @@ def distributedRayTrace(job: Rendering, spp: int = 64, seed: int = 24, offsets=N
     return _trace(job, spp, offsets, offset_tile, **kw)
 
 
-class Accumulator:
+class _PixelState:
+    """Per-pixel state of one view that the library keeps between calls: the shard geometry of its rows (as for render)
+    and the handle `create` makes, released by close() through `destroy`."""
+    _what = "state"  # (for the error of a call after close())
+
+    def __init__(self, job: Rendering, stream_spp: int, shard_index: int, shard_count: int, band_height: int, device: bool,
+                 create, destroy):
+        init()
+        self.job, self.device, self.stream_spp = job, bool(device), int(stream_spp)
+        self.shard_index, self.shard_count = shard_index, shard_count
+        self.band_height, self.rows = _shard_rows(job, shard_count, band_height)
+        self._destroy, self._h = destroy, C.c_void_p()
+        check(create(job.width, job.height, shard_index, shard_count, self.band_height, self.stream_spp, C.byref(self._h)))
+
+    def _handle(self):
+        if not self._h:
+            raise ValueError(f"the {self._what} is closed")
+        return self._h
+
+    def close(self) -> None:
+        if getattr(self, "_h", None):
+            self._destroy(self._h)
+        self._h = None
+
+    def __del__(self):
+        try:
+            self.close()
+        except Exception:
+            pass
+
+
+class Accumulator(_PixelState):
     """Progressive rendering (rh_render_accumulate): running per-pixel sums of the sample colours of one view, kept on
     the device between calls, so that an image can be refined over several calls instead of rendered again.  Each
     add(spp) traces spp new samples per pixel exactly as render would, continues the sums in sample order and returns
@@ -831,16 +801,12 @@ class Accumulator:
     shard-compact).  `device`: outputs are CUDA tensors (and `offsets` may be one); else numpy arrays.  The first add()
     after creation or reset() fixes the scene, camera and max_depth of the job; reset() returns to 0 samples."""
 
+    _what = "accumulator"
+
     def __init__(self, job: Rendering, stream_spp: int = 0, shard_index: int = 0, shard_count: int = 1, band_height: int = 0,
                  device: bool = False):
         L = lib()
-        init()
-        self.job, self.device = job, bool(device)
-        self.shard_index, self.shard_count = shard_index, shard_count
-        self.band_height = band_height or L.rh_default_band_height(job.height, shard_count)
-        self.rows = L.rh_shard_rows(job.height, shard_count, self.band_height)
-        self._h = C.c_void_p()
-        check(L.rh_accum_create(job.width, job.height, shard_index, shard_count, self.band_height, int(stream_spp), C.byref(self._h)))
+        super().__init__(job, stream_spp, shard_index, shard_count, band_height, device, L.rh_accum_create, L.rh_accum_destroy)
         self._n = 0
 
     @property
@@ -858,49 +824,21 @@ class Accumulator:
         first); `seed`: the next spp samples of the accumulator's SplitMix64
         stream instead; neither: one sample at the pixel coordinate per spp.  `profile`: time every launch on its own
         (stats ms_trace / ms_shadow / ms_resolve; slower)."""
-        if self._h is None or not self._h:
-            raise ValueError("the accumulator is closed")
-        L = lib()
+        h = self._handle()
         job = self.job
-        mode, off = _offset_mode(offsets, 0)
-        off_ptr, seed_box = None, None
-        flags = ((capi.RH_FLAG_HIT_IDS if want_hit_ids else 0) | (capi.RH_FLAG_EXACT_BOXES if exact_boxes else 0)
-                 | _shadow_flag(shadow) | (0 if light_maps else capi.RH_FLAG_NO_LIGHT_MAPS)
-                 | (capi.RH_FLAG_DEVICE_OUT if self.device else 0) | (capi.RH_FLAG_PROFILE if profile else 0))
-        if seed is not None:
-            if offsets is not None:
-                raise ValueError("pass either offsets or seed")
-            seed_box = C.c_uint64(seed)
-            mode, off_ptr = capi.RH_OFFSETS_SPLITMIX64, C.addressof(seed_box)
-        elif off is not None:
-            have = off.numel() if hasattr(off, "numel") else off.size
-            if have != job.width * job.height * spp * 2:
-                raise ValueError(f"offsets has {have} values, expected {job.width * job.height * spp * 2}")
-            if getattr(off, "is_cuda", False):
-                if not self.device:
-                    raise ValueError("CUDA offsets need an accumulator with device=True")
-                flags |= capi.RH_FLAG_DEVICE_OFFSETS
-            # a slice of one stream, offsets[:, n:n + spp], is a strided view: the library reads a dense array
-            off = off.contiguous() if hasattr(off, "contiguous") else np.ascontiguousarray(off)
-            off_ptr = _ptr(off)
+        mode, off_ptr, keep, dev_off = _offsets(job, spp, offsets, seed, 0)
+        if dev_off and not self.device:
+            raise ValueError("CUDA offsets need an accumulator with device=True")
+        flags = (_flags(want_hit_ids=want_hit_ids, exact_boxes=exact_boxes, shadow=shadow, light_maps=light_maps, device=self.device,
+                        profile=profile) | (capi.RH_FLAG_DEVICE_OFFSETS if dev_off else 0))
         o = _opts(job, spp, mode, off_ptr, 0, self.shard_index, self.shard_count, self.band_height, chunk_samples, flags)
-        shapes = {"rgb": (self.rows, job.width, 3), "linear": (self.rows, job.width, 3), "ids": (self.rows, job.width, spp, 2)}
-        if self.device:
-            import torch
-
-            def empty(shape, dtype):
-                return torch.empty(shape, dtype=getattr(torch, dtype), device="cuda")
-
-            torch.cuda.current_stream().synchronize()  # the library runs on its own stream
-        else:
-            def empty(shape, dtype):
-                return np.empty(shape, dtype=dtype)
-        px = empty(shapes["rgb"], "uint8") if rgb else None
-        lin = empty(shapes["linear"], "float64") if linear else None
-        ids = empty(shapes["ids"], "int32") if want_hit_ids else None
+        empty = _alloc(self.device)
+        px = empty((self.rows, job.width, 3), "uint8") if rgb else None
+        lin = empty((self.rows, job.width, 3), "float64") if linear else None
+        ids = empty((self.rows, job.width, spp, 2), "int32") if want_hit_ids else None
         st = capi.rh_stats()
-        check(L.rh_render_accumulate(job.scene.device, C.byref(job.camera), C.byref(o), self._h,
-                                     *(_ptr(a) if a is not None else None for a in (px, lin, ids)), C.byref(st)))
+        check(lib().rh_render_accumulate(job.scene.device, C.byref(job.camera), C.byref(o), h,
+                                         *(_ptr(a) if a is not None else None for a in (px, lin, ids)), C.byref(st)))
         self._n += spp
         return Image(job.width, self.rows, px, st.as_dict(), ids, lin)
 
@@ -908,17 +846,6 @@ class Accumulator:
         """Back to 0 samples; the next add() may use another scene, camera or max_depth."""
         check(lib().rh_accum_reset(self._h))
         self._n = 0
-
-    def close(self) -> None:
-        if getattr(self, "_h", None):
-            lib().rh_accum_destroy(self._h)
-        self._h = None
-
-    def __del__(self):
-        try:
-            self.close()
-        except Exception:
-            pass
 
 
 def progressiveRayTrace(job: Rendering, spp: int = 64, batch: int = 8, seed: int = 24):
@@ -939,7 +866,7 @@ def progressiveRayTrace(job: Rendering, spp: int = 64, batch: int = 8, seed: int
         acc.close()
 
 
-class AdaptiveAccumulator:
+class AdaptiveAccumulator(_PixelState):
     """Adaptive sampling (rh_render_adaptive): progressive rendering that traces new samples only for the pixels whose
     standard error of the mean is still above a threshold in some channel.  Every pixel continues its own slice of the
     SplitMix64 stream sample_offsets(n, stream_spp, seed), so a pixel that ends with n samples has exactly the bytes of
@@ -949,17 +876,12 @@ class AdaptiveAccumulator:
     `shard_index` / `shard_count` / `band_height` as for render (the outputs are shard-compact).  `device`: outputs are
     CUDA tensors, else numpy arrays.  The first add() after creation or reset() fixes the scene, camera and max_depth."""
 
+    _what = "adaptive accumulator"
+
     def __init__(self, job: Rendering, stream_spp: int, shard_index: int = 0, shard_count: int = 1, band_height: int = 0,
                  device: bool = False):
         L = lib()
-        init()
-        self.job, self.device, self.stream_spp = job, bool(device), int(stream_spp)
-        self.shard_index, self.shard_count = shard_index, shard_count
-        self.band_height = band_height or L.rh_default_band_height(job.height, shard_count)
-        self.rows = L.rh_shard_rows(job.height, shard_count, self.band_height)
-        self._h = C.c_void_p()
-        check(L.rh_adaptive_create(job.width, job.height, shard_index, shard_count, self.band_height, self.stream_spp,
-                                   C.byref(self._h)))
+        super().__init__(job, stream_spp, shard_index, shard_count, band_height, device, L.rh_adaptive_create, L.rh_adaptive_destroy)
 
     def add(self, spp: int, seed: int, threshold: float, min_spp: int = 8, rgb: bool = True, linear: bool = True,
             shadow: str | None = None, exact_boxes: bool = False, light_maps: bool = True, chunk_samples: int = 0,
@@ -968,33 +890,23 @@ class AdaptiveAccumulator:
         `min_spp` samples, or a channel's standard error above `threshold`, and room left in the stream).  Returns the
         Image of every pixel's samples so far: `pixels` (RGB8, when `rgb`), `linear` (float64, when `linear`) and this
         call's stats, with stats["n_active"] the number of pixels traced."""
-        if self._h is None or not self._h:
-            raise ValueError("the adaptive accumulator is closed")
-        L = lib()
+        h = self._handle()
         job = self.job
         seed_box = C.c_uint64(seed)
-        flags = ((capi.RH_FLAG_EXACT_BOXES if exact_boxes else 0) | _shadow_flag(shadow)
-                 | (0 if light_maps else capi.RH_FLAG_NO_LIGHT_MAPS) | (capi.RH_FLAG_DEVICE_OUT if self.device else 0)
-                 | (capi.RH_FLAG_PROFILE if profile else 0) | (capi.RH_FLAG_COUNT if count else 0))
+        flags = _flags(exact_boxes=exact_boxes, shadow=shadow, light_maps=light_maps, device=self.device, profile=profile, count=count)
         o = _opts(job, spp, capi.RH_OFFSETS_SPLITMIX64, C.addressof(seed_box), 0, self.shard_index, self.shard_count,
                   self.band_height, chunk_samples, flags)
         ao = capi.rh_adaptive_opts()
         ao.threshold, ao.min_spp = float(threshold), int(min_spp)
         shape = (self.rows, job.width, 3)
-        if self.device:
-            import torch
-
-            torch.cuda.current_stream().synchronize()  # the library runs on its own stream
-            px = torch.empty(shape, dtype=torch.uint8, device="cuda") if rgb else None
-            lin = torch.empty(shape, dtype=torch.float64, device="cuda") if linear else None
-        else:
-            px = np.empty(shape, dtype=np.uint8) if rgb else None
-            lin = np.empty(shape, dtype=np.float64) if linear else None
+        empty = _alloc(self.device)
+        px = empty(shape, "uint8") if rgb else None
+        lin = empty(shape, "float64") if linear else None
         n_active = C.c_uint64()
         st = capi.rh_stats()
-        check(L.rh_render_adaptive(job.scene.device, C.byref(job.camera), C.byref(o), C.byref(ao), self._h,
-                                   _ptr(px) if px is not None else None, _ptr(lin) if lin is not None else None,
-                                   C.byref(n_active), C.byref(st)))
+        check(lib().rh_render_adaptive(job.scene.device, C.byref(job.camera), C.byref(o), C.byref(ao), h,
+                                       _ptr(px) if px is not None else None, _ptr(lin) if lin is not None else None,
+                                       C.byref(n_active), C.byref(st)))
         stats = st.as_dict()
         stats["n_active"] = n_active.value
         return Image(job.width, self.rows, px, stats, None, lin)
@@ -1003,36 +915,15 @@ class AdaptiveAccumulator:
         """(counts uint32 [rows, width], sums float64 [rows, width, 3], sums of squares float64 [rows, width, 3]), numpy
         arrays or, with device=True, CUDA tensors."""
         shape = (self.rows, self.job.width)
-        if self.device:
-            import torch
-
-            counts = torch.empty(shape, dtype=torch.int32, device="cuda")  # (torch has no uint32 arithmetic to speak of)
-            sums = torch.empty(shape + (3,), dtype=torch.float64, device="cuda")
-            sumsq = torch.empty(shape + (3,), dtype=torch.float64, device="cuda")
-            torch.cuda.current_stream().synchronize()
-            flags = capi.RH_FLAG_DEVICE_OUT
-        else:
-            counts = np.empty(shape, dtype=np.uint32)
-            sums = np.empty(shape + (3,), dtype=np.float64)
-            sumsq = np.empty(shape + (3,), dtype=np.float64)
-            flags = 0
-        check(lib().rh_adaptive_state(self._h, _ptr(counts), _ptr(sums), _ptr(sumsq), flags))
+        empty = _alloc(self.device)
+        counts = empty(shape, "int32" if self.device else "uint32")  # (torch has no uint32 arithmetic to speak of)
+        sums, sumsq = empty(shape + (3,), "float64"), empty(shape + (3,), "float64")
+        check(lib().rh_adaptive_state(self._h, _ptr(counts), _ptr(sums), _ptr(sumsq), _flags(device=self.device)))
         return counts, sums, sumsq
 
     def reset(self) -> None:
         """Every count and sum back to 0; the next add() may use another scene, camera or max_depth."""
         check(lib().rh_adaptive_reset(self._h))
-
-    def close(self) -> None:
-        if getattr(self, "_h", None):
-            lib().rh_adaptive_destroy(self._h)
-        self._h = None
-
-    def __del__(self):
-        try:
-            self.close()
-        except Exception:
-            pass
 
 
 def adaptiveRayTrace(job: Rendering, max_spp: int = 64, batch: int = 4, min_spp: int = 8, threshold: float = 0.5 / 255,
