@@ -564,6 +564,40 @@ typedef struct rh_light_groups {
 int rh_render_light_groups(const rh_scene* scene, const rh_camera* camera, const rh_render_opts* opts,
                            const rh_light_groups* groups, uint8_t* rgb_out, int32_t* hit_ids_out, rh_stats* stats);
 
+/* ---- camera batches ------------------------------------------------- */
+/* Many views of one scene in one wavefront (cube-map faces, stereo pairs and rigs, thumbnails, multi-view image sets). */
+typedef struct rh_views {
+  const rh_camera* cameras; /* n_views cameras (host memory)                                                     */
+  uint32_t n_views;         /* 1 .. 65536                                                                        */
+  uint32_t reserved_;       /* must be 0                                                                         */
+  const uint64_t* seeds;    /* RH_OFFSETS_SPLITMIX64 only: n_views seeds (host), or NULL = every view uses
+                               *opts->offsets; non-NULL with another offset mode is RH_ERR_ARG                     */
+} rh_views;                 /* 24 bytes */
+/* View v is exactly rh_render(scene, &cameras[v], opts'), where opts' is opts with *offsets = seeds[v] when seeds is
+ * given: the same rays (every offset mode, host, device and shard-compact offsets, shard and band selection), bytes,
+ * hit ids and ray counts, up to the 1-LSB wobble of Transparent forks that two rh_render calls already show.  All views
+ * share width, height, spp, max_depth and the offsets; the cameras may differ in anything, projection included.
+ * Outputs are view-major over shard-compact rows (rows = rh_shard_rows(height, shard_count, band_height)):
+ *   rgb_out      uint8[n_views][rows][width][3], as rh_render writes it (padding rows of the last band: 0);
+ *   linear_out   double[n_views][rows][width][3], the colour toIntC is applied to: the linear_out a single
+ *                rh_render_accumulate call on a freshly created accumulator writes for that view (padding rows: 0);
+ *   hit_ids_out  (RH_FLAG_HIT_IDS) int32[n_views][rows][width][spp][2].
+ * rgb_out and linear_out are each optional (NULL), but not both.  RH_FLAG_DEVICE_OUT covers all three outputs
+ * (linear_out 8-byte aligned).  RH_FLAG_DEVICE_OFFSETS, RH_FLAG_SHARD_OFFSETS, RH_FLAG_EXACT_BOXES,
+ * RH_FLAG_NO_LIGHT_MAPS, the shadow-schedule flags, RH_FLAG_PROFILE and chunk_samples behave as in rh_render; host
+ * per-pixel offsets (F64 / F32) are uploaded once per call to device scratch (RH_ERR_OOM when they do not fit).
+ * RH_ERR_ARG: RH_FLAG_PEER_FRAMES, RH_FLAG_COUNT, n_views 0 or above 65536, a null cameras, a nonzero reserved_, a
+ * camera with an unknown projection (the message names the view), seeds with an offset mode other than SplitMix64, and
+ * rh_render's own checks.  The call uses the scene's decided shadow schedule (else pooled).  Its queues start at the
+ * larger of the scene's queue factor (else 2) and the factor the scene's last views call needed, reduced while the
+ * queues would outgrow the memory the library plans for a chunk, and grow by the overflow retry; the call remembers
+ * its own factor for the next views call.  It changes neither the schedule, nor the queue factor renders use, nor the
+ * row costs.  stats: ray counts summed over the views (rays_primary = n_views times one
+ * view's), negative_channels of rgb_out, and chunks, queue_factor, shadow_split and ms_total as rh_render fills
+ * them (ms_total includes the upload of the camera table, the seeds and host offsets).  A call refused for its arguments writes nothing. */
+int rh_render_views(const rh_scene* scene, const rh_views* views, const rh_render_opts* opts, uint8_t* rgb_out,
+                    double* linear_out, int32_t* hit_ids_out, rh_stats* stats);
+
 /* Rows owned by one shard (equal for all shards: bands are padded). */
 int rh_shard_rows(int height, int shard_count, int band_height);
 int rh_default_band_height(int height, int shard_count);

@@ -136,6 +136,10 @@ class rh_light_groups(C.Structure):
     _fields_ = [("group_of_light", C.c_void_p), ("n_groups", C.c_uint32), ("reserved_", C.c_uint32), ("out", C.c_void_p)]
 
 
+class rh_views(C.Structure):
+    _fields_ = [("cameras", C.POINTER(rh_camera)), ("n_views", C.c_uint32), ("reserved_", C.c_uint32), ("seeds", C.POINTER(C.c_uint64))]
+
+
 class rh_update_info(C.Structure):
     _fields_ = [("colours_only", C.c_uint32), ("occluders_rebuilt", C.c_uint32), ("maps_rasterised", C.c_uint32),
                 ("maps_kept", C.c_uint32), ("lit_queries", C.c_uint64)]
@@ -146,6 +150,7 @@ assert C.sizeof(rh_material) == 96 and C.sizeof(rh_light) == 64 and C.sizeof(rh_
 assert C.sizeof(rh_tri) == 80 and C.sizeof(rh_tri_shade) == 128 and C.sizeof(rh_object) == 96
 assert C.sizeof(rh_hit) == 80 and C.sizeof(rh_trace_opts) == 16 and C.sizeof(rh_adaptive_opts) == 16
 assert C.sizeof(rh_update_info) == 24 and C.sizeof(rh_features) == 40 and C.sizeof(rh_light_groups) == 24
+assert C.sizeof(rh_views) == 24
 
 vp = C.c_void_p
 
@@ -179,6 +184,7 @@ SIGNATURES = {
     "rh_render_features": (C.c_int, [vp, C.POINTER(rh_camera), C.POINTER(rh_render_opts), C.POINTER(rh_features), vp, C.POINTER(rh_stats)]),
     "rh_render_light_groups": (C.c_int, [vp, C.POINTER(rh_camera), C.POINTER(rh_render_opts), C.POINTER(rh_light_groups), vp, vp,
                                          C.POINTER(rh_stats)]),
+    "rh_render_views": (C.c_int, [vp, C.POINTER(rh_views), C.POINTER(rh_render_opts), vp, vp, vp, C.POINTER(rh_stats)]),
     "rh_shard_rows": (C.c_int, [C.c_int, C.c_int, C.c_int]),
     "rh_default_band_height": (C.c_int, [C.c_int, C.c_int]),
     "rh_deinterleave_bands": (C.c_int, [vp, vp, C.c_int, C.c_int, C.c_int, C.c_int]),

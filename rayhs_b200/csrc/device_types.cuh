@@ -106,6 +106,7 @@ struct OccSphere { double c[3], r; };     // Geometry.hs:63
 constexpr int kOccPlanes = 16, kOccSpheres = 16, kOccMeshes = 8, kFastLights = 12;
 constexpr int kMaskLights = 32;  // lights whose per-hit state fits the 32-bit walk / settled masks of a shadow task
 constexpr int kMaxGroups = 16;   // light groups of rh_render_light_groups
+constexpr uint32_t kMaxViews = 65536;  // cameras of one rh_render_views call
 
 struct SceneView {
   const WideNode* wide;      // exact double boxes: rays with a zero direction component, RH_FLAG_EXACT_BOXES
@@ -278,6 +279,12 @@ struct ChunkParams {
   uint32_t group_stride;
   uint32_t n_groups;
   uint32_t group_mask[kMaxGroups];  // bit l: light l is in group g
+  // rh_render_views (after the render's fields: their offsets stay as they were): the frame's local rows are
+  // [view][view_rows]; pass 0 builds local row r's rays with cams[r / view_rows] and, with view_seeds, SplitMix64 seed
+  // view_seeds[r / view_rows].  view_rows 0 (cams null): not a views frame.
+  const CameraParams* cams;
+  const unsigned long long* view_seeds;
+  uint32_t view_rows;
 };
 
 // rh_render_accumulate's end of a chunk instead of the resolve: the running per-pixel sums of the accumulator.
@@ -334,7 +341,8 @@ struct FeatureParams {
 };
 
 // Launchers (kernels.cu).  `count` selects the instrumented instantiation (box/tri counters); launch_trace runs the
-// uninstrumented ray instantiation for P.offset_mode == kOffsetsRays and the pixel-list one when P.list.pixels is set.
+// uninstrumented ray instantiation for P.offset_mode == kOffsetsRays, the pixel-list one when P.list.pixels is set and
+// the uninstrumented views one when P.cams is set.
 // (followed by a one-thread kernel that closes the pass's range of the hit queue, ChunkCtl::hit_start)
 void launch_trace(const SceneView& S, const CameraParams& cam, const ChunkParams& P, bool count, int grid, void* stream);
 // classify_kernel, then the walks of the hits it queued — refill: the per-lane-refill kernel (incoherent rays) instead of
@@ -347,6 +355,10 @@ void launch_resolve(const ChunkParams& P, void* stream);
 // folded per pixel in sample order and times 1 / spp, to out + g * out_group_stride + (out_px0 + pixel) * 3, where
 // pixel is chunk-local (padding rows: 0)
 void launch_light_groups_resolve(const ChunkParams& P, double* out, size_t out_group_stride, size_t out_px0, void* stream);
+// rh_render_views' end of a chunk instead of the resolve: resolve_kernel's RGB8 (P.rgb, may be null) and, to
+// linear + (first_row * width + pixel) * 3 (may be null), the linear colours toIntC is applied to, with the padding
+// rows of each view decided per view (0 in both outputs)
+void launch_views_resolve(const ChunkParams& P, double* linear, void* stream);
 // rh_trace_rays' end of a chunk instead of the resolve: the accumulators of its rays to colors (double[n][3], all rays)
 void launch_store_colors(const ChunkParams& P, double* colors, void* stream);
 // rh_render_accumulate's end of a chunk instead of the resolve: adds the chunk's samples to the running sums and writes

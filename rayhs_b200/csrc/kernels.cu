@@ -14,6 +14,8 @@
 //   accumulate_resolve_kernel  K6 of rh_render_accumulate: running per-pixel sums across calls, RGB8 and linear colours.
 //   adaptive_*            rh_render_adaptive: selection and compaction of the pixels still above the threshold, the
 //                         sink of their samples (trace_kernel<.., Source::kPixelList>), commit, RGB8 and linear output.
+//   views_resolve_kernel  K6 of rh_render_views: RGB8 and linear colours of a batch of views (trace_kernel<.., Source::kViews>),
+//                         padding rows decided per view.
 //   feature_kernel        rh_render_features: per pixel the albedo, normal, depth and hit count of its camera rays' first
 //                         hits (closest hit + Hit + colorAt, no shading), for denoisers and compositing.
 //   deinterleave          K7: band re-assembly after the all-gather.
@@ -1427,13 +1429,33 @@ __device__ __forceinline__ bool offset_slot(const ChunkParams& P, uint32_t item,
 // RayHs.hs:178-181) or a queued secondary ray with its weight and tags.  False for a padding row of the last band.
 // What pass 0's work items are: camera samples of the chunk's image rows (rh_render), caller-built rays (kRays:
 // rh_trace_rays, P.offset_mode == kOffsetsRays) or samples of the entries of a pixel list (kPixelList:
-// rh_render_adaptive, P.list).  The last two are false past the chunk's items (P.ray_items).
-enum class Source { kCamera, kRays, kPixelList };
+// rh_render_adaptive, P.list).  The last two are false past the chunk's items (P.ray_items).  kViews (rh_render_views):
+// camera samples as kCamera's, each local row with its view's camera and the rows, offsets and seed of that view's frame.
+enum class Source { kCamera, kRays, kPixelList, kViews };
 
 // Image row of a shard-compact row of the list's image (global_row with the PixelList's bands).
 __device__ __forceinline__ uint32_t list_image_row(const PixelList& L, uint32_t local_row) {
   const uint32_t lb = local_row / L.band_height, rib = local_row % L.band_height;
   return (lb * L.shard_count + L.shard_index) * L.band_height + rib;
+}
+
+// rh_render_views: view v's camera, through the read-only path (the items of a warp almost always share a view)
+__device__ __forceinline__ CameraParams view_camera(const ChunkParams& P, uint32_t v) {
+  const CameraParams* src = P.cams + v;
+  CameraParams c;
+#pragma unroll
+  for (int k = 0; k < 9; k++) c.m[k] = __ldg(src->m + k);
+#pragma unroll
+  for (int k = 0; k < 3; k++) c.pos[k] = __ldg(src->pos + k);
+  c.w = __ldg(&src->w);
+  c.h = __ldg(&src->h);
+  c.half_w = __ldg(&src->half_w);
+  c.half_h = __ldg(&src->half_h);
+  c.apw = __ldg(&src->apw);
+  c.aph = __ldg(&src->aph);
+  c.f = __ldg(&src->f);
+  c.projection = __ldg(&src->projection);
+  return c;
 }
 
 template <Source SRC>
@@ -1460,6 +1482,41 @@ __device__ __forceinline__ bool load_item(const ChunkParams& P, const CameraPara
     const double ox = splitmix01(P.offset_seed, 2 * g) - 0.5;
     const double oy = splitmix01(P.offset_seed, 2 * g + 1) - 0.5;
     r = camera_ray(cam, (double)col + ox, (double)grow + oy);
+    return true;
+  }
+  if (SRC == Source::kViews && primary) {
+    // local row lr is row lr_v of view v: the ray rh_render casts for pixel sample (lr_v, col, s) with cams[v], its
+    // offsets indexed as offset_slot indexes the render's (shard-compact ones by lr_v from the array's start)
+    const uint32_t lp = item / P.spp, s = item - lp * P.spp;
+    const uint32_t lrow = lp / P.width, col = lp - lrow * P.width;
+    const uint32_t lr = P.first_row + lrow, v = lr / P.view_rows, lr_v = lr - v * P.view_rows;
+    const uint32_t grow = global_row(P, lr_v);
+    if (grow >= P.height) return false;
+    double ox = 0, oy = 0;
+    if (P.offset_mode == RH_OFFSETS_SPLITMIX64) {
+      const unsigned long long seed = P.view_seeds ? __ldg(P.view_seeds + v) : P.offset_seed;
+      const unsigned long long g = ((unsigned long long)grow * P.width + col) * P.stream_spp + P.stream_base + s;
+      ox = splitmix01(seed, 2 * g) - 0.5;
+      oy = splitmix01(seed, 2 * g + 1) - 0.5;
+    } else if (P.offset_mode == RH_OFFSETS_F64 || P.offset_mode == RH_OFFSETS_F32 || P.offset_mode == RH_OFFSETS_TILED_F64) {
+      size_t idx;
+      if (P.offset_mode == RH_OFFSETS_TILED_F64)
+        idx = ((size_t)(grow % P.offset_tile) * P.offset_tile + (col % P.offset_tile)) * P.spp + s;
+      else if (P.offset_index == kOffIndexGlobal)
+        idx = ((size_t)grow * P.width + col) * P.spp + s;
+      else
+        idx = ((size_t)lr_v * P.width + col) * P.spp + s;
+      if (P.offset_mode == RH_OFFSETS_F32) {
+        const float2 o2 = __ldg((const float2*)P.offsets + idx);
+        ox = (double)o2.x;
+        oy = (double)o2.y;
+      } else {
+        const double2 o2 = __ldg((const double2*)P.offsets + idx);
+        ox = o2.x;
+        oy = o2.y;
+      }
+    }
+    r = camera_ray(view_camera(P, v), (double)col + ox, (double)grow + oy);
     return true;
   }
   if (primary) {
@@ -2663,6 +2720,76 @@ __global__ void __launch_bounds__(kBlock) accumulate_resolve_kernel(const __grid
   }
 }
 
+// ------------------------------------------------------------------ K6'''': rh_render_views' sink
+// resolve_kernel's RGB8 and accumulate_resolve_kernel's linear colours of a fresh accumulator (the same loads, association
+// and 1 / spp), with a padding row decided in its own view: local row lr is row lr % view_rows of its view.  Its own
+// kernel rather than a template parameter of those two, so that the render's sinks stay as they are; negative channels
+// count RGB8 output only, as in accumulate_resolve_kernel.
+__global__ void __launch_bounds__(kBlock) views_resolve_kernel(const __grid_constant__ ChunkParams P, double* __restrict__ linear) {
+  __shared__ __align__(16) double lin[kBlock * 3];
+  __shared__ __align__(16) uint8_t bytes[kBlock * 3];
+  const uint32_t n_pixels = P.n_rows * P.width;
+  const uint32_t lp = blockIdx.x * kBlock + threadIdx.x;
+  bool negative = false;
+  if (lp < n_pixels) {
+    double cr = 0, cg = 0, cb = 0;
+    const uint32_t lr = P.first_row + lp / P.width;
+    if (global_row(P, lr % P.view_rows) < P.height) {
+      double sr = 0, sg = 0, sb = 0;  // foldl (+) black
+      const double* a = P.accum + (size_t)lp * P.spp;
+      if ((P.spp & 1u) == 0 && (P.accum_stride & 1u) == 0) {
+        const double2* a0 = (const double2*)a;
+        const double2* a1 = (const double2*)(a + P.accum_stride);
+        const double2* a2 = (const double2*)(a + 2 * (size_t)P.accum_stride);
+        for (uint32_t s = 0; s < P.spp / 2; s++) {
+          const double2 r2 = a0[s], g2 = a1[s], b2 = a2[s];
+          sr = (sr + r2.x) + r2.y;
+          sg = (sg + g2.x) + g2.y;
+          sb = (sb + b2.x) + b2.y;
+        }
+      } else {
+        for (uint32_t s = 0; s < P.spp; s++) {
+          sr = sr + a[s];
+          sg = sg + a[P.accum_stride + s];
+          sb = sb + a[2 * (size_t)P.accum_stride + s];
+        }
+      }
+      const double inv = 1.0 / (double)P.spp;
+      cr = inv * sr;
+      cg = inv * sg;
+      cb = inv * sb;
+    }
+    bool neg = false;
+    bytes[3 * threadIdx.x] = (uint8_t)to_int_c(cr, neg);
+    bytes[3 * threadIdx.x + 1] = (uint8_t)to_int_c(cg, neg);
+    bytes[3 * threadIdx.x + 2] = (uint8_t)to_int_c(cb, neg);
+    negative = neg && P.rgb;
+    lin[3 * threadIdx.x] = cr;
+    lin[3 * threadIdx.x + 1] = cg;
+    lin[3 * threadIdx.x + 2] = cb;
+  }
+  const unsigned neg = __ballot_sync(kFull, negative);
+  if ((threadIdx.x & 31) == 0 && neg) atomicAdd(&P.counters->negative_channels, (unsigned long long)__popc(neg));
+  __syncthreads();
+  const uint32_t n_here = min((uint32_t)kBlock, n_pixels - blockIdx.x * kBlock) * 3;
+  const size_t first = (size_t)P.first_row * P.width + (size_t)blockIdx.x * kBlock;
+  if (P.rgb) {
+    uint8_t* dst = P.rgb + first * 3;
+    if ((((uintptr_t)dst) & 3) == 0) {
+      const uint32_t words = n_here / 4;
+      if (threadIdx.x < words) ((uint32_t*)dst)[threadIdx.x] = ((const uint32_t*)bytes)[threadIdx.x];
+      const uint32_t tail = words * 4 + threadIdx.x;
+      if (tail < n_here) dst[tail] = bytes[tail];
+    } else {
+      for (uint32_t i = threadIdx.x; i < n_here; i += kBlock) dst[i] = bytes[i];
+    }
+  }
+  if (linear) {
+    double* dst = linear + first * 3;
+    for (uint32_t i = threadIdx.x; i < n_here; i += kBlock) dst[i] = lin[i];
+  }
+}
+
 // ------------------------------------------------------------------ K6''': rh_render_light_groups' images
 // Beside resolve_kernel: per group (and the remainder), each pixel's samples folded in sample order with resolve_kernel's
 // loads and association, times 1 / spp; the linear triples leave coalesced through shared memory, as in
@@ -3001,6 +3128,7 @@ int configure_kernels() {
   set((const void*)trace_kernel<false, Source::kRays>, kTraceSmem);
   set((const void*)trace_kernel<true, Source::kPixelList>, kTraceSmem);
   set((const void*)trace_kernel<false, Source::kPixelList>, kTraceSmem);
+  set((const void*)trace_kernel<false, Source::kViews>, kTraceSmem);
   set((const void*)shadow_pooled_kernel<true>, kShadowSmem);
   set((const void*)shadow_pooled_kernel<false>, kShadowSmem);
   set((const void*)shadow_refill_kernel<true>, kWalkSmem);
@@ -3046,6 +3174,7 @@ void launch_trace(const SceneView& S, const CameraParams& cam, const ChunkParams
   if (P.offset_mode == kOffsetsRays) trace_kernel<false, Source::kRays><<<grid * kTracePerSm, kTraceBlock, kTraceSmem, st>>>(S, cam, P);
   else if (P.list.pixels && count) trace_kernel<true, Source::kPixelList><<<grid * kTracePerSm, kTraceBlock, kTraceSmem, st>>>(S, cam, P);
   else if (P.list.pixels) trace_kernel<false, Source::kPixelList><<<grid * kTracePerSm, kTraceBlock, kTraceSmem, st>>>(S, cam, P);
+  else if (P.cams) trace_kernel<false, Source::kViews><<<grid * kTracePerSm, kTraceBlock, kTraceSmem, st>>>(S, cam, P);
   else if (count) trace_kernel<true, Source::kCamera><<<grid * kTracePerSm, kTraceBlock, kTraceSmem, st>>>(S, cam, P);
   else trace_kernel<false, Source::kCamera><<<grid * kTracePerSm, kTraceBlock, kTraceSmem, st>>>(S, cam, P);
   close_hit_range_kernel<<<1, 1, 0, st>>>(P.ctl, P.pass);
@@ -3091,6 +3220,10 @@ void launch_resolve(const ChunkParams& P, void* stream) {
 void launch_light_groups_resolve(const ChunkParams& P, double* out, size_t out_group_stride, size_t out_px0, void* stream) {
   const uint32_t n_pixels = P.n_rows * P.width;
   light_groups_resolve_kernel<<<(n_pixels + kBlock - 1) / kBlock, kBlock, 0, (cudaStream_t)stream>>>(P, out, out_group_stride, out_px0);
+}
+void launch_views_resolve(const ChunkParams& P, double* linear, void* stream) {
+  const uint32_t n_pixels = P.n_rows * P.width;
+  views_resolve_kernel<<<(n_pixels + kBlock - 1) / kBlock, kBlock, 0, (cudaStream_t)stream>>>(P, linear);
 }
 void launch_store_colors(const ChunkParams& P, double* colors, void* stream) {
   store_colors_kernel<<<(P.ray_items + kBlock - 1) / kBlock, kBlock, 0, (cudaStream_t)stream>>>(P, colors);

@@ -22,6 +22,11 @@ struct ChunkPlan {
   bool ramped = false;         // the compute-bound plan of a streamed frame whose row costs are known
 };
 
+// The largest chunk (samples) the library plans on its own: as many samples as 45 % of the device memory holds.
+inline size_t max_chunk_samples(size_t device_mem, size_t bytes_per_sample = kBytesPerSample) {
+  return std::min<size_t>((size_t)(0.45 * (double)device_mem) / bytes_per_sample, (size_t)0x3ffffff0u);
+}
+
 // Mean cost per row of rows [row0, row0 + n).
 inline double cost_density(const float* row_cost, int row0, int n) {
   double c = 0;
@@ -46,7 +51,7 @@ inline ChunkPlan plan_chunks(int rows_local, size_t row_samples, int chunk_sampl
   std::vector<int>& plan = p.rows;
   size_t want = (size_t)chunk_samples, first = want;
   if (chunk_samples <= 0) {
-    want = std::min<size_t>((size_t)(0.45 * (double)device_mem) / bytes_per_sample, (size_t)0x3ffffff0u);
+    want = max_chunk_samples(device_mem, bytes_per_sample);
     // a frame that needs several chunks has two of them in flight, each with its own scratch: half the budget each
     if ((size_t)rows_local * row_samples > want) want /= kLanes;
     if (host_offsets) want = std::min<size_t>(want, kStreamChunk);

@@ -101,6 +101,7 @@ struct Device {
   } lane[2];
   DevBuf ctl, counters, offsets, rgb, ids, linear;
   DevBuf query;  // ray queries: claim cursor, then (host buffers) one chunk of rays and of results
+  DevBuf views;  // rh_render_views: the camera table, then the seeds
   void* pinned = nullptr;  // ctl + counters read-back
   size_t pinned_bytes = 0;
   int max_threads = 0;  // largest grid * block of the traversal kernels (one block per SM)
@@ -155,7 +156,7 @@ struct Device {
         e = nullptr;
       }
     }
-    for (DevBuf* b : {&ctl, &counters, &offsets, &rgb, &ids, &linear, &query})
+    for (DevBuf* b : {&ctl, &counters, &offsets, &rgb, &ids, &linear, &query, &views})
       b->release();
     if (pinned) cudaFreeHost(pinned);
     pinned = nullptr;
@@ -205,6 +206,7 @@ struct rh_scene {
   mutable std::vector<int> cost_key;      // {W, H, spp, shards, shard, band height} the row costs belong to
   mutable std::vector<float> row_cost;    // kernel ms per local row (its chunk's time / its chunk's rows)
   mutable uint32_t queue_factor = 2;          // the queue capacity factor the scene's last frame needed
+  mutable uint32_t views_queue_factor = 2;    // ... and its last rh_render_views frame (which leaves the one above alone)
   mutable bool stream_compute_bound = false;  // ... and in that frame the kernels, not the upload, finished last
   // What derive_tables needs to rebuild the material- and light-derived tables for rh_scene_update (DESIGN.md "Scene
   // updates"), on the host: the object records, the linear object list, the sphere-tree root, both tree depths, the
@@ -1545,7 +1547,7 @@ void scene_update_commit(rh_scene* S, std::unique_ptr<rh_scene> N, int cls) {
     S->tune_ns_per_pair[0] = S->tune_ns_per_pair[1] = 0;
     S->cost_key.clear();
     S->row_cost.clear();
-    S->queue_factor = 2;
+    S->queue_factor = S->views_queue_factor = 2;
     S->stream_compute_bound = false;
   }
   S->generation++;
@@ -1622,19 +1624,30 @@ struct Frame {
   uint32_t n_groups = 0;
   uint32_t group_mask[kMaxGroups] = {};
   double* group_out = nullptr;
+  // rh_render_views: the local rows are [view][view_rows]; pass 0 takes each view's camera from cams (device) and, with
+  // view_seeds (device), its SplitMix64 seed; the sink decides padding rows per view and writes RGB8 (optional) and the
+  // linear colours (`linear`, optional).  Device offsets are read from the start of the array for every view.
+  bool views = false;
+  uint32_t view_rows = 0;
+  const CameraParams* cams = nullptr;
+  const unsigned long long* view_seeds = nullptr;
+  // host data the kernels read, copied to the device at the start of each attempt (rh_render_views: the camera table,
+  // the seeds and host per-pixel offsets)
+  struct Upload { void* dst; const void* src; size_t bytes; };
+  std::vector<Upload> uploads;
   const char* overflow_error = "rh_render: ray queue overflow; lower chunk_samples";
-  // renders (not traces, list frames or light-group frames) tune the scene's shadow schedule and record its queue factor
-  // and row costs
-  bool learns() const { return !trace && !pixel_list && !n_groups; }
+  // renders (not traces, list frames, light-group or views frames) tune the scene's shadow schedule and record its queue
+  // factor and row costs
+  bool learns() const { return !trace && !pixel_list && !n_groups && !views; }
 };
 
 // rh_render's argument checks (`who` names the entry point in the messages).  With f->accumulate, f->pixel_list,
-// f->features or f->n_groups set, rgb_out may be null.
+// f->features, f->n_groups or f->views set, rgb_out may be null.
 int render_frame(Device* D, const rh_scene* scene, const rh_camera* camera, const rh_render_opts* o, uint8_t* rgb_out,
                  int32_t* hit_ids_out, Frame* f, const char* who = "rh_render") {
   const std::string w(who);
   const bool peer_frames = o && (o->flags & RH_FLAG_PEER_FRAMES) != 0;
-  if (!scene || !camera || !o || (!rgb_out && !peer_frames && !f->accumulate && !f->pixel_list && !f->features && !f->n_groups))
+  if (!scene || !camera || !o || (!rgb_out && !peer_frames && !f->accumulate && !f->pixel_list && !f->features && !f->n_groups && !f->views))
     return rh::set_error(RH_ERR_ARG, w + ": null argument");
   if (peer_frames && (!o->peer_frames || o->n_peer_frames <= 0 || o->n_peer_frames > kMaxPeers))
     return rh::set_error(RH_ERR_ARG, w + ": RH_FLAG_PEER_FRAMES needs 1..16 peer frame pointers");
@@ -1866,11 +1879,14 @@ struct FrameRun {
       chunk_ev.push_back(prof_event(lane_stream));  // after the wait: the span holds kernel time only
     }
 
-    if ((o.flags & RH_FLAG_DEVICE_OFFSETS) && (o.flags & RH_FLAG_SHARD_OFFSETS) && d_offsets)
+    if ((o.flags & RH_FLAG_DEVICE_OFFSETS) && (o.flags & RH_FLAG_SHARD_OFFSETS) && d_offsets && !f.views)
       P.offsets = (const char*)d_offsets + (size_t)first_row * row_samples * f.off_elem;
     P.offset_base = (P.offset_index == kOffIndexLocal) ? 0ull : (unsigned long long)first_row * row_samples;
     if (f.trace || f.pixel_list) P.ray_items = (uint32_t)std::min<uint64_t>(P.n_samples, f.n_rays - (uint64_t)first_row * row_samples);
     P.list = f.list;
+    P.cams = f.cams;
+    P.view_seeds = f.view_seeds;
+    P.view_rows = f.view_rows;
     for (int plane = 0; plane < 3; plane++)  // (three 1-D memsets: a 2-D one is limited to 2 GB of pitch)
       RH_CUDA(cudaMemsetAsync((double*)sc.accum.p + (size_t)plane * chunk_samples, 0, (size_t)P.n_samples * sizeof(double), lane_stream));
     if (f.n_groups) {
@@ -1921,6 +1937,8 @@ struct FrameRun {
       launch_accumulate_resolve(P, A, lane_stream);
     } else if (f.pixel_list) {
       launch_adaptive_fold(P, f.ad, lane_stream);
+    } else if (f.views) {
+      launch_views_resolve(P, d_linear, lane_stream);
     } else if (!f.n_groups) {
       launch_resolve(P, lane_stream);
     } else {
@@ -2226,8 +2244,16 @@ int run_frame(Device* D, const rh_scene* scene, const Frame& f, rh_stats* stats)
   }
 
   // queue capacity = factor * chunk samples; doubled when a chunk overflows (and remembered by the scene's renders; a
-  // trace starts from 2, a list frame from the scene's factor)
+  // trace starts from 2, a list frame from the scene's factor).  A views frame starts from the larger of the scene's
+  // factor and the one its own last views frame needed, halved while the lanes' queues would hold more entries than
+  // factor 2 gives the largest chunk plan_chunks makes: a factor learned on small frames, whose per-warp slack is
+  // large, must not size the queues of a batch many times their size (measured on dragon_full: 128² renders leave 32,
+  // which asked a batch of 256 such views for 32 x 67 M queue entries and failed with RH_ERR_OOM).
   uint32_t factor = f.trace ? 2u : std::max(2u, scene->queue_factor);
+  if (f.views) {
+    factor = std::max(factor, scene->views_queue_factor);
+    while (factor > 2 && (size_t)factor * R.chunk_samples * R.n_lanes > 2 * rh::max_chunk_samples(D->total_mem)) factor /= 2;
+  }
   for (;;) {
     if ((rc = R.reserve_queues(factor))) return rc;
     R.launches = 0;
@@ -2240,6 +2266,10 @@ int run_frame(Device* D, const rh_scene* scene, const Frame& f, rh_stats* stats)
     RH_CUDA(cudaMemsetAsync(D->counters.p, 0, sizeof(FrameCounters), D->stream));
     if (mode == RH_OFFSETS_TILED_F64 && !dev_off)
       RH_CUDA(cudaMemcpyAsync((void*)R.d_offsets, o.offsets, tile_bytes, cudaMemcpyHostToDevice, D->stream));
+    for (const Frame::Upload& u : f.uploads) {
+      RH_CUDA(cudaMemcpyAsync(u.dst, u.src, u.bytes, cudaMemcpyHostToDevice, D->stream));
+      R.upload_bytes += u.bytes;
+    }
     if (R.n_lanes > 1) {  // lane 1 starts after the control blocks are zeroed
       RH_CUDA(cudaEventRecord(D->ev_lane, D->stream));
       RH_CUDA(cudaStreamWaitEvent(D->stream2, D->ev_lane, 0));
@@ -2268,6 +2298,7 @@ int run_frame(Device* D, const rh_scene* scene, const Frame& f, rh_stats* stats)
       if (R.cap >= 0x7fffff00u || factor >= (1u << 16)) return rh::set_error(RH_ERR_OVERFLOW, f.overflow_error);
       factor *= 2;
       if (f.learns()) scene->queue_factor = factor;
+      if (f.views) scene->views_queue_factor = factor;
       continue;
     }
     if (stats) R.read_stats(stats, factor);
@@ -2915,6 +2946,77 @@ int light_groups_on(Device* D, const rh_scene* scene, const rh_camera* camera, c
   return run_frame(D, scene, f, stats);
 }
 
+// ------------------------------------------------------------------ camera batches
+// rh_render_views is one render (render_frame's checks, run_frame's plan, queues, overflow retry and passes) of a tall
+// frame whose local rows are [view][rows]: pass 0 builds each row's rays with its view's camera, and the chunks end with
+// a sink that decides padding rows per view.  Like a list frame it uses the scene's learned state without changing it.
+int views_on(Device* D, const rh_scene* scene, const rh_views* vw, const rh_render_opts* o, uint8_t* rgb_out, double* linear_out,
+             int32_t* hit_ids_out, rh_stats* stats) {
+  const std::string w = "rh_render_views";
+  if (!vw || !o) return rh::set_error(RH_ERR_ARG, w + ": null argument");
+  if (o->flags & (RH_FLAG_PEER_FRAMES | RH_FLAG_COUNT))
+    return rh::set_error(RH_ERR_ARG, w + ": RH_FLAG_PEER_FRAMES and RH_FLAG_COUNT are not supported");
+  if (vw->n_views < 1 || vw->n_views > kMaxViews) return rh::set_error(RH_ERR_ARG, w + ": n_views must be 1..65536");
+  if (!vw->cameras) return rh::set_error(RH_ERR_ARG, w + ": cameras is null");
+  if (vw->reserved_) return rh::set_error(RH_ERR_ARG, w + ": reserved_ must be 0");
+  if (vw->seeds && o->offset_mode != RH_OFFSETS_SPLITMIX64)
+    return rh::set_error(RH_ERR_ARG, w + ": seeds go with RH_OFFSETS_SPLITMIX64 only");
+  if (!rgb_out && !linear_out) return rh::set_error(RH_ERR_ARG, w + ": rgb_out and linear_out are both null");
+  const uint32_t V = vw->n_views;
+  for (uint32_t v = 0; v < V; v++) {
+    const int32_t proj = vw->cameras[v].projection;
+    if (proj != RH_PROJ_ORTHOGRAPHIC && proj != RH_PROJ_PERSPECTIVE)
+      return rh::set_error(RH_ERR_ARG, w + ": cameras[" + std::to_string(v) + "] has an unknown projection");
+  }
+  Frame f;
+  f.views = true;
+  int rc = render_frame(D, scene, &vw->cameras[0], o, rgb_out, hit_ids_out, &f, "rh_render_views");
+  if (rc) return rc;
+  const int rows = f.rows_local, W = f.o.width;
+  if ((uint64_t)V * rows > 0x7fffffffu) return rh::set_error(RH_ERR_ARG, w + ": n_views x shard rows must be below 2^31");
+  if (o->flags & RH_FLAG_DEVICE_OUT) {
+    if ((uintptr_t)linear_out % 8) return rh::set_error(RH_ERR_ARG, w + ": device linear_out must be 8-byte aligned");
+    RH_CUDA(cudaSetDevice(D->dev));
+    if ((rc = check_device_pointers({rgb_out, linear_out, (o->flags & RH_FLAG_HIT_IDS) ? hit_ids_out : nullptr},
+                                    w + ": RH_FLAG_DEVICE_OUT with a pointer that is not device memory")))
+      return rc;
+  }
+  RH_CUDA(cudaSetDevice(D->dev));
+  // the camera table and the seeds, behind one another in one buffer
+  std::vector<CameraParams> cams(V);
+  for (uint32_t v = 0; v < V; v++) cams[v] = make_camera(vw->cameras[v], W, f.o.height);
+  const size_t cam_bytes = V * sizeof(CameraParams), seed_bytes = vw->seeds ? V * sizeof(uint64_t) : 0;
+  if ((rc = D->views.reserve(cam_bytes + seed_bytes))) return rc;
+  f.cams = (const CameraParams*)D->views.p;
+  f.uploads.push_back({D->views.p, cams.data(), cam_bytes});
+  if (vw->seeds) {
+    f.view_seeds = (const unsigned long long*)((char*)D->views.p + cam_bytes);
+    f.uploads.push_back({(char*)D->views.p + cam_bytes, vw->seeds, seed_bytes});
+  }
+  // host per-pixel offsets are the same for every view: staged once, then read as device offsets are
+  const int mode = f.o.offset_mode;
+  if ((mode == RH_OFFSETS_F64 || mode == RH_OFFSETS_F32) && !(f.o.flags & RH_FLAG_DEVICE_OFFSETS)) {
+    const int off_rows = (f.o.flags & RH_FLAG_SHARD_OFFSETS) ? rows : f.o.height;
+    const size_t bytes = (size_t)off_rows * W * f.o.spp * f.off_elem;
+    if (D->offsets.reserve(bytes)) {
+      cudaGetLastError();  // (clears the failed allocation)
+      return rh::set_error(RH_ERR_OOM, w + ": the host offsets (" + std::to_string(bytes) + " bytes) do not fit in device memory");
+    }
+    f.uploads.push_back({D->offsets.p, f.o.offsets, bytes});
+    f.o.offsets = D->offsets.p;
+    f.o.flags |= RH_FLAG_DEVICE_OFFSETS;
+  }
+  f.view_rows = (uint32_t)rows;
+  f.rows_local = (int)(V * rows);
+  f.out_bytes *= V;
+  f.ids_bytes *= V;
+  f.rays_primary *= V;
+  f.linear = linear_out;
+  f.linear_bytes = (size_t)f.rows_local * W * 3 * sizeof(double);
+  f.overflow_error = "rh_render_views: ray queue overflow; lower chunk_samples";
+  return run_frame(D, scene, f, stats);
+}
+
 }  // namespace
 
 // ================================================================== C ABI
@@ -3110,6 +3212,12 @@ int rh_render_light_groups(const rh_scene* scene, const rh_camera* camera, const
                            const rh_light_groups* groups, uint8_t* rgb_out, int32_t* hit_ids_out, rh_stats* stats) {
   if (!g_dev) return rh::set_error(RH_ERR_STATE, "rh_render_light_groups: call rh_init first");
   return light_groups_on(g_dev.get(), scene, camera, opts, groups, rgb_out, hit_ids_out, stats);
+}
+
+int rh_render_views(const rh_scene* scene, const rh_views* views, const rh_render_opts* opts, uint8_t* rgb_out,
+                    double* linear_out, int32_t* hit_ids_out, rh_stats* stats) {
+  if (!g_dev) return rh::set_error(RH_ERR_STATE, "rh_render_views: call rh_init first");
+  return views_on(g_dev.get(), scene, views, opts, rgb_out, linear_out, hit_ids_out, stats);
 }
 
 int rh_default_band_height(int height, int shard_count) {

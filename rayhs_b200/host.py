@@ -568,6 +568,67 @@ def renderLightGroups(job: Rendering, spp: int = 1, offsets=None, seed: int | No
     return LightGroups(out[:G], out[G], image, ids, st.as_dict())
 
 
+# ---- camera batches (many views of one scene in one wavefront)
+
+@dataclass
+class Views:
+    """rh_render_views of a batch of cameras, view-major over the shard's rows: pixels [V, rows, w, 3] uint8 (None unless
+    asked for), view v being render(camera v)'s RGB8 rows; linear [V, rows, w, 3] float64 (None unless asked for), the
+    colours toIntC is applied to, as a fresh Accumulator's first add returns them; hit_ids [V, rows, w, spp, 2] when
+    asked for; and the call's stats (ray counts summed over the views).  numpy arrays, or CUDA tensors with device
+    outputs."""
+    pixels: object = None
+    linear: object = None
+    hit_ids: object = None
+    stats: dict = field(default_factory=dict)
+
+
+def renderViews(job: Rendering, cameras, spp: int = 1, offsets=None, seed: int | None = None, seeds=None, rgb: bool = True,
+                linear: bool = False, want_hit_ids: bool = False, device: bool = False, shard_index: int = 0, shard_count: int = 1,
+                band_height: int = 0, chunk_samples: int = 0, exact_boxes: bool = False, shadow: str | None = None,
+                light_maps: bool = True, offset_tile: int = 0, shard_offsets: bool = False, profile: bool = False) -> Views:
+    """One wavefront for a batch of views of job's scene: view v is render(job with cameras[v], spp, offsets / seed,
+    ...).  `cameras`: a sequence of capi.rh_camera (job.camera is not used; width, height and maxDepth are job's).
+    `offsets`: full-frame [width*height, spp, 2] float64 / float32 (with `shard_offsets`, the shard's rows only; with
+    `offset_tile`, the [tile*tile, spp, 2] tile), numpy, a CPU tensor or a CUDA tensor, the same for every view; `seed`:
+    the SplitMix64 stream instead; `seeds`: one SplitMix64 seed per view.  CUDA offsets or device=True: the outputs are
+    CUDA tensors.  `rgb` / `linear`: which of the two images to return (at least one)."""
+    cams = list(cameras)
+    V = len(cams)
+    if not rgb and not linear:
+        raise ValueError("ask for rgb, linear or both")
+    if seeds is not None:
+        seeds = [int(x) for x in seeds]
+        if len(seeds) != V:
+            raise ValueError(f"seeds has {len(seeds)} entries for {V} cameras")
+        if offsets is not None:
+            raise ValueError("pass either offsets or seeds")
+        if seed is None:
+            seed = seeds[0] if seeds else 0
+    bh, rows = _shard_rows(job, shard_count, band_height)
+    mode, off_ptr, keep, dev_off = _offsets(job, spp, offsets, seed, offset_tile, rows if shard_offsets else None)
+    device = device or dev_off
+    flags = (_flags(want_hit_ids=want_hit_ids, exact_boxes=exact_boxes, shadow=shadow, light_maps=light_maps, profile=profile,
+                    device=device) | (capi.RH_FLAG_DEVICE_OFFSETS if dev_off else 0)
+             | (capi.RH_FLAG_SHARD_OFFSETS if shard_offsets else 0))
+    o = _opts(job, spp, mode, off_ptr, offset_tile, shard_index, shard_count, bh, chunk_samples, flags)
+    empty = _alloc(device)
+    shape = (V, rows, job.width)
+    out = Views(empty(shape + (3,), "uint8") if rgb else None, empty(shape + (3,), "float64") if linear else None,
+                empty(shape + (spp, 2), "int32") if want_hit_ids else None)
+    table = (capi.rh_camera * max(V, 1))(*cams)
+    seed_table = (C.c_uint64 * max(V, 1))(*seeds) if seeds is not None else None
+    vw = capi.rh_views()
+    vw.cameras, vw.n_views = C.cast(table, C.POINTER(capi.rh_camera)), V
+    if seed_table is not None:
+        vw.seeds = C.cast(seed_table, C.POINTER(C.c_uint64))
+    st = capi.rh_stats()
+    check(lib().rh_render_views(job.scene.device, C.byref(vw), C.byref(o), _ptr(out.pixels) if rgb else None,
+                                _ptr(out.linear) if linear else None, _ptr(out.hit_ids) if want_hit_ids else None, C.byref(st)))
+    out.stats = st.as_dict()
+    return out
+
+
 def scene_setup_ms(scene: Scene) -> dict:
     """Milliseconds rh_scene_create spent on its parts (host-side trees, light-space tables, uploads)."""
     ms, info = scene._info()
