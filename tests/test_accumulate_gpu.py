@@ -12,13 +12,12 @@ import pytest
 
 import rayhs_b200 as rh
 from rayhs_b200 import capi, host
-from tests.test_trace_rays_gpu import growth_scene, has_transparent, to_int_c
-from tests.util import GOLDEN, SCENES, assert_parity, load_scene
+from tests.test_trace_rays_gpu import growth_scene, has_transparent
+from tests.util import ATOL, GOLDEN, RTOL, SCENES, assert_parity, load_scene, to_int_c
 
 pytestmark = pytest.mark.gpu
 
 W, H, SPP, BATCHES = 64, 48, 8, (1, 3, 4)  # odd and even batches: both fold paths of the sink
-RTOL, ATOL = 1e-9, 1e-12
 PLAIN = "dragon_low"  # no Transparent material: renders are deterministic to the byte
 
 

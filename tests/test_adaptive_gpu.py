@@ -11,8 +11,8 @@ import pytest
 import rayhs_b200 as rh
 from rayhs_b200 import capi, host
 from tests.adaptive_rule import active_pixels, fold
-from tests.test_trace_rays_gpu import growth_scene, has_transparent, to_int_c
-from tests.util import SCENES, assert_parity, load_scene
+from tests.test_trace_rays_gpu import growth_scene, has_transparent
+from tests.util import SCENES, assert_parity, load_scene, to_int_c
 
 pytestmark = pytest.mark.gpu
 

@@ -13,8 +13,8 @@ from oracle.orc import OracleScene
 from rayhs_b200 import capi
 from tests import value_cases as vc
 from tests.test_features_gpu import BUILT, SIZES
-from tests.test_trace_rays_gpu import ATOL, RTOL, growth_scene, has_transparent
-from tests.util import SCENES, assert_parity, load_scene
+from tests.test_trace_rays_gpu import growth_scene, has_transparent
+from tests.util import ATOL, RTOL, SCENES, assert_parity, load_scene
 
 pytestmark = pytest.mark.gpu
 

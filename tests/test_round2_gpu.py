@@ -56,22 +56,33 @@ def test_a_shard_of_single_row_bands_picks_arbitrary_rows():
     assert np.array_equal(ids.cpu().numpy().reshape(rows, w, spp, 2)[:len(ys)], full.hit_ids.reshape(h, w, spp, 2)[ys])
 
 
-@pytest.mark.parametrize("name", ["dragon_low", "dragon_full", "transform", "cornellBox"])
+# hand-built scenes at the limits of the packed tables (tests/test_limits_gpu.py): 42 maps at 512^2 cells per face, 48
+# at 256^2, and 12 lights x 8 meshes with directional lights first (lit bit 11 and map index 11 * 8 + 7 in use)
+LIMIT_SCENES = {"map_res_42": lambda L: L.map_res_scene(7), "map_res_48": lambda L: L.map_res_scene(8),
+                "packed_12x8": lambda L: L.packed_scene(12)}
+
+
+@pytest.mark.parametrize("name", ["dragon_low", "dragon_full", "transform", "cornellBox"] + list(LIMIT_SCENES))
 def test_device_built_light_tables_equal_the_host_built_ones(name, monkeypatch):
     """rh_scene_create builds the cube maps and the lit-triangle flags with CUDA kernels (setup_kernels.cu); the host
     builders of light_maps.cpp (RAYHS_B200_SETUP=host) run the same geometry code (light_geom.h) and must produce the
     same tables bit for bit — the host builders are what tests/test_light_maps.py checks against brute force."""
     import os
 
-    from tests.util import GOLDEN
+    from tests import test_limits_gpu
+    from tests.util import GOLDEN, RawScene
 
-    path = os.path.join(GOLDEN, name + ".pack")
+    def make():
+        if name in LIMIT_SCENES:
+            return RawScene(*LIMIT_SCENES[name](test_limits_gpu), camera=test_limits_gpu.CAMERA)
+        return rh.Scene.from_pack(os.path.join(GOLDEN, name + ".pack"))
+
     monkeypatch.delenv("RAYHS_B200_SETUP", raising=False)
-    dev = rh.Scene.from_pack(path)
-    t_dev = dev.light_tables()
+    dev = make()
+    t_dev = rh.Scene.light_tables(dev)
     monkeypatch.setenv("RAYHS_B200_SETUP", "host")
-    host = rh.Scene.from_pack(path)
-    t_host = host.light_tables()
+    host = make()
+    t_host = rh.Scene.light_tables(host)
     assert t_dev["res"] == t_host["res"]
     assert np.array_equal(t_dev["index"], t_host["index"])
     assert t_dev["maps"].shape == t_host["maps"].shape
@@ -81,5 +92,8 @@ def test_device_built_light_tables_equal_the_host_built_ones(name, monkeypatch):
         assert np.array_equal(t_dev["lit"], t_host["lit"])
         if name.startswith("dragon"):
             assert (t_dev["lit"] & 0x0fff).astype(bool).mean() > 0.3   # the flags are not trivially empty
+    if name in LIMIT_SCENES:   # the tables are not trivially empty either
+        assert len(t_dev["maps"]) and t_dev["lit"] is not None and (t_dev["lit"] & 0x0fff).any(), name
+    print(name, "res", t_dev["res"], "maps", len(t_dev["maps"]))
     dev.close()
     host.close()

@@ -12,23 +12,14 @@ import rayhs_b200 as rh
 from rayhs_b200 import capi
 from tests.test_ray_query_gpu import BUILT, CAM_H, CAM_W, MAX_GRAZING, adversarial_rays, geometry, incoherent_rays
 from tests.trace_oracle import COUNT_NAMES, TraceOracle
-from tests.util import SCENES, assert_parity, load_scene
+from tests.util import ATOL, RTOL, SCENES, assert_parity, load_scene, to_int_c
 
 pytestmark = pytest.mark.gpu
-
-# the tolerance tests/test_pyref_pins_oracle.py uses: the wavefront adds a ray's light terms in its own order (DESIGN §3)
-RTOL, ATOL = 1e-9, 1e-12
 
 
 def has_transparent(sc):
     raw = sc.raw.contents
     return any(raw.materials[i].kind == capi.RH_MAT_TRANSPARENT for i in range(raw.n_materials))
-
-
-def to_int_c(c):
-    """Image.hs:54-55 toIntC, clamped into 0..255 as rh_render stores it (NaN: hs_min NaN 1 = 1, so 255)."""
-    v = 255 * np.where(c <= 1, c, 1.0)
-    return np.where(v < 0, 0, np.minimum(np.trunc(np.where(v < 0, 0, v)), 255)).astype(np.uint8)
 
 
 def trace(sc, rays, max_depth, **kw):

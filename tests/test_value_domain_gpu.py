@@ -10,9 +10,8 @@ import pytest
 
 import rayhs_b200 as rh
 from oracle.orc import OracleScene
-from tests.test_trace_rays_gpu import ATOL, RTOL
 from tests.trace_oracle import COUNT_NAMES, TraceOracle
-from tests.util import load_scene
+from tests.util import ATOL, RTOL, load_scene
 from tests import value_cases as vc
 
 pytestmark = pytest.mark.gpu

@@ -58,6 +58,56 @@ def assert_parity(gpu_u8, ref_u8, what=""):
     return m
 
 
+# The tolerance of a linear colour against the oracle's (tests/test_pyref_pins_oracle.py uses it too): the wavefront adds
+# a sample's terms in its own order, <= 1 ulp per term, and Transparent forks with atomics (DESIGN §3).
+RTOL, ATOL = 1e-9, 1e-12
+
+
+def to_int_c(c):
+    """Image.hs:54-55 toIntC, clamped into 0..255 as rh_render stores it (NaN: hs_min NaN 1 = 1, so 255)."""
+    v = 255 * np.where(c <= 1, c, 1.0)
+    return np.where(v < 0, 0, np.minimum(np.trunc(np.where(v < 0, 0, v)), 255)).astype(np.uint8)
+
+
+def assert_oracle_exact(pixels, linear, ref, what=""):
+    """The image equals the oracle's (`ref`: OracleScene.render) up to the departures of DESIGN §3, channel by channel:
+    the linear colour is within RTOL / ATOL of the oracle's (NaN equals NaN); the bytes are toIntC of the device's own
+    linear colour; and they are the oracle's bytes, except where the two linear colours, that close, straddle a
+    quantisation step — there they differ by exactly 1.  Returns the number of such straddled channels."""
+    want_lin, want_u8 = ref["rgb_f64"], ref["rgb_u8"]
+    linear = np.asarray(linear, dtype=np.float64).reshape(want_lin.shape)
+    pixels = np.asarray(pixels).reshape(want_u8.shape)
+    ok = np.isclose(linear, want_lin, rtol=RTOL, atol=ATOL, equal_nan=True)
+    bad = np.argwhere(~ok)[:5]
+    assert ok.all(), (what, f"{int((~ok).sum())} linear channels off the oracle's", bad.tolist(),
+                      [(linear[tuple(b)], want_lin[tuple(b)]) for b in bad])
+    own = to_int_c(linear)
+    bad = np.argwhere(pixels != own)[:5]
+    assert not len(bad), (what, f"{int((pixels != own).sum())} bytes are not toIntC of the linear colour", bad.tolist(),
+                          [(int(pixels[tuple(b)]), int(own[tuple(b)]), linear[tuple(b)]) for b in bad])
+    straddled = own != to_int_c(want_lin)
+    d = pixels.astype(np.int32) - want_u8.astype(np.int32)
+    wrong = np.where(straddled, np.abs(d) != 1, d != 0)
+    bad = np.argwhere(wrong)[:5]
+    assert not wrong.any(), (what, f"{int(wrong.sum())} bytes off the oracle's ({int(straddled.sum())} channels straddle a "
+                                   "quantisation step and may differ by 1)", bad.tolist(),
+                             [(int(pixels[tuple(b)]), int(want_u8[tuple(b)])) for b in bad])
+    return int(straddled.sum())
+
+
+def render_linear(job, spp=1, offsets=None, seed=None, **kw):
+    """The frame rh_render makes (progressive rendering's first call traces the same samples and stores the same bytes;
+    tests/test_accumulate_gpu.py pins that) with its linear colours, hit ids and stats.  `seed`: the samples of
+    sample_offsets(width * height, spp, seed), regenerated on the device."""
+    import rayhs_b200 as rh
+
+    acc = rh.Accumulator(job, stream_spp=spp if seed is not None else 0)
+    try:
+        return acc.add(spp, offsets=offsets, seed=seed, want_hit_ids=True, **kw)
+    finally:
+        acc.close()
+
+
 # ---------------------------------------------------------------------------------------------
 # Hand-built raw scenes (rh_raw_scene) for analytic and edge-case tests.
 class RawScene:
@@ -163,6 +213,16 @@ class RawScene:
             self._dev = C.c_void_p()
             capi.check(capi.lib().rh_scene_create(self.flat, C.byref(self._dev)))
         return self._dev
+
+    def close(self):
+        """Releases the device scene and the flattened scene (a scene with many light maps holds hundreds of MB)."""
+        from rayhs_b200 import capi
+
+        if self._dev:
+            capi.lib().rh_scene_destroy(self._dev)
+        if self._flat:
+            capi.lib().rh_flat_destroy(self._flat)
+        self._dev = self._flat = None
 
 
 def grid_mesh(n, z=0.0, wobble=0.0, seed=1):
