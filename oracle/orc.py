@@ -4,6 +4,11 @@ TEST INFRASTRUCTURE ONLY (see the header of oracle.cpp): imported by tests/, by
 __graft_entry__.smoke() and by bench.py's cpu_baseline / --impl reference legs, never by
 rayhs_b200/.  The scene is handed over as the POD `rh_raw_scene` (objects before any tree
 build); the oracle builds its own tree with the KDTree.hs rule.
+
+Besides renders and one-ray queries, the library answers the tests' batch questions over
+caller-built rays [n, 6] (origin, direction) on host threads: closest hits, shadow verdicts,
+traceRay colours and first-hit features (OracleScene.*_batch), and camera rays (camera_rays);
+batch.cpp defines them, after oracle.cpp, in the same library.
 """
 from __future__ import annotations
 
@@ -14,6 +19,13 @@ import numpy as np
 
 _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.path.join(_HERE, "_build", "liborc.so")
+
+# one rh_hit record (include/rayhs_b200.h), as orc_closest_batch writes it; declared here on its own so that the tests
+# can hold it against the product's rayhs_b200.HIT_DTYPE and the header
+HIT_DTYPE = np.dtype([("t", "<f8"), ("p", "<f8", 3), ("n", "<f8", 3), ("uv", "<f8", 2), ("object", "<i4"), ("tri", "<i4")])
+assert HIT_DTYPE.itemsize == 80
+# orc_trace_batch's ray counts, in its order, under the names of the product's stats
+COUNT_NAMES = ("rays_primary", "rays_reflect", "rays_probe", "rays_exit", "rays_shadow")
 
 
 class orc_result_counts(C.Structure):
@@ -44,6 +56,11 @@ def lib() -> C.CDLL:
                                  vp, C.POINTER(orc_result_counts)]
         L.orc_render2.argtypes = [vp, vp, C.c_int, C.c_int, C.c_int, C.c_int, vp, C.c_int, C.c_uint64, C.c_int, C.c_int, C.c_int,
                                   C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, vp, vp, vp, vp, C.POINTER(orc_result_counts)]
+        L.orc_camera_rays.argtypes = [vp, C.c_double, C.c_double, vp, C.c_uint64, vp]
+        L.orc_closest_batch.argtypes = [vp, vp, C.c_uint64, vp, C.c_int]
+        L.orc_shadow_batch.argtypes = [vp, C.c_uint32, vp, C.c_uint64, vp, C.c_int]
+        L.orc_trace_batch.argtypes = [vp, vp, C.c_uint64, C.c_int, vp, vp, vp, C.c_int]
+        L.orc_feature_batch.argtypes = [vp, vp, C.c_uint64, vp, vp, vp, vp, vp, C.c_int]
         _lib = L
     return _lib
 
@@ -87,6 +104,40 @@ class OracleScene:
         out = (C.c_double * 3)()
         lib().orc_color_at(self._h, material, u, v, out)
         return np.array(out[:])
+
+    def closest_batch(self, rays, threads=0):
+        """closestIntersection for every row of rays [n, 6] (origin, direction): a record array of HIT_DTYPE."""
+        rays = _rays(rays)
+        out = np.empty(len(rays), dtype=HIT_DTYPE)
+        assert lib().orc_closest_batch(self._h, rays.ctypes.data, len(rays), out.ctypes.data, threads) == 0
+        return out
+
+    def shadow_batch(self, light, rays, threads=0):
+        """shadowIntersection towards light `light` for every row of rays [n, 6]: a bool array."""
+        rays = _rays(rays)
+        out = np.empty(len(rays), dtype=np.uint8)
+        assert lib().orc_shadow_batch(self._h, int(light), rays.ctypes.data, len(rays), out.ctypes.data, threads) == 0
+        return out.view(np.bool_)
+
+    def trace_batch(self, rays, max_depth, threads=0):
+        """traceRay sc 0 max_depth for every row of rays [n, 6]: (colors [n, 3], ids [n, 2], counts dict of COUNT_NAMES)."""
+        rays = _rays(rays)
+        colors = np.empty((len(rays), 3))
+        ids = np.empty((len(rays), 2), dtype=np.int32)
+        counts = np.zeros(5, dtype=np.uint64)
+        assert lib().orc_trace_batch(self._h, rays.ctypes.data, len(rays), int(max_depth), colors.ctypes.data, ids.ctypes.data,
+                                     counts.ctypes.data, threads) == 0
+        return colors, ids, dict(zip(COUNT_NAMES, (int(c) for c in counts)))
+
+    def features_batch(self, rays, threads=0):
+        """The first-hit features of every row of rays [n, 6]: dict of t [n], n and albedo [n, 3], ids and uv [n, 2]."""
+        rays = _rays(rays)
+        n = len(rays)
+        t, nn, al, uv = np.empty(n), np.empty((n, 3)), np.empty((n, 3)), np.empty((n, 2))
+        ids = np.empty((n, 2), dtype=np.int32)
+        assert lib().orc_feature_batch(self._h, rays.ctypes.data, n, t.ctypes.data, nn.ctypes.data, al.ctypes.data, ids.ctypes.data,
+                                       uv.ctypes.data, threads) == 0
+        return dict(t=t, n=nn, albedo=al, ids=ids, uv=uv)
 
     def render(self, camera, w, h, max_depth, spp=1, offsets=None, rows=(0, None, 1), threads=0, want_ids=True):
         """rayTrace / distributedRayTrace over rows[0]:rows[1]:rows[2].  Returns a dict with full-frame arrays
@@ -136,6 +187,22 @@ class OracleScene:
         return dict(rows=ys, cols=xs, rgb_f64=rgb_f64, rgb_u8=rgb_u8, hit_ids=ids,
                     rays={n: int(cnt.rays[i]) for i, n in enumerate(names)}, rays_total=int(sum(cnt.rays)),
                     seconds=cnt.seconds, threads=cnt.threads)
+
+
+def _rays(rays):
+    return np.ascontiguousarray(rays, dtype=np.float64).reshape(-1, 6)
+
+
+def camera_rays(camera, w, h, xy=None):
+    """rayFromPixel (Projection.hs:22-46) of a w x h view at pixel coordinates xy [n, 2] (default: every pixel's (x, y),
+    row-major), in one call: rays [n, 6] = origin, direction."""
+    if xy is None:
+        rows, cols = np.divmod(np.arange(h * w), w)
+        xy = np.stack([cols, rows], axis=1)
+    xy = np.ascontiguousarray(xy, dtype=np.float64).reshape(-1, 2)
+    rays = np.empty((len(xy), 6))
+    lib().orc_camera_rays(C.cast(C.pointer(camera), C.c_void_p), w, h, xy.ctypes.data, len(xy), rays.ctypes.data)
+    return rays
 
 
 def mod1(n: float, d: float) -> float:

@@ -20,6 +20,7 @@ OBJ = os.path.join(ROOT, "build", "obj")
 LIB = os.path.join(ROOT, "rayhs_b200", "librayhs_b200.so")
 CLI = os.path.join(ROOT, "rayhs_b200", "rayhs")
 ORACLE_SRC = os.path.join(ROOT, "oracle", "oracle.cpp")
+ORACLE_LIB_SRC = os.path.join(ROOT, "oracle", "batch.cpp")  # includes ORACLE_SRC
 ORACLE_LIB = os.path.join(ROOT, "oracle", "_build", "liborc.so")
 
 NVCC = os.environ.get("NVCC") or shutil.which("nvcc") or "/usr/local/cuda/bin/nvcc"
@@ -106,9 +107,10 @@ def build_cli(force: bool = False) -> str:
 def build_oracle(force: bool = False) -> str:
     os.makedirs(os.path.dirname(ORACLE_LIB), exist_ok=True)
     flags = ["-std=c++17", "-O2", "-ffp-contract=off", "-fPIC", "-shared"]
-    if force or _stale(ORACLE_LIB, [ORACLE_SRC, HEADERS[-1]], flags):
-        _run([CXX, *flags, ORACLE_SRC, "-o", ORACLE_LIB, "-lpthread"])
-        _stamp(ORACLE_LIB, [ORACLE_SRC, HEADERS[-1]], flags)
+    deps = [ORACLE_LIB_SRC, ORACLE_SRC, HEADERS[-1]]
+    if force or _stale(ORACLE_LIB, deps, flags):
+        _run([CXX, *flags, ORACLE_LIB_SRC, "-o", ORACLE_LIB, "-lpthread"])
+        _stamp(ORACLE_LIB, deps, flags)
     return ORACLE_LIB
 
 

@@ -1,4 +1,4 @@
-"""GPU tests of the feature buffers (rh_render_features / renderFeatures) against the oracle (tests/feature_oracle.cpp):
+"""GPU tests of the feature buffers (rh_render_features / renderFeatures) against the oracle (orc_feature_batch):
 every shipped pack and a built scene with every material kind, checker and texture maps on planes and meshes and a
 ShowUV sphere, seen through both projections; the render's own hits; every offset mode, shards, device buffers, the
 exact walk and chunked host buffers giving the same bytes; scene updates; argument errors."""
@@ -8,8 +8,8 @@ import numpy as np
 import pytest
 
 import rayhs_b200 as rh
+from oracle.orc import OracleScene, camera_rays
 from rayhs_b200 import capi
-from tests.feature_oracle import FeatureOracle
 from tests.util import SCENES, RawScene, load_scene
 
 pytestmark = pytest.mark.gpu
@@ -56,7 +56,7 @@ _cache = {}
 def scene(name):
     if name not in _cache:
         sc = BUILT[name]() if name in BUILT else load_scene(name)
-        _cache[name] = (sc, FeatureOracle(sc.raw))
+        _cache[name] = (sc, OracleScene(sc.raw))
     return _cache[name]
 
 
@@ -76,10 +76,44 @@ def uv_dependent(sc):
     return np.array(out + [False])  # (index -1: a miss)
 
 
+def samples(orc, camera, w, h, ox, oy):
+    """The camera rays at pixel coordinates (col + ox, row + oy) for ox, oy [h * w, spp] (float64, pixel-major), through
+    the batch: dict of rays [h*w*spp, 6] and, per pixel and sample, t [h*w, spp], n and albedo [h*w, spp, 3], ids and
+    uv [h*w, spp, 2]."""
+    spp = ox.shape[1]
+    rows, cols = np.divmod(np.arange(h * w), w)
+    xy = np.empty((h * w, spp, 2))
+    xy[..., 0] = cols[:, None] + ox
+    xy[..., 1] = rows[:, None] + oy
+    rays = camera_rays(camera, w, h, xy.reshape(-1, 2))
+    f = orc.features_batch(rays)
+    return dict(rays=rays, t=f["t"].reshape(h * w, spp), n=f["n"].reshape(h * w, spp, 3), albedo=f["albedo"].reshape(h * w, spp, 3),
+                ids=f["ids"].reshape(h * w, spp, 2), uv=f["uv"].reshape(h * w, spp, 2))
+
+
+def fold(s, w, h):
+    """The per-pixel buffers of samples `s`: albedo [h, w, 3], normal [h, w, 3], depth [h, w], hits [h, w] and ids
+    [h, w, spp, 2]; foldl (+) 0 over the samples in sample order, per channel, then times 1.0 / spp (depth: 1.0 / hits
+    over the hitting samples' t)."""
+    spp = s["t"].shape[1]
+    hit = s["ids"][..., 0] >= 0
+    a, nn, ts = np.zeros((h * w, 3)), np.zeros((h * w, 3)), np.zeros(h * w)
+    for k in range(spp):
+        a = a + s["albedo"][:, k]
+        nn = nn + s["n"][:, k]
+        ts = ts + np.where(hit[:, k], s["t"][:, k], 0.0)
+    inv = 1.0 / spp
+    hits = hit.sum(axis=1).astype(np.uint32)
+    with np.errstate(divide="ignore", invalid="ignore"):
+        depth = np.where(hits > 0, (1.0 / hits.astype(np.float64)) * ts, np.inf)
+    return dict(albedo=(inv * a).reshape(h, w, 3), normal=(inv * nn).reshape(h, w, 3), depth=depth.reshape(h, w),
+                hits=hits.reshape(h, w), ids=s["ids"].reshape(h, w, spp, 2))
+
+
 def expected(sc, orc, w, h, ox, oy):
     """The oracle's buffers for pixel offsets ox, oy [h*w, spp].  A sample on a sphere whose albedo depends on its uv takes
     the device's uv (rh_closest_intersection of the same ray), which must be within SPHERE_UV_ULP of the oracle's."""
-    s = orc.samples(sc.camera, w, h, ox, oy)
+    s = samples(orc, sc.camera, w, h, ox, oy)
     dep = uv_dependent(sc)[s["ids"][..., 0]]
     if dep.any():
         rays = s["rays"].reshape(h * w, -1, 6)[dep]
@@ -93,7 +127,7 @@ def expected(sc, orc, w, h, ox, oy):
         for m, (u, v) in zip(mats, got):
             al.append((u, v, 0.0) if raw.materials[m].kind == capi.RH_MAT_SHOWUV else orc.color_at(m, u, v))
         s["albedo"][dep] = np.array(al)
-    return orc.fold(s, w, h)
+    return fold(s, w, h)
 
 
 def assert_same(fe, e, what, rows=None):

@@ -1,6 +1,6 @@
 """CPU tests of the batched ray queries: the rh_hit layout of the header against the ctypes / numpy mirrors, loud
-failure without a device, and the batch oracle of the query tests (tests/query_oracle.cpp: orc_closest_batch /
-orc_shadow_batch) against the oracle's one-ray entry point and against hand-derived answers."""
+failure without a device, and the oracle's batch queries (oracle/batch.cpp: orc_closest_batch / orc_shadow_batch)
+against the oracle's one-ray entry point and against hand-derived answers."""
 import ctypes as C
 import math
 import os
@@ -10,10 +10,8 @@ import numpy as np
 import pytest
 
 import rayhs_b200 as rh
-from oracle.orc import OracleScene
+from oracle.orc import HIT_DTYPE as ORC_HIT_DTYPE, OracleScene
 from rayhs_b200 import capi
-from tests.query_oracle import HIT_DTYPE as ORC_HIT_DTYPE
-from tests.query_oracle import BatchOracle
 from tests.util import RawScene, load_scene
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
@@ -59,7 +57,7 @@ def test_closest_batch_equals_the_one_ray_entry_point():
     d = rng.normal(size=(2000, 3))
     d[::7, rng.randint(0, 3)] = 0.0  # zero components
     rays = np.concatenate([np.array(cam), np.concatenate([o, d], axis=1)])
-    got = BatchOracle(sc.raw).closest_batch(rays, threads=4)
+    got = OracleScene(sc.raw).closest_batch(rays, threads=4)
     hits = 0
     for i, r in enumerate(rays):
         one = orc.closest(r[:3], r[3:])
@@ -81,7 +79,7 @@ SPHERE = {"kind": "sphere", "center": (0, 0, 0), "radius": 1.0}
 def test_closest_batch_hand_derived_answers():
     rs = RawScene([SPHERE, {"kind": "plane", "point": (0, -2, 0), "normal": (0, 1, 0), "tangent": (1, 0, 0)}],
                   [{"kind": "diffuse"}], [])
-    orc = BatchOracle(rs.raw)
+    orc = OracleScene(rs.raw)
     rays = np.array([[0, 0, -5, 0, 0, 1],     # from outside at the centre: t = distance - 1
                      [0, 0, 0, 0, 0, 1],      # from the centre: the far root
                      [0, 0, 0.5, 0, 0, 2],    # from inside, direction of length 2: far root at z = 1, t = 0.25
@@ -101,22 +99,22 @@ def test_shadow_batch_hand_derived_answers():
     # the only blocker is an emitter: isOccluder (RayHs.hs:81-82) drops it
     emitter = RawScene([{"kind": "sphere", "center": (0, 0, 3), "radius": 0.5}], [{"kind": "emmit", "color1": (1, 1, 1)}],
                        [{"kind": "point", "vec": (0, 0, 6)}])
-    assert not BatchOracle(emitter.raw).shadow_batch(0, ray)[0]
+    assert not OracleScene(emitter.raw).shadow_batch(0, ray)[0]
     # the same sphere as a diffuse object does block
     diffuse = RawScene([{"kind": "sphere", "center": (0, 0, 3), "radius": 0.5}], [{"kind": "diffuse"}],
                        [{"kind": "point", "vec": (0, 0, 6)}])
-    assert BatchOracle(diffuse.raw).shadow_batch(0, ray)[0]
+    assert OracleScene(diffuse.raw).shadow_batch(0, ray)[0]
     # a blocker behind a point light is not in front of it (inFrontOfLight, RayHs.hs:84-87) ...
     behind = [{"kind": "sphere", "center": (0, 0, 5), "radius": 0.5}]
     point = RawScene(behind, [{"kind": "diffuse"}], [{"kind": "point", "vec": (0, 0, 2)}])
-    assert not BatchOracle(point.raw).shadow_batch(0, ray)[0]
+    assert not OracleScene(point.raw).shadow_batch(0, ray)[0]
     # ... while for a directional light every hit counts
     directional = RawScene(behind, [{"kind": "diffuse"}], [{"kind": "directional", "vec": (0, 0, 1)}])
-    assert BatchOracle(directional.raw).shadow_batch(0, ray)[0]
+    assert OracleScene(directional.raw).shadow_batch(0, ray)[0]
     # two lights in one scene: the index selects the light
     both = RawScene(behind, [{"kind": "diffuse"}], [{"kind": "point", "vec": (0, 0, 2)}, {"kind": "directional", "vec": (0, 0, 1)}])
-    assert BatchOracle(both.raw).shadow_batch(0, np.repeat(ray, 3, axis=0)).tolist() == [False] * 3
-    assert BatchOracle(both.raw).shadow_batch(1, np.repeat(ray, 3, axis=0)).tolist() == [True] * 3
+    assert OracleScene(both.raw).shadow_batch(0, np.repeat(ray, 3, axis=0)).tolist() == [False] * 3
+    assert OracleScene(both.raw).shadow_batch(1, np.repeat(ray, 3, axis=0)).tolist() == [True] * 3
 
 
 def test_python_layer_rejects_bad_shapes_and_dtypes_before_any_call():

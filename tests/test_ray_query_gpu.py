@@ -9,8 +9,8 @@ import numpy as np
 import pytest
 
 import rayhs_b200 as rh
+from oracle.orc import OracleScene
 from rayhs_b200 import capi
-from tests.query_oracle import BatchOracle
 from tests.util import SCENES, RawScene, load_scene
 
 pytestmark = pytest.mark.gpu
@@ -41,7 +41,7 @@ BUILT = {"many_objects": many_objects_scene, "spheres_1000": lambda: rh.Scene.sy
 def case(request):
     name = request.param
     sc = BUILT[name]() if name in BUILT else load_scene(name)
-    orc = BatchOracle(sc.raw)
+    orc = OracleScene(sc.raw)
     return name, sc, orc, geometry(sc)
 
 
@@ -249,7 +249,7 @@ def test_more_rays_than_one_launch_and_one_host_chunk():
     import torch
 
     sc = load_scene("dragon_full")
-    orc = BatchOracle(sc.raw)
+    orc = OracleScene(sc.raw)
     g = geometry(sc)
     n = (1 << 24) + 5
     rng = np.random.RandomState(2024)

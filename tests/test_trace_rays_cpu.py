@@ -1,6 +1,6 @@
 """CPU tests of the radiance queries (rh_trace_rays / traceRay): the rh_trace_opts layout of the header against the
 ctypes mirror, loud failure without a device, argument checks of the Python layer, and the batch oracle of the GPU
-tests (tests/trace_oracle.cpp: orc_trace_batch) against hand-derived answers and against the oracle's own render."""
+tests (oracle/batch.cpp: orc_trace_batch) against hand-derived answers and against the oracle's own render."""
 import ctypes as C
 import os
 import subprocess
@@ -10,9 +10,8 @@ import numpy as np
 import pytest
 
 import rayhs_b200 as rh
-from oracle.orc import OracleScene
+from oracle.orc import OracleScene, camera_rays
 from rayhs_b200 import capi
-from tests.trace_oracle import TraceOracle
 from tests.util import SCENES, RawScene, load_scene
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
@@ -70,7 +69,7 @@ RAY = np.array([[1.0, 1, 0, -1, -1, 0]])
 
 
 def trace(raw_scene, rays, max_depth):
-    return TraceOracle(raw_scene.raw).trace_batch(rays, max_depth)
+    return OracleScene(raw_scene.raw).trace_batch(rays, max_depth)
 
 
 def test_trace_batch_diffuse_plane_under_a_point_light():
@@ -124,8 +123,8 @@ def test_trace_batch_equals_the_oracle_render_at_one_sample(name):
     bit for bit: the same traceRay, called per pixel by rayTrace (RayHs.hs:156-166)."""
     sc = load_scene(name)
     ref = OracleScene(sc.raw).render(sc.camera, W, H, sc.max_depth)
-    orc = TraceOracle(sc.raw)
-    col, ids, counts = orc.trace_batch(orc.camera_rays(sc.camera, W, H), sc.max_depth)
+    orc = OracleScene(sc.raw)
+    col, ids, counts = orc.trace_batch(camera_rays(sc.camera, W, H), sc.max_depth)
     assert col.tobytes() == ref["rgb_f64"].reshape(-1, 3).tobytes(), name
     assert np.array_equal(ids, ref["hit_ids"].reshape(-1, 2)), name
     assert [counts[k] for k in ("rays_primary", "rays_reflect", "rays_probe", "rays_exit", "rays_shadow")] == \

@@ -9,9 +9,9 @@ import numpy as np
 import pytest
 
 import rayhs_b200 as rh
+from oracle.orc import COUNT_NAMES, OracleScene, camera_rays
 from rayhs_b200 import capi
 from tests.test_ray_query_gpu import BUILT, CAM_H, CAM_W, MAX_GRAZING, adversarial_rays, geometry, incoherent_rays
-from tests.trace_oracle import COUNT_NAMES, TraceOracle
 from tests.util import ATOL, RTOL, SCENES, assert_parity, load_scene, to_int_c
 
 pytestmark = pytest.mark.gpu
@@ -38,12 +38,12 @@ def close(a, b):
 def case(request):
     name = request.param
     sc = BUILT[name]() if name in BUILT else load_scene(name)
-    return name, sc, TraceOracle(sc.raw), geometry(sc)
+    return name, sc, OracleScene(sc.raw), geometry(sc)
 
 
 def rays_of(name, sc, g):
     rng = np.random.RandomState(zlib.crc32(name.encode()) ^ 0x7ACE)
-    return {"camera": TraceOracle.camera_rays(sc.camera, CAM_W, CAM_H), "incoherent": incoherent_rays(g, rng),
+    return {"camera": camera_rays(sc.camera, CAM_W, CAM_H), "incoherent": incoherent_rays(g, rng),
             "adversarial": adversarial_rays(g, rng)}
 
 
@@ -53,7 +53,7 @@ def test_camera_rays_give_the_renders_bytes_and_hit_ids(name, size):
     sc = load_scene(name)
     w, h = size
     img = rh.render(rh.Rendering(sc, sc.camera, w, h, sc.max_depth), want_hit_ids=True)
-    rays = TraceOracle.camera_rays(sc.camera, w, h)
+    rays = camera_rays(sc.camera, w, h)
     r = trace(sc, rays, sc.max_depth, want_hit_ids=True)
     assert r.colors.shape == (w * h, 3) and r.colors.dtype == np.float64 and r.stats["rays_primary"] == w * h
     assert np.array_equal(r.hit_ids, img.hit_ids.reshape(-1, 2)), name
@@ -168,7 +168,7 @@ def test_queue_growth_retries_and_keeps_the_colours():
     assert r.stats["queue_factor"] > 2, r.stats
     assert r.stats["rays_reflect"] + r.stats["rays_probe"] > 3 * n, r.stats
     idx = np.unique(np.concatenate([np.random.RandomState(4).randint(0, n, 1500), [0, 1, 4095, 4096, n - 1]]))
-    want, want_ids, _ = TraceOracle(sc.raw).trace_batch(rays[idx], 8)
+    want, want_ids, _ = OracleScene(sc.raw).trace_batch(rays[idx], 8)
     assert close(r.colors[idx], want).all(), np.flatnonzero(~close(r.colors[idx], want))[:10]
     assert np.array_equal(r.hit_ids[idx], want_ids)
     assert (want > 0).any()

@@ -9,8 +9,7 @@ import numpy as np
 import pytest
 
 import rayhs_b200 as rh
-from oracle.orc import OracleScene
-from tests.trace_oracle import COUNT_NAMES, TraceOracle
+from oracle.orc import COUNT_NAMES, OracleScene, camera_rays
 from tests.util import ATOL, RTOL, load_scene
 from tests import value_cases as vc
 
@@ -75,7 +74,7 @@ def check(rs, depth, exact, spp=1, offsets=None, seed=None, what=""):
         assert a.stats["negative_channels"] == neg, (tag, "accumulate negative_channels")
         assert_bytes(a.pixels, ref, (tag, "accumulate"))
         if spp == 1 and offsets is None and seed is None:
-            rays = TraceOracle.camera_rays(rs.camera, w, h)
+            rays = camera_rays(rs.camera, w, h)
             r = rh.traceRay(rs, np.ascontiguousarray(rays[:, :3]), np.ascontiguousarray(rays[:, 3:]), depth, want_hit_ids=True, **kw)
             assert_linear(r.colors, ref["rgb_f64"], exact, (tag, "traceRay"))
             assert np.array_equal(r.hit_ids, ref["hit_ids"].reshape(-1, 2)), (tag, "traceRay hit ids")
@@ -137,16 +136,15 @@ def test_far_sample_offsets(dtype):
 def test_non_finite_sample_offsets(dtype):
     """NaN and +-inf offsets make NaN and infinite camera rays: every sample's hit id is the oracle's, except the
     documented departure (the oracle's hit time NaN or +inf), where the wavefront reports a miss."""
-    from tests.query_oracle import BatchOracle
-
     rs = vc.lit_stage(vc.point())
     w, h, spp = rs.width, rs.height, 4
     off = offsets_frame(dtype, [math.nan, math.inf, -math.inf, 0.5])
     off64 = off.astype(np.float64).reshape(h, w, spp, 2)
-    ref = OracleScene(rs.raw).render(rs.camera, w, h, 0, spp=spp, offsets=off64)
-    rays = np.array([np.concatenate(BatchOracle.ray_from_pixel(rs.camera, w, h, x + off64[y, x, k, 0], y + off64[y, x, k, 1]))
+    orc = OracleScene(rs.raw)
+    ref = orc.render(rs.camera, w, h, 0, spp=spp, offsets=off64)
+    rays = np.array([np.concatenate(orc.ray_from_pixel(rs.camera, w, h, x + off64[y, x, k, 0], y + off64[y, x, k, 1]))
                      for y in range(h) for x in range(w) for k in range(spp)])
-    dep = departure(BatchOracle(rs.raw).closest_batch(rays)).reshape(h, w, spp)
+    dep = departure(orc.closest_batch(rays)).reshape(h, w, spp)
     assert dep.any() and not dep.all()
     for kw in VARIANTS:
         ids = rh.render(rh.Rendering(rs, rs.camera, w, h, 0), spp=spp, offsets=off, want_hit_ids=True, **kw).hit_ids.reshape(h, w, spp, 2)
@@ -179,7 +177,7 @@ EDGE = [math.nan, math.inf, -math.inf, 5e-324, 2.0 ** 100, 2.0 ** -100, 1e300, -
 
 
 def edge_rays(sc, n=2000, seed=4):
-    rays = TraceOracle.camera_rays(sc.camera, 40, 30)
+    rays = camera_rays(sc.camera, 40, 30)
     rng = np.random.RandomState(seed)
     rays = rays[rng.randint(0, len(rays), n)].copy()
     pick = rng.randint(0, len(EDGE), size=rays.shape)
@@ -193,12 +191,10 @@ def test_caller_rays_with_extreme_components(which):
     """closestIntersection and traceRay of rays with NaN, +-inf, subnormal, 2^+-100 and 1e300 components against the
     oracle: equal on every ray outside the documented departure, a miss on the rays inside it.  (mesh_nan's NaN vertex
     normals reflect into NaN rays, which are inside it: its radiance is compared without reflections.)"""
-    from tests.query_oracle import BatchOracle
-
     sc = {"cornellBox": lambda: load_scene("cornellBox"), "lambert": lambda: vc.lambert(1, "diffuse", "flat"),
           "mesh_nan": lambda: vc.NORMALS["mesh_nan"][0](*vc.NORMALS["mesh_nan"][1])}[which]()
     rays = edge_rays(sc)
-    want = BatchOracle(sc.raw).closest_batch(rays)
+    want = OracleScene(sc.raw).closest_batch(rays)
     dep = departure(want)
     assert dep.any() and not dep.all()
     hits = rh.closestIntersection(sc, np.ascontiguousarray(rays[:, :3]), np.ascontiguousarray(rays[:, 3:]))
@@ -206,7 +202,7 @@ def test_caller_rays_with_extreme_components(which):
     assert np.array_equal(got[~dep], np.stack([want["object"], want["tri"]], axis=1)[~dep]), which
     assert (got[dep] == -1).all(), which
     keep = rays[~dep]
-    orc = TraceOracle(sc.raw)
+    orc = OracleScene(sc.raw)
     for depth in ((0,) if which == "mesh_nan" else (0, 2)):
         colors, ids, counts = orc.trace_batch(keep, depth)
         for kw in VARIANTS:
@@ -230,7 +226,7 @@ def test_product_order_departure_is_the_documented_one(bounces):
             {"kind": "sphere", "center": (2.0 * bounces, 0, 1), "radius": 0.3, "material": 1}]
     rs = vc.scene(objs, mats, [])
     rays = np.array([[0.0, 0.0, 1.0, 1.0, 0.0, -1.0]])
-    want, _, counts = TraceOracle(rs.raw).trace_batch(rays, bounces)
+    want, _, counts = OracleScene(rs.raw).trace_batch(rays, bounces)
     assert counts["rays_reflect"] == bounces
     assert want[0, 0] == 2.0 ** (108 * bounces - 1000)
     got = rh.traceRay(rs, rays[:, :3], rays[:, 3:], bounces).colors
@@ -254,7 +250,7 @@ def test_black_under_an_overflowed_weight_is_absorbed_by_the_addition(kind, max_
             {"kind": "sphere", "center": (20.0, 0, 1), "radius": 0.3, "material": 1}]
     rs = vc.scene(objs, mats, [vc.point(vec=(19.4, 0, 1), color=(1, 1, 1))])
     rays = np.array([[0.0, 0.0, 1.0, 1.0, 0.0, -1.0]])
-    want, ids, counts = TraceOracle(rs.raw).trace_batch(rays, max_depth)
+    want, ids, counts = OracleScene(rs.raw).trace_batch(rays, max_depth)
     if kind == "plastic" and max_depth == 10:
         assert np.isneginf(want[0, 0]) and np.isposinf(want[0, 1:]).all(), want
     for kw in VARIANTS:
