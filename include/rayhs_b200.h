@@ -53,8 +53,8 @@ enum {
 enum { RH_CMAP_FLAT = 0, RH_CMAP_CHECKER = 1, RH_CMAP_TEXTURE = 2 };
 /* Light.hs:8-10                                                          */
 enum { RH_LIGHT_DIRECTIONAL = 0, RH_LIGHT_POINT = 1 };
-/* Projection.hs:10-15                                                    */
-enum { RH_PROJ_ORTHOGRAPHIC = 0, RH_PROJ_PERSPECTIVE = 1 };
+/* Projection.hs:10-15, and RH_PROJ_THIN_LENS (a perspective camera with a circular thin lens; see rh_camera) */
+enum { RH_PROJ_ORTHOGRAPHIC = 0, RH_PROJ_PERSPECTIVE = 1, RH_PROJ_THIN_LENS = 2 };
 /* sample-offset formats for rh_render (RayHs.hs:173-188)                 */
 enum {
   RH_OFFSETS_NONE = 0,     /* 1 sample at the integer pixel coordinate (generatePixels, Image.hs:34-36) */
@@ -102,16 +102,35 @@ typedef struct rh_texture {
   uint64_t offset;
 } rh_texture;
 
-/* Projection.hs:17-20 + 10-15 */
+/* Projection.hs:17-20 + 10-15.
+ *
+ * RH_PROJ_THIN_LENS: position, target, up and fovy as for RH_PROJ_PERSPECTIVE; proj_width is the lens (aperture)
+ * radius R >= 0 in world units, proj_height the focus distance F > 0 (the plane perpendicular to the view axis at
+ * distance F from position is in focus); near_ is ignored.  R, F and fovy must be finite, else the render returns
+ * RH_ERR_ARG.  The ray of image position (px, py) (the same doubles the pinhole ray is built from, col + ox and
+ * row + oy), all in IEEE double in this order, without fused multiply-add:
+ *   1. vx, vy, f, d = normalize(vx, vy, f), M = lookAt(position, target, up) and p = position, as RH_PROJ_PERSPECTIVE;
+ *   2. R == 0: the perspective ray, bit for bit;
+ *   3. lens sample: mix64(z) = SplitMix64's output function (z ^= z >> 30; z *= 0xBF58476D1CE4E5B9; z ^= z >> 27;
+ *      z *= 0x94D049BB133111EB; z ^= z >> 31, mod 2^64); key = bits(px) ^ mix64(bits(py)) (IEEE-754 bit patterns);
+ *      U(key, k) = value k of the SplitMix64 stream seeded with key, as a double in [0, 1) (RH_OFFSETS_SPLITMIX64's
+ *      generator).  For j = 0 .. 15: a = 2 U(key, 2j) - 1, b = 2 U(key, 2j + 1) - 1; the first pair with
+ *      (a*a) + (b*b) < 1 is taken; if none is, a = b = 0;
+ *   4. in camera space L = (R*a, R*b, 0), s = F / d.z, P = (s*d.x, s*d.y, s*d.z), e = normalize(P - L);
+ *   5. origin = apply(M, L) + p, direction = apply(M, e).
+ * The lens point depends on the image position only, so every entry point that casts rh_render's camera rays casts
+ * the same lens rays.  It is a hash, not stratified, whatever the pixel offsets are; with RH_OFFSETS_NONE a pixel has
+ * one fixed lens point.  The reference's perspective camera never reads proj_width or proj_height, so the layout is
+ * unchanged. */
 typedef struct rh_camera {
   double position[3];
   double target[3];
   double up[3];
   int32_t projection; /* RH_PROJ_* */
   int32_t pad_;
-  double fovy;        /* perspective only                       */
-  double proj_width;  /* parsed but unused by the reference     */
-  double proj_height; /* (Projection.hs:34)                     */
+  double fovy;        /* perspective and thin lens                              */
+  double proj_width;  /* perspective: parsed but unused by the reference        */
+  double proj_height; /* (Projection.hs:34); thin lens: R and F, see above      */
   double near_;
 } rh_camera;
 

@@ -33,6 +33,10 @@ NVCC_FLAGS = [
     "-Xcompiler", "-fPIC,-ffp-contract=off", "-Xptxas", "-v",
 ]
 CXX_FLAGS = ["-std=c++17", "-O2", "-fPIC", "-ffp-contract=off", "-Wall", "-Wno-unused-function"]
+# The oracle's flags: liborc.so and every test library that includes oracle/oracle.cpp (tests/lens_oracle.py) are built
+# with them, so that all of them compare the GPU against one and the same restatement (-ffp-contract=off: no fused
+# multiply-add, as in the reference).
+ORACLE_FLAGS = ["-std=c++17", "-O2", "-ffp-contract=off", "-fPIC", "-shared"]
 
 CUDA_SOURCES = ["kernels.cu", "runtime.cu", "setup_kernels.cu"]
 CXX_SOURCES = ["frontend.cpp", "host_build.cpp", "light_maps.cpp"]
@@ -106,7 +110,7 @@ def build_cli(force: bool = False) -> str:
 
 def build_oracle(force: bool = False) -> str:
     os.makedirs(os.path.dirname(ORACLE_LIB), exist_ok=True)
-    flags = ["-std=c++17", "-O2", "-ffp-contract=off", "-fPIC", "-shared"]
+    flags = ORACLE_FLAGS
     deps = [ORACLE_LIB_SRC, ORACLE_SRC, HEADERS[-1]]
     if force or _stale(ORACLE_LIB, deps, flags):
         _run([CXX, *flags, ORACLE_LIB_SRC, "-o", ORACLE_LIB, "-lpthread"])

@@ -151,8 +151,9 @@ struct CameraParams {
   double m[9];  // lookAt matrix rows (Mat.hs:83-93)
   double pos[3];
   double w, h, half_w, half_h, apw, aph, f;
-  int32_t projection;
+  int32_t projection;  // RH_PROJ_*; a thin lens of radius 0 is RH_PROJ_PERSPECTIVE here
   int32_t pad_;
+  double lens_r, focus;  // RH_PROJ_THIN_LENS: aperture radius R and focus distance F
 };
 
 // Per-chunk control block in device memory (zeroed before each chunk).

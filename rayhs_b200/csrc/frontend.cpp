@@ -459,6 +459,11 @@ void parse_camera(const JValue& o, rh_camera& c) {  // JSON.hs:99-105, 74-84
     c.proj_width = num(p, "width");
     c.proj_height = num(p, "height");
     c.near_ = num(p, "near");
+  } else if (kind == "thinLens") {  // no JSON tag in the reference: depth of field (rh_camera, RH_PROJ_THIN_LENS)
+    c.projection = RH_PROJ_THIN_LENS;
+    c.fovy = num(p, "fovy");
+    c.proj_width = num(p, "aperture");
+    c.proj_height = num(p, "focusDistance");
   } else bad("Unknown type for projection " + kind);
 }
 

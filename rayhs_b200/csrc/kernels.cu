@@ -1089,25 +1089,6 @@ __device__ __forceinline__ uint32_t global_row(const ChunkParams& P, uint32_t lo
   return (lb * P.shard_count + P.shard_index) * P.band_height + rib;
 }
 
-// Projection.hs:22-39 rayFromPixel with the per-frame constants hoisted into CameraParams.
-__device__ __forceinline__ Ray camera_ray(const CameraParams& cam, double px, double py) {
-  const double vx = cam.apw * (px - cam.half_w) / cam.w;
-  const double vy = cam.aph * ((-py) + cam.half_h) / cam.h;
-  V3 o, d;
-  if (cam.projection == RH_PROJ_ORTHOGRAPHIC) {
-    o = mk(vx, vy, 0);
-    d = mk(0, 0, 1);
-  } else {
-    d = normalize(mk(vx, vy, cam.f));
-    o = mk(0, 0, 0);
-  }
-  Ray r;
-  r.o = o + ld3(cam.pos);
-  r.d = mk(cam.m[0] * d.x + cam.m[1] * d.y + cam.m[2] * d.z, cam.m[3] * d.x + cam.m[4] * d.y + cam.m[5] * d.z,
-           cam.m[6] * d.x + cam.m[7] * d.y + cam.m[8] * d.z);  // Mat.hs:40-44
-  return r;
-}
-
 // Value k (0-based) of the SplitMix64 stream seeded with `seed`, as a double in [0, 1): the generator's state after
 // k + 1 steps is seed + (k + 1) * gamma, so any value can be produced on its own (csrc/frontend.cpp SplitMix64).
 __device__ __forceinline__ double splitmix01(unsigned long long seed, unsigned long long k) {
@@ -1116,6 +1097,61 @@ __device__ __forceinline__ double splitmix01(unsigned long long seed, unsigned l
   z = (z ^ (z >> 27)) * 0x94D049BB133111EBull;
   z = z ^ (z >> 31);
   return (double)(z >> 11) * (1.0 / 9007199254740992.0);
+}
+
+// Mat.hs:40-44 with the row-major matrix of CameraParams
+__device__ __forceinline__ V3 apply(const double* m, V3 v) {
+  return mk(m[0] * v.x + m[1] * v.y + m[2] * v.z, m[3] * v.x + m[4] * v.y + m[5] * v.z, m[6] * v.x + m[7] * v.y + m[8] * v.z);
+}
+
+// RH_PROJ_THIN_LENS (include/rayhs_b200.h, rh_camera): the ray of image position (px, py) whose perspective direction
+// in camera space is d, with the camera read from `c` (the kernel parameter, or the views' table in global memory).
+// The lens point is drawn from a hash of (px, py) by rejection from the square, at most 16 attempts.  Not inlined, and
+// handed a pointer rather than the caller's copy: the pinhole path of trace_kernel, which runs at its register cap,
+// keeps its own code, registers and stack frame, and pays one uniform branch (DESIGN.md, "Thin-lens cameras").
+__device__ __noinline__ Ray lens_ray(const CameraParams* c, double px, double py, V3 d) {
+  const CameraParams& cam = *c;
+  unsigned long long z = (unsigned long long)__double_as_longlong(py);  // mix64, SplitMix64's output function
+  z = (z ^ (z >> 30)) * 0xBF58476D1CE4E5B9ull;
+  z = (z ^ (z >> 27)) * 0x94D049BB133111EBull;
+  z = z ^ (z >> 31);
+  const unsigned long long key = (unsigned long long)__double_as_longlong(px) ^ z;
+  double a = 0, b = 0;
+  for (unsigned j = 0; j < 16; j++) {
+    const double x = 2 * splitmix01(key, 2 * j) - 1, y = 2 * splitmix01(key, 2 * j + 1) - 1;  // (both exact)
+    if ((x * x) + (y * y) < 1) {
+      a = x;
+      b = y;
+      break;
+    }
+  }
+  const V3 L = mk(cam.lens_r * a, cam.lens_r * b, 0);
+  const double s = cam.focus / d.z;
+  const V3 e = normalize(mk(s * d.x, s * d.y, s * d.z) - L);
+  Ray r;
+  r.o = apply(cam.m, L) + ld3(cam.pos);
+  r.d = apply(cam.m, e);
+  return r;
+}
+
+// Projection.hs:22-39 rayFromPixel with the per-frame constants hoisted into CameraParams, and the thin lens (`src`:
+// where cam lives, for lens_ray).
+__device__ __forceinline__ Ray camera_ray(const CameraParams& cam, const CameraParams* src, double px, double py) {
+  const double vx = cam.apw * (px - cam.half_w) / cam.w;
+  const double vy = cam.aph * ((-py) + cam.half_h) / cam.h;
+  V3 o, d;
+  if (cam.projection == RH_PROJ_ORTHOGRAPHIC) {
+    o = mk(vx, vy, 0);
+    d = mk(0, 0, 1);
+  } else {
+    d = normalize(mk(vx, vy, cam.f));
+    if (cam.projection == RH_PROJ_THIN_LENS) return lens_ray(src, px, py, d);
+    o = mk(0, 0, 0);
+  }
+  Ray r;
+  r.o = o + ld3(cam.pos);
+  r.d = apply(cam.m, d);
+  return r;
 }
 
 // ------------------------------------------------------------------ accumDiffuse (RayHs.hs:89-97): the light fold
@@ -1439,7 +1475,8 @@ __device__ __forceinline__ uint32_t list_image_row(const PixelList& L, uint32_t 
   return (lb * L.shard_count + L.shard_index) * L.band_height + rib;
 }
 
-// rh_render_views: view v's camera, through the read-only path (the items of a warp almost always share a view)
+// rh_render_views: view v's camera, through the read-only path (the items of a warp almost always share a view); the
+// pinhole fields only (lens_ray reads a lens from the table)
 __device__ __forceinline__ CameraParams view_camera(const ChunkParams& P, uint32_t v) {
   const CameraParams* src = P.cams + v;
   CameraParams c;
@@ -1481,7 +1518,7 @@ __device__ __forceinline__ bool load_item(const ChunkParams& P, const CameraPara
     const unsigned long long g = ((unsigned long long)grow * L.width + col) * P.stream_spp + __ldg(L.counts + p) + s;
     const double ox = splitmix01(P.offset_seed, 2 * g) - 0.5;
     const double oy = splitmix01(P.offset_seed, 2 * g + 1) - 0.5;
-    r = camera_ray(cam, (double)col + ox, (double)grow + oy);
+    r = camera_ray(cam, &cam, (double)col + ox, (double)grow + oy);
     return true;
   }
   if (SRC == Source::kViews && primary) {
@@ -1516,7 +1553,7 @@ __device__ __forceinline__ bool load_item(const ChunkParams& P, const CameraPara
         oy = o2.y;
       }
     }
-    r = camera_ray(view_camera(P, v), (double)col + ox, (double)grow + oy);
+    r = camera_ray(view_camera(P, v), P.cams + v, (double)col + ox, (double)grow + oy);
     return true;
   }
   if (primary) {
@@ -1542,7 +1579,7 @@ __device__ __forceinline__ bool load_item(const ChunkParams& P, const CameraPara
         oy = o2.y;
       }
     }
-    r = camera_ray(cam, (double)col + ox, (double)grow + oy);
+    r = camera_ray(cam, &cam, (double)col + ox, (double)grow + oy);
     return true;
   }
   const size_t cap = P.q_in.capacity;

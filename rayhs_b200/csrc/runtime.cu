@@ -1583,8 +1583,22 @@ CameraParams make_camera(const rh_camera& c, int width, int height) {
   if (aspect > 1) { p.apw = w; p.aph = w / aspect; }
   else { p.apw = aspect * h; p.aph = h; }
   p.f = 0.5 * h / (std::tan(0.5) * c.fovy);  // Projection.hs:35 — `tan 0.5 * fovy` (SURVEY App. A-C1)
-  p.projection = c.projection;
+  // a lens of radius 0 casts the perspective rays bit for bit (rh_camera), so the kernels take the pinhole path for it
+  p.projection = (c.projection == RH_PROJ_THIN_LENS && c.proj_width == 0) ? RH_PROJ_PERSPECTIVE : c.projection;
+  if (p.projection == RH_PROJ_THIN_LENS) {
+    p.lens_r = c.proj_width;
+    p.focus = c.proj_height;
+  }
   return p;
+}
+
+// RH_PROJ_THIN_LENS's argument checks: "" when the camera is not a lens or its R, F and fovy are valid, else what is wrong
+std::string lens_error(const rh_camera& c) {
+  if (c.projection != RH_PROJ_THIN_LENS) return "";
+  if (!std::isfinite(c.proj_width) || !(c.proj_width >= 0)) return "thin-lens aperture radius proj_width must be finite and >= 0";
+  if (!std::isfinite(c.proj_height) || !(c.proj_height > 0)) return "thin-lens focus distance proj_height must be finite and > 0";
+  if (!std::isfinite(c.fovy) || !(c.fovy > 0)) return "thin-lens fovy must be finite and > 0";
+  return "";
 }
 
 // ------------------------------------------------------------------ render
@@ -1657,8 +1671,10 @@ int render_frame(Device* D, const rh_scene* scene, const rh_camera* camera, cons
   const int W = o->width, H = o->height, spp = o->spp;
   if (W <= 0 || H <= 0 || spp <= 0 || o->max_depth < 0 || o->max_depth > kMaxDepth)
     return rh::set_error(RH_ERR_ARG, w + ": bad width/height/spp/max_depth");
-  if (camera->projection != RH_PROJ_ORTHOGRAPHIC && camera->projection != RH_PROJ_PERSPECTIVE)
+  if (camera->projection != RH_PROJ_ORTHOGRAPHIC && camera->projection != RH_PROJ_PERSPECTIVE && camera->projection != RH_PROJ_THIN_LENS)
     return rh::set_error(RH_ERR_ARG, w + ": unknown projection");
+  const std::string lens = lens_error(*camera);
+  if (!lens.empty()) return rh::set_error(RH_ERR_ARG, w + ": " + lens);
   const int G = o->shard_count <= 0 ? 1 : o->shard_count;
   if (o->shard_index < 0 || o->shard_index >= G) return rh::set_error(RH_ERR_ARG, w + ": shard_index out of range");
   const int bh = o->band_height > 0 ? o->band_height : rh_default_band_height(H, G);
@@ -2965,8 +2981,10 @@ int views_on(Device* D, const rh_scene* scene, const rh_views* vw, const rh_rend
   const uint32_t V = vw->n_views;
   for (uint32_t v = 0; v < V; v++) {
     const int32_t proj = vw->cameras[v].projection;
-    if (proj != RH_PROJ_ORTHOGRAPHIC && proj != RH_PROJ_PERSPECTIVE)
+    if (proj != RH_PROJ_ORTHOGRAPHIC && proj != RH_PROJ_PERSPECTIVE && proj != RH_PROJ_THIN_LENS)
       return rh::set_error(RH_ERR_ARG, w + ": cameras[" + std::to_string(v) + "] has an unknown projection");
+    const std::string lens = lens_error(vw->cameras[v]);
+    if (!lens.empty()) return rh::set_error(RH_ERR_ARG, w + ": cameras[" + std::to_string(v) + "]: " + lens);
   }
   Frame f;
   f.views = true;

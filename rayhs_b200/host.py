@@ -224,6 +224,17 @@ def renderingFromScene(sc: Scene, width: int | None = None, height: int | None =
     return Rendering(sc, sc.camera, width or sc.width, height or sc.height, sc.max_depth if maxDepth is None else maxDepth)
 
 
+def thinLens(camera: capi.rh_camera, aperture: float, focus_distance: float) -> capi.rh_camera:
+    """A copy of `camera` as a thin-lens camera (RH_PROJ_THIN_LENS: depth of field): the same position, target, up and
+    fovy, a circular lens of radius `aperture` (world units; 0 casts the perspective rays) and the plane at
+    `focus_distance` along the view axis in focus.  Every render entry point takes it; see rh_camera in
+    include/rayhs_b200.h for the rays."""
+    c = capi.rh_camera.from_buffer_copy(camera)
+    c.projection = capi.RH_PROJ_THIN_LENS
+    c.proj_width, c.proj_height = float(aperture), float(focus_distance)
+    return c
+
+
 @dataclass
 class Image:
     """Image.hs:21-23, already quantised by toIntC (Image.hs:54-55): uint8 [height, width, 3].  `linear` (progressive
