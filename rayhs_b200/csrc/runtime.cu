@@ -1592,8 +1592,11 @@ CameraParams make_camera(const rh_camera& c, int width, int height) {
   return p;
 }
 
-// RH_PROJ_THIN_LENS's argument checks: "" when the camera is not a lens or its R, F and fovy are valid, else what is wrong
-std::string lens_error(const rh_camera& c) {
+// A camera's argument checks: "" when its projection is known and, for RH_PROJ_THIN_LENS, its R, F and fovy are valid,
+// else what is wrong
+std::string camera_error(const rh_camera& c) {
+  if (c.projection != RH_PROJ_ORTHOGRAPHIC && c.projection != RH_PROJ_PERSPECTIVE && c.projection != RH_PROJ_THIN_LENS)
+    return "unknown projection";
   if (c.projection != RH_PROJ_THIN_LENS) return "";
   if (!std::isfinite(c.proj_width) || !(c.proj_width >= 0)) return "thin-lens aperture radius proj_width must be finite and >= 0";
   if (!std::isfinite(c.proj_height) || !(c.proj_height > 0)) return "thin-lens focus distance proj_height must be finite and > 0";
@@ -1631,8 +1634,6 @@ struct Frame {
   AccumParams acc{};
   double* linear = nullptr;
   size_t linear_bytes = 0;
-  // rh_render_features: render_frame's checks and geometry only (features_on runs the frame, not run_frame); no RGB8 sink
-  bool features = false;
   // rh_render_light_groups: the shadow kernels also add each group's terms, and a sink beside the resolve writes the
   // group images to group_out (device, or host through a chunk of scratch); RGB8 is optional
   uint32_t n_groups = 0;
@@ -1649,20 +1650,19 @@ struct Frame {
   // the seeds and host per-pixel offsets)
   struct Upload { void* dst; const void* src; size_t bytes; };
   std::vector<Upload> uploads;
-  const char* overflow_error = "rh_render: ray queue overflow; lower chunk_samples";
+  const char* who = "rh_render";  // the entry point, in run_frame's messages
   // renders (not traces, list frames, light-group or views frames) tune the scene's shadow schedule and record its queue
   // factor and row costs
   bool learns() const { return !trace && !pixel_list && !n_groups && !views; }
 };
 
-// rh_render's argument checks (`who` names the entry point in the messages).  With f->accumulate, f->pixel_list,
-// f->features, f->n_groups or f->views set, rgb_out may be null.
+// rh_render's argument checks (`who` names the entry point in the messages).  rgb_out may be null: each entry point
+// decides which of its outputs it needs.
 int render_frame(Device* D, const rh_scene* scene, const rh_camera* camera, const rh_render_opts* o, uint8_t* rgb_out,
                  int32_t* hit_ids_out, Frame* f, const char* who = "rh_render") {
   const std::string w(who);
-  const bool peer_frames = o && (o->flags & RH_FLAG_PEER_FRAMES) != 0;
-  if (!scene || !camera || !o || (!rgb_out && !peer_frames && !f->accumulate && !f->pixel_list && !f->features && !f->n_groups && !f->views))
-    return rh::set_error(RH_ERR_ARG, w + ": null argument");
+  if (!scene || !camera || !o) return rh::set_error(RH_ERR_ARG, w + ": null argument");
+  const bool peer_frames = (o->flags & RH_FLAG_PEER_FRAMES) != 0;
   if (peer_frames && (!o->peer_frames || o->n_peer_frames <= 0 || o->n_peer_frames > kMaxPeers))
     return rh::set_error(RH_ERR_ARG, w + ": RH_FLAG_PEER_FRAMES needs 1..16 peer frame pointers");
   if (peer_frames && (o->flags & RH_FLAG_HIT_IDS))
@@ -1671,10 +1671,8 @@ int render_frame(Device* D, const rh_scene* scene, const rh_camera* camera, cons
   const int W = o->width, H = o->height, spp = o->spp;
   if (W <= 0 || H <= 0 || spp <= 0 || o->max_depth < 0 || o->max_depth > kMaxDepth)
     return rh::set_error(RH_ERR_ARG, w + ": bad width/height/spp/max_depth");
-  if (camera->projection != RH_PROJ_ORTHOGRAPHIC && camera->projection != RH_PROJ_PERSPECTIVE && camera->projection != RH_PROJ_THIN_LENS)
-    return rh::set_error(RH_ERR_ARG, w + ": unknown projection");
-  const std::string lens = lens_error(*camera);
-  if (!lens.empty()) return rh::set_error(RH_ERR_ARG, w + ": " + lens);
+  const std::string cam_err = camera_error(*camera);
+  if (!cam_err.empty()) return rh::set_error(RH_ERR_ARG, w + ": " + cam_err);
   const int G = o->shard_count <= 0 ? 1 : o->shard_count;
   if (o->shard_index < 0 || o->shard_index >= G) return rh::set_error(RH_ERR_ARG, w + ": shard_index out of range");
   const int bh = o->band_height > 0 ? o->band_height : rh_default_band_height(H, G);
@@ -1686,6 +1684,7 @@ int render_frame(Device* D, const rh_scene* scene, const rh_camera* camera, cons
   if ((o->flags & RH_FLAG_HIT_IDS) && !hit_ids_out) return rh::set_error(RH_ERR_ARG, w + ": RH_FLAG_HIT_IDS without hit_ids_out");
   if (mode == RH_OFFSETS_SPLITMIX64 && (o->flags & RH_FLAG_DEVICE_OFFSETS))
     return rh::set_error(RH_ERR_ARG, w + ": RH_OFFSETS_SPLITMIX64 takes a host pointer to the seed");
+  f->who = who;
   f->o = *o;
   f->o.shard_count = G;
   f->o.band_height = bh;
@@ -1760,6 +1759,33 @@ int upload_offset_rows(const Frame& f, size_t row_samples, int first_row, int n_
   return RH_OK;
 }
 
+// The chunk parameters that follow from the frame alone and are the same for every chunk of it, whichever kernels
+// (run_frame's or rh_render_features's) take them.
+ChunkParams frame_chunk_params(const Frame& f) {
+  const rh_render_opts& o = f.o;
+  ChunkParams P{};
+  P.spp = o.spp;
+  P.width = o.width;
+  P.height = o.height;
+  P.shard_index = o.shard_index;
+  P.shard_count = o.shard_count;
+  P.band_height = o.band_height;
+  P.offset_mode = o.offset_mode;
+  P.offset_tile = o.offset_tile;
+  if (o.offset_mode == RH_OFFSETS_SPLITMIX64) memcpy(&P.offset_seed, o.offsets, sizeof P.offset_seed);
+  P.stream_spp = f.stream_spp;
+  P.stream_base = f.stream_base;
+  if (o.flags & RH_FLAG_PEER_FRAMES) {
+    P.n_peers = (uint32_t)o.n_peer_frames;
+    for (int g = 0; g < o.n_peer_frames; g++) P.peer[g] = (uint8_t*)o.peer_frames[g];
+  }
+  P.list = f.list;
+  P.cams = f.cams;
+  P.view_seeds = f.view_seeds;
+  P.view_rows = f.view_rows;
+  return P;
+}
+
 // One frame on one device: its plan and buffers, and what the enqueued chunks recorded.
 struct FrameRun {
   Device* D;
@@ -1779,7 +1805,6 @@ struct FrameRun {
   size_t group_out_stride = 0;
   const void* d_offsets = nullptr;
   int off_index = kOffIndexLocal;
-  unsigned long long offset_seed = 0;
   int ring = 2;                  // slots of the offset upload ring
   size_t cap = 0, walk_cap = 0;  // queue capacities in entries
   // recorded by the enqueue, per attempt
@@ -1836,34 +1861,19 @@ struct FrameRun {
     Device::Scratch& sc = D->lane[ln];
     const cudaStream_t lane_stream = ln ? D->stream2 : D->stream;
     double* group_out = group_out_dev ? f.group_out : (double*)sc.group_out.p;
-    ChunkParams P{};
+    ChunkParams P = frame_chunk_params(f);
     P.first_row = first_row;
     P.n_rows = n_rows;
     P.n_samples = (uint32_t)((size_t)n_rows * row_samples);
-    P.spp = o.spp;
-    P.width = o.width;
-    P.height = o.height;
-    P.shard_index = o.shard_index;
-    P.shard_count = o.shard_count;
-    P.band_height = o.band_height;
     P.max_depth = o.max_depth;
     P.exact_boxes = (o.flags & RH_FLAG_EXACT_BOXES) ? 1 : 0;
     P.no_light_maps = (o.flags & RH_FLAG_NO_LIGHT_MAPS) ? 1 : 0;
-    P.offset_mode = o.offset_mode;
     P.offset_index = off_index;
-    P.offset_tile = o.offset_tile;
     P.offsets = d_offsets;
-    P.offset_seed = offset_seed;
-    P.stream_spp = f.stream_spp;
-    P.stream_base = f.stream_base;
     P.accum = (double*)sc.accum.p;
     P.accum_stride = (uint32_t)chunk_samples;
     P.hit_ids = d_ids;
     P.rgb = d_rgb;
-    if (o.flags & RH_FLAG_PEER_FRAMES) {
-      P.n_peers = (uint32_t)o.n_peer_frames;
-      for (int g = 0; g < o.n_peer_frames; g++) P.peer[g] = (uint8_t*)o.peer_frames[g];
-    }
     P.ctl = (ChunkCtl*)D->ctl.p + ck;
     P.counters = (FrameCounters*)D->counters.p;
     P.q_hits.plane = (double2*)sc.hitq.p;
@@ -1899,10 +1909,6 @@ struct FrameRun {
       P.offsets = (const char*)d_offsets + (size_t)first_row * row_samples * f.off_elem;
     P.offset_base = (P.offset_index == kOffIndexLocal) ? 0ull : (unsigned long long)first_row * row_samples;
     if (f.trace || f.pixel_list) P.ray_items = (uint32_t)std::min<uint64_t>(P.n_samples, f.n_rays - (uint64_t)first_row * row_samples);
-    P.list = f.list;
-    P.cams = f.cams;
-    P.view_seeds = f.view_seeds;
-    P.view_rows = f.view_rows;
     for (int plane = 0; plane < 3; plane++)  // (three 1-D memsets: a 2-D one is limited to 2 GB of pitch)
       RH_CUDA(cudaMemsetAsync((double*)sc.accum.p + (size_t)plane * chunk_samples, 0, (size_t)P.n_samples * sizeof(double), lane_stream));
     if (f.n_groups) {
@@ -2152,6 +2158,18 @@ void FrameRun::learn() const {
   }
 }
 
+// Sets *d to where the kernels write an output: nowhere when the caller asked for none (user null), the caller's buffer
+// when it is device memory, else `scratch`, which the caller copies back to `user` after the kernels.
+template <class T>
+int stage_output(DevBuf& scratch, T* user, size_t bytes, bool dev_out, T** d) {
+  *d = user;
+  if (!user || dev_out) return RH_OK;
+  const int rc = scratch.reserve(bytes);
+  if (rc) return rc;
+  *d = (T*)scratch.p;
+  return RH_OK;
+}
+
 // Runs a validated frame: chunk plan, scratch, the chunks' launches, and — when a chunk's queues overflowed — the whole
 // frame again with twice the queue capacity.
 int run_frame(Device* D, const rh_scene* scene, const Frame& f, rh_stats* stats) {
@@ -2180,25 +2198,14 @@ int run_frame(Device* D, const rh_scene* scene, const Frame& f, rh_stats* stats)
                            rh::kBytesPerSample + group_bytes * (dev_out ? 1 : 2));
   R.n_chunks = (int)R.plan.rows.size();
   R.chunk_samples = (size_t)*std::max_element(R.plan.rows.begin(), R.plan.rows.end()) * R.row_samples;
-  if (R.chunk_samples > 0x7fffffffu) return rh::set_error(RH_ERR_ARG, "rh_render: chunk too large");
+  const std::string w(f.who);
+  if (R.chunk_samples > 0x7fffffffu) return rh::set_error(RH_ERR_ARG, w + ": chunk too large");
 
   int rc;
-  if (peer_frames || !f.out) R.d_rgb = nullptr;
-  else if (dev_out) R.d_rgb = f.out;
-  else {
-    if ((rc = D->rgb.reserve(f.out_bytes))) return rc;
-    R.d_rgb = (uint8_t*)D->rgb.p;
-  }
-  if (want_ids && dev_out) R.d_ids = (int2*)f.ids_out;
-  else if (want_ids) {
-    if ((rc = D->ids.reserve(f.ids_bytes))) return rc;
-    R.d_ids = (int2*)D->ids.p;
-  }
-  if (f.linear && dev_out) R.d_linear = f.linear;
-  else if (f.linear) {
-    if ((rc = D->linear.reserve(f.linear_bytes))) return rc;
-    R.d_linear = (double*)D->linear.p;
-  }
+  if ((rc = stage_output(D->rgb, peer_frames ? nullptr : f.out, f.out_bytes, dev_out, &R.d_rgb)) ||
+      (rc = stage_output(D->ids, want_ids ? (int2*)f.ids_out : nullptr, f.ids_bytes, dev_out, &R.d_ids)) ||
+      (rc = stage_output(D->linear, f.linear, f.linear_bytes, dev_out, &R.d_linear)))
+    return rc;
   // Two chunks in flight (two streams, two sets of queues) when the frame has several: the kernels are persistent and
   // fill the GPU, so a chunk's next kernel starts on the SMs the other chunk's kernel frees as its warps run out of
   // work — the tail of every launch is filled instead of idle.  One lane when every launch is timed on its own.
@@ -2239,9 +2246,7 @@ int run_frame(Device* D, const rh_scene* scene, const Frame& f, rh_stats* stats)
       if ((rc = D->offsets.reserve(tile_bytes))) return rc;
       R.d_offsets = D->offsets.p;
     }
-  } else if (mode == RH_OFFSETS_SPLITMIX64) {
-    memcpy(&R.offset_seed, o.offsets, sizeof R.offset_seed);
-  } else if (mode != RH_OFFSETS_NONE && dev_off) {
+  } else if (mode != RH_OFFSETS_NONE && dev_off) {  // (RH_OFFSETS_SPLITMIX64 takes a host seed: frame_chunk_params's)
     R.d_offsets = o.offsets;
     R.off_index = (o.flags & RH_FLAG_SHARD_OFFSETS) ? kOffIndexLocal : kOffIndexGlobal;  // (compact: each chunk's slice is in work-item order)
   } else if (R.host_offsets) {
@@ -2311,7 +2316,8 @@ int run_frame(Device* D, const rh_scene* scene, const Frame& f, rh_stats* stats)
     bool overflow = false;
     for (int ck = 0; ck < R.n_chunks; ck++) overflow |= R.ctl()[ck].overflow != 0;
     if (overflow) {
-      if (R.cap >= 0x7fffff00u || factor >= (1u << 16)) return rh::set_error(RH_ERR_OVERFLOW, f.overflow_error);
+      if (R.cap >= 0x7fffff00u || factor >= (1u << 16))
+        return rh::set_error(RH_ERR_OVERFLOW, w + ": ray queue overflow; lower " + (f.trace ? "chunk_rays" : "chunk_samples"));
       factor *= 2;
       if (f.learns()) scene->queue_factor = factor;
       if (f.views) scene->views_queue_factor = factor;
@@ -2326,18 +2332,34 @@ int run_frame(Device* D, const rh_scene* scene, const Frame& f, rh_stats* stats)
 
 int render_on(Device* D, const rh_scene* scene, const rh_camera* camera, const rh_render_opts* o, uint8_t* rgb_out,
               int32_t* hit_ids_out, rh_stats* stats) {
+  // (rh_multi_render's shards store into the peer frames instead)
+  if (!rgb_out && !(o && (o->flags & RH_FLAG_PEER_FRAMES))) return rh::set_error(RH_ERR_ARG, "rh_render: null argument");
   Frame f;
   const int rc = render_frame(D, scene, camera, o, rgb_out, hit_ids_out, &f);
   return rc ? rc : run_frame(D, scene, f, stats);
 }
 
-// Returns RH_OK when every non-null pointer is device (or managed) memory, else the argument error `msg`.
-int check_device_pointers(std::initializer_list<const void*> ptrs, const std::string& msg) {
-  for (const void* p : ptrs) {
-    if (!p) continue;
-    cudaPointerAttributes a{};
-    RH_CUDA(cudaPointerGetAttributes(&a, p));
-    if (a.type != cudaMemoryTypeDevice && a.type != cudaMemoryTypeManaged) return rh::set_error(RH_ERR_ARG, msg);
+// A buffer an entry point takes with RH_FLAG_DEVICE_OUT: null when the call does not use it, and the alignment of the
+// words its kernels move (1: none).
+struct DeviceArg {
+  const void* p;
+  size_t align;
+  const char* name;
+};
+
+// RH_FLAG_DEVICE_OUT's checks: every listed buffer aligned, then device (or managed) memory of D's GPU, which this
+// makes the current one.
+int check_device_outputs(Device* D, const std::string& who, std::initializer_list<DeviceArg> args) {
+  for (const DeviceArg& a : args)
+    if ((uintptr_t)a.p % a.align)
+      return rh::set_error(RH_ERR_ARG, who + ": device " + a.name + " must be " + std::to_string(a.align) + "-byte aligned");
+  RH_CUDA(cudaSetDevice(D->dev));
+  for (const DeviceArg& a : args) {
+    if (!a.p) continue;
+    cudaPointerAttributes attr{};
+    RH_CUDA(cudaPointerGetAttributes(&attr, a.p));
+    if (attr.type != cudaMemoryTypeDevice && attr.type != cudaMemoryTypeManaged)
+      return rh::set_error(RH_ERR_ARG, who + ": RH_FLAG_DEVICE_OUT with a pointer that is not device memory");
   }
   return RH_OK;
 }
@@ -2385,6 +2407,14 @@ void shard_state_fix_view(ShardState* S, const rh_scene* scene, const rh_camera*
   S->max_depth = max_depth;
 }
 
+// RH_OFFSETS_SPLITMIX64's window check: "" when samples [base, base + spp) lie inside a stream of stream_spp samples per
+// pixel, else what is wrong
+std::string stream_window_error(uint32_t base, uint32_t spp, uint32_t stream_spp) {
+  if ((uint64_t)base + spp <= stream_spp) return "";
+  return "RH_OFFSETS_SPLITMIX64 past the end of the stream (" + std::to_string(base) + " + spp " + std::to_string(spp) +
+         " > stream_spp " + std::to_string(stream_spp) + ")";
+}
+
 // ------------------------------------------------------------------ progressive accumulation
 // rh_render_accumulate's argument checks: rh_render's (render_frame), then those of the accumulator.
 int accumulate_frame(Device* D, const rh_scene* scene, const rh_camera* camera, const rh_render_opts* o, rh_accum* acc,
@@ -2403,19 +2433,14 @@ int accumulate_frame(Device* D, const rh_scene* scene, const rh_camera* camera, 
   if (o->offset_mode == RH_OFFSETS_SPLITMIX64) {
     if (acc->stream_spp == 0)
       return rh::set_error(RH_ERR_ARG, w + ": RH_OFFSETS_SPLITMIX64 needs an accumulator created with stream_spp > 0");
-    if ((uint64_t)acc->n + spp > acc->stream_spp)
-      return rh::set_error(RH_ERR_ARG, w + ": RH_OFFSETS_SPLITMIX64 past the end of the stream (" + std::to_string(acc->n) + " + " +
-                                           std::to_string(spp) + " > stream_spp " + std::to_string(acc->stream_spp) + ")");
+    const std::string window = stream_window_error(acc->n, spp, acc->stream_spp);
+    if (!window.empty()) return rh::set_error(RH_ERR_ARG, w + ": " + window);
   }
   if ((rc = shard_state_matches(acc, *f, acc->n > 0, scene, camera, w, "accumulator", "rh_accum_reset"))) return rc;
   const bool want_ids = (o->flags & RH_FLAG_HIT_IDS) != 0;
-  if (o->flags & RH_FLAG_DEVICE_OUT) {
-    if ((uintptr_t)linear_out % 8) return rh::set_error(RH_ERR_ARG, w + ": device linear_out must be 8-byte aligned");
-    RH_CUDA(cudaSetDevice(D->dev));
-    if ((rc = check_device_pointers({rgb_out, linear_out, want_ids ? hit_ids_out : nullptr},
-                                    w + ": RH_FLAG_DEVICE_OUT with a pointer that is not device memory")))
-      return rc;
-  }
+  if ((o->flags & RH_FLAG_DEVICE_OUT) &&
+      (rc = check_device_outputs(D, w, {{rgb_out, 1, "rgb_out"}, {linear_out, 8, "linear_out"}, {want_ids ? hit_ids_out : nullptr, 1, "hit_ids_out"}})))
+    return rc;
   const size_t half = 3 * acc->plane;
   f->stream_spp = acc->stream_spp;
   f->stream_base = acc->n;
@@ -2426,7 +2451,6 @@ int accumulate_frame(Device* D, const rh_scene* scene, const rh_camera* camera, 
   f->acc.n_total = acc->n + spp;
   f->linear = linear_out;
   f->linear_bytes = (size_t)f->rows_local * f->o.width * 3 * sizeof(double);
-  f->overflow_error = "rh_render_accumulate: ray queue overflow; lower chunk_samples";
   return RH_OK;
 }
 
@@ -2477,12 +2501,8 @@ int adaptive_frame(Device* D, const rh_scene* scene, const rh_camera* camera, co
   f->pixel_list = true;
   if ((rc = render_frame(D, scene, camera, o, rgb_out, nullptr, f, "rh_render_adaptive"))) return rc;
   if ((rc = shard_state_matches(ad, *f, ad->fixed, scene, camera, w, "adaptive state", "rh_adaptive_reset"))) return rc;
-  if (o->flags & RH_FLAG_DEVICE_OUT) {
-    if ((uintptr_t)linear_out % 8) return rh::set_error(RH_ERR_ARG, w + ": device linear_out must be 8-byte aligned");
-    RH_CUDA(cudaSetDevice(D->dev));
-    if ((rc = check_device_pointers({rgb_out, linear_out}, w + ": RH_FLAG_DEVICE_OUT with a pointer that is not device memory")))
-      return rc;
-  }
+  if ((o->flags & RH_FLAG_DEVICE_OUT) && (rc = check_device_outputs(D, w, {{rgb_out, 1, "rgb_out"}, {linear_out, 8, "linear_out"}})))
+    return rc;
   f->ad = ad->A;
   f->ad.spp = (uint32_t)o->spp;
   f->ad.min_spp = ao->min_spp;
@@ -2490,7 +2510,6 @@ int adaptive_frame(Device* D, const rh_scene* scene, const rh_camera* camera, co
   f->stream_spp = ad->stream_spp;
   f->list = {f->ad.list, f->ad.counts, (uint32_t)ad->width, (uint32_t)ad->height, (uint32_t)ad->shard_index,
              (uint32_t)ad->shard_count, (uint32_t)ad->band_height};
-  f->overflow_error = "rh_render_adaptive: ray queue overflow; lower chunk_samples";
   return RH_OK;
 }
 
@@ -2533,14 +2552,9 @@ int adaptive_on(Device* D, const rh_scene* scene, const rh_camera* camera, const
   const size_t px = ad->plane;
   unsigned long long negative = 0;
   if (rgb_out || linear_out) {
-    A.rgb = rgb_out;
-    A.linear = linear_out;
-    if (!dev_out) {
-      if (rgb_out && (rc = D->rgb.reserve(px * 3))) return rc;
-      if (linear_out && (rc = D->linear.reserve(px * 3 * sizeof(double)))) return rc;
-      A.rgb = rgb_out ? (uint8_t*)D->rgb.p : nullptr;
-      A.linear = linear_out ? (double*)D->linear.p : nullptr;
-    }
+    if ((rc = stage_output(D->rgb, rgb_out, px * 3, dev_out, &A.rgb)) ||
+        (rc = stage_output(D->linear, linear_out, px * 3 * sizeof(double), dev_out, &A.linear)))
+      return rc;
     RH_CUDA(cudaMemsetAsync(A.negative, 0, sizeof(unsigned long long), D->stream));
     launch_adaptive_output(A, D->stream);
     launches += 1;
@@ -2645,22 +2659,19 @@ int adaptive_state_on(Device* D, const rh_adaptive* ad, uint32_t* counts_out, do
   if (flags & ~RH_FLAG_DEVICE_OUT) return rh::set_error(RH_ERR_ARG, w + ": flags must be 0 or RH_FLAG_DEVICE_OUT");
   const bool dev = (flags & RH_FLAG_DEVICE_OUT) != 0;
   RH_CUDA(cudaSetDevice(D->dev));
-  if (dev) {
-    if ((uintptr_t)sums_out % 8 || (uintptr_t)sumsq_out % 8)
-      return rh::set_error(RH_ERR_ARG, w + ": device sums_out and sumsq_out must be 8-byte aligned");
-    if ((rc = check_device_pointers({counts_out, sums_out, sumsq_out}, w + ": RH_FLAG_DEVICE_OUT with a pointer that is not device memory")))
-      return rc;
-  }
+  if (dev && (rc = check_device_outputs(D, w, {{counts_out, 1, "counts_out"}, {sums_out, 8, "sums_out"}, {sumsq_out, 8, "sumsq_out"}})))
+    return rc;
   const size_t px = ad->plane, bytes = px * 3 * sizeof(double);
   if (counts_out)
     RH_CUDA(cudaMemcpyAsync(counts_out, ad->A.counts, px * sizeof(uint32_t), dev ? cudaMemcpyDeviceToDevice : cudaMemcpyDeviceToHost, D->stream));
-  if (!dev && (sums_out || sumsq_out) && (rc = D->linear.reserve(bytes))) return rc;
   const double* planes[2] = {ad->A.sum, ad->A.sumsq};
   double* outs[2] = {sums_out, sumsq_out};
   for (int k = 0; k < 2; k++) {
-    if (!outs[k]) continue;
-    launch_adaptive_interleave(planes[k], px, dev ? outs[k] : (double*)D->linear.p, D->stream);
-    if (!dev) RH_CUDA(cudaMemcpyAsync(outs[k], D->linear.p, bytes, cudaMemcpyDeviceToHost, D->stream));
+    double* d;
+    if ((rc = stage_output(D->linear, outs[k], bytes, dev, &d))) return rc;
+    if (!d) continue;
+    launch_adaptive_interleave(planes[k], px, d, D->stream);
+    if (!dev) RH_CUDA(cudaMemcpyAsync(outs[k], d, bytes, cudaMemcpyDeviceToHost, D->stream));
   }
   RH_CUDA(cudaGetLastError());
   RH_CUDA(cudaStreamSynchronize(D->stream));
@@ -2687,15 +2698,11 @@ int query_on(Device* D, const rh_scene* scene, int64_t light, const double* rays
   if (!rays || !out) return rh::set_error(RH_ERR_ARG, w + ": null buffer");
   const bool shadow = light >= 0, dev = (flags & RH_FLAG_DEVICE_OUT) != 0;
   const size_t out_bytes = shadow ? sizeof(uint8_t) : sizeof(rh_hit);
-  RH_CUDA(cudaSetDevice(D->dev));
-  if (dev) {
-    // the kernels move rays and records in 16-byte words
-    if ((uintptr_t)rays % 16 || (!shadow && (uintptr_t)out % 16))
-      return rh::set_error(RH_ERR_ARG, w + ": device buffers must be 16-byte aligned");
-  }
   int rc;
-  if (dev && (rc = check_device_pointers({rays, out}, w + ": RH_FLAG_DEVICE_OUT with a pointer that is not device memory")))
+  // the kernels move rays and records in 16-byte words
+  if (dev && (rc = check_device_outputs(D, w, {{rays, 16, "rays"}, {out, shadow ? 1u : 16u, shadow ? "occluded_out" : "hits_out"}})))
     return rc;
+  RH_CUDA(cudaSetDevice(D->dev));
   Device::Scratch& sc = D->lane[0];  // the render's deep-stack scratch covers grid x block of the query kernels
   if ((rc = sc.deep.reserve((size_t)scene->deep_entries * D->max_threads * sizeof(uint2)))) return rc;
   const uint64_t chunk = dev ? kQueryLaunch : kQueryChunk;
@@ -2751,16 +2758,14 @@ int trace_on(Device* D, const rh_scene* scene, const double* rays, uint64_t n, c
   if (want_ids && !hit_ids_out) return rh::set_error(RH_ERR_ARG, "rh_trace_rays: RH_FLAG_HIT_IDS without hit_ids_out");
   const uint64_t rows = (n + kTraceRowRays - 1) / kTraceRowRays;
   if (rows > 0x7fffffffu) return rh::set_error(RH_ERR_ARG, "rh_trace_rays: too many rays");
-  RH_CUDA(cudaSetDevice(D->dev));
+  // rays are read as 16-byte words; colours and ids are written as 8-byte words
   if (dev) {
-    // rays are read as 16-byte words; colours and ids are written as 8-byte words
-    if ((uintptr_t)rays % 16 || (uintptr_t)colors_out % 8 || (want_ids && (uintptr_t)hit_ids_out % 8))
-      return rh::set_error(RH_ERR_ARG, "rh_trace_rays: device rays must be 16-byte aligned, colours and ids 8-byte aligned");
-    const int rc = check_device_pointers({rays, colors_out, want_ids ? hit_ids_out : nullptr},
-                                         "rh_trace_rays: RH_FLAG_DEVICE_OUT with a pointer that is not device memory");
+    const int rc = check_device_outputs(D, "rh_trace_rays", {{rays, 16, "rays"}, {colors_out, 8, "colors_out"},
+                                                             {want_ids ? hit_ids_out : nullptr, 8, "hit_ids_out"}});
     if (rc) return rc;
   }
   Frame f;
+  f.who = "rh_trace_rays";
   f.o.width = kTraceRowRays;
   f.o.height = f.o.band_height = f.rows_local = (int)rows;
   f.o.max_depth = o->max_depth;
@@ -2778,7 +2783,6 @@ int trace_on(Device* D, const rh_scene* scene, const double* rays, uint64_t n, c
   f.rays_primary = n;
   f.trace = true;
   f.n_rays = n;
-  f.overflow_error = "rh_trace_rays: ray queue overflow; lower chunk_rays";
   return run_frame(D, scene, f, stats);
 }
 
@@ -2801,26 +2805,19 @@ int features_on(Device* D, const rh_scene* scene, const rh_camera* camera, const
   if (o->offset_mode != RH_OFFSETS_SPLITMIX64 && (ft->stream_spp || ft->stream_base))
     return rh::set_error(RH_ERR_ARG, w + ": stream_spp and stream_base are for RH_OFFSETS_SPLITMIX64 only");
   Frame f;
-  f.features = true;
   int rc = render_frame(D, scene, camera, o, nullptr, hit_ids_out, &f, "rh_render_features");
   if (rc) return rc;
   const uint32_t spp = (uint32_t)o->spp;
   if (ft->stream_spp) f.stream_spp = ft->stream_spp;
   f.stream_base = ft->stream_base;
-  if ((uint64_t)f.stream_base + spp > f.stream_spp)
-    return rh::set_error(RH_ERR_ARG, w + ": RH_OFFSETS_SPLITMIX64 past the end of the stream (stream_base " + std::to_string(f.stream_base) +
-                                         " + spp " + std::to_string(spp) + " > stream_spp " + std::to_string(f.stream_spp) + ")");
+  const std::string window = stream_window_error(f.stream_base, spp, f.stream_spp);
+  if (!window.empty()) return rh::set_error(RH_ERR_ARG, w + ": " + window);
   const int mode = o->offset_mode;
   const bool dev = (o->flags & RH_FLAG_DEVICE_OUT) != 0, dev_off = (o->flags & RH_FLAG_DEVICE_OFFSETS) != 0;
+  if (dev && (rc = check_device_outputs(D, w, {{ft->albedo, 8, "albedo"}, {ft->normal, 8, "normal"}, {ft->depth, 8, "depth"},
+                                               {ft->hits, 8, "hits"}, {want_ids ? hit_ids_out : nullptr, 8, "hit_ids_out"}})))
+    return rc;
   RH_CUDA(cudaSetDevice(D->dev));
-  if (dev) {
-    for (const void* p : {(const void*)ft->albedo, (const void*)ft->normal, (const void*)ft->depth, (const void*)ft->hits,
-                          (const void*)(want_ids ? hit_ids_out : nullptr)})
-      if ((uintptr_t)p % 8) return rh::set_error(RH_ERR_ARG, w + ": device outputs must be 8-byte aligned");
-    if ((rc = check_device_pointers({ft->albedo, ft->normal, ft->depth, ft->hits, want_ids ? hit_ids_out : nullptr},
-                                    w + ": RH_FLAG_DEVICE_OUT with a pointer that is not device memory")))
-      return rc;
-  }
   const bool host_offsets = (mode == RH_OFFSETS_F64 || mode == RH_OFFSETS_F32) && !dev_off;
   const size_t W = (size_t)o->width, row_samples = W * spp;
   const int rows = f.rows_local;
@@ -2845,18 +2842,7 @@ int features_on(Device* D, const rh_scene* scene, const rh_camera* camera, const
   if ((rc = D->query.reserve(at))) return rc;
   char* scratch = (char*)D->query.p;
 
-  ChunkParams P{};
-  P.spp = spp;
-  P.width = o->width;
-  P.height = o->height;
-  P.shard_index = f.o.shard_index;
-  P.shard_count = f.o.shard_count;
-  P.band_height = f.o.band_height;
-  P.offset_mode = mode;
-  P.offset_tile = o->offset_tile;
-  P.stream_spp = f.stream_spp;
-  P.stream_base = f.stream_base;
-  if (mode == RH_OFFSETS_SPLITMIX64) memcpy(&P.offset_seed, o->offsets, sizeof P.offset_seed);
+  ChunkParams P = frame_chunk_params(f);
   QueryParams Q{};
   Q.exact_boxes = (o->flags & RH_FLAG_EXACT_BOXES) ? 1 : 0;
   Q.deep_stack = (uint2*)sc.deep.p;
@@ -2953,12 +2939,7 @@ int light_groups_on(Device* D, const rh_scene* scene, const rh_camera* camera, c
     f.group_mask[g] |= 1u << l;
   }
   f.group_out = lg->out;
-  f.overflow_error = "rh_render_light_groups: ray queue overflow; lower chunk_samples";
-  if (o->flags & RH_FLAG_DEVICE_OUT) {
-    if ((uintptr_t)lg->out % 8) return rh::set_error(RH_ERR_ARG, w + ": device out must be 8-byte aligned");
-    RH_CUDA(cudaSetDevice(D->dev));
-    if ((rc = check_device_pointers({lg->out}, w + ": RH_FLAG_DEVICE_OUT with a pointer that is not device memory"))) return rc;
-  }
+  if ((o->flags & RH_FLAG_DEVICE_OUT) && (rc = check_device_outputs(D, w, {{lg->out, 8, "out"}}))) return rc;
   return run_frame(D, scene, f, stats);
 }
 
@@ -2980,11 +2961,8 @@ int views_on(Device* D, const rh_scene* scene, const rh_views* vw, const rh_rend
   if (!rgb_out && !linear_out) return rh::set_error(RH_ERR_ARG, w + ": rgb_out and linear_out are both null");
   const uint32_t V = vw->n_views;
   for (uint32_t v = 0; v < V; v++) {
-    const int32_t proj = vw->cameras[v].projection;
-    if (proj != RH_PROJ_ORTHOGRAPHIC && proj != RH_PROJ_PERSPECTIVE && proj != RH_PROJ_THIN_LENS)
-      return rh::set_error(RH_ERR_ARG, w + ": cameras[" + std::to_string(v) + "] has an unknown projection");
-    const std::string lens = lens_error(vw->cameras[v]);
-    if (!lens.empty()) return rh::set_error(RH_ERR_ARG, w + ": cameras[" + std::to_string(v) + "]: " + lens);
+    const std::string cam_err = camera_error(vw->cameras[v]);
+    if (!cam_err.empty()) return rh::set_error(RH_ERR_ARG, w + ": cameras[" + std::to_string(v) + "]: " + cam_err);
   }
   Frame f;
   f.views = true;
@@ -2992,13 +2970,10 @@ int views_on(Device* D, const rh_scene* scene, const rh_views* vw, const rh_rend
   if (rc) return rc;
   const int rows = f.rows_local, W = f.o.width;
   if ((uint64_t)V * rows > 0x7fffffffu) return rh::set_error(RH_ERR_ARG, w + ": n_views x shard rows must be below 2^31");
-  if (o->flags & RH_FLAG_DEVICE_OUT) {
-    if ((uintptr_t)linear_out % 8) return rh::set_error(RH_ERR_ARG, w + ": device linear_out must be 8-byte aligned");
-    RH_CUDA(cudaSetDevice(D->dev));
-    if ((rc = check_device_pointers({rgb_out, linear_out, (o->flags & RH_FLAG_HIT_IDS) ? hit_ids_out : nullptr},
-                                    w + ": RH_FLAG_DEVICE_OUT with a pointer that is not device memory")))
-      return rc;
-  }
+  if ((o->flags & RH_FLAG_DEVICE_OUT) &&
+      (rc = check_device_outputs(D, w, {{rgb_out, 1, "rgb_out"}, {linear_out, 8, "linear_out"},
+                                        {(o->flags & RH_FLAG_HIT_IDS) ? hit_ids_out : nullptr, 1, "hit_ids_out"}})))
+    return rc;
   RH_CUDA(cudaSetDevice(D->dev));
   // the camera table and the seeds, behind one another in one buffer
   std::vector<CameraParams> cams(V);
@@ -3031,7 +3006,6 @@ int views_on(Device* D, const rh_scene* scene, const rh_views* vw, const rh_rend
   f.rays_primary *= V;
   f.linear = linear_out;
   f.linear_bytes = (size_t)f.rows_local * W * 3 * sizeof(double);
-  f.overflow_error = "rh_render_views: ray queue overflow; lower chunk_samples";
   return run_frame(D, scene, f, stats);
 }
 
