@@ -51,8 +51,8 @@ enum {
 };
 /* ColorMap.hs:11-16                                                      */
 enum { RH_CMAP_FLAT = 0, RH_CMAP_CHECKER = 1, RH_CMAP_TEXTURE = 2 };
-/* Light.hs:8-10                                                          */
-enum { RH_LIGHT_DIRECTIONAL = 0, RH_LIGHT_POINT = 1 };
+/* Light.hs:8-10, and RH_LIGHT_SPHERE (a point light that emits from a ball; see rh_light) */
+enum { RH_LIGHT_DIRECTIONAL = 0, RH_LIGHT_POINT = 1, RH_LIGHT_SPHERE = 2 };
 /* Projection.hs:10-15, and RH_PROJ_THIN_LENS (a perspective camera with a circular thin lens; see rh_camera) */
 enum { RH_PROJ_ORTHOGRAPHIC = 0, RH_PROJ_PERSPECTIVE = 1, RH_PROJ_THIN_LENS = 2 };
 /* sample-offset formats for rh_render (RayHs.hs:173-188)                 */
@@ -86,7 +86,27 @@ typedef struct rh_material {
   double pad2_[2];
 } rh_material;
 
-/* Light.hs:8-10.  vec = direction (un-normalised, Light.hs:14) or position. */
+/* Light.hs:8-10.  vec = direction (un-normalised, Light.hs:14) or position.
+ *
+ * RH_LIGHT_SPHERE: a point light whose radius is also the radius r of the ball it emits from (the reference's falloff
+ * c / (1 + d/r)^2 is the inverse-square law of such a ball): vec is the centre, color and radius mean what they mean
+ * for RH_LIGHT_POINT.  radius must be finite and >= 0, else rh_scene_create and rh_scene_update return RH_ERR_ARG.
+ * Each shading point samples one point of the ball per light, all in IEEE double in this order, without fused
+ * multiply-add.  For the point p that accumDiffuse (RayHs.hs:89-97) receives and light index l:
+ *   1. key = bits(p.x) ^ mix64(bits(p.y) ^ mix64(bits(p.z) ^ mix64(l))), with bits the IEEE-754 bit pattern, l as a
+ *      uint64 and mix64 SplitMix64's output function (as for RH_PROJ_THIN_LENS, see rh_camera);
+ *   2. for j = 0 .. 15: a = 2 U(key, 3j) - 1, b = 2 U(key, 3j + 1) - 1, c = 2 U(key, 3j + 2) - 1, with U(key, k) value k
+ *      of the SplitMix64 stream seeded with key, as a double in [0, 1) (as for the lens); the first triple with
+ *      ((a*a) + (b*b)) + (c*c) < 1 is taken; if none is, a = b = c = 0 (the centre);
+ *   3. L' = (vec[0] + r*a, vec[1] + r*b, vec[2] + r*c);
+ *   4. the pair (p, l) is then exactly an RH_LIGHT_POINT at L' with the same color and radius: lightAt (Light.hs:15-17)
+ *      gives the direction and the falloff, the shadow ray is rayEps p ld, and inFrontOfLight (RayHs.hs:84-87) compares
+ *      against L'.
+ * The sample depends on p and l only, so every entry point that shades the same hit uses the same light point, and K
+ * accumulate calls of s samples still equal one call of K*s samples.  The penumbra converges as the camera samples of
+ * a pixel land on different points.  The points are a hash, not stratified: with RH_OFFSETS_NONE a hit point has one
+ * fixed light point.  A radius of 0 gives RH_LIGHT_POINT's image.  rh_shadow_intersection takes caller-built rays and
+ * compares a sphere light's hits against its centre, as for a point light. */
 typedef struct rh_light {
   int32_t kind;  /* RH_LIGHT_* */
   int32_t pad_;

@@ -6,8 +6,8 @@ csrc/kernels.cu and are reached through librayhs_b200.so (include/rayhs_b200.h).
 """
 from .host import (HIT_DTYPE, Accumulator, AdaptiveAccumulator, Features, Hits, Image, LightGroups, PeerFrames, Radiance, Rendering, Scene, Views, assemble_bands, buildRendering, closestIntersection, distributedRayTrace, init, main,
                    adaptiveRayTrace, progressiveRayTrace, rayTrace, shadowIntersection, traceRay,
-                   render, renderFeatures, renderLightGroups, renderViews, render_device, render_multi, multi_shutdown, renderingFromScene, sample_offsets, scene_setup_ms, shard_global_rows, shutdown, thinLens, writePPM)
+                   render, renderFeatures, renderLightGroups, renderViews, render_device, render_multi, multi_shutdown, renderingFromScene, sample_offsets, scene_setup_ms, shard_global_rows, shutdown, sphereLight, thinLens, writePPM)
 
 __all__ = ["HIT_DTYPE", "Accumulator", "AdaptiveAccumulator", "Features", "Hits", "Image", "LightGroups", "PeerFrames", "Radiance", "Rendering", "Scene", "Views", "assemble_bands", "buildRendering", "closestIntersection",
            "adaptiveRayTrace", "distributedRayTrace", "init", "main", "progressiveRayTrace", "rayTrace", "shadowIntersection", "traceRay", "render", "renderFeatures", "renderLightGroups", "renderViews", "render_device", "render_multi", "multi_shutdown", "renderingFromScene", "sample_offsets", "scene_setup_ms", "shard_global_rows", "shutdown",
-           "thinLens", "writePPM"]
+           "sphereLight", "thinLens", "writePPM"]

@@ -18,7 +18,7 @@ RH_OK, RH_ERR_ARG, RH_ERR_CUDA, RH_ERR_NCCL, RH_ERR_OOM, RH_ERR_STATE, RH_ERR_IO
 RH_OBJ_PLANE, RH_OBJ_SPHERE, RH_OBJ_MESH = 0, 1, 2
 RH_MAT_MIRROR, RH_MAT_DIFFUSE, RH_MAT_PLASTIC, RH_MAT_EMMIT, RH_MAT_TRANSPARENT, RH_MAT_SHOWNORMAL, RH_MAT_SHOWUV = range(7)
 RH_CMAP_FLAT, RH_CMAP_CHECKER, RH_CMAP_TEXTURE = 0, 1, 2
-RH_LIGHT_DIRECTIONAL, RH_LIGHT_POINT = 0, 1
+RH_LIGHT_DIRECTIONAL, RH_LIGHT_POINT, RH_LIGHT_SPHERE = 0, 1, 2
 RH_PROJ_ORTHOGRAPHIC, RH_PROJ_PERSPECTIVE, RH_PROJ_THIN_LENS = 0, 1, 2
 RH_OFFSETS_NONE, RH_OFFSETS_F64, RH_OFFSETS_F32, RH_OFFSETS_TILED_F64, RH_OFFSETS_SPLITMIX64 = 0, 1, 2, 3, 4
 RH_FLAG_HIT_IDS, RH_FLAG_DEVICE_OUT, RH_FLAG_DEVICE_OFFSETS, RH_FLAG_COUNT, RH_FLAG_PROFILE, RH_FLAG_EXACT_BOXES = 1, 2, 4, 8, 16, 32

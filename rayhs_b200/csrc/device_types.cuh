@@ -350,7 +350,8 @@ void launch_trace(const SceneView& S, const CameraParams& cam, const ChunkParams
 // the pooled one (coherent rays).  Returns the number of launches.  P.groups set: the instantiations that also add the
 // light-group terms (count must be false).
 // `classified`: a cudaEvent_t recorded after the classify kernel (or null).
-int launch_shadow(const SceneView& S, const ChunkParams& P, bool count, bool refill, int grid, void* stream, void* classified);
+int launch_shadow(const SceneView& S, const ChunkParams& P, bool count, bool refill, int grid, void* stream, void* classified,
+                  bool sphere_lights);
 void launch_resolve(const ChunkParams& P, void* stream);
 // rh_render_light_groups' sink, beside the resolve: each group's (and the remainder's) per-sample sums of the chunk,
 // folded per pixel in sample order and times 1 / spp, to out + g * out_group_stride + (out_px0 + pixel) * 3, where
@@ -392,8 +393,8 @@ int preload_setup_kernels();
 int device_light_map(const double L[3], const rh_tri* d_tris, const uint32_t* d_slots, size_t n, int R, float* d_out, double min_empty,
                      unsigned long long* d_words, int* useful, double* empty_fraction, void* stream);
 int device_lit_flags(const rh_tri* d_tris, const WideNode32* d_nodes, const double center[3], uint32_t root, const uint32_t* d_slots,
-                     uint32_t n_slots, const rh_light* d_lights, uint32_t n_lights, uint32_t mask, uint32_t mesh, uint16_t* d_lit,
-                     unsigned long long* d_flagged, void* stream);
+                     uint32_t n_slots, const rh_light* d_lights, uint32_t n_lights, uint32_t mask, uint32_t no_query, uint32_t mesh,
+                     uint16_t* d_lit, unsigned long long* d_flagged, void* stream);
 // micro-benchmarks
 void launch_gather_bench(const double2* buf, uint64_t n_records, uint32_t loads_per_thread, double2* sink, int grid, int block,
                          void* stream);

@@ -439,6 +439,9 @@ rh_light parse_light(const JValue& o) {  // JSON.hs:63-72
   std::string kind = str(o, "type");
   if (kind == "directional") { l.kind = RH_LIGHT_DIRECTIONAL; vec3(o, "direction", l.vec); color3(o, "color", l.color); }
   else if (kind == "point") { l.kind = RH_LIGHT_POINT; vec3(o, "position", l.vec); color3(o, "color", l.color); l.radius = num(o, "radius"); }
+  else if (kind == "sphere") {  // no JSON tag in the reference: a point light that emits from its ball (rh_light, RH_LIGHT_SPHERE)
+    l.kind = RH_LIGHT_SPHERE; vec3(o, "position", l.vec); color3(o, "color", l.color); l.radius = num(o, "radius");
+  }
   else bad("Unknown type for light " + kind);
   return l;
 }

@@ -161,7 +161,9 @@ struct Ctx {
   const rh_light* lights;
 };
 
-// Root boxes and light sides of the staged occluder tables (threads 0 .. n_roots * n_lights of the block).
+// Root boxes and light sides of the staged occluder tables (threads 0 .. n_roots * n_lights of the block).  SPH (the
+// scene has sphere lights): a sphere light's sides hold for every point of its ball (include/rayhs_b200.h, rh_light).
+template <bool SPH>
 __device__ __forceinline__ void stage_roots(SmemTables& sm, const SceneView& S) {
   const uint32_t n_meshes = S.n_occ_meshes, n_lights = S.n_lights;
   const uint32_t n_roots = n_meshes + (S.sphere_root != kEmpty ? 1u : 0u);
@@ -179,11 +181,21 @@ __device__ __forceinline__ void stage_roots(SmemTables& sm, const SceneView& S) 
   if (threadIdx.x < n_roots * n_lights) {
     const uint32_t li = threadIdx.x / n_roots, m = threadIdx.x % n_roots;
     uint32_t side = 0;
-    if (sm.lights[li].kind != RH_LIGHT_DIRECTIONAL)
+    if constexpr (SPH) {
+      // a coordinate of L' = c + r*a (|a| < 1) lies in [c - r, c + r] after both roundings (rounding is monotonic)
+      const rh_light& L = sm.lights[li];
+      const double r = L.kind == RH_LIGHT_SPHERE ? L.radius : 0.0;
+      if (L.kind != RH_LIGHT_DIRECTIONAL)
+        for (int a = 0; a < 3; a++) {
+          if (L.vec[a] + r < sm.rootbox[m][a]) side |= 1u << a;
+          if (L.vec[a] - r > sm.rootbox[m][3 + a]) side |= 8u << a;
+        }
+    } else if (sm.lights[li].kind != RH_LIGHT_DIRECTIONAL) {
       for (int a = 0; a < 3; a++) {
         if (sm.lights[li].vec[a] < sm.rootbox[m][a]) side |= 1u << a;
         if (sm.lights[li].vec[a] > sm.rootbox[m][3 + a]) side |= 8u << a;
       }
+    }
     sm.light_side[li][m] = (uint8_t)side;
     sm.light_map[li][m] = (S.light_map_index && m < n_meshes) ? S.light_map_index[li * kOccMeshes + m] : kEmpty;
   }
@@ -203,7 +215,15 @@ __device__ __forceinline__ void stage_roots(SmemTables& sm, const SceneView& S) 
       const double l1 = fabs(lp.x) + fabs(lp.y) + fabs(lp.z);
       for (uint32_t k = 0; k < S.n_occ_planes; k++) {
         const double f = dot(ld3(sm.planes[k].n), lp - ld3(sm.planes[k].p));
-        const double m = sm.plane_margin[k][0] + sm.plane_margin[k][1] * l1;
+        double m = sm.plane_margin[k][0] + sm.plane_margin[k][1] * l1;
+        if constexpr (SPH) {
+          // a sphere light: the whole ball by the margin of its farthest point (|L'|_1 <= |c|_1 + 3r), which also covers
+          // the roundings of c + r*a, plus r |n|_1 >= |n.(L' - c)|
+          if (L.kind == RH_LIGHT_SPHERE) {
+            const double r = L.radius, n1 = fabs(sm.planes[k].n[0]) + fabs(sm.planes[k].n[1]) + fabs(sm.planes[k].n[2]);
+            m = (sm.plane_margin[k][0] + sm.plane_margin[k][1] * (l1 + 3 * r)) + r * n1;
+          }
+        }
         if (f > m) front |= 1u << k;
         if (f < -m) behind |= 1u << k;
       }
@@ -213,6 +233,7 @@ __device__ __forceinline__ void stage_roots(SmemTables& sm, const SceneView& S) 
   }
 }
 
+template <bool SPH = false>
 __device__ __forceinline__ void stage_tables(SmemTables& sm, const SceneView& S, Ctx& cx) {
   copy16(sm.nodes, S.wide32, S.n_smem_nodes * (uint32_t)sizeof(WideNode32));
   if (S.tables_in_smem) {
@@ -226,7 +247,7 @@ __device__ __forceinline__ void stage_tables(SmemTables& sm, const SceneView& S,
     if (!S.tables_in_smem) copy16(sm.lights, S.lights, S.n_lights * (uint32_t)sizeof(rh_light));
   }
   __syncthreads();
-  if (S.shadow_fast) stage_roots(sm, S);
+  if (S.shadow_fast) stage_roots<SPH>(sm, S);
   __syncthreads();
   cx.S = &S;
   cx.sm_nodes = sm.nodes;
@@ -821,13 +842,16 @@ __device__ __forceinline__ void rebuild_hit(const SceneView& S, const DObject& o
 }
 
 // RayHs.hs:74-87 shadowIntersection: true when some non-emitter object has a hit in front of the light.
-// (General form over the object list; the kernels for <= 32 lights use the compact occluder tables instead.)
-template <bool COUNT>
-__device__ __forceinline__ bool occluded(const Ctx& cx, const Ray& r, bool exact, const rh_light& L, Stack& st, Cnt<COUNT>& cnt) {
+// (General form over the object list; the kernels for <= 32 lights use the compact occluder tables instead.)  SPH: lpos
+// is where the pair sees the light (light_pos), the point inFrontOfLight compares against; else L's position.
+template <bool COUNT, bool SPH = false>
+__device__ __forceinline__ bool occluded(const Ctx& cx, const Ray& r, bool exact, const rh_light& L, const V3& lpos, Stack& st,
+                                         Cnt<COUNT>& cnt) {
   const RayF f = make_rayf(r, *cx.S);
   AnyHit sink;
   sink.directional = (L.kind == RH_LIGHT_DIRECTIONAL);
-  sink.lpos = ld3(L.vec);
+  if constexpr (SPH) sink.lpos = lpos;
+  else sink.lpos = ld3(L.vec);
   sink.dl2 = sink.directional ? 0.0 : sqrDist(r.o, sink.lpos);
   // hits farther than the light cannot be in front of it; 1e-6 relative slack covers |d| != 1 rounding
   const double far = sink.directional ? __longlong_as_double(0x7ff0000000000000LL)
@@ -1155,13 +1179,50 @@ __device__ __forceinline__ Ray camera_ray(const CameraParams& cam, const CameraP
 }
 
 // ------------------------------------------------------------------ accumDiffuse (RayHs.hs:89-97): the light fold
-// Light.hs:12-17
-__device__ __forceinline__ void light_at(const rh_light& L, const V3& p, V3& ld, V3& lc) {
+// RH_LIGHT_SPHERE (include/rayhs_b200.h, rh_light): the point L' of the ball (centre c, radius r) of light li that the
+// shading point p samples, by rejection from the cube [-1, 1)^3 with a hash of (p, li), at most 16 attempts.  Not inlined:
+// only the kernels instantiated for scenes with sphere lights call it.
+__device__ __forceinline__ unsigned long long mix64(unsigned long long z) {  // SplitMix64's output function
+  z = (z ^ (z >> 30)) * 0xBF58476D1CE4E5B9ull;
+  z = (z ^ (z >> 27)) * 0x94D049BB133111EBull;
+  return z ^ (z >> 31);
+}
+__device__ __noinline__ V3 sphere_point(V3 c, double r, uint32_t li, V3 p) {
+  const unsigned long long key =
+      (unsigned long long)__double_as_longlong(p.x) ^
+      mix64((unsigned long long)__double_as_longlong(p.y) ^ mix64((unsigned long long)__double_as_longlong(p.z) ^ mix64(li)));
+  double a = 0, b = 0, e = 0;
+  for (unsigned j = 0; j < 16; j++) {
+    const double x = 2 * splitmix01(key, 3 * j) - 1, y = 2 * splitmix01(key, 3 * j + 1) - 1, z = 2 * splitmix01(key, 3 * j + 2) - 1;
+    if (((x * x) + (y * y)) + (z * z) < 1) {
+      a = x;
+      b = y;
+      e = z;
+      break;
+    }
+  }
+  return mk(c.x + r * a, c.y + r * b, c.z + r * e);
+}
+// Where the (hit p, light li) pair sees light L: its position (or direction), or, in the kernels for scenes with sphere
+// lights (SPH), a sphere light's sample L'.  With it every pair is a point or directional light of the reference.
+template <bool SPH>
+__device__ __forceinline__ V3 light_pos(const rh_light& L, uint32_t li, const V3& p) {
+  if constexpr (SPH) {
+    if (L.kind == RH_LIGHT_SPHERE) return sphere_point(ld3(L.vec), L.radius, li, p);
+  }
+  return ld3(L.vec);
+}
+
+// Light.hs:12-17 for the pair (p, light li); SPH: also where the pair sees the light (light_pos) in *lpos, if given.
+template <bool SPH = false>
+__device__ __forceinline__ void light_at(const rh_light& L, uint32_t li, const V3& p, V3& ld, V3& lc, V3* lpos = nullptr) {
   if (L.kind == RH_LIGHT_DIRECTIONAL) {  // Light.hs:14
     ld = ld3(L.vec);
     lc = ld3(L.color);
+    if constexpr (SPH) if (lpos) *lpos = ld;
   } else {  // Light.hs:15-17
-    const V3 lp = ld3(L.vec);
+    const V3 lp = light_pos<SPH>(L, li, p);
+    if constexpr (SPH) if (lpos) *lpos = lp;
     const double dd = sqrt(sqrDist(lp, p));
     const double s = 1.0 + dd / L.radius;
     const double falloff = 1.0 / (s * s);
@@ -1178,10 +1239,11 @@ struct LightPair {
   double dd, far;
   bool directional;
 };
-__device__ __forceinline__ LightPair make_light_pair(const rh_light& L, const V3& p) {
+template <bool SPH = false>
+__device__ __forceinline__ LightPair make_light_pair(const rh_light& L, uint32_t li, const V3& p) {
   LightPair q;
   q.directional = (L.kind == RH_LIGHT_DIRECTIONAL);
-  q.lp = ld3(L.vec);
+  q.lp = light_pos<SPH>(L, li, p);
   if (q.directional) {
     q.ld = q.lp;
     q.dd = 0;
@@ -1348,7 +1410,7 @@ struct LightFold {
   V3 acc;
 };
 // FAST: the occluder tables are the staged shared-memory ones (SceneView::shadow_fast), read with LDS.
-template <bool COUNT, bool FAST>
+template <bool COUNT, bool FAST, bool SPH>
 __device__ __forceinline__ LightFold fold_lights(const SmemTables& sm, const Ctx& cx, const ChunkParams& P, const V3& p, const V3& n,
                                                 const V3& cd, uint32_t lit, Cnt<COUNT>& cnt) {
   const SceneView& S = *cx.S;
@@ -1385,7 +1447,7 @@ __device__ __forceinline__ LightFold fold_lights(const SmemTables& sm, const Ctx
   }
   for (uint32_t li = 0; li < n_lights; li++) {
     const rh_light& L = lights[li];
-    const LightPair q = make_light_pair(L, p);
+    const LightPair q = make_light_pair<SPH>(L, li, p);
     const double ldn = dot(q.ld, n);
     if (ldn <= 0 && cd_tame && light_is_tame(L)) {
       F.culled++;
@@ -1420,12 +1482,13 @@ __device__ __forceinline__ LightFold fold_lights(const SmemTables& sm, const Ctx
 }
 
 // The fold of a queued hit once its walks are done: `vis` bit l = light l adds nothing.
+template <bool SPH>
 __device__ __forceinline__ V3 fold_visible(const Ctx& cx, uint32_t n_lights, uint32_t vis, const V3& p, const V3& n, const V3& cd) {
   V3 acc = mk(0, 0, 0);  // foldl ... black lts
   for (uint32_t li = 0; li < n_lights; li++) {
     if ((vis >> li) & 1u) continue;  // Just _ -> black (or l.n <= 0: the term is exactly 0)
     V3 ld, lc;
-    light_at(cx.lights[li], p, ld, lc);
+    light_at<SPH>(cx.lights[li], li, p, ld, lc);
     acc = acc + mul(hs_max(dot(ld, n), 0) * kPiInv, cmul(cd, lc));  // diffuse, Material.hs:31-33
   }
   return acc;
@@ -1434,13 +1497,14 @@ __device__ __forceinline__ V3 fold_visible(const Ctx& cx, uint32_t n_lights, uin
 // rh_render_light_groups, beside a folded hit's add to its sample: the same fold restricted to each group's lights (a
 // group without a visible light adds nothing), and Diffuse's ambient term to the remainder.  `sbits`: the queue's sample
 // word (bit 31: ambient term).
+template <bool SPH>
 __device__ __forceinline__ void accumulate_groups(const Ctx& cx, const ChunkParams& P, uint32_t n_lights, uint32_t vis, uint32_t sbits,
                                                   const V3& p, const V3& n, const V3& cd, double w) {
   const uint32_t sample = sbits & 0x7fffffffu;
 #pragma unroll 1
   for (uint32_t g = 0; g < P.n_groups; g++) {
     const uint32_t mask = P.group_mask[g];
-    if (mask & ~vis) accumulate_group(P, g, sample, w, fold_visible(cx, n_lights, vis | ~mask, p, n, cd));
+    if (mask & ~vis) accumulate_group(P, g, sample, w, fold_visible<SPH>(cx, n_lights, vis | ~mask, p, n, cd));
   }
   if (sbits & 0x80000000u) accumulate_group(P, P.n_groups, sample, w, mul(0.2, cd));
 }
@@ -1865,12 +1929,12 @@ constexpr size_t kClassifySmem = sizeof(SmemTables) + (kClassifyBlock / 32) * si
 
 // GROUPS (rh_render_light_groups): a hit folded here also adds its light-group terms (accumulate_groups; a finished
 // kHitDirect term goes to the remainder).
-template <bool COUNT, bool FAST, bool GROUPS = false>
+template <bool COUNT, bool FAST, bool GROUPS = false, bool SPH = false>
 __global__ void __launch_bounds__(kClassifyBlock, RH_CLASSIFY_MINB) classify_kernel(const __grid_constant__ SceneView S,
                                                                      const __grid_constant__ ChunkParams P) {
   SmemTables& sm = *reinterpret_cast<SmemTables*>(rh_smem);
   Ctx cx;
-  stage_tables(sm, S, cx);
+  stage_tables<SPH>(sm, S, cx);
   const uint32_t lane = threadIdx.x & 31;
   SlabWriter& out = reinterpret_cast<ClassifyWarpSmem*>(rh_smem + sizeof(SmemTables))[threadIdx.x >> 5].out;
   if (lane == 0) out.init();
@@ -1912,7 +1976,7 @@ __global__ void __launch_bounds__(kClassifyBlock, RH_CLASSIFY_MINB) classify_ker
           F.walk = F.settled = F.culled = 0;
           F.acc = task.cd;
         } else {
-          F = fold_lights<COUNT, FAST>(sm, cx, P, task.p, task.n, task.cd, lit, cnt);
+          F = fold_lights<COUNT, FAST, SPH>(sm, cx, P, task.p, task.n, task.cd, lit, cnt);
         }
         n_culled += F.culled;
         if (F.walk) {
@@ -1925,7 +1989,7 @@ __global__ void __launch_bounds__(kClassifyBlock, RH_CLASSIFY_MINB) classify_ker
           accumulate(P, task.sample & 0x7fffffffu, task.w, total);
           if constexpr (GROUPS) {
             if (lit & kHitDirect) accumulate_group(P, P.n_groups, task.sample, task.w, task.cd);
-            else accumulate_groups(cx, P, S.n_lights, F.settled, task.sample, task.p, task.n, task.cd, task.w);
+            else accumulate_groups<SPH>(cx, P, S.n_lights, F.settled, task.sample, task.p, task.n, task.cd, task.w);
           }
         }
       }
@@ -1948,11 +2012,11 @@ __global__ void __launch_bounds__(kClassifyBlock, RH_CLASSIFY_MINB) classify_ker
 // ------------------------------------------------------------------ K3: the tree walks of the queued hits
 // The (hit, light) pair's any-hit walk over the occluding trees (RayHs.hs:74-87 for the mesh objects and the sphere
 // tree; planes and linear spheres were settled by the trace kernel).  True = occluded.
-template <bool COUNT>
+template <bool COUNT, bool SPH>
 __device__ __forceinline__ bool walk_pair(const Ctx& cx, const ChunkParams& P, const uint32_t* mesh_roots, uint32_t n_meshes,
-                                          const rh_light& L, const V3& p, Stack& st, Cnt<COUNT>& cnt) {
+                                          const rh_light& L, uint32_t li, const V3& p, Stack& st, Cnt<COUNT>& cnt) {
   const SceneView& S = *cx.S;
-  const LightPair q = make_light_pair(L, p);
+  const LightPair q = make_light_pair<SPH>(L, li, p);
   Ray r;
   r.o = q.o;
   r.d = q.ld;
@@ -2005,7 +2069,7 @@ constexpr size_t kShadowSmem = sizeof(WalkTables) + (kShadowBlock / 32) * sizeof
                                (size_t)kShortStack * kShadowBlock * sizeof(uint2);
 static_assert(kShadowSmem <= 227 * 1024, "pooled shadow kernel shared memory");
 
-template <bool COUNT, bool GROUPS = false>  // GROUPS: phase 3 also adds the light-group terms
+template <bool COUNT, bool GROUPS = false, bool SPH = false>  // GROUPS: phase 3 also adds the light-group terms
 __global__ void __launch_bounds__(kShadowBlock, kShadowPerSm) shadow_pooled_kernel(const __grid_constant__ SceneView S,
                                                                         const __grid_constant__ ChunkParams P) {
   WalkTables& sm = *reinterpret_cast<WalkTables*>(rh_smem);
@@ -2087,7 +2151,7 @@ __global__ void __launch_bounds__(kShadowBlock, kShadowPerSm) shadow_pooled_kern
         unsigned dn0 = 0, dt0 = 0;
         if constexpr (!COUNT) { dn0 = cnt.dn; dt0 = cnt.dt; }
 #endif
-        if (walk_pair<COUNT>(cx, P, mesh_roots, n_meshes, cx.lights[lw], mk(a.x, a.y, b.x), st, cnt)) atomicOr(&ws.vis[j], 1u << lw);
+        if (walk_pair<COUNT, SPH>(cx, P, mesh_roots, n_meshes, cx.lights[lw], lw, mk(a.x, a.y, b.x), st, cnt)) atomicOr(&ws.vis[j], 1u << lw);
 #ifdef RH_WARP_TIMES
         if constexpr (!COUNT) {
           unsigned dn1 = cnt.dn - dn0, dt1 = cnt.dt - dt0;
@@ -2127,10 +2191,10 @@ __global__ void __launch_bounds__(kShadowBlock, kShadowPerSm) shadow_pooled_kern
       const double2 a = qp[item], b = qp[cap + item], c = qp[2 * cap + item], d = qp[3 * cap + item], e = qp[4 * cap + item];
       const uint32_t sbits = P.q_shadow.sample[item];
       const V3 p = mk(a.x, a.y, b.x), n = mk(b.y, c.x, c.y), cd = mk(d.x, d.y, e.x);
-      const V3 acc = fold_visible(cx, n_lights, ws.vis[j], p, n, cd);
+      const V3 acc = fold_visible<SPH>(cx, n_lights, ws.vis[j], p, n, cd);
       const V3 total = (sbits & 0x80000000u) ? mul(0.2, cd) + acc : acc;  // Diffuse adds the ambient term, RayHs.hs:111-114
       accumulate(P, sbits & 0x7fffffffu, e.y, total);
-      if constexpr (GROUPS) accumulate_groups(cx, P, n_lights, ws.vis[j], sbits, p, n, cd, e.y);
+      if constexpr (GROUPS) accumulate_groups<SPH>(cx, P, n_lights, ws.vis[j], sbits, p, n, cd, e.y);
     }
     __syncwarp();
   }
@@ -2165,7 +2229,7 @@ constexpr size_t kWalkSmem = sizeof(WalkTables) + (size_t)kWalkColumns * kWalkBl
                              (size_t)kShortStack * kWalkBlock * sizeof(uint2);
 static_assert(kWalkSmem <= 227 * 1024, "refill shadow kernel shared memory");
 
-template <bool COUNT, bool GROUPS = false>  // GROUPS: the final fold also adds the light-group terms
+template <bool COUNT, bool GROUPS = false, bool SPH = false>  // GROUPS: the final fold also adds the light-group terms
 __global__ void __launch_bounds__(kWalkBlock, 1) shadow_refill_kernel(const __grid_constant__ SceneView S,
                                                                       const __grid_constant__ ChunkParams P) {
   WalkTables& sm = *reinterpret_cast<WalkTables*>(rh_smem);
@@ -2206,10 +2270,10 @@ __global__ void __launch_bounds__(kWalkBlock, 1) shadow_refill_kernel(const __gr
         const double2 bq = qp[cap + item], c = qp[2 * cap + item], d = qp[3 * cap + item], e = qp[4 * cap + item];
         const uint32_t sbits = P.q_shadow.sample[item];
         const V3 p = mk(lane_slot(8), lane_slot(9), lane_slot(10)), n = mk(bq.y, c.x, c.y), cd = mk(d.x, d.y, e.x);
-        const V3 acc = fold_visible(cx, n_lights, vis, p, n, cd);
+        const V3 acc = fold_visible<SPH>(cx, n_lights, vis, p, n, cd);
         const V3 total = (sbits & 0x80000000u) ? mul(0.2, cd) + acc : acc;  // Diffuse adds the ambient term, RayHs.hs:111-114
         accumulate(P, sbits & 0x7fffffffu, e.y, total);
-        if constexpr (GROUPS) accumulate_groups(cx, P, n_lights, vis, sbits, p, n, cd, e.y);
+        if constexpr (GROUPS) accumulate_groups<SPH>(cx, P, n_lights, vis, sbits, p, n, cd, e.y);
         has_task = false;
       }
       const unsigned empty = __ballot_sync(kFull, !has_task);
@@ -2243,7 +2307,7 @@ __global__ void __launch_bounds__(kWalkBlock, 1) shadow_refill_kernel(const __gr
       if (!walking && has_task && rest != 0) {  // the walk towards the hit's next light
         cur = __ffs(rest) - 1;
         rest &= rest - 1;
-        const LightPair q = make_light_pair(cx.lights[cur], mk(lane_slot(8), lane_slot(9), lane_slot(10)));
+        const LightPair q = make_light_pair<SPH>(cx.lights[cur], cur, mk(lane_slot(8), lane_slot(9), lane_slot(10)));
         Ray r;
         r.o = q.o;
         r.d = q.ld;
@@ -2321,12 +2385,12 @@ __global__ void __launch_bounds__(kWalkBlock, 1) shadow_refill_kernel(const __gr
 // Simple form, for scenes with more than 32 lights (the masks of a queued hit hold 32): every Diffuse / Plastic hit is
 // queued unclassified; one hit per lane, lights in sequence, each query over the whole object list run to completion.
 constexpr size_t kSimpleSmem = sizeof(SmemTables) + (size_t)kShortStack * kShadowBlock * sizeof(uint2);
-template <bool COUNT>
+template <bool COUNT, bool SPH = false>
 __global__ void __launch_bounds__(kShadowBlock, 1) shadow_simple_kernel(const __grid_constant__ SceneView S,
                                                                         const __grid_constant__ ChunkParams P) {
   SmemTables& sm = *reinterpret_cast<SmemTables*>(rh_smem);
   Ctx cx;
-  stage_tables(sm, S, cx);
+  stage_tables<SPH>(sm, S, cx);
   Stack st = make_stack(rh_smem + sizeof(SmemTables), kShadowBlock, P);
   Cnt<COUNT> cnt;
   cnt.zero();
@@ -2358,8 +2422,8 @@ __global__ void __launch_bounds__(kShadowBlock, 1) shadow_simple_kernel(const __
       V3 acc = mk(0, 0, 0);  // foldl ... black lts
       for (uint32_t li = 0; li < S.n_lights; li++) {
         const rh_light& L = cx.lights[li];
-        V3 ld, lc;
-        light_at(L, p, ld, lc);
+        V3 ld, lc, lp;  // (lp: SPH only)
+        light_at<SPH>(L, li, p, ld, lc, &lp);
         // diffuse (Material.hs:31-33) = (max (l.n) 0 / pi) * (cd (*) lc): exactly zero when l.n <= 0 (and cd (*) lc is
         // finite, light_is_tame), whether or not the point is shadowed, so the occlusion query cannot change the sum
         const double ldn = dot(ld, n);
@@ -2368,7 +2432,7 @@ __global__ void __launch_bounds__(kShadowBlock, 1) shadow_simple_kernel(const __
           continue;
         }
         const Ray sr = rayEps(p, ld);
-        const bool shadowed = occluded<COUNT>(cx, sr, P.exact_boxes || needs_exact_walk(sr, S), L, st, cnt);
+        const bool shadowed = occluded<COUNT, SPH>(cx, sr, P.exact_boxes || needs_exact_walk(sr, S), L, lp, st, cnt);
         if (!shadowed) acc = acc + mul(hs_max(ldn, 0) * kPiInv, cmul(cd, lc));
       }
       const V3 total = (sbits & 0x80000000u) ? mul(0.2, cd) + acc : acc;
@@ -2490,7 +2554,7 @@ __global__ void __launch_bounds__(kQueryBlock, 1) query_shadow_kernel(const __gr
   claim_rays(Q, lane, [&](uint32_t first, uint32_t count) {
     const Ray r = load_query_ray(Q, first, count, tile, lane);
     if (lane < count)
-      Q.occluded[first + lane] = occluded<false>(cx, r, Q.exact_boxes || needs_exact_walk(r, S), L, st, cnt) ? 1 : 0;
+      Q.occluded[first + lane] = occluded<false>(cx, r, Q.exact_boxes || needs_exact_walk(r, S), L, ld3(L.vec), st, cnt) ? 1 : 0;
   });
 }
 
@@ -3153,8 +3217,48 @@ __global__ void stream_bench_kernel(const double2* __restrict__ buf, uint64_t n_
 }  // namespace
 
 // ------------------------------------------------------------------ launchers
-static int g_classify_grid[2] = {148, 148};
-static int g_groups_classify_grid[2] = {148, 148};  // classify_kernel<false, FAST, true>, by FAST
+static int g_classify_grid[2][2] = {{148, 148}, {148, 148}};         // classify_kernel<COUNT, true, false, SPH>, by SPH, COUNT
+static int g_groups_classify_grid[2][2] = {{148, 148}, {148, 148}};  // classify_kernel<false, FAST, true, SPH>, by SPH, FAST
+
+// The shadow kernels' instantiations of one value of SPH (the scene has sphere lights).
+template <bool SPH>
+cudaError_t configure_shadow_kernels() {
+  cudaError_t e = cudaSuccess;
+  auto set = [&](const void* fn, size_t bytes) {
+    if (e == cudaSuccess) e = cudaFuncSetAttribute(fn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bytes);
+  };
+  set((const void*)shadow_pooled_kernel<true, false, SPH>, kShadowSmem);
+  set((const void*)shadow_pooled_kernel<false, false, SPH>, kShadowSmem);
+  set((const void*)shadow_refill_kernel<true, false, SPH>, kWalkSmem);
+  set((const void*)shadow_refill_kernel<false, false, SPH>, kWalkSmem);
+  set((const void*)shadow_simple_kernel<true, SPH>, kSimpleSmem);
+  set((const void*)shadow_simple_kernel<false, SPH>, kSimpleSmem);
+  set((const void*)classify_kernel<true, true, false, SPH>, kClassifySmem);
+  set((const void*)classify_kernel<false, true, false, SPH>, kClassifySmem);
+  set((const void*)classify_kernel<true, false, false, SPH>, kClassifySmem);
+  set((const void*)classify_kernel<false, false, false, SPH>, kClassifySmem);
+  set((const void*)shadow_pooled_kernel<false, true, SPH>, kShadowSmem);
+  set((const void*)shadow_refill_kernel<false, true, SPH>, kWalkSmem);
+  set((const void*)classify_kernel<false, true, true, SPH>, kClassifySmem);
+  set((const void*)classify_kernel<false, false, true, SPH>, kClassifySmem);
+  if (e != cudaSuccess) return e;
+  int dev = 0, sms = 0, nb = 0;
+  cudaGetDevice(&dev);
+  cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
+  for (int c = 0; c < 2; c++) {
+    if (c) cudaOccupancyMaxActiveBlocksPerMultiprocessor(&nb, classify_kernel<true, true, false, SPH>, kClassifyBlock, kClassifySmem);
+    else cudaOccupancyMaxActiveBlocksPerMultiprocessor(&nb, classify_kernel<false, true, false, SPH>, kClassifyBlock, kClassifySmem);
+    g_classify_grid[SPH][c] = sms * (nb > 0 ? nb : 1);
+  }
+  for (int fast = 0; fast < 2; fast++) {
+    nb = 0;
+    if (fast) cudaOccupancyMaxActiveBlocksPerMultiprocessor(&nb, classify_kernel<false, true, true, SPH>, kClassifyBlock, kClassifySmem);
+    else cudaOccupancyMaxActiveBlocksPerMultiprocessor(&nb, classify_kernel<false, false, true, SPH>, kClassifyBlock, kClassifySmem);
+    g_groups_classify_grid[SPH][fast] = sms * (nb > 0 ? nb : 1);
+  }
+  return cudaSuccess;
+}
+
 int configure_kernels() {
   cudaError_t e = cudaSuccess;
   auto set = [&](const void* fn, size_t bytes) {
@@ -3166,39 +3270,11 @@ int configure_kernels() {
   set((const void*)trace_kernel<true, Source::kPixelList>, kTraceSmem);
   set((const void*)trace_kernel<false, Source::kPixelList>, kTraceSmem);
   set((const void*)trace_kernel<false, Source::kViews>, kTraceSmem);
-  set((const void*)shadow_pooled_kernel<true>, kShadowSmem);
-  set((const void*)shadow_pooled_kernel<false>, kShadowSmem);
-  set((const void*)shadow_refill_kernel<true>, kWalkSmem);
-  set((const void*)shadow_refill_kernel<false>, kWalkSmem);
-  set((const void*)shadow_simple_kernel<true>, kSimpleSmem);
-  set((const void*)shadow_simple_kernel<false>, kSimpleSmem);
-  set((const void*)classify_kernel<true, true>, kClassifySmem);
-  set((const void*)classify_kernel<false, true>, kClassifySmem);
-  set((const void*)classify_kernel<true, false>, kClassifySmem);
-  set((const void*)classify_kernel<false, false>, kClassifySmem);
-  set((const void*)shadow_pooled_kernel<false, true>, kShadowSmem);
-  set((const void*)shadow_refill_kernel<false, true>, kWalkSmem);
-  set((const void*)classify_kernel<false, true, true>, kClassifySmem);
-  set((const void*)classify_kernel<false, false, true>, kClassifySmem);
   set((const void*)query_closest_kernel, kQuerySmem);
   set((const void*)query_shadow_kernel, kQuerySmem);
   set((const void*)feature_kernel, kQuerySmem);
-  if (e == cudaSuccess) {
-    int dev = 0, sms = 0, nb = 0;
-    cudaGetDevice(&dev);
-    cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
-    for (int c = 0; c < 2; c++) {
-      if (c) cudaOccupancyMaxActiveBlocksPerMultiprocessor(&nb, classify_kernel<true, true>, kClassifyBlock, kClassifySmem);
-      else cudaOccupancyMaxActiveBlocksPerMultiprocessor(&nb, classify_kernel<false, true>, kClassifyBlock, kClassifySmem);
-      g_classify_grid[c] = sms * (nb > 0 ? nb : 1);
-    }
-    for (int fast = 0; fast < 2; fast++) {
-      nb = 0;
-      if (fast) cudaOccupancyMaxActiveBlocksPerMultiprocessor(&nb, classify_kernel<false, true, true>, kClassifyBlock, kClassifySmem);
-      else cudaOccupancyMaxActiveBlocksPerMultiprocessor(&nb, classify_kernel<false, false, true>, kClassifyBlock, kClassifySmem);
-      g_groups_classify_grid[fast] = sms * (nb > 0 ? nb : 1);
-    }
-  }
+  if (e == cudaSuccess) e = configure_shadow_kernels<false>();
+  if (e == cudaSuccess) e = configure_shadow_kernels<true>();
   return (int)e;
 }
 int max_threads_per_launch(int n_sms) {
@@ -3216,39 +3292,46 @@ void launch_trace(const SceneView& S, const CameraParams& cam, const ChunkParams
   else trace_kernel<false, Source::kCamera><<<grid * kTracePerSm, kTraceBlock, kTraceSmem, st>>>(S, cam, P);
   close_hit_range_kernel<<<1, 1, 0, st>>>(P.ctl, P.pass);
 }
-int launch_shadow(const SceneView& S, const ChunkParams& P, bool count, bool refill, int grid, void* stream, void* classified) {
+template <bool SPH>
+int launch_shadow_kernels(const SceneView& S, const ChunkParams& P, bool count, bool refill, int grid, void* stream, void* classified) {
   cudaStream_t st = (cudaStream_t)stream;
   if (S.n_lights > (uint32_t)kMaskLights) {
-    if (count) shadow_simple_kernel<true><<<grid, kShadowBlock, kSimpleSmem, st>>>(S, P);
-    else shadow_simple_kernel<false><<<grid, kShadowBlock, kSimpleSmem, st>>>(S, P);
+    if (count) shadow_simple_kernel<true, SPH><<<grid, kShadowBlock, kSimpleSmem, st>>>(S, P);
+    else shadow_simple_kernel<false, SPH><<<grid, kShadowBlock, kSimpleSmem, st>>>(S, P);
     if (classified) cudaEventRecord((cudaEvent_t)classified, st);
     return 1;
   }
   if (P.groups) {  // rh_render_light_groups (never counting)
-    if (S.shadow_fast) classify_kernel<false, true, true><<<g_groups_classify_grid[1], kClassifyBlock, kClassifySmem, st>>>(S, P);
-    else classify_kernel<false, false, true><<<g_groups_classify_grid[0], kClassifyBlock, kClassifySmem, st>>>(S, P);
+    if (S.shadow_fast) classify_kernel<false, true, true, SPH><<<g_groups_classify_grid[SPH][1], kClassifyBlock, kClassifySmem, st>>>(S, P);
+    else classify_kernel<false, false, true, SPH><<<g_groups_classify_grid[SPH][0], kClassifyBlock, kClassifySmem, st>>>(S, P);
     if (classified) cudaEventRecord((cudaEvent_t)classified, st);
-    if (refill) shadow_refill_kernel<false, true><<<grid, kWalkBlock, kWalkSmem, st>>>(S, P);
-    else shadow_pooled_kernel<false, true><<<grid * kShadowPerSm, kShadowBlock, kShadowSmem, st>>>(S, P);
+    if (refill) shadow_refill_kernel<false, true, SPH><<<grid, kWalkBlock, kWalkSmem, st>>>(S, P);
+    else shadow_pooled_kernel<false, true, SPH><<<grid * kShadowPerSm, kShadowBlock, kShadowSmem, st>>>(S, P);
     return 2;
   }
   // FAST: the occluder tables are the staged shared-memory ones (SceneView::shadow_fast)
   if (S.shadow_fast) {
-    if (count) classify_kernel<true, true><<<g_classify_grid[1], kClassifyBlock, kClassifySmem, st>>>(S, P);
-    else classify_kernel<false, true><<<g_classify_grid[0], kClassifyBlock, kClassifySmem, st>>>(S, P);
+    if (count) classify_kernel<true, true, false, SPH><<<g_classify_grid[SPH][1], kClassifyBlock, kClassifySmem, st>>>(S, P);
+    else classify_kernel<false, true, false, SPH><<<g_classify_grid[SPH][0], kClassifyBlock, kClassifySmem, st>>>(S, P);
   } else {
-    if (count) classify_kernel<true, false><<<g_classify_grid[1], kClassifyBlock, kClassifySmem, st>>>(S, P);
-    else classify_kernel<false, false><<<g_classify_grid[0], kClassifyBlock, kClassifySmem, st>>>(S, P);
+    if (count) classify_kernel<true, false, false, SPH><<<g_classify_grid[SPH][1], kClassifyBlock, kClassifySmem, st>>>(S, P);
+    else classify_kernel<false, false, false, SPH><<<g_classify_grid[SPH][0], kClassifyBlock, kClassifySmem, st>>>(S, P);
   }
   if (classified) cudaEventRecord((cudaEvent_t)classified, st);  // the pass's slabs of the hit queue are free again
   if (refill) {
-    if (count) shadow_refill_kernel<true><<<grid, kWalkBlock, kWalkSmem, st>>>(S, P);
-    else shadow_refill_kernel<false><<<grid, kWalkBlock, kWalkSmem, st>>>(S, P);
+    if (count) shadow_refill_kernel<true, false, SPH><<<grid, kWalkBlock, kWalkSmem, st>>>(S, P);
+    else shadow_refill_kernel<false, false, SPH><<<grid, kWalkBlock, kWalkSmem, st>>>(S, P);
   } else {
-    if (count) shadow_pooled_kernel<true><<<grid * kShadowPerSm, kShadowBlock, kShadowSmem, st>>>(S, P);
-    else shadow_pooled_kernel<false><<<grid * kShadowPerSm, kShadowBlock, kShadowSmem, st>>>(S, P);
+    if (count) shadow_pooled_kernel<true, false, SPH><<<grid * kShadowPerSm, kShadowBlock, kShadowSmem, st>>>(S, P);
+    else shadow_pooled_kernel<false, false, SPH><<<grid * kShadowPerSm, kShadowBlock, kShadowSmem, st>>>(S, P);
   }
   return 2;
+}
+// sphere_lights: the scene has an RH_LIGHT_SPHERE light; only those scenes run the kernels that sample the balls.
+int launch_shadow(const SceneView& S, const ChunkParams& P, bool count, bool refill, int grid, void* stream, void* classified,
+                  bool sphere_lights) {
+  return sphere_lights ? launch_shadow_kernels<true>(S, P, count, refill, grid, stream, classified)
+                       : launch_shadow_kernels<false>(S, P, count, refill, grid, stream, classified);
 }
 void launch_resolve(const ChunkParams& P, void* stream) {
   const uint32_t n_pixels = P.n_rows * P.width;

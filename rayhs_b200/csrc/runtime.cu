@@ -191,6 +191,7 @@ struct rh_scene {
   uint32_t deep_entries = 1;     // per-thread entries of the deep-stack scratch this scene's walks can need
   bool refill_possible = true;   // the per-lane-refill shadow kernel stacks every tree root: not with hundreds of meshes
   bool has_transparent = false;  // some material is Transparent (Material.hs:18): frames need the probe passes
+  bool has_sphere_lights = false;  // some light is RH_LIGHT_SPHERE: frames run the shadow kernels that sample the balls
   // Shadow-walk schedule of this scene: 0 = undecided, 1 = pooled, 2 = per-lane refill.  Decided by timing one large
   // frame with each (render_on); frames too small to time use the pooled kernel and do not count, and after
   // kTuneGiveUp of those the scene stays pooled.
@@ -846,8 +847,13 @@ int check_tables(const rh_material* mats, uint32_t n_materials, const rh_texture
       }
     }
   }
-  for (uint32_t i = 0; i < n_lights; i++)
-    if (lights[i].kind != RH_LIGHT_DIRECTIONAL && lights[i].kind != RH_LIGHT_POINT) return rh::set_error(RH_ERR_ARG, w + ": unknown light kind");
+  for (uint32_t i = 0; i < n_lights; i++) {
+    const rh_light& L = lights[i];
+    if (L.kind != RH_LIGHT_DIRECTIONAL && L.kind != RH_LIGHT_POINT && L.kind != RH_LIGHT_SPHERE)
+      return rh::set_error(RH_ERR_ARG, w + ": unknown light kind");
+    if (L.kind == RH_LIGHT_SPHERE && !(std::isfinite(L.radius) && L.radius >= 0))
+      return rh::set_error(RH_ERR_ARG, w + ": lights[" + std::to_string(i) + "]: a sphere light's radius must be finite and >= 0");
+  }
   return RH_OK;
 }
 
@@ -1187,6 +1193,8 @@ int derive_tables(Device* D, const rh_scene& G, const rh_material* mats, uint32_
   v.tables_in_smem = (objs.size() <= (size_t)kSmemObjects && n_materials <= (uint32_t)kSmemObjects && n_lights <= (uint32_t)kSmemLights);
   T->has_transparent = false;
   for (uint32_t i = 0; i < n_materials; i++) T->has_transparent |= mats[i].kind == RH_MAT_TRANSPARENT;
+  T->has_sphere_lights = false;
+  for (uint32_t i = 0; i < n_lights; i++) T->has_sphere_lights |= lights[i].kind == RH_LIGHT_SPHERE;
   {
     // Deep-stack scratch (entries beyond the shared-memory short stack, and the exact walk's whole stack): a walk
     // stacks at most one entry per level of its tree; the per-lane-refill shadow kernel also stacks the other roots.
@@ -1196,8 +1204,9 @@ int derive_tables(Device* D, const rh_scene& G, const rh_material* mats, uint32_
     T->deep_entries = std::max<uint32_t>(G.ref_depth + 4, float_need > (uint32_t)kShortStack ? float_need - kShortStack : 1u);
   }
   // Light-space tables of the shadow kernels (light_maps.cpp): cube maps of the nearest possible occluder distance, one
-  // per (point light, occluder mesh), and lit-triangle flags per (triangle, light of either kind).  Only the
-  // shared-memory-table shadow kernels read them.
+  // per (point light, occluder mesh), and lit-triangle flags per (triangle, point or directional light).  Only the
+  // shared-memory-table shadow kernels read them.  Both hold for one light point, so a sphere light has neither, and
+  // neither the map budget nor the lit-query limit counts it: the other lights get the tables of the scene without it.
   v.light_maps = nullptr;
   v.lit_flags = nullptr;
   v.light_map_index = nullptr;
@@ -1211,8 +1220,13 @@ int derive_tables(Device* D, const rh_scene& G, const rh_material* mats, uint32_
   auto mesh_slots = [&](size_t m) { return G.mesh_slots.data() + G.slot_begin[occ_objs[m]]; };
   auto mesh_n_slots = [&](size_t m) { return G.slot_begin[occ_objs[m] + 1] - G.slot_begin[occ_objs[m]]; };
   {
-    uint32_t n_point = 0;
-    for (uint32_t li = 0; li < n_lights; li++) n_point += lights[li].kind == RH_LIGHT_POINT;
+    uint32_t n_point = 0, n_sphere = 0, sphere_bits = 0;  // (sphere_bits: of the light indices that have lit bits)
+    for (uint32_t li = 0; li < n_lights; li++) {
+      n_point += lights[li].kind == RH_LIGHT_POINT;
+      n_sphere += lights[li].kind == RH_LIGHT_SPHERE;
+      if (lights[li].kind == RH_LIGHT_SPHERE && li < 12) sphere_bits |= 1u << li;
+    }
+    const uint32_t n_table_lights = n_lights - n_sphere;
     const size_t n_pairs = (size_t)n_point * occ_meshes.size();
     if (v.shadow_fast && !occ_meshes.empty() && n_lights) {
       int R = kLightMapRes;
@@ -1269,7 +1283,7 @@ int derive_tables(Device* D, const rh_scene& G, const rh_material* mats, uint32_
                 useful_maps++;
               }
             }
-            want[m] = n_slots * (size_t)n_lights <= kLitMaxQueriesDevice && (n_point == 0 || useful_maps > 0);
+            want[m] = n_slots * (size_t)n_table_lights <= kLitMaxQueriesDevice && (n_point == 0 || useful_maps > 0);
           }
           // lit triangles: the old bits of every light index whose light kept its kind and position stay, as long as
           // every mesh that had bits still has them (a mesh that gains them is queried for every light)
@@ -1291,9 +1305,9 @@ int derive_tables(Device* D, const rh_scene& G, const rh_material* mats, uint32_
             const uint32_t mask = reuse_lit && old->mesh_lit[m] ? changed : all;
             RH_CUDA((cudaError_t)device_lit_flags(d_tris, (const WideNode32*)G.wide32.p, G.view.center, occ_meshes[m],
                                                   (const uint32_t*)scratch.bufs[m].p, (uint32_t)mesh_n_slots(m),
-                                                  (const rh_light*)T->lights.p, n_lights, mask, (uint32_t)m, (uint16_t*)T->lit_flags.p,
-                                                  (unsigned long long*)words.p + 2, D->stream));
-            if (info) info->lit_queries += (uint64_t)mesh_n_slots(m) * (uint64_t)__builtin_popcount(mask & all);
+                                                  (const rh_light*)T->lights.p, n_lights, mask, sphere_bits, (uint32_t)m,
+                                                  (uint16_t*)T->lit_flags.p, (unsigned long long*)words.p + 2, D->stream));
+            if (info) info->lit_queries += (uint64_t)mesh_n_slots(m) * (uint64_t)__builtin_popcount(mask & all & ~sphere_bits);
           }
           unsigned long long flagged = 0;
           RH_CUDA(cudaMemcpyAsync(&flagged, (unsigned long long*)words.p + 2, 8, cudaMemcpyDeviceToHost, D->stream));
@@ -1319,7 +1333,7 @@ int derive_tables(Device* D, const rh_scene& G, const rh_material* mats, uint32_
             const std::vector<uint32_t> slots(mesh_slots(m), mesh_slots(m) + mesh_n_slots(m));
           // lit triangles: per triangle and light, can another triangle of this mesh shadow it at all?  The queries
           // run on their own threads while this one builds the mesh's cube maps.
-          const bool want_lit = slots.size() * (size_t)n_lights <= kLitMaxQueries;
+          const bool want_lit = slots.size() * (size_t)n_table_lights <= kLitMaxQueries;
           if (want_lit && lit.empty()) lit.assign(dtris.size(), 0);
           size_t lit_found = 0;
           bool lit_failed = false;
@@ -1338,6 +1352,7 @@ int derive_tables(Device* D, const rh_scene& G, const rh_material* mats, uint32_
                   const uint32_t s0 = slots[at];
                   uint32_t bits = 0;
                   for (uint32_t li = 0; li < n_lights && li < 12; li++) {
+                    if ((sphere_bits >> li) & 1u) continue;
                     rh::LitQuery q;
                     if (!rh::lit_query_make(dtris[s0], lights[li].vec, lights[li].kind == RH_LIGHT_DIRECTIONAL, &q)) continue;
                     bool blocked = false;
@@ -1450,6 +1465,7 @@ void swap_tables(rh_scene& a, rh_scene& b) {
   std::swap(a.deep_entries, b.deep_entries);
   std::swap(a.refill_possible, b.refill_possible);
   std::swap(a.has_transparent, b.has_transparent);
+  std::swap(a.has_sphere_lights, b.has_sphere_lights);
   std::swap(a.n_light_maps, b.n_light_maps);
   std::swap(a.ms_light_tables, b.ms_light_tables);
   std::swap(a.objs_host, b.objs_host);
@@ -1941,7 +1957,7 @@ struct FrameRun {
         P.deep_stack = (uint2*)sc.deep_shadow.p;
       }
       const int n_shadow = launch_shadow(scene->view, P, counting, sh.use_refill, D->n_sms, shadow_stream,
-                                         pipelined ? (void*)D->ev_classified[ln][pass] : nullptr);
+                                         pipelined ? (void*)D->ev_classified[ln][pass] : nullptr, scene->has_sphere_lights);
       if (sh.profile) spans.push_back({a, prof_event(lane_stream), 1});
       launches += 2 + n_shadow;  // (trace, the one-thread kernel that closes its hit range, classify, walk)
     }

@@ -12,7 +12,7 @@ namespace rh {
 
 enum UpdateClass : int {
   kUpdateNone = 0,      // no byte of a named field changed
-  kUpdateColours = 1,   // light color / radius and material color1 / color2 / size only: upload the tables, nothing else
+  kUpdateColours = 1,   // light color / radius (not a sphere light's) and material color1 / color2 / size only: upload the tables
   kUpdateEmitters = 2,  // some object became or stopped being an emitter: occluder tables and all light tables anew
   kUpdateTables = 3,    // same occluders, other lights or material kinds: rebuild only the light tables that changed
 };
@@ -20,8 +20,11 @@ enum UpdateClass : int {
 template <class T>
 inline bool same_bytes(const T& a, const T& b) { return memcmp(&a, &b, sizeof a) == 0; }
 
-// What a light's cube maps and lit-triangle bits depend on.
-inline bool same_light_geometry(const rh_light& a, const rh_light& b) { return a.kind == b.kind && same_bytes(a.vec, b.vec); }
+// What a light's cube maps and lit-triangle bits depend on, and, for a sphere light, its ball: a sphere light's radius is
+// geometry (its light points, and whether it has those tables at all follows from its kind).
+inline bool same_light_geometry(const rh_light& a, const rh_light& b) {
+  return a.kind == b.kind && same_bytes(a.vec, b.vec) && (a.kind != RH_LIGHT_SPHERE || same_bytes(a.radius, b.radius));
+}
 
 inline UpdateClass classify_update(const rh_material* old_m, const rh_material* new_m, uint32_t n_materials, const rh_light* old_l,
                                    uint32_t n_old_lights, const rh_light* new_l, uint32_t n_new_lights,

@@ -201,16 +201,16 @@ int device_light_map(const double L[3], const rh_tri* d_tris, const uint32_t* d_
 
 // Device version of the lit-triangle queries of one mesh (runtime.cu's host loop) for the light indices in `mask` (bits
 // below 12): clears those bits on the mesh's slots, writes the mesh into bits 12-15 and queries those of the lights
-// 0 .. n_lights-1 only; the other bits stay.  mask 0 only counts.  Enqueues only; the flags of the mesh's slots are
+// 0 .. n_lights-1 that are not in `no_query` (sphere lights) only; the other bits stay.  mask 0 only counts.  Enqueues only; the flags of the mesh's slots are
 // complete when the stream has run.  d_flagged: device counter, incremented by the number of triangles of this mesh with
 // at least one flag.
 int device_lit_flags(const rh_tri* d_tris, const WideNode32* d_nodes, const double center[3], uint32_t root, const uint32_t* d_slots,
-                     uint32_t n_slots, const rh_light* d_lights, uint32_t n_lights, uint32_t mask, uint32_t mesh, uint16_t* d_lit,
-                     unsigned long long* d_flagged, void* stream_) {
+                     uint32_t n_slots, const rh_light* d_lights, uint32_t n_lights, uint32_t mask, uint32_t no_query, uint32_t mesh,
+                     uint16_t* d_lit, unsigned long long* d_flagged, void* stream_) {
   cudaStream_t st = (cudaStream_t)stream_;
   if (!n_slots) return 0;
   mask &= 0x0fffu;
-  const uint32_t query = mask & (n_lights >= 12 ? 0x0fffu : (1u << n_lights) - 1), n_query = (uint32_t)__builtin_popcount(query);
+  const uint32_t query = mask & ~no_query & (n_lights >= 12 ? 0x0fffu : (1u << n_lights) - 1), n_query = (uint32_t)__builtin_popcount(query);
   if (mask) lit_init_kernel<<<(n_slots + 255) / 256, 256, 0, st>>>(d_slots, n_slots, mesh, mask, d_lit);
   if (n_query) {
     const unsigned long long threads = (unsigned long long)n_slots * n_query;

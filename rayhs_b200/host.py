@@ -235,6 +235,18 @@ def thinLens(camera: capi.rh_camera, aperture: float, focus_distance: float) -> 
     return c
 
 
+def sphereLight(position, color, radius: float) -> capi.rh_light:
+    """A sphere light (RH_LIGHT_SPHERE: soft shadows): a point light at `position` whose falloff radius `radius` (finite,
+    >= 0) is also the radius of the ball it emits from; each shaded point samples one point of the ball (see rh_light in
+    include/rayhs_b200.h).  For Scene.update's light table, or to turn a scene's point lights into sphere lights."""
+    L = capi.rh_light()
+    L.kind = capi.RH_LIGHT_SPHERE
+    L.vec[:] = [float(x) for x in position]
+    L.color[:] = [float(x) for x in color]
+    L.radius = float(radius)
+    return L
+
+
 @dataclass
 class Image:
     """Image.hs:21-23, already quantised by toIntC (Image.hs:54-55): uint8 [height, width, 3].  `linear` (progressive
